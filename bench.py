@@ -2,6 +2,7 @@
 """bench.py — plans/sec of the batched plan-generation-and-validation path (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c5]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
 
 Workloads (benchmarks/workloads.py; weak scaling: the per-GPU share is fixed):
@@ -29,6 +30,10 @@ cpu_baseline  the CPU oracle port process-parallel on all host cores over a boun
            (BRUTE-FORCE per-cell integer raster in C: a checker, not an optimised CPU rasteriser)
 --impl reference   the same CPU arm as its own JSON line (the reference is pure Python + Shapely and cannot be
            installed here; the oracle port is what runs — see DESIGN.md), same `config` as the GPU arm
+--dump-outputs DIR   after the K timed steps, write what the last of them computed as DIR/<name>.npy (float64): the
+           per-field argmin, the summary columns and the paths + speed profiles of a fixed, seeded sample of candidates
+           (see dump_outputs).  The inputs are generated deterministically, so two builds can be compared file by file.
+           With N > 1 rank 0 writes: the argmin is the merged one, summaries and paths cover rank 0's candidate range.
 """
 from __future__ import annotations
 
@@ -203,6 +208,59 @@ def numpy_merge(parts):
     return cost, cand
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SUMMARY_ROWS = 65536     # candidates whose summaries --dump-outputs writes (a seeded sample above that)
+DUMP_PATH_ROWS = 256          # candidates whose paths and speed profiles it writes
+
+
+def dump_outputs(bufs, n_cand: int, n_fields: int, cand_base: int, with_paths: bool):
+    """What one device step left in ``bufs`` (the arrays run_device_batch hands its caller), as float64 host arrays:
+      best_cost, best_cand            [F]       per-field argmin (-1: no valid candidate)
+      summary_cand                    [S]       global indices of the candidates whose summaries follow
+      summary_<column>                [S, ...]  every fcpp_summary column but `reserved`
+      path_cand, path_offsets         [P], [P+1]  (paths mode) the candidates whose points follow, and their ranges
+      path_xy, speeds_kmh             [n, 2], [n]
+    Batches of more than DUMP_SUMMARY_ROWS / DUMP_PATH_ROWS candidates are sampled with fixed seeds, so the same
+    arguments give the same rows.  Integer outputs are exact in float64."""
+    import torch
+    from field_coverage_path_planning_b200 import _lib
+
+    def sample(k: int, seed: int) -> np.ndarray:
+        if n_cand <= k:
+            return np.arange(n_cand)
+        return np.sort(np.random.default_rng(seed).choice(n_cand, k, replace=False))
+
+    out = {"best_cost": bufs.d_cost[:n_fields].cpu().numpy().astype(np.float64),
+           "best_cand": bufs.d_best[:n_fields].cpu().numpy().astype(np.float64)}
+    rows = sample(DUMP_SUMMARY_ROWS, 1)
+    isz = _lib.SUMMARY_DTYPE.itemsize
+    raw = bufs.d_sum[:n_cand * isz].view(n_cand, isz)[torch.as_tensor(rows, device=bufs.d_sum.device)]
+    s = np.ascontiguousarray(raw.cpu().numpy()).view(_lib.SUMMARY_DTYPE).reshape(-1)
+    out["summary_cand"] = (rows + cand_base).astype(np.float64)
+    for name in _lib.SUMMARY_DTYPE.names:
+        if name != "reserved":
+            out["summary_" + name] = s[name].astype(np.float64)
+    if with_paths:
+        rows = sample(DUMP_PATH_ROWS, 2)
+        off = bufs.d_off[:n_cand + 1].cpu().numpy()
+        idx = np.concatenate([np.arange(off[b], off[b + 1]) for b in rows] + [np.zeros(0, dtype=np.int64)])
+        ti = torch.as_tensor(idx, device=bufs.d_path.device)
+        out["path_cand"] = (rows + cand_base).astype(np.float64)
+        out["path_offsets"] = np.concatenate([[0], np.cumsum(off[rows + 1] - off[rows])]).astype(np.float64)
+        out["path_xy"] = bufs.d_path[ti].cpu().numpy()
+        out["speeds_kmh"] = bufs.d_spd[ti].cpu().numpy()
+    nbytes = sum(a.nbytes for a in out.values())
+    if nbytes > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {nbytes} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    return out
+
+
+def write_dump(directory: str, arrays) -> None:
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -217,7 +275,13 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the argmin check against the whole job")
     ap.add_argument("--e2e-explicit", action="store_true",
                     help="e2e leg with explicit per-candidate arrays instead of the factored candidate axes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -358,6 +422,8 @@ def main():
     total_cands = w.n_cand
     value = total_cands * args.steps / (dev_ms_max / 1e3)
     step_ms = dev_ms_max / args.steps
+    # taken before the sustained region runs further steps through the same buffers
+    dumped = dump_outputs(bufs, B, F, lo, w.outputs == "paths") if args.dump_outputs and rank == 0 else None
 
     # ---- merged argmin of the timed steps vs the whole job evaluated shard by shard on this GPU ----
     argmin_ok = None
@@ -525,6 +591,8 @@ def main():
                          f"brute-force integer coverage raster) with the CPU oracle, {cores} processes, {rc['wall']:.1f} s wall",
                "note": CPU_NOTE}
 
+    if dumped is not None:
+        write_dump(args.dump_outputs, dumped)
     if rank == 0:
         print(json.dumps({
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": n_gpus, "steps": args.steps,
