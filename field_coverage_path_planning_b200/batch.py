@@ -910,6 +910,8 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     ranks in contiguous ranges, each rank plans its shard on its own GPU and the per-field best
     is merged with ONE all-gather of the (cost, candidate) words + a merge kernel (see ``dist.py``);
     ``winner_paths`` then holds the fields whose winner this rank owns."""
+    if cost not in ("length", "time"):
+        raise ValueError(f"cost must be 'length' or 'time', not {cost!r}")
     vehicle = vehicle or VehicleParams()
     if distributed:
         from . import dist

@@ -30,13 +30,17 @@ def fc():
 
 def _oracle_one(job):
     from oracle import batch as ob, ref_planner as rp
-    (verts, R, heading, corner, obst, h), coverage, keep = job
-    return ob.evaluate_candidate(verts, rp.VehicleParams(), R=R, heading=heading, start_corner=corner, obstacles=obst,
-                                 grid_h=h, coverage=coverage, keep_paths=keep)
+    (verts, R, heading, corner, obst, h), coverage, keep = job[:3]
+    veh = rp.VehicleParams(**(job[3] if len(job) > 3 else {}))
+    extra = job[4] if len(job) > 4 else {}
+    return ob.evaluate_candidate(verts, veh, R=R, heading=heading, start_corner=corner, obstacles=obst,
+                                 grid_h=h, coverage=coverage, keep_paths=keep, **extra)
 
 
 def oracle_many(jobs):
-    """[(oracle_args, coverage, keep_paths)] -> oracle records, in a fork pool (the children never touch CUDA)."""
+    """[(oracle_args, coverage, keep_paths[, vehicle fields[, evaluate_candidate keywords]])] -> oracle records, in a
+    fork pool (the children never touch CUDA).  The vehicle fields are a dict of rp.VehicleParams fields (the
+    defaults when absent); the keywords are e.g. turn_model / clothoid_share."""
     from oracle import raster
     raster.build()
     n = min(len(jobs), os.cpu_count() or 1)
