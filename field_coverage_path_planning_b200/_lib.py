@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # FCPP_LIB selects another build of the same library (A/B timing of kernel variants); there is still
 # no fallback: the file must exist and export the ABI
 LIB_PATH = os.environ.get("FCPP_LIB") or os.path.join(_HERE, "libfcpp.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 FLAG_CORNER_MASK = 3
 FLAG_REVERSE_ORDER = 4
@@ -132,9 +132,9 @@ assert SUMMARY_DTYPE.itemsize == 176, SUMMARY_DTYPE.itemsize
 
 EXPORTS = [
     "fcpp_abi_version", "fcpp_create", "fcpp_destroy", "fcpp_last_error", "fcpp_set_trig_tables",
-    "fcpp_layout", "fcpp_plan_batch", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_field_argmin_exchange", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
+    "fcpp_layout", "fcpp_plan_batch", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
     "fcpp_tour_lengths", "fcpp_distance_matrix", "fcpp_connection_matrix", "fcpp_ga_init_population", "fcpp_ga_next_size", "fcpp_ga_generation", "fcpp_ga_solve", "fcpp_kmeans_lloyd", "fcpp_tsp_two_opt",
-    "fcpp_launch_count", "fcpp_last_fused", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
+    "fcpp_launch_count", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
 ]
 
 _lib = None
@@ -201,8 +201,6 @@ def load():
         L.fcpp_kmeans_lloyd.argtypes = [vp, i32, vp, vp, vp, i32, vp, vp, i32, dbl, vp, vp, vp]
         L.fcpp_tsp_two_opt.restype = C.c_int
         L.fcpp_tsp_two_opt.argtypes = [vp, i32, vp, vp, vp, i32, vp, vp, vp, i32, vp]
-        L.fcpp_last_fused.restype = i32
-        L.fcpp_last_fused.argtypes = [vp]
         L.fcpp_last_max_points.restype = i32
         L.fcpp_last_max_points.argtypes = [vp]
         L.fcpp_last_max_head_points.restype = i32
@@ -211,8 +209,6 @@ def load():
         L.fcpp_set_profiling.argtypes = [vp, C.c_int]
         L.fcpp_last_total_points.restype = C.c_int64
         L.fcpp_last_total_points.argtypes = [vp]
-        L.fcpp_field_argmin_exchange.restype = C.c_int
-        L.fcpp_field_argmin_exchange.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, vp, vp, vp, vp, vp]
         L.fcpp_set_cover_mode.restype = C.c_int
         L.fcpp_set_cover_mode.argtypes = [vp, C.c_int]
         L.fcpp_kernel_times.restype = C.c_int

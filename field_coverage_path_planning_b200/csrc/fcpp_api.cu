@@ -136,9 +136,6 @@ int fcpp_create(int device, fcpp_handle **out)
         fcpp_destroy(h);
         return FCPP_ERR_CUDA;
     }
-#ifdef FCPP_COVER_EXPERIMENT
-    if (getenv("FCPP_EXP")) h->cover_mode = atoi(getenv("FCPP_EXP"));
-#endif
     *out = h;
     return FCPP_OK;
 }
@@ -166,14 +163,15 @@ const char *fcpp_last_error(const fcpp_handle *h) { return h ? h->err : "invalid
 
 int64_t fcpp_launch_count(const fcpp_handle *h) { return h ? h->launches : 0; }
 
-int32_t fcpp_last_fused(const fcpp_handle *h) { return h ? h->last_fused : 0; }
 int32_t fcpp_last_max_points(const fcpp_handle *h) { return h ? h->last_maxn : 0; }
 int32_t fcpp_last_max_head_points(const fcpp_handle *h) { return h ? h->last_maxhead : 0; }
 int64_t fcpp_last_total_points(const fcpp_handle *h) { return h ? h->last_total : -1; }
 
 int fcpp_set_cover_mode(fcpp_handle *h, int mode)
 {
+    constexpr int known = 1 | 2 | 64 | 128;  // the bits documented in fcpp.h
     if (!h) return FCPP_ERR_INVALID;
+    if (mode & ~known) return fail(h, FCPP_ERR_INVALID, "fcpp_set_cover_mode: unknown mode bits 0x%x", mode & ~known);
     h->cover_mode = mode;
     return FCPP_OK;
 }
@@ -285,27 +283,12 @@ int fcpp_plan_batch(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outputs 
         if (rc) return rc;
     }
     if (prof) cudaEventRecord(h->ev[1], st);
-    cudaError_t e;
-    h->last_fused = 0;
+    cudaError_t e = fcpp_launch_plan(h, *batch, *out, st);
+    if (e != cudaSuccess) return cuda_fail(h, e, "plan kernel");
+    if (prof) cudaEventRecord(h->ev[2], st);
     if (batch->do_coverage) {
-        // plan + coverage: two launches (the profiling event sits between them), or — opt-in, cover mode bit 2 —
-        // ONE fused kernel with CTA roles when it fits (fcpp_hot.cu)
-        int fused = 0;
-        if (!(h->cover_mode & 4)) {
-            e = fcpp_launch_plan(h, *batch, *out, st, nullptr);
-            if (e != cudaSuccess) return cuda_fail(h, e, "plan kernel");
-            if (prof) cudaEventRecord(h->ev[2], st);
-            e = fcpp_launch_cover(h, *batch, *out, st);
-        } else {
-            if (prof) cudaEventRecord(h->ev[2], st);
-            e = fcpp_launch_plan_cover(h, *batch, *out, st, &fused);
-        }
-        if (e != cudaSuccess) return cuda_fail(h, e, "plan / coverage kernels");
-        h->last_fused = fused;
-    } else {
-        e = fcpp_launch_plan(h, *batch, *out, st, nullptr);
-        if (e != cudaSuccess) return cuda_fail(h, e, "plan kernel");
-        if (prof) cudaEventRecord(h->ev[2], st);
+        e = fcpp_launch_cover(h, *batch, *out, st);
+        if (e != cudaSuccess) return cuda_fail(h, e, "coverage kernels");
     }
     if (prof) cudaEventRecord(h->ev[3], st);
     h->layout_valid = false;  // one layout per plan call
@@ -362,21 +345,6 @@ int fcpp_status_count(fcpp_handle *h, const fcpp_summary *d_summary, int64_t n_c
     cudaSetDevice(h->device);
     cudaError_t e = fcpp_launch_status_count(h, d_summary, n_cand, mask, d_count, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(h, e, "status count kernel");
-    return FCPP_OK;
-}
-
-int fcpp_field_argmin_exchange(fcpp_handle *h, int32_t world, int32_t rank, int32_t n_fields, uint32_t epoch,
-                               const uint64_t *peer_bufs, const uint64_t *peer_flags, double *d_best_cost,
-                               int64_t *d_best_cand, void *stream)
-{
-    if (!h) return FCPP_ERR_INVALID;
-    if (world < 1 || world > FCPP_MAX_PEERS || rank < 0 || rank >= world || n_fields < 0 || !peer_bufs || !peer_flags ||
-        (n_fields > 0 && (!d_best_cost || !d_best_cand)))
-        return fail(h, FCPP_ERR_INVALID, "fcpp_field_argmin_exchange: bad argument");
-    cudaSetDevice(h->device);
-    cudaError_t e = fcpp_launch_argmin_exchange(h, world, rank, n_fields, epoch, peer_bufs, peer_flags, d_best_cost,
-                                                d_best_cand, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(h, e, "argmin exchange kernel");
     return FCPP_OK;
 }
 

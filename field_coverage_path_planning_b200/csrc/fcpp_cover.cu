@@ -615,7 +615,7 @@ __device__ __forceinline__ int rect_cover(const CoverFixed &s, int nr, int j, in
 // Returns false (nothing counted) when the zones overlap or are too large; the caller then runs
 // the row-tiled evaluation of the whole band.
 __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_ent, int rq, int H, double invH, int nx, int ny,
-                           unsigned long long &my_total, unsigned long long &my_cov, int mode)
+                           unsigned long long &my_total, unsigned long long &my_cov)
 {
     const int tid = threadIdx.x;
     const int nr = min(s.nrect, RECT_CAP);
@@ -709,9 +709,6 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
             zrow = 0;
         }
         if (nt == 0) break;
-#ifdef FCPP_COVER_EXPERIMENT
-        if (mode & 16) continue;  // timing experiment: no zone bitmaps (wrong counts)
-#endif
         __syncthreads();
         // row windows of the resident rows, clipped to their zone's columns
         for (int k = tid; k < used_r; k += T) {
@@ -748,9 +745,6 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
     // the same lattice index on the first and the last row of the run it has it on every row, and
     // the run is counted once and multiplied.  Runs with slanted boundaries go row by row. ----
     __syncthreads();  // the last pass is done with the tile: reuse it for the breakpoints
-#ifdef FCPP_COVER_EXPERIMENT
-    if (mode & 32) return true;  // timing experiment: no closed-form rows (wrong counts)
-#endif
     int *bp = reinterpret_cast<int *>(s.tile);  // [nb] sorted breakpoints, then [nb] slow runs (lo, hi)
     const int nb = 10 + 2 * nr + 8;
     static_assert(T >= 2 * (10 + 2 * RECT_CAP + 8), "one thread per (run, end)");
@@ -843,8 +837,7 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
     return true;
 }
 
-// One candidate's coverage by the T threads of a CTA (stand-alone cover_kernel, or a coverage-role CTA of the fused
-// plan + coverage kernel in fcpp_hot.cu).
+// One candidate's coverage by the T threads of a CTA (cover_kernel, or one listed item of cover_work_kernel).
 __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *__restrict__ recs,
                                            const TrigTables *__restrict__ trig, fcpp_summary *__restrict__ summary,
                                            int pc, int mode, const int32_t *__restrict__ rep /*[2][n_cand]*/,
@@ -894,11 +887,7 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
     // =====================================================================================
     // A10: four verification corner windows (lattice POINTS, h = 0.1 m)
     // =====================================================================================
-#ifdef FCPP_COVER_EXPERIMENT
-    if (do10 && !(mode & 8)) {
-#else
     if (do10) {
-#endif
         const double fl = b.field_extent[2 * r.field], fw = b.field_extent[2 * r.field + 1];
         const int g = r.corner_g;
         const int rw = (g + 31) >> 5;
@@ -1069,7 +1058,7 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
             if (tid == 0) s.next_w0 = 0;
             // axis-aligned straights: bitmap only around the corners, the rest in closed form
             if (FCPP_COVER_RECT && !(mode & 1) && s.nrect > 0 &&
-                band_zoned(s, d, nh - 1, rq, H, invH, nx, ny, my_total, my_cov, mode))
+                band_zoned(s, d, nh - 1, rq, H, invH, nx, ny, my_total, my_cov))
                 j0 = ny;
             while (j0 < ny) {
                 // --- how many rows to try: from the word count of the first row.  The previous pass
@@ -1332,16 +1321,6 @@ __global__ void __launch_bounds__(128) cover_copy_kernel(fcpp_summary *__restric
 
 }  // namespace
 
-// What a coverage launch needs besides the batch: shared-memory size and the de-duplication tables.
-struct CoverLaunch {
-    int pc = 0;
-    size_t bytes = 0;
-    int32_t *d_rep = nullptr;
-    unsigned long long *keys = nullptr, *hash = nullptr;
-    unsigned int *vals = nullptr;
-    int32_t *work = nullptr, *counters = nullptr;  // de-duplicated batches: the listed candidates (cover_work_kernel)
-};
-
 // few representatives expected (a heading search): persistent grid over the listed candidates.  (Measured: config 3
 // coverage 4.0 -> 2.8 ms per 737 280 candidates; batches where most candidates rasterise a part — configs 2 and 5 —
 // run 1.5-2.5 % slower that way, hence the hint.  Cover mode bits 6 / 7 force either.)
@@ -1352,16 +1331,23 @@ static bool cover_use_work_list(const fcpp_handle *h, const fcpp_batch &b)
 
 static int dedupe_threads(const fcpp_handle *h, int64_t n) { return n <= 2 * 32 * (int64_t)h->sm_count ? 32 : 128; }
 
-// sizes + (when the batch asks for it) the de-duplication kernels that precede the coverage kernel
-static cudaError_t cover_prepare(fcpp_handle *h, const fcpp_batch &b, cudaStream_t st, CoverLaunch &L)
+// Coverage of a batch: (when the batch asks for it) the de-duplication kernels, the coverage kernel, then the copy of
+// the representatives' counts to the other members of their groups, which also empties the hash table.
+cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st)
 {
+    if (b.n_cand == 0) return cudaSuccess;
     int pc = cover_point_capacity(h->cover_pcap);
     while (cover_smem_bytes(pc) > (size_t)h->max_smem_optin && pc > 4 * VPOLY_CAP + 16) pc -= 64;
-    L.pc = pc;
-    L.bytes = cover_smem_bytes(pc);
-    cudaError_t e = cudaSuccess;
+    const size_t bytes = cover_smem_bytes(pc);
+    int32_t *d_rep = nullptr;
+    unsigned long long *keys = nullptr, *hash = nullptr;
+    unsigned int *vals = nullptr;
+    int32_t *work = nullptr, *counters = nullptr;  // de-duplicated batches: the listed candidates (cover_work_kernel)
+    cudaError_t e;
     // de-duplication (asked for by the batch, unless switched off by cover mode bit 1)
     const int64_t n = b.n_cand;
+    // (one thread per candidate, latency bound: small batches use 32-thread CTAs to reach more SMs)
+    const int th = dedupe_threads(h, n);
     if (b.cover_dedupe && n > 1 && !(h->cover_mode & 2) && n < (1ll << 28)) {
         uint32_t cap = 1024;
         while ((int64_t)cap < 4 * n) cap <<= 1;  // two keys per candidate, load factor <= 1/2
@@ -1377,72 +1363,49 @@ static cudaError_t cover_prepare(fcpp_handle *h, const fcpp_batch &b, cudaStream
         }
         // layout: keys [cap] | vals [cap] | hash / slot [2][n] | rep [2][n] | work [n] | counters [2]; a different
         // capacity moves the arrays, so the table is zeroed again
-        L.keys = (unsigned long long *)h->d_dedupe;
-        L.vals = (unsigned int *)(L.keys + cap);
-        L.hash = (unsigned long long *)(L.vals + cap);
-        L.d_rep = (int32_t *)(L.hash + 2 * n);
-        L.work = L.d_rep + 2 * n;
-        L.counters = L.work + n;
+        keys = (unsigned long long *)h->d_dedupe;
+        vals = (unsigned int *)(keys + cap);
+        hash = (unsigned long long *)(vals + cap);
+        d_rep = (int32_t *)(hash + 2 * n);
         if (h->dedupe_cap != cap) {
             e = cudaMemsetAsync(h->d_dedupe, 0, (size_t)cap * 12, st);
             if (e != cudaSuccess) return e;
             h->dedupe_cap = cap;
         }
-        // (one thread per candidate, latency bound: small batches use 32-thread CTAs to reach more SMs)
-        const int th = dedupe_threads(h, n);
         const unsigned g = (unsigned)((n + th - 1) / th);
-        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, L.keys, L.vals, cap - 1, L.hash);
-        cover_rep_kernel<<<g, th, 0, st>>>(h->d_rec, n, L.keys, L.vals, cap - 1, L.hash, L.d_rep);
+        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash);
+        cover_rep_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, d_rep);
         h->launches += 2;
         if (cover_use_work_list(h, b)) {
-            e = cudaMemsetAsync(L.counters, 0, 2 * sizeof(int32_t), st);
+            work = d_rep + 2 * n;
+            counters = work + n;
+            e = cudaMemsetAsync(counters, 0, 2 * sizeof(int32_t), st);
             if (e != cudaSuccess) return e;
-            cover_list_kernel<<<g, th, 0, st>>>(n, L.d_rep, L.work, L.counters);
+            cover_list_kernel<<<g, th, 0, st>>>(n, d_rep, work, counters);
             h->launches++;
-        } else {
-            L.work = nullptr;
         }
         e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
     }
-    return e;
-}
-
-// hands the representatives' counts to the other members of their groups and empties the hash table
-static cudaError_t cover_finish(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st,
-                                const CoverLaunch &L)
-{
-    if (!L.d_rep) return cudaSuccess;
-    const int64_t n = b.n_cand;
-    const int th = dedupe_threads(h, n);
-    cover_copy_kernel<<<(unsigned)((n + th - 1) / th), th, 0, st>>>(o.summary, n, L.d_rep, L.keys, L.vals, L.hash);
-    h->launches++;
-    return cudaGetLastError();
-}
-
-cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st)
-{
-    if (b.n_cand == 0) return cudaSuccess;
-    CoverLaunch L;
-    cudaError_t e = cover_prepare(h, b, st, L);
-    if (e != cudaSuccess) return e;
-    if (L.work) {
-        e = cudaFuncSetAttribute(cover_work_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.bytes);
+    if (work) {
+        e = cudaFuncSetAttribute(cover_work_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         if (e != cudaSuccess) return e;
         int64_t grid = (int64_t)FCPP_COVER_MINBLOCKS * h->sm_count;
-        if (grid > b.n_cand) grid = b.n_cand;
-        cover_work_kernel<<<(unsigned)grid, T, L.bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, L.pc, h->cover_mode,
-                                                              L.d_rep, o.corner_bits, o.corner_bits_stride, L.work,
-                                                              L.counters);
+        if (grid > n) grid = n;
+        cover_work_kernel<<<(unsigned)grid, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
+                                                            o.corner_bits, o.corner_bits_stride, work, counters);
     } else {
-        e = cudaFuncSetAttribute(cover_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.bytes);
+        e = cudaFuncSetAttribute(cover_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         if (e != cudaSuccess) return e;
-        cover_kernel<<<(unsigned)b.n_cand, T, L.bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, L.pc, h->cover_mode,
-                                                              L.d_rep, o.corner_bits, o.corner_bits_stride);
+        cover_kernel<<<(unsigned)n, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
+                                                    o.corner_bits, o.corner_bits_stride);
     }
     h->launches++;
     e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    return cover_finish(h, b, o, st, L);
+    if (e != cudaSuccess || !d_rep) return e;
+    cover_copy_kernel<<<(unsigned)((n + th - 1) / th), th, 0, st>>>(o.summary, n, d_rep, keys, vals, hash);
+    h->launches++;
+    return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------------

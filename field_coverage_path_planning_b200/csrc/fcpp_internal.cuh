@@ -82,9 +82,8 @@ struct fcpp_handle {
     int64_t last_total;      // total points of the last synchronous layout pass with offsets (-1: unknown)
     int cover_pcap;          // point capacity of the coverage kernel's staging for the next launch
     int cover_mode;          // diagnostics (fcpp_set_cover_mode): bit 0 = never use the zoned band evaluation,
-                             // bit 1 = no coverage de-duplication, bit 2 = plan and coverage as ONE fused kernel,
-                             // bits 6 / 7 = de-duplicated batches: force one coverage CTA per candidate / the persistent work list
-    int last_fused;          // the last fcpp_plan_batch ran the fused plan + coverage kernel
+                             // bit 1 = no coverage de-duplication, bits 6 / 7 = de-duplicated batches: force one
+                             // coverage CTA per candidate / the persistent work list
     void *d_dedupe;          // coverage de-duplication: hash table, hashes, representatives
     size_t dedupe_bytes;
     uint32_t dedupe_cap;     // slots of the (currently zeroed) table inside d_dedupe; 0 = not initialised
@@ -681,11 +680,8 @@ __device__ __forceinline__ void gen_point(const CandRec &r, const TrigTables &tt
 // launchers (defined in the .cu files, called from fcpp_api.cu)
 cudaError_t fcpp_launch_layout(fcpp_handle *h, const fcpp_batch &b, int32_t *d_n_pts, int64_t *d_offsets,
                                cudaStream_t st);
-cudaError_t fcpp_launch_plan(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st,
-                             int *too_large);
+cudaError_t fcpp_launch_plan(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st);
 cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st);
-cudaError_t fcpp_launch_plan_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st,
-                                   int *fused_out);
 cudaError_t fcpp_launch_speed_verify(fcpp_handle *h, const fcpp_vehicle &veh, const double *d_path,
                                      const double *d_speeds_in, const int64_t *d_offsets, int64_t n_paths,
                                      int64_t max_len, int do_speed_plan, double *d_speeds_out, double *d_curv,
@@ -711,9 +707,6 @@ cudaError_t fcpp_launch_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, 
                                      double *d_best_cost, int64_t *d_best_cand, cudaStream_t st);
 cudaError_t fcpp_launch_winner_records(fcpp_handle *h, const fcpp_summary *d_summary, int64_t lo, int64_t hi,
                                        const int64_t *d_best_cand, int32_t n_fields, void *d_out, cudaStream_t st);
-cudaError_t fcpp_launch_argmin_exchange(fcpp_handle *h, int32_t world, int32_t rank, int32_t n_fields, uint32_t epoch,
-                                        const uint64_t *peer_bufs, const uint64_t *peer_flags, double *d_best_cost,
-                                        int64_t *d_best_cand, cudaStream_t st);
 cudaError_t fcpp_launch_distance_matrix(fcpp_handle *h, const double *d_pos, int32_t n, double *d_D, cudaStream_t st);
 cudaError_t fcpp_launch_connection_matrix(fcpp_handle *h, const double *d_verts, int32_t n_fields, double depot_x,
                                           double depot_y, double *d_C, int32_t *d_arg, cudaStream_t st);

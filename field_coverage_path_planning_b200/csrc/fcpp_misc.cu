@@ -202,82 +202,6 @@ __global__ void argmin_merge_kernel(const long long *__restrict__ g, int world, 
     best_cand[f] = bi;
 }
 
-// multi-GPU, fused: exchange of the ranks' (cost, candidate) words over PEER MEMORY (NVLink P2P stores
-// into every rank's symmetric buffer + a release/acquire flag per rank) and the merge, in ONE kernel —
-// no NCCL call, no separate merge launch.  slots = [2 parities][world][2 F] words on every rank; a rank
-// can run at most one call ahead of a peer (it needs the peer's flag of the current call to finish),
-// so two parities are enough.  Flags hold the epoch (monotonic) of the rank's last completed write.
-struct ExchangePeers {
-    unsigned long long buf[FCPP_MAX_PEERS];   // peer p's slot array, mapped into this process
-    unsigned long long flag[FCPP_MAX_PEERS];  // peer p's flag array (uint32 [world])
-};
-
-__device__ __forceinline__ void st_release_sys(unsigned int *p, unsigned int v)
-{
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int *p)
-{
-    unsigned int v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-constexpr int EXCH_THREADS = 512;
-__global__ void __launch_bounds__(EXCH_THREADS) argmin_exchange_kernel(const ExchangePeers peers, int world, int rank,
-                                                                        int n_fields, unsigned int epoch,
-                                                                        double *best_cost, long long *best_cand,
-                                                                        long long timeout_cycles)
-{
-    const int tid = threadIdx.x;
-    const int64_t words = 2 * (int64_t)n_fields;                    // cost bits [F] then candidates [F]
-    const int64_t par = (int64_t)(epoch & 1u) * world * words;
-    // 1. my words into slot `rank` of every rank (peer stores; own copy too)
-    for (int p = 0; p < world; ++p) {
-        long long *dst = reinterpret_cast<long long *>(peers.buf[p]) + par + (int64_t)rank * words;
-        for (int64_t i = tid; i < words; i += EXCH_THREADS)
-            dst[i] = (i < n_fields) ? __double_as_longlong(best_cost[i]) : best_cand[i - n_fields];
-    }
-    __threadfence_system();
-    __syncthreads();
-    // 2. publish: my flag on every rank; 3. wait for every rank's flag here
-    __shared__ int timed_out;
-    if (tid == 0) timed_out = 0;
-    __syncthreads();
-    if (tid < world) {
-        st_release_sys(reinterpret_cast<unsigned int *>(peers.flag[tid]) + rank, epoch);
-        const unsigned int *mine = reinterpret_cast<const unsigned int *>(peers.flag[rank]) + tid;
-        // gentle polling: relaxed loads with a back-off (a tight acquire loop on the line the peers are
-        // writing to slows their stores down), one acquire at the end
-        const long long t0 = clock64();
-        while ((int)(*reinterpret_cast<const volatile unsigned int *>(mine) - epoch) < 0) {
-            __nanosleep(256);
-            if (clock64() - t0 > timeout_cycles) {
-                timed_out = 1;
-                break;
-            }
-        }
-        (void)ld_acquire_sys(mine);
-    }
-    __syncthreads();
-    // 4. merge (the rule of argmin_merge_kernel); a peer that never arrived poisons the result
-    const volatile long long *g = reinterpret_cast<const volatile long long *>(peers.buf[rank]) + par;
-    for (int f = tid; f < n_fields; f += EXCH_THREADS) {
-        double bc = INFINITY;
-        long long bi = -1;
-        for (int r = 0; r < world; ++r) {
-            const double c = __longlong_as_double(g[(int64_t)r * words + f]);
-            const long long i = g[(int64_t)r * words + n_fields + f];
-            if (i >= 0 && (bi < 0 || c < bc || (c == bc && i < bi))) {
-                bc = c;
-                bi = i;
-            }
-        }
-        best_cost[f] = timed_out ? __longlong_as_double(0x7ff8000000000000ll) : bc;
-        best_cand[f] = timed_out ? -2 : bi;
-    }
-}
-
 // multi-GPU: this rank's contribution to the all-gather of the winners' summary records — the 176-byte record of
 // every field whose global winner lies in [lo, hi), zeros elsewhere (a SUM over the ranks then is the record)
 __global__ void winner_records_kernel(const fcpp_summary *__restrict__ sm, int64_t lo, int64_t hi,
@@ -376,22 +300,6 @@ cudaError_t fcpp_launch_winner_records(fcpp_handle *h, const fcpp_summary *d_sum
     const int64_t n = (int64_t)n_fields * (sizeof(fcpp_summary) / 16);
     winner_records_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_summary, lo, hi, (const long long *)d_best_cand,
                                                                        n_fields, (int4 *)d_out);
-    h->launches++;
-    return cudaGetLastError();
-}
-
-cudaError_t fcpp_launch_argmin_exchange(fcpp_handle *h, int32_t world, int32_t rank, int32_t n_fields, uint32_t epoch,
-                                        const uint64_t *peer_bufs, const uint64_t *peer_flags, double *d_best_cost,
-                                        int64_t *d_best_cand, cudaStream_t st)
-{
-    if (n_fields == 0) return cudaSuccess;
-    ExchangePeers pp{};
-    for (int p = 0; p < world; ++p) {
-        pp.buf[p] = peer_bufs[p];
-        pp.flag[p] = peer_flags[p];
-    }
-    argmin_exchange_kernel<<<1, EXCH_THREADS, 0, st>>>(pp, world, rank, n_fields, epoch, d_best_cost,
-                                                        (long long *)d_best_cand, 20000000000ll /* ~10 s */);
     h->launches++;
     return cudaGetLastError();
 }

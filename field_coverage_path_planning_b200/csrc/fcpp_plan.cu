@@ -84,16 +84,6 @@ __device__ inline Smem carve(unsigned char *base, int ncap)
     return s;
 }
 
-// Barrier of the group of threads that works on one plan: the whole CTA in the stand-alone kernels, a 128-thread
-// quarter of a 512-thread CTA (named barrier) when four plans share a CTA of the fused plan + coverage kernel
-struct CtaSync {
-    __device__ __forceinline__ void operator()() const { __syncthreads(); }
-};
-struct QuarterSync {
-    int id;  // hardware barrier 1 .. 4
-    __device__ __forceinline__ void operator()() const { asm volatile("bar.sync %0, 128;" ::"r"(id) : "memory"); }
-};
-
 // ---------------------------------------------------------------------------------------------
 // min-plus scan element: the map u -> min(M, u + C)
 // ---------------------------------------------------------------------------------------------
@@ -117,8 +107,7 @@ __device__ __forceinline__ MP mp_shfl_up(const MP &v, int d)
 
 // exclusive block scan of per-thread aggregates in thread order; returns the carry-in value
 // (the M of the composition of all earlier threads; +inf for thread 0)
-template <class Sync>
-__device__ __forceinline__ double mp_block_exclusive(MP agg, double *sh /*>= 2*NWARP*/, int tid, const Sync &sync)
+__device__ __forceinline__ double mp_block_exclusive(MP agg, double *sh /*>= 2*NWARP*/, int tid)
 {
     const int lane = tid & 31, warp = tid >> 5;
     MP inc = agg;
@@ -131,8 +120,8 @@ __device__ __forceinline__ double mp_block_exclusive(MP agg, double *sh /*>= 2*N
         sh[2 * warp] = inc.C;
         sh[2 * warp + 1] = inc.M;
     }
-    sync();
-    // composition of all earlier warps (serial over the few warps of the group)
+    __syncthreads();
+    // composition of all earlier warps (serial over the few warps of the CTA)
     MP pre;
     pre.C = 0.0;
     pre.M = INFINITY;
@@ -149,7 +138,7 @@ __device__ __forceinline__ double mp_block_exclusive(MP agg, double *sh /*>= 2*N
         ex.M = INFINITY;
     }
     const MP tot = mp_combine(pre, ex);
-    sync();
+    __syncthreads();
     return tot.M;
 }
 
@@ -166,19 +155,19 @@ __device__ __forceinline__ double warp_max(double v)
     return v;
 }
 
-// reduce NV sums / maxes across the group (deterministic order); result valid in thread 0
-template <int NV, bool IS_MAX, int NWARP, class Sync>
-__device__ __forceinline__ void block_reduce(double (&v)[NV], double *sh, int tid, const Sync &sync)
+// reduce NV sums / maxes across the CTA (deterministic order); result valid in thread 0
+template <int NV, bool IS_MAX, int NWARP>
+__device__ __forceinline__ void block_reduce(double (&v)[NV], double *sh, int tid)
 {
     const int lane = tid & 31, warp = tid >> 5;
 #pragma unroll
     for (int k = 0; k < NV; ++k) v[k] = IS_MAX ? warp_max(v[k]) : warp_sum(v[k]);
-    sync();
+    __syncthreads();
     if (lane == 0) {
 #pragma unroll
         for (int k = 0; k < NV; ++k) sh[warp * NV + k] = v[k];
     }
-    sync();
+    __syncthreads();
     if (tid == 0) {
 #pragma unroll
         for (int k = 0; k < NV; ++k) {
@@ -266,7 +255,7 @@ __device__ __forceinline__ double vlimit(double v0, double kappa, const fcpp_veh
 #endif
 constexpr int TG = FCPP_PLAN_GEN_THREADS;
 #ifndef FCPP_PLAN_GEN_MIN_CTAS
-// CTAs of 128 threads per SM the register allocation aims at.  Measured (tools/fused_ab.py, plan kernel of config
+// CTAs of 128 threads per SM the register allocation aims at.  Measured (tools/cover_ab.py, plan kernel of config
 // 2 / 5 / 3): 8 CTAs (64 registers, 308 B of spills) 0.207 / 0.624 / 4.50 ms, 7 (72 registers) 0.193 / 0.602 / 4.20,
 // 6 (80) 0.203 / 0.598 / 4.25, 5 (96) 0.220 / 0.641 / 4.36, 4 (120, no spills) 0.240 / 0.680 / 4.80.
 #define FCPP_PLAN_GEN_MIN_CTAS 7
@@ -286,7 +275,7 @@ struct GenFixed {
     uint16_t mixed[MIXED_CAP];   // main passes whose turn samples need the per-point tests (phase 0c)
     int32_t n_mixed;
     double gvl[N_GENERIC];       // curvature-limited speed of the generic points
-    double scratch[9 * (FCPP_PLAN_GEN_THREADS / 32) + 8];  // group reductions: 9 values per warp; scans: 2 per warp
+    double scratch[9 * (FCPP_PLAN_GEN_THREADS / 32) + 8];  // block reductions: 9 values per warp; scans: 2 per warp
     union {
         struct {
             double chain_v[CHAIN_POINTS];  // final speed (km/h) of the regular chain's points
@@ -409,10 +398,9 @@ __device__ __forceinline__ void point_tests(const GenSmem &s, int n_obs_poly, do
 }
 
 
-// One generated plan by the TG threads of a group (tid = 0 .. TG-1) in their own shared-memory region.
-template <class Sync, bool OMEGA = false>
-__device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *smem, const int tid, const int64_t cand,
-                                              const Sync &sync)
+// One generated plan by the TG threads of a CTA (tid = 0 .. TG-1).
+template <bool OMEGA = false>
+__device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *smem, const int tid, const int64_t cand)
 {
     constexpr int T = TG;
     const GenSmem s = gen_carve(smem, a.ncap, a.obs_cap_verts, a.obs_cap_polys);
@@ -421,7 +409,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
     const fcpp_vehicle &veh = a.b.vehicle;
     fcpp_summary *sum = a.out.summary ? a.out.summary + cand : nullptr;
     if (tid == 0) mbar_init(&f.bar, 1);
-    sync();
+    __syncthreads();
 
     int n_obs_poly = 0;
     {
@@ -445,12 +433,12 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
         for (int k = tid; k < (int)(sizeof(TrigTables) / sizeof(double)); k += T)
             ((double *)&f.tt)[k] = ((const double *)a.trig)[k];
         for (int k = tid; k < N_GENERIC; k += T) f.glist[k] = -1;
-        // ONE thread polls the mbarrier, the group barrier releases the rest, and every thread then observes the
+        // ONE thread polls the mbarrier, the CTA barrier releases the rest, and every thread then observes the
         // completed phase itself (acquire of the async-proxy writes)
         if (tid == 0)
             while (!mbar_try_wait(&f.bar, 0)) {
             }
-        sync();
+        __syncthreads();
         while (!mbar_try_wait(&f.bar, 0)) {
         }
     }
@@ -462,8 +450,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
         for (int k = tid; k <= n_obs_poly; k += T) s.obs_vs[k] = a.b.obs_vert_start[p0 + k] - base;
     }
     const int N = r.n_total, n_main = r.n_main;
-    FCPP_ASSERT(gen_smem_bytes(a.ncap, a.obs_cap_verts, a.obs_cap_polys) <= fcpp_dynamic_smem_bytes() + 0u ||
-                blockDim.x != TG /* fused kernel: four plans share one allocation, checked by the host */);
+    FCPP_ASSERT(gen_smem_bytes(a.ncap, a.obs_cap_verts, a.obs_cap_polys) <= fcpp_dynamic_smem_bytes() + 0u);
     const int n_skip = main_skip(n_main);  // regular chain points: i in [2, 2 + n_skip)
     const int NS = N - n_skip;             // staged points
     const int64_t off = a.out.offsets ? a.out.offsets[cand] : 0;
@@ -498,7 +485,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
             return;
         }
     }
-    sync();  // obs_vs is complete
+    __syncthreads();  // obs_vs is complete
     const double W = veh.working_width;
     TurnModel tm;
     tm.model = a.b.turn_model;
@@ -554,7 +541,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
         s.obs_bb[4 * p + 2] = x1 + rr + 1e-6;
         s.obs_bb[4 * p + 3] = y1 + rr + 1e-6;
     }
-    sync();
+    __syncthreads();
     // one thread per table slot (two rounds when the CTA has fewer threads than slots' thread ids)
     for (int vt = tid; vt < 96 + 4 * FCPP_MAX_LOOPS; vt += T) {
         int slot = -1;
@@ -616,7 +603,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
             f.tbl[slot] = e;
         }
     }
-    sync();
+    __syncthreads();
 
     // ------------------------------------------------------------------------------------
     // phase 0c (summary-only batches): the turns of the regular main passes, classified per PASS.  The 20 turn samples
@@ -649,7 +636,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
     };
     if (cull) {
         if (tid == 0) f.n_mixed = 0;
-        sync();
+        __syncthreads();
         const double rad = r.R + 1e-6;
         for (int idx = tid; idx * CHAIN_POINTS + 1 < i_end; idx += T) {
             // the pass's points j >= 1 inside the regular range (pass 0: its two ends are staged)
@@ -783,7 +770,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
         }
         point_tests(s, n_obs_poly, r2, x, y, n_bviol, n_oviol);
     }
-    sync();  // glist, chain_v
+    __syncthreads();  // glist, chain_v
     // ------------------------------------------------------------------------------------
     // phase 1b: the regular chains' points (most of a plan): generated, tested, written with the chain's speeds
     // ------------------------------------------------------------------------------------
@@ -933,7 +920,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
             }
         }
     }
-    sync();
+    __syncthreads();
 
     // ------------------------------------------------------------------------------------
     // phases 3 / 4 over the staged sequence (the zero-length segment after point 1 separates the two staged ends
@@ -953,7 +940,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
                 agg.M = fmin(s.U[q], agg.M + c);
                 agg.C = agg.C + c;
             }
-            double carry = mp_block_exclusive(agg, f.scratch, tid, sync);
+            double carry = mp_block_exclusive(agg, f.scratch, tid);
             for (int q = cs; q < ce; ++q) {
                 const double dsp = (q > 0) ? s.X[q - 1] : 0.0;
                 const double c = (q > 0 && !(dsp < FCPP_ZERO_LEN)) ? two_a * dsp : INFINITY;
@@ -961,7 +948,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
                 s.U[q] = carry;
             }
         }
-        sync();
+        __syncthreads();
         {
             const int rt = T - 1 - tid;
             const int rs = min(NS, rt * chunk);
@@ -975,7 +962,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
                 agg.M = fmin(s.U[q], agg.M + c);
                 agg.C = agg.C + c;
             }
-            double carry = mp_block_exclusive(agg, f.scratch, tid, sync);
+            double carry = mp_block_exclusive(agg, f.scratch, tid);
             for (int q = re - 1; q >= rs; --q) {
                 const double dsn = s.X[q];
                 const double c = (q + 1 < NS && !(dsn < FCPP_ZERO_LEN)) ? two_a * dsn : INFINITY;
@@ -983,7 +970,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
                 s.U[q] = carry;
             }
         }
-        sync();
+        __syncthreads();
     }
 
     // ------------------------------------------------------------------------------------
@@ -1035,7 +1022,7 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
         }
         finish_point(act, act ? (i < 2 ? i : i - n_skip) : 0, u_lim, vl);
     }
-    sync();
+    __syncthreads();
     // ------------------------------------------------------------------------------------
     // phase 5b: work time with the adjusted speeds (mlp3:423-431, :1298-1311)
     // ------------------------------------------------------------------------------------
@@ -1052,8 +1039,8 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
     }
     double sums[9] = {acc_len_m, acc_len_h, acc_tpre_m, acc_tpre_h, acc_t_m,
                       acc_t_h,   (double)n_aviol, (double)n_bviol, (double)n_oviol};
-    block_reduce<9, false, T / 32>(sums, f.scratch, tid, sync);
-    block_reduce<3, true, T / 32>(mx, f.scratch, tid, sync);
+    block_reduce<9, false, T / 32>(sums, f.scratch, tid);
+    block_reduce<3, true, T / 32>(mx, f.scratch, tid);
     if (tid == 0 && sum) {
         // the regular chains: one chain's sums times their number
         const double nreg = (double)(n_skip / CHAIN_POINTS);
@@ -1089,13 +1076,13 @@ __device__ __forceinline__ void plan_gen_body(const PlanArgs &a, unsigned char *
 __global__ void __launch_bounds__(TG, FCPP_PLAN_GEN_MIN_CTAS) plan_gen_omega_kernel(const PlanArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    plan_gen_body<CtaSync, true>(a, smem_raw, threadIdx.x, blockIdx.x, CtaSync());
+    plan_gen_body<true>(a, smem_raw, threadIdx.x, blockIdx.x);
 }
 
 __global__ void __launch_bounds__(TG, FCPP_PLAN_GEN_MIN_CTAS) plan_gen_kernel(const PlanArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    plan_gen_body(a, smem_raw, threadIdx.x, blockIdx.x, CtaSync());
+    plan_gen_body(a, smem_raw, threadIdx.x, blockIdx.x);
 }
 
 // One caller-supplied path (A7 / A8 / A13 of the drop-in API): every point from its coordinates.
@@ -1202,7 +1189,7 @@ __device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s,
                 agg.M = fmin(s.U[i], agg.M + c);
                 agg.C = agg.C + c;
             }
-            double carry = mp_block_exclusive(agg, s.scratch, tid, CtaSync());
+            double carry = mp_block_exclusive(agg, s.scratch, tid);
             for (int i = cs; i < ce; ++i) {
                 const double dsp = (i > 0) ? s.X[i - 1] : 0.0;
                 const double c = (i > 0 && !(dsp < FCPP_ZERO_LEN)) ? two_a * dsp : INFINITY;
@@ -1224,7 +1211,7 @@ __device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s,
                 agg.M = fmin(s.U[i], agg.M + c);
                 agg.C = agg.C + c;
             }
-            double carry = mp_block_exclusive(agg, s.scratch, tid, CtaSync());
+            double carry = mp_block_exclusive(agg, s.scratch, tid);
             for (int i = re - 1; i >= rs; --i) {
                 const double dsn = s.X[i];
                 const double c = (i + 1 < N && !(dsn < FCPP_ZERO_LEN)) ? two_a * dsn : INFINITY;
@@ -1270,8 +1257,8 @@ __device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s,
     for (int i = tid; i + 1 < N; i += T)
         acc_t_m += div_z(s.X[i], fmax(div36((s.U[i] + s.U[i + 1]) / 2), FCPP_MIN_SPEED_MS));
     double sums[4] = {acc_len_m, acc_tpre_m, acc_t_m, (double)n_aviol};
-    block_reduce<4, false, T / 32>(sums, s.scratch, tid, CtaSync());
-    block_reduce<3, true, T / 32>(mx, s.scratch, tid, CtaSync());
+    block_reduce<4, false, T / 32>(sums, s.scratch, tid);
+    block_reduce<3, true, T / 32>(mx, s.scratch, tid);
     if (tid == 0 && sum) {
         sum->status = 0;
         sum->n_passes = 0;
@@ -1412,9 +1399,10 @@ cudaError_t launch_big(fcpp_handle *h, PlanArgs &a, int64_t n_items, int max_poi
 // Generated plans: one CTA per candidate.  Only the first 2 + last 22 main points and the headland are staged in
 // shared memory (~25 B per point), so the staging depends on the longest HEADLAND of the batch, not on the plan
 // length: no length tiers, no HBM staging, 7-8 CTAs of 128 threads per SM at every field size.
-static size_t plan_gen_args(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, PlanArgs &a)
+cudaError_t fcpp_launch_plan(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st)
 {
-    a = PlanArgs{};
+    if (b.n_cand == 0) return cudaSuccess;
+    PlanArgs a{};
     a.b = b;
     a.recs = h->d_rec;
     a.trig = h->d_trig;
@@ -1423,16 +1411,7 @@ static size_t plan_gen_args(fcpp_handle *h, const fcpp_batch &b, const fcpp_outp
     a.obs_cap_polys = b.obs_poly_start ? b.max_obs_polys : 0;
     a.ncap = (MAIN_STAGED + (h->cover_pcap > 0 ? h->cover_pcap : 0) + 63) / 64 * 64;
     a.n_items = b.n_cand;
-    return gen_smem_bytes(a.ncap, a.obs_cap_verts, a.obs_cap_polys);
-}
-
-cudaError_t fcpp_launch_plan(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st,
-                             int *ncap_out)
-{
-    if (b.n_cand == 0) return cudaSuccess;
-    PlanArgs a;
-    const size_t bytes = plan_gen_args(h, b, o, a);
-    if (ncap_out) *ncap_out = a.ncap;
+    const size_t bytes = gen_smem_bytes(a.ncap, a.obs_cap_verts, a.obs_cap_polys);
     if (bytes > (size_t)h->max_smem_optin) return cudaErrorInvalidValue;  // obstacle tables / headland beyond shared memory
     const bool omega = b.turn_model == FCPP_TURN_OMEGA;  // its own instance: the default patterns do not carry its code
     cudaError_t e = cudaFuncSetAttribute(omega ? plan_gen_omega_kernel : plan_gen_kernel,

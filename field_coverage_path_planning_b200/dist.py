@@ -11,8 +11,7 @@ Works on NCCL (CUDA tensors) and gloo (CPU tensors — used by the world_size-2 
 """
 from __future__ import annotations
 
-import os
-from typing import Dict, Optional, Tuple
+from typing import Dict, Tuple
 
 import numpy as np
 import torch
@@ -43,73 +42,17 @@ def shard_candidates(cands: Dict[str, np.ndarray], world: int, rank: int) -> Tup
     return {k: v[lo:hi] for k, v in cands.items()}, lo
 
 
-class _PeerExchange:
-    """Symmetric-memory buffers for fcpp_field_argmin_exchange: per rank [2][world][2 F] int64 slots + a
-    flag array, mapped into every process of the group (torch symmetric memory over NVLink P2P).  One
-    instance per (device, F, group); set-up is a collective.  ``ok`` is False — on EVERY rank — when
-    symmetric memory is unavailable on any of them, and reduce_best falls back to NCCL."""
-    _cache: Dict[tuple, "_PeerExchange"] = {}
-
-    def __init__(self, dev: torch.device, F: int, group):
-        import ctypes as C
-        self.ok = False
-        self.epoch = 0
-        world = dist.get_world_size(group)
-        good = 0
-        try:
-            import torch.distributed._symmetric_memory as symm
-            if world <= 16:
-                words = 2 * world * 2 * F
-                self.nbytes = words * 8 + 256
-                self.t = symm.empty(self.nbytes, dtype=torch.uint8, device=dev)
-                self.t.zero_()
-                self.hdl = symm.rendezvous(self.t, dist.group.WORLD if group is None else group)
-                ptrs = [int(p) for p in self.hdl.buffer_ptrs]
-                self.bufs = (C.c_uint64 * world)(*ptrs)
-                self.flags = (C.c_uint64 * world)(*[p + words * 8 for p in ptrs])
-                self.rank, self.world = int(self.hdl.rank), int(self.hdl.world_size)
-                good = 1
-        except Exception:           # no symmetric memory in this build / on this box
-            good = 0
-        agree = torch.tensor([good], dtype=torch.int32, device=dev)
-        dist.all_reduce(agree, op=dist.ReduceOp.MIN, group=group)     # also orders the zeroing before any use
-        torch.cuda.synchronize(dev)
-        self.ok = bool(agree.item())
-
-    @classmethod
-    def get(cls, dev: torch.device, F: int, group) -> "_PeerExchange":
-        key = (dev.index, F, id(group))
-        ex = cls._cache.get(key)
-        if ex is None:
-            ex = cls._cache[key] = cls(dev, F, group)
-        return ex
-
-
-def reduce_best(best_cost: torch.Tensor, best_cand: torch.Tensor, group=None, peer: Optional[bool] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+def reduce_best(best_cost: torch.Tensor, best_cand: torch.Tensor, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Global per-field (cost, candidate) from the local ones.  ``best_cand`` holds GLOBAL
     candidate indices (-1 = this rank has no valid candidate for the field).  In place.
 
     CUDA tensors: one NCCL all-gather of the (cost, candidate) words + the library's merge kernel
-    (fcpp_field_argmin_merge).  ``peer=True`` / FCPP_PEER_EXCHANGE=1 (opt-in): ONE kernel that exchanges
-    the words over peer memory and merges them (fcpp_field_argmin_exchange) — bit-identical, 16 vs 42 us
-    per isolated call at N=2, but measured slower inside the 8-GPU bench loop (DESIGN.md §6), hence not
-    the default.  CPU tensors (gloo tests): the same rule with torch ops."""
+    (fcpp_field_argmin_merge).  CPU tensors (gloo tests): the same rule with torch ops."""
     if best_cost.is_cuda:
         import ctypes as C
         F = best_cost.numel()
         world = dist.get_world_size(group)
         dev = best_cost.device
-        use_peer = (os.environ.get("FCPP_PEER_EXCHANGE", "0") == "1") if peer is None else peer
-        if (use_peer and world > 1 and best_cost.dtype == torch.float64 and best_cand.dtype == torch.int64
-                and best_cost.is_contiguous() and best_cand.is_contiguous()):
-            ex = _PeerExchange.get(dev, F, group)
-            if ex.ok:
-                ex.epoch += 1
-                h = _lib.handle(dev.index)
-                st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-                h.check(h.lib.fcpp_field_argmin_exchange(h.h, ex.world, ex.rank, F, ex.epoch, ex.bufs, ex.flags,
-                                                         best_cost.data_ptr(), best_cand.data_ptr(), st))
-                return best_cost, best_cand
         adjacent = (best_cost.dtype == torch.float64 and best_cand.dtype == torch.int64 and best_cost.is_contiguous()
                     and best_cand.is_contiguous() and best_cand.data_ptr() == best_cost.data_ptr() + 8 * F
                     and best_cost.untyped_storage().data_ptr() == best_cand.untyped_storage().data_ptr())

@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define FCPP_ABI_VERSION 3
+#define FCPP_ABI_VERSION 4
 
 /* hard-coded sample counts of the reference (SURVEY.md §5) */
 #define FCPP_UTURN_POINTS 20      /* mlp3:807  */
@@ -256,18 +256,6 @@ int fcpp_winner_records(fcpp_handle *h, const fcpp_summary *d_summary, int64_t c
 int fcpp_status_count(fcpp_handle *h, const fcpp_summary *d_summary, int64_t n_cand, int32_t mask, int32_t *d_count,
                       void *stream);
 
-/* Multi-GPU, fused form of all-gather + fcpp_field_argmin_merge: ONE kernel writes this rank's (cost, candidate)
- * words into every rank's symmetric buffer over peer memory (NVLink P2P stores), publishes a flag per rank,
- * waits for the other ranks' flags and merges — no NCCL call.  d_best_cost / d_best_cand hold the local result
- * on entry and the global one on exit.  peer_bufs[p] / peer_flags[p] (HOST arrays of `world` device addresses):
- * rank p's slot array of 2 * world * 2 * n_fields 8-byte words and its flag array of `world` uint32, zeroed
- * before the first call and mapped into this process (e.g. torch symmetric memory); epoch = 1, 2, 3, ... per
- * call, identical on every rank.  A rank that does not arrive within ~10 s poisons the result (NaN, -2). */
-#define FCPP_MAX_PEERS 16
-int fcpp_field_argmin_exchange(fcpp_handle *h, int32_t world, int32_t rank, int32_t n_fields, uint32_t epoch,
-                               const uint64_t *peer_bufs, const uint64_t *peer_flags, double *d_best_cost,
-                               int64_t *d_best_cand, void *stream);
-
 /* Generic A7/A8/A13 on caller-supplied paths (ragged batch, path p = points offsets[p]..offsets[p+1]):
  * speed planning mlp3:467-589 (d_speeds_out may alias d_speeds_in), curvature verification
  * mlp3:1373-1424 and length/time mlp3:1290-1311 into d_summary (fields n_accel_viol, max_*,
@@ -406,9 +394,6 @@ int64_t fcpp_last_total_points(const fcpp_handle *h);
  * CUDA events on the launching stream; fcpp_kernel_times (call after synchronising the stream)
  * returns the milliseconds of the last call: [0] layout (+scan), [1] plan, [2] coverage. */
 int fcpp_set_profiling(fcpp_handle *h, int on);
-/* 1 when the last fcpp_plan_batch ran plan and coverage as ONE fused kernel (CTA roles, fcpp_hot.cu): the kernel
- * times then are [0] layout, [1] ~0, [2] the fused kernel.  Opt-in: fcpp_set_cover_mode bit 2. */
-int32_t fcpp_last_fused(const fcpp_handle *h);
 int fcpp_kernel_times(fcpp_handle *h, float *ms3);
 
 /* Diagnostics: coverage-kernel evaluation mode of the following fcpp_plan_batch calls.  0 = automatic
@@ -416,10 +401,10 @@ int fcpp_kernel_times(fcpp_handle *h, float *ms3);
  * (bitmap around the corners, closed form elsewhere), any other field row-tiled.  Bit 0 set = always
  * row-tiled.  Bit 1 set = no coverage de-duplication (by default candidates whose coverage inputs are
  * identical — same field, R, start corner; e.g. the headings of a heading search — are rasterised once
- * and share the counts).  Bit 2 set = plan and coverage as ONE fused kernel with CTA roles (measured slower on
- * config 2, see fcpp_hot.cu; default: two launches).  Bits 6 / 7 override fcpp_batch.cover_dedupe's choice
- * between one coverage CTA per candidate (bit 6) and the persistent grid over the listed representatives (bit 7).
- * All modes give identical results (tests/test_gpu_parity.py compares them). */
+ * and share the counts).  Bits 6 / 7 override fcpp_batch.cover_dedupe's choice between one coverage CTA per
+ * candidate (bit 6) and the persistent grid over the listed representatives (bit 7).  Any other bit is
+ * FCPP_ERR_INVALID and leaves the mode unchanged.  All modes give identical results (tests/test_gpu_parity.py
+ * compares them). */
 int fcpp_set_cover_mode(fcpp_handle *h, int mode);
 
 #ifdef __cplusplus

@@ -1,6 +1,5 @@
-"""Multi-GPU results on hardware (skipped below 2 GPUs; the driver's 1-GPU box skips it, `gpurun --gpus 2 --
-python -m pytest tests/test_gpu_multi.py -m gpu` runs it): the peer-memory exchange kernel and the NCCL
-merge path against the numpy rule, and plan_batch(distributed=True) against the single-process result."""
+"""Multi-GPU results on hardware (skipped below 2 GPUs): the per-field argmin exchange (NCCL all-gather +
+merge kernel) against the numpy rule, and plan_batch(distributed=True) against the single-process result."""
 import os
 import socket
 import subprocess

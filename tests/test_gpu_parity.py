@@ -361,6 +361,9 @@ def test_band_zoned_equals_row_tiled_and_oracle(fc):
     from field_coverage_path_planning_b200 import _lib
     from oracle import batch as ob, ref_planner as rp
     h = _lib.handle(0)
+    # mode bits other than 0, 1, 6 and 7 are rejected (bit 2 once selected a fused plan + coverage kernel)
+    for bad in (4, 5, 8, 16, 32):
+        assert h.lib.fcpp_set_cover_mode(h.h, bad) == -1, bad  # FCPP_ERR_INVALID
 
     def both(fields, veh, cand, modes=(1, 2, 3), **kw):
         """mode bit 0: row-tiled band only; bit 1: no coverage de-duplication (on by default in batches with a
@@ -626,41 +629,6 @@ def test_verify_all_corners_returns_grid_and_origin(fc):
             assert c["grid"].shape == (g, g) and c["grid"].dtype == bool
             assert np.array_equal(c["grid"], want), (R, k)
             assert (c["cells_before"], c["cells_after"]) == (n1, n2) and int(c["grid"].sum()) == n2
-
-
-def test_fused_plan_cover_kernel_identical(fc):
-    """Opt-in fused plan + coverage kernel (CTA roles: four plans per 512-thread CTA on named barriers next to
-    coverage CTAs, fcpp_hot.cu) == the two separate launches, bit for bit: summaries, paths, speeds, argmin;
-    batch sizes that are not a multiple of four, dead candidates, obstacles, a heading search."""
-    import torch
-    from field_coverage_path_planning_b200 import _lib
-    h = _lib.handle(0)
-    veh = fc.VehicleParams()
-    tiny = [(0, 0), (30, 0), (30, 15), (0, 15)]
-    para = [(100, 50), (600, 120), (640, 330), (140, 260)]
-    cases = [
-        ([RECT], fc.make_candidates(1, radii=np.linspace(5.0, 12.0, 257), start_corners=[0, 1, 2, 3]), [OBST2]),
-        ([RECT, tiny, para], fc.make_candidates(3, radii=[6.0, 8.0, 11.0], start_corners=[0, 2, 3]), None),
-        ([para, RECT], fc.make_candidates(2, headings=np.deg2rad(np.arange(0.0, 180.0, 9.0)), radii=[7.0]), None),
-        ([RECT], fc.make_candidates(1, radii=[8.0]), None),
-    ]
-    n_fused = 0
-    for fields, cand, obst in cases:
-        a = fc.plan_batch(fields, veh, cand, obstacles=obst, outputs="paths")
-        assert int(h.lib.fcpp_last_fused(h.h)) == 0
-        try:
-            h.check(h.lib.fcpp_set_cover_mode(h.h, 4))
-            b = fc.plan_batch(fields, veh, cand, obstacles=obst, outputs="paths")
-            # (a batch whose longest headland does not leave room for four plans per CTA falls back to two launches)
-            n_fused += int(h.lib.fcpp_last_fused(h.h))
-        finally:
-            h.check(h.lib.fcpp_set_cover_mode(h.h, 0))
-        assert a.summary.tobytes() == b.summary.tobytes()
-        assert np.array_equal(a.best_cand, b.best_cand) and np.array_equal(a.best_cost, b.best_cost)
-        n = int(a.offsets[-1])
-        assert np.array_equal(a.offsets, b.offsets)
-        assert torch.equal(a.d_path[:n], b.d_path[:n]) and torch.equal(a.d_speeds[:n], b.d_speeds[:n])
-    assert n_fused >= 2
 
 
 def test_factored_candidate_sets_identical_to_explicit_arrays(fc):

@@ -195,40 +195,6 @@ def test_plan_longer_than_shared_memory_staging_per_vehicle(fc, name):
 
 
 @gpu
-@pytest.mark.parametrize("name", ["sf1.5", "alat0.001"])
-def test_fused_plan_cover_kernel_identical_per_vehicle(fc, name):
-    """The opt-in fused plan + coverage kernel (fcpp_set_cover_mode bit 2) == the two separate launches, bit for
-    bit, under a vehicle with many violations and one with speeds below the time floor."""
-    import torch
-    from field_coverage_path_planning_b200 import _lib
-    h = _lib.handle(0)
-    veh, _, _ = vehicles(fc, name)
-    tiny = [(0, 0), (30, 0), (30, 15), (0, 15)]
-    cases = [
-        ([RECT], fc.make_candidates(1, radii=np.linspace(5.0, 12.0, 257), start_corners=CORNERS), [OBST2]),
-        ([RECT, tiny, PARA], fc.make_candidates(3, radii=[6.0, 8.0, 11.0], start_corners=[0, 2, 3]), None),
-        ([PARA, RECT], fc.make_candidates(2, headings=np.deg2rad(np.arange(0.0, 180.0, 9.0)), radii=[7.0]), None),
-        ([RECT], fc.make_candidates(1, radii=np.linspace(5.0, 8.0, 65), start_corners=CORNERS), [OBST2]),
-        ([RECT], fc.make_candidates(1, radii=[8.0]), None),
-    ]
-    n_fused = 0
-    for fields, cand, obst in cases:
-        a = fc.plan_batch(fields, veh, cand, obstacles=obst, outputs="paths")
-        try:
-            h.check(h.lib.fcpp_set_cover_mode(h.h, 4))
-            b = fc.plan_batch(fields, veh, cand, obstacles=obst, outputs="paths")
-            n_fused += int(h.lib.fcpp_last_fused(h.h))
-        finally:
-            h.check(h.lib.fcpp_set_cover_mode(h.h, 0))
-        assert a.summary.tobytes() == b.summary.tobytes()
-        assert np.array_equal(a.best_cand, b.best_cand) and np.array_equal(a.best_cost, b.best_cost)
-        n = int(a.offsets[-1])
-        assert np.array_equal(a.offsets, b.offsets)
-        assert torch.equal(a.d_path[:n], b.d_path[:n]) and torch.equal(a.d_speeds[:n], b.d_speeds[:n])
-    assert n_fused >= 2
-
-
-@gpu
 @pytest.mark.parametrize("turn_model", ["omega", "clothoid"])
 @pytest.mark.parametrize("name", ["sf1.5", "along0.02"])
 def test_opt_in_turn_models_vs_oracle_per_vehicle(fc, name, turn_model):

@@ -29,7 +29,7 @@ def test_library_exports_every_declared_symbol(built):
     for name in declared:
         assert hasattr(L, name), name
     assert declared == set(_lib.EXPORTS)
-    assert L.fcpp_abi_version() == _lib.ABI_VERSION == 3
+    assert L.fcpp_abi_version() == _lib.ABI_VERSION == 4
 
 
 def test_struct_mirrors_match_c_layout(built, tmp_path):
