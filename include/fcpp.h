@@ -260,7 +260,10 @@ int fcpp_status_count(fcpp_handle *h, const fcpp_summary *d_summary, int64_t n_c
  * speed planning mlp3:467-589 (d_speeds_out may alias d_speeds_in), curvature verification
  * mlp3:1373-1424 and length/time mlp3:1290-1311 into d_summary (fields n_accel_viol, max_*,
  * len_main, time_main, time_main_pre; the split point n_main = whole path).
- * do_speed_plan = 0 verifies the given speeds without adjusting them. */
+ * do_speed_plan = 0 verifies the given speeds without adjusting them.
+ * max_path_len sizes the per-path staging: paths of up to max_path_len rounded up to a multiple of 256 points (0: up
+ * to the largest shared-memory staging, ~9500 points on a B200) are processed; a longer path gets status
+ * FCPP_CAND_TOO_LARGE, zero lengths, times, counts and maxima, and no speeds or curvature written. */
 int fcpp_speed_verify(fcpp_handle *h, const fcpp_vehicle *veh, const double *d_path_xy,
                       const double *d_speeds_in, const int64_t *d_offsets, int64_t n_paths,
                       int64_t max_path_len, int do_speed_plan, double *d_speeds_out,

@@ -365,9 +365,11 @@ def test_band_zoned_equals_row_tiled_and_oracle(fc):
     for bad in (4, 5, 8, 16, 32):
         assert h.lib.fcpp_set_cover_mode(h.h, bad) == -1, bad  # FCPP_ERR_INVALID
 
-    def both(fields, veh, cand, modes=(1, 2, 3), **kw):
+    def both(fields, veh, cand, modes=(1, 2, 3, 64, 128, 65, 129), **kw):
         """mode bit 0: row-tiled band only; bit 1: no coverage de-duplication (on by default in batches with a
-        heading or start-corner axis: corner windows shared per (field, R), bands per (field, R, corner))"""
+        heading or start-corner axis: corner windows shared per (field, R), bands per (field, R, corner)); bits 6 / 7:
+        one coverage CTA per candidate / the persistent work list over the representatives, whichever the batch
+        would choose (a heading search takes the work list, every other de-duplicated batch one CTA per candidate)"""
         auto = fc.plan_batch(fields, veh, cand, **kw).summary
         for mode in modes:
             try:
@@ -404,12 +406,12 @@ def test_band_zoned_equals_row_tiled_and_oracle(fc):
     # rasterising every candidate (mode 2), also with duplicated and dead candidates in the batch
     hc = fc.make_candidates(len(fields), headings=np.deg2rad(np.arange(0.0, 180.0, 15.0)), radii=[6.0, 8.0],
                             start_corners=[0, 2])
-    s = both(fields, veh, hc, modes=(1, 2, 3))
+    s = both(fields, veh, hc)
     per = s["cov_cells"].reshape(len(fields), 12, 4)
     assert (per == per[:, :1, :]).all() and (s["cov_cells"] > 0).all()
     tiny = [[(0, 0), (30, 0), (30, 15), (0, 15)]] + fields[:2]       # field 0: inset empty -> dead candidates
     tc = fc.make_candidates(3, headings=[0.0, 0.3], radii=[8.0, 8.0], start_corners=[1])
-    s = both(tiny, veh, tc, modes=(2,))
+    s = both(tiny, veh, tc, modes=(2, 64, 128))
     assert (s["status"][:4] != 0).all() and (s["cov_total"][:4] == 0).all() and (s["cov_total"][4:] > 0).all()
     # many narrow loops: K = 12, 15 and 16 headland loops (48-64 chain rectangles = the cap)
     narrow = [[(0, 0), (120, 0), (120, 90), (0, 90)]]
