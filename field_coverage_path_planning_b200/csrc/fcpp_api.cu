@@ -223,7 +223,7 @@ int fcpp_layout(fcpp_handle *h, const fcpp_batch *batch, int32_t *d_n_pts, int64
     if (rc) return rc;
     cudaError_t e = fcpp_launch_layout(h, *batch, d_n_pts, d_offsets, st);
     if (e != cudaSuccess) return cuda_fail(h, e, "layout kernel");
-    // the plan kernel sizes its shared-memory staging by the longest plan of the batch
+    // the plan and coverage kernels size their shared-memory staging by the longest headland of the batch
     int maxn = batch->max_points_hint, maxhead = batch->max_head_points_hint;
     if (maxn <= 0 || maxhead <= 0) {
         h->h_maxn[0] = h->h_maxn[1] = 0;
@@ -245,9 +245,6 @@ int fcpp_layout(fcpp_handle *h, const fcpp_batch *batch, int32_t *d_n_pts, int64
         h->last_total = -1;  // asynchronous pass: nothing was read back
     }
     h->cover_pcap = maxhead;
-    int want = (maxn + 63) / 64 * 64;
-    if (want < 256) want = 256;
-    h->plan_ncap_hint = want;
     h->layout_valid = true;
     h->layout_ncand = batch->n_cand;
     h->layout_id[0] = batch->cand_field ? (const void *)batch->cand_R : (const void *)batch->ax_radii;

@@ -64,11 +64,10 @@ struct fcpp_handle {
     CandRec *d_rec;
     int64_t rec_cap;
     void *d_scan_tmp;
-    void *d_big;             // HBM staging of plans that do not fit shared memory
+    void *d_big;             // HBM staging of caller-supplied paths that do not fit shared memory
     int64_t big_cap;
     int64_t scan_tmp_cap;
     int64_t launches;
-    int plan_ncap_hint;      // smem point capacity wanted by the next plan launch (0 = maximum)
     int *d_maxn;             // device: [max n_total, max n_head] of the last layout pass
     int *h_maxn;             // pinned host mirror
     int max_smem_optin;

@@ -23,32 +23,38 @@
 
 namespace {
 
-constexpr int T0 = FCPP_PLAN_THREADS;  // threads per CTA of the smallest variant; plan_kernel also runs at 2x and 4x
+constexpr int T0 = FCPP_PLAN_THREADS;  // threads per CTA of the smallest variant; path_kernel also runs at 2x and 4x
 
+// generated plans (plan_gen_kernel, plan_gen_omega_kernel)
 struct PlanArgs {
-    // GEN
     fcpp_batch b;
     const CandRec *recs;
     const TrigTables *trig;
     fcpp_outputs out;
-    // generic (GEN = false)
+    int obs_cap_verts; // smem capacity for obstacle vertices
+    int obs_cap_polys;
+    int ncap;          // smem capacity in staged points
+};
+
+// caller-supplied paths (path_kernel, path_big_kernel)
+struct PathArgs {
     fcpp_vehicle veh;
     const double *in_path;
     const double *in_speeds;
     const int64_t *in_offsets;
     int do_speed_plan;
-    // both
-    int ncap;          // smem capacity in (staged) points
-    int nmin;          // this launch handles nmin < N <= ncap (tiers by plan length, see launch_tiers)
+    double *speeds_kmh;
+    double *curvature;
+    fcpp_summary *summary;
+    int ncap;          // smem capacity in points
+    int nmin;          // this launch handles nmin < N <= ncap (tiers by path length, see launch_tiers)
     int defer;         // 1: a later launch with a larger staging handles N > ncap
-    int obs_cap_verts; // smem capacity for obstacle vertices
-    int obs_cap_polys;
-    // plans longer than the shared-memory staging go through plan_big_kernel (HBM/L2 staging)
-    int big_enabled;          // regular kernel: leave candidates with N > ncap to the big kernel
+    // paths longer than the shared-memory staging go through path_big_kernel (HBM/L2 staging)
+    int big_enabled;          // regular kernel: leave paths with N > ncap to the big kernel
     int big_ncap;             // big kernel: point capacity of one CTA's scratch slice
     unsigned char *big_scratch;
     int64_t big_stride;       // bytes per CTA slice
-    int64_t n_items;          // candidates / paths in the batch
+    int64_t n_items;          // paths in the batch
 };
 
 // per-candidate table entry of a structure slot: segment length to the next point, curvature, curvature-limited
@@ -1087,11 +1093,11 @@ __global__ void __launch_bounds__(TG, FCPP_PLAN_GEN_MIN_CTAS) plan_gen_kernel(co
 
 // One caller-supplied path (A7 / A8 / A13 of the drop-in API): every point from its coordinates.
 template <bool BIG, int T>
-__device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s, const int64_t cand, const int cap)
+__device__ __forceinline__ void plan_body_path(const PathArgs &a, const Smem &s, const int64_t cand, const int cap)
 {
     const int tid = threadIdx.x;
     const fcpp_vehicle &veh = a.veh;
-    fcpp_summary *sum = a.out.summary ? a.out.summary + cand : nullptr;
+    fcpp_summary *sum = a.summary ? a.summary + cand : nullptr;
     const int64_t off = a.in_offsets[cand];
     const int N = (int)(a.in_offsets[cand + 1] - off);
     const int n_main = N;
@@ -1225,8 +1231,8 @@ __device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s,
     int n_aviol = 0;
     double mx[3] = {0.0, 0.0, 0.0};
     {
-        double *gs = a.out.speeds_kmh ? a.out.speeds_kmh + off : nullptr;
-        double *gk = a.out.curvature ? a.out.curvature + off : nullptr;
+        double *gs = a.speeds_kmh ? a.speeds_kmh + off : nullptr;
+        double *gk = a.curvature ? a.curvature + off : nullptr;
         for (int i = tid; i < N; i += T) {
             const double kap = s.Y[i];
             const double v0 = a.in_speeds[off + i];
@@ -1289,7 +1295,7 @@ __device__ __forceinline__ void plan_body_path(const PlanArgs &a, const Smem &s,
 // Caller-supplied paths.  T threads per CTA: T0 (256) when four or more CTAs fit an SM, 2*T0 / 4*T0 when the
 // staging of long paths leaves room for only two / one: the SM keeps ~32 resident warps either way
 template <int T>
-__global__ void __launch_bounds__(T, (T0 * FCPP_PLAN_MIN_CTAS) / T) path_kernel(const PlanArgs a)
+__global__ void __launch_bounds__(T, (T0 * FCPP_PLAN_MIN_CTAS) / T) path_kernel(const PathArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     if (a.nmin >= 0 || a.defer) {  // tiered launch: is this path in this tier's length range?
@@ -1302,7 +1308,7 @@ __global__ void __launch_bounds__(T, (T0 * FCPP_PLAN_MIN_CTAS) / T) path_kernel(
 
 // Paths that do not fit the shared-memory staging (N > ~9000 points): a few persistent CTAs walk the batch and
 // run the same body with x/y/u staged in a per-CTA slice of library-owned HBM (L2-resident in practice).
-__global__ void __launch_bounds__(T0, 3) path_big_kernel(const PlanArgs a)
+__global__ void __launch_bounds__(T0, 3) path_big_kernel(const PathArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem s = carve(smem_raw, 0);
@@ -1320,7 +1326,7 @@ __global__ void __launch_bounds__(T0, 3) path_big_kernel(const PlanArgs a)
 }
 
 template <int T>
-cudaError_t launch_variant(const PlanArgs &a, int64_t n, size_t bytes, cudaStream_t st)
+cudaError_t launch_variant(const PathArgs &a, int64_t n, size_t bytes, cudaStream_t st)
 {
     cudaError_t e = cudaFuncSetAttribute(path_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
@@ -1341,7 +1347,7 @@ int capacity_for_ctas(fcpp_handle *h, int ctas)
 // into up to three TIERS by length — N <= cap4 at T0 threads and four CTAs per SM, cap4 < N <= cap2 at 2*T0 and
 // two, longer at 4*T0 and one — so that short paths do not inherit the occupancy of the longest.  Every tier
 // launches one CTA per path; CTAs outside the tier's range exit on one read.
-cudaError_t launch_tiers(fcpp_handle *h, PlanArgs &a, int64_t n, int want, int cap_max, bool big, cudaStream_t st)
+cudaError_t launch_tiers(fcpp_handle *h, PathArgs &a, int64_t n, int want, int cap_max, bool big, cudaStream_t st)
 {
     const int cap4 = capacity_for_ctas(h, 4);
     const int cap2 = capacity_for_ctas(h, 2);
@@ -1371,7 +1377,7 @@ cudaError_t launch_tiers(fcpp_handle *h, PlanArgs &a, int64_t n, int want, int c
 
 // launch path_big_kernel when the longest path exceeds the shared-memory capacity.  The HBM staging (h->d_big) is
 // owned and resized here only.
-cudaError_t launch_big(fcpp_handle *h, PlanArgs &a, int64_t n_items, int max_points, cudaStream_t st)
+cudaError_t launch_big(fcpp_handle *h, PathArgs &a, int64_t n_items, int max_points, cudaStream_t st)
 {
     const int big_ncap = (max_points + 255) / 256 * 256;
     const int64_t stride = (int64_t)(3 * align16(sizeof(double) * (size_t)big_ncap));
@@ -1410,7 +1416,6 @@ cudaError_t fcpp_launch_plan(fcpp_handle *h, const fcpp_batch &b, const fcpp_out
     a.obs_cap_verts = b.obs_poly_start ? b.max_obs_verts : 0;
     a.obs_cap_polys = b.obs_poly_start ? b.max_obs_polys : 0;
     a.ncap = (MAIN_STAGED + (h->cover_pcap > 0 ? h->cover_pcap : 0) + 63) / 64 * 64;
-    a.n_items = b.n_cand;
     const size_t bytes = gen_smem_bytes(a.ncap, a.obs_cap_verts, a.obs_cap_polys);
     if (bytes > (size_t)h->max_smem_optin) return cudaErrorInvalidValue;  // obstacle tables / headland beyond shared memory
     const bool omega = b.turn_model == FCPP_TURN_OMEGA;  // its own instance: the default patterns do not carry its code
@@ -1431,15 +1436,15 @@ cudaError_t fcpp_launch_speed_verify(fcpp_handle *h, const fcpp_vehicle &veh, co
                                      fcpp_summary *d_summary, cudaStream_t st)
 {
     if (n_paths == 0) return cudaSuccess;
-    PlanArgs a{};
+    PathArgs a{};
     a.veh = veh;
     a.in_path = d_path;
     a.in_speeds = d_speeds_in;
     a.in_offsets = d_offsets;
     a.do_speed_plan = do_speed_plan;
-    a.out.summary = d_summary;
-    a.out.speeds_kmh = d_speeds_out;
-    a.out.curvature = d_curv;
+    a.summary = d_summary;
+    a.speeds_kmh = d_speeds_out;
+    a.curvature = d_curv;
     const int cap_max = capacity_for_ctas(h, 1);
     const int want = max_len > 0 ? (int)((max_len + 255) / 256 * 256) : 0;
     a.ncap = (want > 0 && want < cap_max) ? want : cap_max;

@@ -160,8 +160,9 @@ def _speed_verify(h, batch, max_len, plan=1, alias=False, base=0):
 def test_speed_verify_ragged_batch_across_tiers_vs_oracle(fc, h, ragged):
     """Speed planning, per-point curvature, length, times and the curvature verification of every path of a batch
     that spans the three shared-memory tiers (256 / 512 / 1024 threads) and the HBM-staged kernel, against
-    oracle/ref_planner; then the same batch without speed planning, with the speeds aliased in place, and at a
-    non-zero base offset inside larger buffers."""
+    oracle/ref_planner; then paths of the batch one per call with max_path_len = n, as the drop-in planner calls it
+    (a path's thread count depends on its own length only, so the bytes are those of the batch), the same batch
+    without speed planning, with the speeds aliased in place, and at a non-zero base offset inside larger buffers."""
     cap4, cap2, cap1 = ragged["caps"]
     lengths, off, ref = ragged["lengths"], ragged["offsets"], ragged["ref"]
     longest = int(lengths.max())
@@ -199,6 +200,18 @@ def test_speed_verify_ragged_batch_across_tiers_vs_oracle(fc, h, ragged):
     print(f"max |speed - oracle| {worst_v:.3e} km/h, max |kappa - oracle| {worst_k:.3e} 1/m")
     total = int(off[-1])
     assert not np.isnan(spd[:total]).any() and not np.isnan(kap[:total]).any()
+
+    # one path per call, max_path_len = n: the same bytes as inside the batch, on both sides of cap4, cap2 and cap1
+    picks = [int(np.flatnonzero((lengths >= 3) & (lengths < cap4))[0])]
+    picks += [int(np.flatnonzero(lengths == n)[0]) for n in (cap4, cap4 + 1, cap2, cap2 + 1, cap1, cap1 + 1, 2 * cap1)]
+    for b in picks:
+        o0, o1 = int(off[b]), int(off[b + 1])
+        n = o1 - o0
+        one = dict(lengths=lengths[b:b + 1], offsets=np.array([0, n], dtype=np.int64), xy=ragged["xy"][o0:o1],
+                   speeds=ragged["speeds"][o0:o1])
+        spd1, kap1, s1, _ = _speed_verify(h, one, n)
+        assert spd1[:n].tobytes() == spd[o0:o1].tobytes() and kap1[:n].tobytes() == kap[o0:o1].tobytes(), (b, n)
+        assert s1.tobytes() == s[b:b + 1].tobytes(), (b, n)
 
     # verification only: speeds pass through, the counts and maxima are those of the input speeds
     spd0, kap0, s0, _ = _speed_verify(h, ragged, longest, plan=0)
