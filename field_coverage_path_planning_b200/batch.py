@@ -35,12 +35,12 @@ def _dev(device) -> torch.device:
 
 
 class _Staging:
-    """Grow-only pinned host buffers of one device: ONE packed host->device copy of a batch's inputs
-    and ONE packed device->host copy of its results, instead of a cudaHostAlloc + copy per array."""
+    """Grow-only pinned host buffer of one device and slot: ONE packed host->device copy of a batch's inputs,
+    instead of a cudaHostAlloc + copy per array.  (Results are read back into ``_ResultPool`` buffers.)"""
     _per_dev: Dict[tuple, "_Staging"] = {}
 
     def __init__(self):
-        self.h_in = self.h_out = None
+        self.h_in = None
         self.in_done = None          # event: the last packed H2D copy has left h_in
 
     @classmethod
@@ -57,11 +57,6 @@ class _Staging:
             self.h_in = torch.empty(max(nbytes * 2, 1 << 20), dtype=torch.uint8).pin_memory()
         return self.h_in
 
-    def host_out(self, nbytes: int) -> torch.Tensor:
-        if self.h_out is None or self.h_out.numel() < nbytes:
-            self.h_out = torch.empty(max(nbytes * 2, 1 << 20), dtype=torch.uint8).pin_memory()
-        return self.h_out
-
 
 class _PinnedView:
     """numpy's owner object of a view into a pinned buffer: alive exactly as long as some array views it."""
@@ -77,7 +72,8 @@ class _ResultPool:
     memcpy out of a staging buffer (at 737 280 candidates that copy cost more than the PCIe transfer).  A buffer
     is reused only when no array views it any more (weak reference to the views' owner object), so a caller that
     drops the previous BatchResult runs allocation-free; one that keeps many results gets new buffers up to
-    ``MAX_BYTES`` and ordinary pageable copies beyond (``get`` returns None)."""
+    ``MAX_BYTES`` and, beyond that, a pinned buffer per read-back that the pool does not keep.  Every device->host
+    read-back takes its host memory from here: no two read-backs that can be in flight share a buffer."""
     MAX_BYTES = 4 << 30
     _bufs: List[list] = []          # [tensor, weakref to the _PinnedView handed out last | None]
 
@@ -87,7 +83,7 @@ class _ResultPool:
 
     @classmethod
     def get(cls, nbytes: int):
-        """-> (pinned uint8 tensor, numpy uint8 view of its first nbytes) or None."""
+        """-> (pinned uint8 tensor, numpy uint8 view of its first nbytes)."""
         import weakref
         nbytes = max(int(nbytes), 256)
         best = None
@@ -97,7 +93,8 @@ class _ResultPool:
         if best is None:
             cls._bufs = [e for e in cls._bufs if not cls._free(e)]      # free ones were too small
             if sum(e[0].numel() for e in cls._bufs) + nbytes > cls.MAX_BYTES:
-                return None
+                t = torch.empty(nbytes, dtype=torch.uint8).pin_memory()   # freed with the last view of it
+                return t, np.asarray(_PinnedView(t, nbytes))
             best = [torch.empty(max(nbytes + (nbytes >> 2), 1 << 20), dtype=torch.uint8).pin_memory(), None]
             cls._bufs.append(best)
         pv = _PinnedView(best[0], nbytes)
@@ -611,12 +608,13 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, co
 
 class _PendingFetch:
     """The read-back of a launched batch, enqueued but not waited for."""
-    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "pooled", "ho", "lay", "event")
+    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "hv", "lay", "win", "hwin", "event")
 
 
 def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
-                   cand_base: int) -> _PendingFetch:
-    """Enqueue the copies of summaries + argmin (+ offsets) into ONE pinned buffer on torch's current stream and
+                   cand_base: int, win: Optional[torch.Tensor] = None) -> _PendingFetch:
+    """Enqueue the copies of summaries + argmin (+ offsets) (+ ``win``: the winners' records and flag-count word
+    of a sharded batch, see dist.gather_winner_records) into ONE pooled pinned buffer on torch's current stream and
     record an event behind them; nothing is waited for."""
     dev = db.dev
     B, F = db.pb.n_cand, db.pb.n_fields
@@ -628,8 +626,10 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
         o_best = o_cost + ((F * 8 + 255) & ~255)
         o_off = o_best + ((F * 8 + 255) & ~255)
         total_out = o_off + ((B + 1) * 8 if need_off else 0)
-        pooled = _ResultPool.get(total_out)
-        ho = pooled[0] if pooled is not None else _Staging.get(dev, db.slot).host_out(max(total_out, 256))
+        o_win = (total_out + 255) & ~255
+        if win is not None:
+            total_out = o_win + win.numel()
+        ho, hv = _ResultPool.get(total_out)
         # the copies run on a COPY stream behind an event of the launching stream: the next batch's kernels (already
         # enqueued by a pipelining caller) must not wait for PCIe — at 737 280 candidates the 130 MB of summaries
         # share the link with the 360 MB of the previous batch's winners' paths
@@ -650,39 +650,33 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
                 ho[o_best:o_best + F * 8].view(torch.int64).copy_(buffers.d_best[:F], non_blocking=True)
             if need_off:
                 ho[o_off:o_off + (B + 1) * 8].view(torch.int64).copy_(buffers.d_off[:B + 1], non_blocking=True)
+            if win is not None:
+                ho[o_win:total_out].copy_(win, non_blocking=True)
             pf.event = torch.cuda.Event()
             pf.event.record(cs)
     pf.db, pf.buffers, pf.outputs, pf.offsets, pf.cand_base = db, buffers, outputs, offsets, cand_base
-    pf.pooled, pf.ho, pf.lay = pooled, ho, (nb_sum, need_off, o_cost, o_best, o_off)
+    pf.hv, pf.lay = hv, (nb_sum, need_off, o_cost, o_best, o_off)
+    pf.win, pf.hwin = win, (hv[o_win:total_out] if win is not None else None)
     return pf
 
 
 def _finish_fetch(pf: _PendingFetch) -> "BatchResult":
-    """Wait for the read-back of ``_enqueue_fetch`` (ONE synchronisation, on its event) and assemble the result."""
-    db, buffers, offsets = pf.db, pf.buffers, pf.offsets
+    """Wait for the read-back of ``_enqueue_fetch`` (ONE synchronisation, on its event) and assemble the result:
+    its arrays are views of the read-back's own pooled buffer."""
+    db, buffers, offsets, hv = pf.db, pf.buffers, pf.offsets, pf.hv
     B, F = db.pb.n_cand, db.pb.n_fields
     nb_sum, need_off, o_cost, o_best, o_off = pf.lay
     pf.event.synchronize()
-    pooled = pf.pooled
-    hv = pooled[1] if pooled is not None else pf.ho.numpy()
-    own = (lambda a: a) if pooled is not None else (lambda a: a.copy())   # pooled: the views ARE the result
-    summary = own(hv[:nb_sum]).view(_lib.SUMMARY_DTYPE)[:B] if nb_sum else np.zeros(0, dtype=_lib.SUMMARY_DTYPE)
-    best_cost = own(hv[o_cost:o_cost + F * 8]).view(np.float64)
-    best_cand = own(hv[o_best:o_best + F * 8]).view(np.int64)
+    summary = hv[:nb_sum].view(_lib.SUMMARY_DTYPE)[:B] if nb_sum else np.zeros(0, dtype=_lib.SUMMARY_DTYPE)
+    best_cost = hv[o_cost:o_cost + F * 8].view(np.float64)
+    best_cand = hv[o_best:o_best + F * 8].view(np.int64)
     if need_off:
-        offsets = own(hv[o_off:o_off + (B + 1) * 8]).view(np.int64)
+        offsets = hv[o_off:o_off + (B + 1) * 8].view(np.int64)
     res = BatchResult(summary=summary, best_cand=best_cand, best_cost=best_cost, n_fields=F, offsets=offsets,
                       d_path=buffers.d_path, d_speeds=buffers.d_spd, d_curvature=buffers.d_kap,
                       d_summary=buffers.d_sum, cand_base=pf.cand_base)
     res.extras["buffers"] = buffers
     return res
-
-
-def _fetch_device_batch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
-                        cand_base: int) -> "BatchResult":
-    """Copy summaries + argmin (+ offsets) of a launched batch back: one pinned buffer, async copies on torch's
-    current stream, ONE synchronisation."""
-    return _finish_fetch(_enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base))
 
 
 _side_streams: Dict[int, "torch.cuda.Stream"] = {}
@@ -709,6 +703,22 @@ def _side_stream(dev: torch.device) -> "torch.cuda.Stream":
     return st
 
 
+def _read_back_paths(d_path: torch.Tensor, d_speeds: torch.Tensor, spans):
+    """The point ranges ``spans`` [(a, b), ...] of a device path and its speeds, back to back in one pooled pinned
+    buffer: async copies on torch's current stream, ONE synchronisation.  -> (path [n, 2], speeds [n]) numpy views."""
+    tot = sum(b - a for a, b in spans)
+    ho, hv = _ResultPool.get(tot * 24 + 256)
+    hp = ho[:tot * 16].view(torch.float64).view(tot, 2)
+    hs = ho[tot * 16:tot * 24].view(torch.float64)
+    at = 0
+    for a, b in spans:
+        hp[at:at + b - a].copy_(d_path[a:b], non_blocking=True)
+        hs[at:at + b - a].copy_(d_speeds[a:b], non_blocking=True)
+        at += b - a
+    torch.cuda.current_stream(d_path.device).synchronize()
+    return hv[:tot * 16].view(np.float64).reshape(tot, 2), hv[tot * 16:tot * 24].view(np.float64)
+
+
 def fetch_winner_paths(db: DeviceBatch, res: BatchResult, outputs: str, best_cand: Optional[np.ndarray] = None,
                        slot: Optional[int] = None) -> int:
     """Bring the path and the speed profile of every field's best candidate to the host
@@ -730,28 +740,12 @@ def fetch_winner_paths(db: DeviceBatch, res: BatchResult, outputs: str, best_can
     if len(own) == 0:
         return 0
     local = (best[own] - res.cand_base).astype(np.int64)
-    nbytes = 0
     with torch.cuda.device(dev):
         if outputs == "paths" and len(own) <= 16 and res.offsets is not None:
             o0, o1 = res.offsets[local], res.offsets[local + 1]
-            tot = int((o1 - o0).sum())
-            pooled = _ResultPool.get(tot * 24 + 256)
-            ho = pooled[0] if pooled is not None else _Staging.get(dev, db.slot).host_out(tot * 24 + 256)
-            hp = ho[:tot * 16].view(torch.float64).view(tot, 2)
-            hs = ho[tot * 16:tot * 24].view(torch.float64)
-            at = 0
-            for a, b in zip(o0, o1):
-                n = int(b - a)
-                hp[at:at + n].copy_(res.d_path[int(a):int(b)], non_blocking=True)
-                hs[at:at + n].copy_(res.d_speeds[int(a):int(b)], non_blocking=True)
-                at += n
-            torch.cuda.current_stream(dev).synchronize()
-            if pooled is not None:
-                P, S = pooled[1][:tot * 16].view(np.float64).reshape(tot, 2), pooled[1][tot * 16:tot * 24].view(np.float64)
-            else:
-                P, S = hp.numpy().copy(), hs.numpy().copy()
+            P, S = _read_back_paths(res.d_path, res.d_speeds, [(int(a), int(b)) for a, b in zip(o0, o1)])
             offs = np.concatenate([[0], np.cumsum(o1 - o0)])
-            nbytes = tot * 24
+            nbytes = len(S) * 24
         else:
             if db.pb.axes is not None:
                 # the winners of a factored set as explicit candidates (a few values per field from the axes)
@@ -772,17 +766,7 @@ def fetch_winner_paths(db: DeviceBatch, res: BatchResult, outputs: str, best_can
             dbw = DeviceBatch(pbw, dev, slot=slot)
             rw = run_device_batch(dbw, "paths", copy_summary=False)
             tot = int(rw.offsets[-1])
-            pooled = _ResultPool.get(tot * 24 + 256)
-            ho = pooled[0] if pooled is not None else _Staging.get(dev, db.slot).host_out(tot * 24 + 256)
-            hp = ho[:tot * 16].view(torch.float64).view(tot, 2)
-            hs = ho[tot * 16:tot * 24].view(torch.float64)
-            hp.copy_(rw.d_path[:tot], non_blocking=True)
-            hs.copy_(rw.d_speeds[:tot], non_blocking=True)
-            torch.cuda.current_stream(dev).synchronize()
-            if pooled is not None:
-                P, S = pooled[1][:tot * 16].view(np.float64).reshape(tot, 2), pooled[1][tot * 16:tot * 24].view(np.float64)
-            else:
-                P, S = hp.numpy().copy(), hs.numpy().copy()
+            P, S = _read_back_paths(rw.d_path, rw.d_speeds, [(0, tot)])
             offs = rw.offsets
             nbytes = tot * 24 + (len(local) + 1) * 8 + 16 * db.pb.n_fields
             res.extras["h2d_bytes"] = res.extras.get("h2d_bytes", 0) + pbw.h2d_bytes()
@@ -807,11 +791,16 @@ class PendingBatch:
             nxt = plan_batch(..., candidates=next_candidates, wait=False)
             res = pend.result()
             pend = nxt
-    """
 
-    def __init__(self, db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits):
+    A sharded batch (``plan_batch(..., distributed=True)``) is collected the same way on every rank; its
+    ``result()`` is COLLECTIVE in one case only: when some rank's remembered launch sizes did not fit its shard,
+    all ranks repeat the batch together."""
+
+    def __init__(self, db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
+                 speculate, shard):
         self.db, self.pf, self.outputs = db, pf, outputs
         self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits)
+        self.speculate, self.shard = speculate, shard
         self._res = None
 
     def __del__(self):
@@ -829,27 +818,35 @@ class PendingBatch:
         db, pf, outputs = self.db, self.pf, self.outputs
         want_curvature, cost, cand_base, copy_summary, winners, corner_bits = self.args
         buffers = pf.buffers
+        B, F = db.pb.n_cand, db.pb.n_fields
+        rec = _lib.SUMMARY_DTYPE.itemsize
         res = _finish_fetch(pf)
-        if buffers.speculative and (not copy_summary or (res.summary["status"] & _SIZE_FLAGS).any()):
+        if self.shard is None:
+            redo = buffers.speculative and (not copy_summary or (res.summary["status"] & _SIZE_FLAGS).any())
+        else:
+            # the number of flagged candidates OF ALL RANKS: every rank reads the same word and decides alike, also
+            # a rank that had no remembered sizes itself
+            redo = self.speculate and int(pf.hwin[F * rec:F * rec + 4].view(np.int32)[0]) != 0
+        if redo:
             # remembered sizes (see _Hints) did not fit this batch, or cannot be checked: once more, sized from its
             # own layout pass.  (A batch with candidates that are genuinely too large takes this path too and comes
             # back with the same flags.)
             _Hints.drop(_Hints.key(db, outputs, want_curvature))
             self._res = run_device_batch(db, outputs, want_curvature, cost, cand_base, copy_summary, None, True,
-                                         winners, corner_bits, speculate=False)
+                                         winners, corner_bits, speculate=False, shard=self.shard)
             return self._res
-        B = db.pb.n_cand
         if corner_bits:   # [B, stride] words on the device; batch.corner_grids() unpacks one candidate's
             res.extras["corner_bits"] = buffers.d_cbits[:B * buffers.cbits_stride].view(B, -1)
         res.extras["h2d_bytes"] = db.pb.h2d_bytes()
-        res.extras["d2h_bytes"] = (len(res.summary) * _lib.SUMMARY_DTYPE.itemsize + 16 * db.pb.n_fields
-                                   + ((B + 1) * 8 if outputs == "paths" else 0))
+        res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F + ((B + 1) * 8 if outputs == "paths" else 0)
+        if self.shard is not None:
+            res.extras["winner_summary"] = pf.hwin[:F * rec].view(_lib.SUMMARY_DTYPE)
+            res.extras["shard"] = self.shard
+            res.extras["d2h_bytes"] += F * rec + 16
         res.extras["speculative"] = bool(buffers.speculative)
         if winners:
             # on the side stream: behind this batch (its event has completed), not behind later batches in flight
-            dev = db.dev
-            side = _side_stream(dev)
-            with torch.cuda.stream(side):
+            with torch.cuda.stream(_side_stream(db.dev)):
                 res.extras["d2h_bytes"] += fetch_winner_paths(db, res, outputs, slot=db.slot + 1)
         self._res = res
         return res
@@ -858,7 +855,8 @@ class PendingBatch:
 def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: bool = False,
                      cost: str = "length", cand_base: int = 0, copy_summary: bool = True,
                      buffers: Optional[BatchBuffers] = None, fetch: bool = True,
-                     winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True):
+                     winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True,
+                     shard: Optional[tuple] = None):
     """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + argmin back.
 
     With ``buffers`` (from a previous run of the same batch shape) and ``db.max_points`` known the
@@ -866,13 +864,22 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
     ``winners``: also bring every field's winning path and speeds to the host (``fetch_winner_paths``).
     ``speculate``: size the launch from remembered batches of the same shape instead of a synchronous layout
     read-back (``_Hints``; checked and repeated when the sizes do not fit).  ``wait=False`` returns a
-    ``PendingBatch``."""
+    ``PendingBatch``.  ``shard=(lo, hi)``: the batch is this rank's candidates [lo, hi) of a batch sharded over the
+    default process group; before the read-back the per-field argmin is merged over the ranks and every field's
+    winning summary record gathered (``dist.reduce_best``, ``dist.gather_winner_records``)."""
     buffers, offsets = _launch_device_batch(db, outputs, want_curvature, cost, cand_base, buffers,
                                             corner_bits=corner_bits, speculate=speculate and copy_summary)
     if not fetch:
         return None
-    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base)
-    pend = PendingBatch(db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits)
+    win = None
+    if shard is not None:
+        from . import dist
+        dist.reduce_best(buffers.d_cost, buffers.d_best)       # in place: now the GLOBAL per-field argmin
+        # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
+        win = dist.gather_winner_records(buffers.d_sum, buffers.d_best, shard[0], shard[1], count_mask=_SIZE_FLAGS)
+    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win)
+    pend = PendingBatch(db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
+                        speculate and copy_summary, shard)
     return pend if not wait else pend.result()
 
 

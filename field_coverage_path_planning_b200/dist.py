@@ -113,83 +113,14 @@ def gather_winner_records(summary_bytes: torch.Tensor, best_cand: torch.Tensor, 
     return words.view(torch.uint8).view(F, rec)
 
 
-class PendingShardedBatch:
-    """A sharded batch in flight on every rank (``plan_batch(..., distributed=True, wait=False)``).  ``result()`` is
-    COLLECTIVE in one case only: when some rank's remembered launch sizes did not fit its shard (every rank sees
-    that in the flag word that rides on the winners' records), all ranks repeat the batch together."""
-
-    def __init__(self, db, pf, hw, outputs, args, lo, hi, speculated):
-        self.db, self.pf, self.hw, self.outputs, self.args = db, pf, hw, outputs, args
-        self.lo, self.hi, self.speculated = lo, hi, speculated
-        self._res = None
-
-    def __del__(self):
-        try:        # an abandoned batch: wait for its read-back before the buffers go back to their pools
-            if self._res is None and self.pf is not None:
-                self.pf.event.synchronize()
-        except Exception:
-            pass
-
-    def result(self):
-        from .batch import _Hints, _finish_fetch, _side_stream, fetch_winner_paths
-        if self._res is not None:
-            return self._res
-        db, pf, outputs = self.db, self.pf, self.outputs
-        want_curvature, cost, winners = self.args
-        pb = db.pb
-        F = pb.n_fields
-        rec = _lib.SUMMARY_DTYPE.itemsize
-        res = _finish_fetch(pf)                                    # ONE synchronisation
-        hv = self.hw[1]
-        if self.speculated and int(hv[F * rec:F * rec + 4].view(np.int32)[0]) != 0:
-            # a rank's remembered sizes were too small (or a candidate is genuinely too large): every rank sees the
-            # same word and launches the batch again, sized from its own layout pass
-            _Hints.drop(_Hints.key(db, outputs, want_curvature))
-            self._res = _submit_sharded(db, outputs, want_curvature, cost, winners, self.lo, self.hi, False).result()
-            return self._res
-        res.extras["winner_summary"] = hv[:F * rec].view(_lib.SUMMARY_DTYPE).reshape(-1)[:F]
-        res.extras["shard"] = (self.lo, self.hi)
-        res.extras["h2d_bytes"] = pb.h2d_bytes()
-        res.extras["d2h_bytes"] = (len(res.summary) * rec + 16 * F + F * rec + 16
-                                   + ((pb.n_cand + 1) * 8 if outputs == "paths" else 0))
-        res.extras["speculative"] = bool(pf.buffers.speculative)
-        if winners:
-            with torch.cuda.stream(_side_stream(db.dev)):      # not behind later batches in flight
-                res.extras["d2h_bytes"] += fetch_winner_paths(db, res, outputs, slot=db.slot + 1)
-        self._res = res
-        return res
-
-
-def _submit_sharded(db, outputs, want_curvature, cost, winners, lo, hi, speculate):
-    """Kernels of this rank's shard, the two collectives and the read-back, all enqueued on the current stream."""
-    from .batch import _SIZE_FLAGS, _ResultPool, _Staging, _enqueue_fetch, _launch_device_batch
-    dev = db.dev
-    F = db.pb.n_fields
-    rec = _lib.SUMMARY_DTYPE.itemsize
-    bufs, offsets = _launch_device_batch(db, outputs, want_curvature, cost, lo, None, speculate=speculate)
-    reduce_best(bufs.d_cost, bufs.d_best)                   # in place: d_cost / d_best now hold the GLOBAL result
-    # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
-    win = gather_winner_records(bufs.d_sum, bufs.d_best, lo, hi, count_mask=_SIZE_FLAGS)
-    with torch.cuda.device(dev):                            # the winners' records ride on the same read-back
-        nb = F * rec + 16
-        pooled = _ResultPool.get(nb)
-        if pooled is None:
-            t = torch.empty(nb, dtype=torch.uint8).pin_memory()
-            pooled = (t, t.numpy())
-        pooled[0][:nb].copy_(win, non_blocking=True)
-    pf = _enqueue_fetch(db, bufs, outputs, offsets, True, lo)
-    # (the numpy view of a pooled buffer must stay referenced: the pool hands a buffer out again once its view is gone)
-    return PendingShardedBatch(db, pf, pooled, outputs, (want_curvature, cost, winners), lo, hi, bool(speculate))
-
-
 def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h, coverage, cost,
                        device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True):
     """plan_batch over all ranks of the default process group (see batch.plan_batch): every rank plans its
     contiguous shard; ONE all-gather + merge kernel gives every rank the per-field argmin, one kernel + one
     all-reduce every winner's summary record; the local summaries, the merged argmin and the winners' records
     come back to the host with ONE synchronisation.  Launch sizes are remembered from earlier batches of the same
-    shape (no layout read-back); ``wait=False`` returns a ``PendingShardedBatch``."""
-    from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch
+    shape (no layout read-back); ``wait=False`` returns a ``batch.PendingBatch``."""
+    from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch, run_device_batch
     if not dist.is_initialized():
         raise RuntimeError("distributed=True needs torch.distributed.init_process_group (backend 'nccl')")
     world, rank = dist.get_world_size(), dist.get_rank()
@@ -203,5 +134,5 @@ def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, out
     dev = _dev(device)
     pb = prepare_batch(fv, vehicle, local, obstacles, sp, grid_h, coverage, turn_model, clothoid_share)
     db = DeviceBatch(pb, dev)
-    pend = _submit_sharded(db, outputs, want_curvature, cost, winners, lo, hi, True)
-    return pend if not wait else pend.result()
+    return run_device_batch(db, outputs, want_curvature, cost, lo, winners=winners, speculate=True, wait=wait,
+                            shard=(lo, hi))
