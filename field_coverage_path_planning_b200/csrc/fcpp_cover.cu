@@ -66,7 +66,7 @@ struct CoverFixed {
     double qedge[2][4][3];  // field / main quad edges: ax, ay, k = ex/ey (relative coordinates)
     int4 qtype[2][4];       // per edge: x = +1 upper bound / -1 lower bound / 0 horizontal, y = ay, z = sign(ex)
     int2 fq[4], mq[4];      // snapped field quad and R-inset, relative to the band lattice origin
-    Target tg[4];
+    Target tg[8];
     int nrows, total_words;
     int next_w0;
     double rconst[2];  // raster_entries: r^2 and the certification margin in cells
@@ -76,9 +76,20 @@ struct CoverFixed {
     int4 rects[RECT_CAP];  // axis-aligned chains: lattice columns [x, y] on lattice rows [z, w] (see setup_entries)
     int nrect;
     // zoned band evaluation (see band_zoned): boxes around the general entries, one per field quadrant
-    int4 zbox[4];      // lattice columns [x, y], rows [z, w]; empty: x > y
-    int ztarget[4];    // zone -> target index of the current pass, -1 = not resident
-    int4 zt[4];        // per target of the current pass: zone, first tile word, words per row, unused
+    // (per corner and variant in band_grouped)
+    int4 zbox[8];      // lattice columns [x, y], rows [z, w]; empty: x > y
+    int ztarget[8];    // zone -> target index of the current pass, -1 = not resident
+    int4 zt[8];        // per target of the current pass: zone, first tile word, words per row, unused
+    // band_grouped: material m (m < 4: the arcs of corner m, m >= 4: the start corner m - 4) owns the points
+    // [moff[m], moff[m + 1]); per zone: covered cells of its bitmap and |U ∩ W ∩ Z|
+    int moff[9];
+    int zquad[8];
+    int zbad;          // materials with a general entry outside their corner's quadrant
+    int zbits[8];
+    unsigned long long zuw[8];
+    double pfill[4][5];  // loop-0 reverse fills by physical corner (the record itself is patched per start corner)
+    int pn[4];
+    unsigned long long gres[4][2];  // per start corner: band cells, covered band cells
 };
 
 // Dynamic part, behind CoverFixed in the same dynamic shared-memory allocation: the scheduling
@@ -614,9 +625,25 @@ __device__ __forceinline__ int rect_cover(const CoverFixed &s, int nr, int j, in
 // W = the row's band windows, Z = the zones' column intervals; the zones are pairwise disjoint).
 // Returns false (nothing counted) when the zones overlap or are too large; the caller then runs
 // the row-tiled evaluation of the whole band.
-__device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_ent, int rq, int H, double invH, int nx, int ny,
-                           unsigned long long &my_total, unsigned long long &my_cov)
+//
+// NZ = 8 (band_grouped): the zones are the materials of the four start corners' bands, the entries are assigned
+// to them by their index (s.moff), `want` is the set of start corners to evaluate.  Returns the start corners
+// whose four zones pass the checks; |U ∩ W| goes to my_total / my_cov, each zone's bitmap count to s.zbits and
+// its |U ∩ W ∩ Z| to s.zuw (the caller combines them per start corner).  NZ = 4 returns 1 or 0.
+__device__ __forceinline__ int material_of(const CoverFixed &s, int e)
 {
+    int m = 0;
+    while (m < 7 && e >= s.moff[m + 1]) ++m;
+    return m;
+}
+// the zones a start corner's band uses: the arc material of the three other corners, its own start material
+__device__ __forceinline__ unsigned zones_of(int sc) { return (0xfu & ~(1u << sc)) | (0x10u << sc); }
+
+template <int NZ>
+__device__ __noinline__ int band_zoned(CoverFixed &s, const CoverDyn &d, int n_ent, int rq, int H, double invH, int nx, int ny,
+                           unsigned long long &my_total, unsigned long long &my_cov, unsigned want = 0)
+{
+    static_assert(NZ == 4 || NZ == 8, "per-candidate quadrants or grouped materials");
     const int tid = threadIdx.x;
     const int nr = min(s.nrect, RECT_CAP);
     const int midx2 = (nx - 1) * H, midy2 = (ny - 1) * H;
@@ -630,7 +657,9 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
             rank += (x < mine.x || (x == mine.x && q < tid)) ? 1 : 0;
         }
     }
-    if (tid < 4) s.zbox[tid] = make_int4(INT_MAX, INT_MIN, INT_MAX, INT_MIN);
+    if (tid < NZ) s.zbox[tid] = make_int4(INT_MAX, INT_MIN, INT_MAX, INT_MIN);
+    if (NZ == 8 && tid < 8) s.zbits[tid] = 0, s.zuw[tid] = 0ull;
+    if (tid == 0) s.zbad = 0;
     __syncthreads();
     if (tid < nr) s.rects[rank] = mine;
     for (int e = tid; e < n_ent; e += T) {
@@ -641,7 +670,13 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
         const int cl = max(floor_div_i(min(sg.x, sg.z) - rq, H, invH), 0);
         const int ch = min(-floor_div_i(-(max(sg.x, sg.z) + rq), H, invH), nx - 1);
         if (jlo > jhi || cl > ch) continue;  // cannot touch the lattice
-        int4 *zb = &s.zbox[seg_quadrant(sg, midx2, midy2)];
+        int z = seg_quadrant(sg, midx2, midy2);
+        if (NZ == 8) {
+            const int m = material_of(s, e);
+            if (z != s.zquad[m]) atomicOr(&s.zbad, 1 << m);
+            z = m;
+        }
+        int4 *zb = &s.zbox[z];
         atomicMin(&zb->x, cl);
         atomicMax(&zb->y, ch);
         atomicMin(&zb->z, jlo);
@@ -649,29 +684,43 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
     }
     __syncthreads();
     // ---- the zones must be pairwise disjoint and small (uniform decision) ----
-    {
+    auto zones_ok = [&](unsigned use) {
         bool okz = true;
         long long words = 0;
-        for (int z = 0; z < 4; ++z) {
+        for (int z = 0; z < NZ; ++z) {
             const int4 a = s.zbox[z];
-            if (a.x > a.y) continue;
+            if (!((use >> z) & 1) || a.x > a.y) continue;
             const int rw = (a.y >> 5) - (a.x >> 5) + 1;
             words += (long long)rw * (a.w - a.z + 1);
             if (rw > TW - 16) okz = false;
-            for (int y = z + 1; y < 4; ++y) {
+            for (int y = z + 1; y < NZ; ++y) {
                 const int4 c = s.zbox[y];
-                if (c.x <= c.y && a.x <= c.y && c.x <= a.y && a.z <= c.w && c.z <= a.w) okz = false;
+                if (((use >> y) & 1) && c.x <= c.y && a.x <= c.y && c.x <= a.y && a.z <= c.w && c.z <= a.w) okz = false;
             }
         }
-        if (words > 12ll * TW) okz = false;
-#ifdef FCPP_COVER_DEBUG
-        if (tid == 0 && (blockIdx.x % 512) == 0) {  // (debug builds only)
-            printf("cand %d nrect %d okz %d words %lld\n", (int)blockIdx.x, nr, (int)okz, words);
-            for (int z = 0; z < 4; ++z) printf("  zone %d cols [%d,%d] rows [%d,%d]\n", z, s.zbox[z].x, s.zbox[z].y, s.zbox[z].z, s.zbox[z].w);
+        return okz && words <= 12ll * TW;
+    };
+    unsigned zuse = 0xffu, done = 1u;
+    if (NZ == 8) {
+        zuse = 0u;
+        done = 0u;
+        for (int sc = 0; sc < 4; ++sc) {
+            const unsigned u = zones_of(sc);
+            if (((want >> sc) & 1) && !(s.zbad & u) && zones_ok(u)) {
+                done |= 1u << sc;
+                zuse |= u;
+            }
         }
-#endif
-        if (!okz) return false;
+    } else {
+        done = zones_ok(0xfu) ? 1u : 0u;
     }
+#ifdef FCPP_COVER_DEBUG
+    if (tid == 0 && (blockIdx.x % 512) == 0) {  // (debug builds only)
+        printf("cand %d nrect %d zones %d done %x\n", (int)blockIdx.x, nr, NZ, done);
+        for (int z = 0; z < NZ; ++z) printf("  zone %d cols [%d,%d] rows [%d,%d]\n", z, s.zbox[z].x, s.zbox[z].y, s.zbox[z].z, s.zbox[z].w);
+    }
+#endif
+    if (!done) return 0;
 
     // ---- bitmap passes over the zones: whole zones are packed into one tile while they fit, a
     // zone larger than the tile is cut into row ranges (every thread derives the same packing) ----
@@ -679,11 +728,11 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
     while (true) {
         int nt = 0, used_w = 0, used_r = 0;
         __syncthreads();  // the previous pass is done with s.tg / s.zt / s.ztarget
-        if (tid < 4) s.ztarget[tid] = -1;
+        if (tid < NZ) s.ztarget[tid] = -1;
         __syncthreads();
-        while (z < 4 && nt < 4) {
+        while (z < NZ && nt < NZ) {
             const int4 box = s.zbox[z];
-            if (box.x > box.y) {
+            if (box.x > box.y || !((zuse >> z) & 1)) {
                 ++z;
                 zrow = 0;
                 continue;
@@ -732,11 +781,18 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
         {
             auto tgt = [&](int e) {
                 const int4 sg = d.ent(e).seg;
-                return (sg.y > sg.w) ? -1 : s.ztarget[seg_quadrant(sg, midx2, midy2)];
+                return (sg.y > sg.w) ? -1 : s.ztarget[NZ == 8 ? material_of(s, e) : seg_quadrant(sg, midx2, midy2)];
             };
             raster_entries(s, d, 0, n_ent, tgt, rq, H, invH);
         }
-        my_cov += (unsigned long long)count_words(s.tile, used_w);
+        if (NZ == 8) {
+            for (int t = 0; t < nt; ++t) {
+                const int c = __reduce_add_sync(0xffffffffu, count_words(s.tile + s.zt[t].y, s.tg[t].nrows * s.zt[t].z));
+                if ((tid & 31) == 0 && c) atomicAdd(&s.zbits[s.zt[t].x], c);
+            }
+        } else {
+            my_cov += (unsigned long long)count_words(s.tile, used_w);
+        }
     }
     // ---- every row in closed form: band cells, rectangle cover outside the zones.  Rows are
     // grouped into runs between BREAKPOINTS (rows where a rectangle or a zone starts or ends, and
@@ -746,9 +802,9 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
     // the run is counted once and multiplied.  Runs with slanted boundaries go row by row. ----
     __syncthreads();  // the last pass is done with the tile: reuse it for the breakpoints
     int *bp = reinterpret_cast<int *>(s.tile);  // [nb] sorted breakpoints, then [nb] slow runs (lo, hi)
-    const int nb = 10 + 2 * nr + 8;
-    static_assert(T >= 2 * (10 + 2 * RECT_CAP + 8), "one thread per (run, end)");
-    static_assert(12 * (10 + 2 * RECT_CAP + 8) <= TW, "breakpoints, slow runs and row intervals live in the tile");
+    const int nb = 10 + 2 * nr + 2 * NZ;
+    static_assert(T >= 2 * (10 + 2 * RECT_CAP + 2 * NZ), "one thread per (run, end)");
+    static_assert(12 * (10 + 2 * RECT_CAP + 2 * NZ) <= TW, "breakpoints, slow runs and row intervals live in the tile");
     {
         int v = -1;
         if (tid == 0) v = 0;
@@ -760,8 +816,9 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
             const int4 rc = s.rects[(tid - 10) >> 1];
             v = (tid & 1) ? rc.w + 1 : rc.z;
         } else if (tid < nb) {
-            const int4 box = s.zbox[(tid - 10 - 2 * nr) >> 1];
-            v = (box.x > box.y) ? 0 : ((tid & 1) ? box.w + 1 : box.z);
+            const int z = (tid - 10 - 2 * nr) >> 1;
+            const int4 box = s.zbox[z];
+            v = (box.x > box.y || !((zuse >> z) & 1)) ? 0 : ((tid & 1) ? box.w + 1 : box.z);
         }
         v = min(max(v, 0), ny);
         int *raw = bp + 2 * nb + 2;
@@ -791,7 +848,7 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
         int4 box = make_int4(INT_MIN, INT_MAX, INT_MIN, INT_MAX);
         if (p > 0) {
             box = s.zbox[p - 1];
-            if (box.x > box.y || j < box.z || j > box.w) return;
+            if (box.x > box.y || j < box.z || j > box.w || !((zuse >> (p - 1)) & 1)) return;
         }
         int cov = 0, cells = 0;
 #pragma unroll
@@ -804,13 +861,15 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
         if (p == 0) {
             my_total += mult * (unsigned long long)cells;
             my_cov += mult * (unsigned long long)cov;
+        } else if (NZ == 8) {
+            if (cov) atomicAdd(&s.zuw[p - 1], mult * (unsigned long long)cov);
         } else {
             my_cov -= mult * (unsigned long long)cov;
         }
     };
     int2 *slow = reinterpret_cast<int2 *>(bp + nb);
-    for (int u = tid; u < 5 * (nb - 1); u += T) {
-        const int i = u / 5, p = u - 5 * i;
+    for (int u = tid; u < (NZ + 1) * (nb - 1); u += T) {
+        const int i = u / (NZ + 1), p = u - (NZ + 1) * i;
         const int lo = bp[i], hi = bp[i + 1] - 1;
         if (lo > hi) continue;
         const int4 v0 = rraw[2 * i], v1 = rraw[2 * i + 1];
@@ -830,23 +889,161 @@ __device__ __noinline__ bool band_zoned(CoverFixed &s, const CoverDyn &d, int n_
         const int2 run = slow[q];
         for (int j = run.x + tid; j <= run.y; j += T) {
             const int4 win = band_row_windows(s, j * H, H, invH, nx);
-            for (int p = 0; p < 5; ++p) row_part(j, win, p, 1ull);
+            for (int p = 0; p <= NZ; ++p) row_part(j, win, p, 1ull);
         }
     }
     __syncthreads();  // the caller may reuse the tile
-    return true;
+    return (int)done;
+}
+
+// Grouped evaluation of the headland bands of the start corners `want` of one (field, R) whose straights are all
+// axis-aligned (CandRec.band_group).  Loop k of start corner sc runs corners[k][sc] -> sc+1 -> sc+2 -> sc+3 -> sc
+// (gen_point_tag): its four straights are the same for every start corner, and what lies at a physical corner c
+// has one of two forms, neither of which depends on sc:
+//   * c != sc, the ARC material: per loop [corner, 15 arc points, (loop 0) the reverse fill of c, corner] — the
+//     last point of the straight into c, the turn, the fill and the first point of the straight out of c;
+//   * c == sc, the START material: [corners[0][c], corners[0][c], corners[1][c], ..., corners[K-1][c]] — the
+//     first point of every loop, the last point of the loop before it and the joins between loops.
+// The straights are rectangles (their end discs are covered by the corner points of the materials), every
+// material segment is a general entry, and the band of sc is band_zoned's identity with the zones
+//     arc(c) for c != sc, start(sc):   cov(sc) = |U ∩ W| + Σ_zones (bits(Z) - |U ∩ W ∩ Z|).
+// So at most 8 zone bitmaps, one rectangle set and one |U ∩ W| serve up to four start corners.  The union of the
+// pieces' segments is the segment set of each start corner's polyline, and both evaluations are exact: the
+// counts equal the per-candidate ones.  Returns the start corners evaluated (s.gres); the others (zones that
+// overlap or are too large, a general entry outside its corner's quadrant, too many points) are left to the
+// per-candidate evaluation.
+__device__ __noinline__ unsigned band_grouped(CoverFixed &s, const CoverDyn &d, unsigned want, int pc, const TurnModel &tm,
+                                              int rq, double rd, int H, double invH, int nx, int ny, int64_t Xc0, int64_t Yc0)
+{
+    const int tid = threadIdx.x;
+    const CandRec &r = s.rec;
+    const int K = r.K;
+    constexpr int LOOP = FCPP_CORNER_POINTS + 2;  // arc material points of a loop without a reverse fill
+    if (tid == 0) {
+        int o = 0;
+        for (int m = 0; m < 8; ++m) {
+            const int c = m & 3;
+            s.moff[m] = o;
+            if (m < 4 && (want & ~(1u << c))) o += LOOP * K + s.pn[c];
+            if (m >= 4 && ((want >> c) & 1)) o += K + 1;
+        }
+        s.moff[8] = o;
+        s.nrect = 4 * K;
+        s.acc[0] = s.acc[1] = 0ull;
+    }
+    __syncthreads();
+    const int np = s.moff[8];
+    if (np > pc || 4 * K > RECT_CAP) return 0u;
+    auto snap = [&](int k, int c) {
+        return make_int2((int)(qfix(r.corners[k][c][0]) - Xc0), (int)(qfix(r.corners[k][c][1]) - Yc0));
+    };
+    // point j of an arc material: loop k, position j in the loop (in place), length of the loop
+    auto arc_pos = [&](int c, int &j, int &k) {
+        const int l0 = LOOP + s.pn[c];
+        k = 0;
+        if (j >= l0) {
+            k = 1 + (j - l0) / LOOP;
+            j = j - l0 - (k - 1) * LOOP;
+        }
+        return k ? LOOP : l0;
+    };
+    for (int i = tid; i < np; i += T) {
+        const int m = material_of(s, i), c = m & 3;
+        int j = i - s.moff[m], k;
+        double x = 0.0, y = 0.0;
+        if (m >= 4) {
+            k = j ? j - 1 : 0;
+            x = r.corners[k][c][0];
+            y = r.corners[k][c][1];
+        } else {
+            const int L = arc_pos(c, j, k);
+            if (j == 0 || j == L - 1) {
+                x = r.corners[k][c][0];
+                y = r.corners[k][c][1];
+            } else if (j <= FCPP_CORNER_POINTS) {
+                corner_arc_pt(s.tt, tm, r.corners[k][c][0], r.corners[k][c][1], r.R, c, j - 1, x, y);
+            } else {  // as gen_point_tag
+                const int mm = j - 1 - FCPP_CORNER_POINTS, nr = s.pn[c];
+                const double len = s.pfill[c][4];
+                const double tt_ = (mm == nr - 1) ? len : mm * (len / (nr - 1));
+                x = s.pfill[c][0] + tt_ * s.pfill[c][2];
+                y = s.pfill[c][1] + tt_ * s.pfill[c][3];
+            }
+        }
+        d.ent(i).erow = make_int2((int)(qfix(x) - Xc0), (int)(qfix(y) - Yc0));
+    }
+    if (tid < 4 * K) {  // straight c -> c + 1 of loop k (exactly axis-aligned: band_group)
+        const int k = tid >> 2, c = tid & 3;
+        const int2 p = snap(k, c), q = snap(k, (c + 1) & 3);
+        if (p.x == q.x) {
+            const int ylo = min(p.y, q.y), yhi = max(p.y, q.y);
+            s.rects[tid] = make_int4(floor_div_i(p.x - rq, H, invH) + 1, -floor_div_i(-(p.x + rq), H, invH) - 1,
+                                     -floor_div_i(-ylo, H, invH), floor_div_i(yhi, H, invH));
+        } else {
+            const int xlo = min(p.x, q.x), xhi = max(p.x, q.x);
+            s.rects[tid] = make_int4(-floor_div_i(-xlo, H, invH), floor_div_i(xhi, H, invH),
+                                     floor_div_i(p.y - rq, H, invH) + 1, -floor_div_i(-(p.y + rq), H, invH) - 1);
+        }
+    }
+    if (tid < 8) {  // quadrant of corner c, as seg_quadrant of the point
+        const int2 p = snap(0, tid & 3);
+        s.zquad[tid] = (2 * p.y >= (ny - 1) * H ? 2 : 0) | (2 * p.x >= (nx - 1) * H ? 1 : 0);
+    }
+    __syncthreads();
+    setup_entries<false, false>(s, d, 0, np - 1, rd, rq, H, invH);
+    __syncthreads();
+    // the segments between two pieces (loops, materials) are not on any path; entries inside the closed R-inset
+    // cover no band cell
+    for (int e = tid; e < np - 1; e += T) {
+        const int m = material_of(s, e);
+        bool dead = e + 1 == s.moff[m + 1];
+        if (m < 4) {
+            int j = e - s.moff[m], k;
+            const int L = arc_pos(m, j, k);
+            dead = dead || j == L - 1;
+        }
+        const int4 sg = d.ent(e).seg;
+        const int x0 = min(sg.x, sg.z) - rq, x1 = max(sg.x, sg.z) + rq, y0 = sg.y - rq, y1 = sg.w + rq;
+        if (dead || (in_quad(s.mq, x0, y0) && in_quad(s.mq, x1, y0) && in_quad(s.mq, x1, y1) && in_quad(s.mq, x0, y1)))
+            write_dead_entry(d, e);
+    }
+    __syncthreads();
+    unsigned long long my_total = 0ull, my_cov = 0ull;
+    const unsigned done = (unsigned)band_zoned<8>(s, d, np - 1, rq, H, invH, nx, ny, my_total, my_cov, want);
+    if (!done) return 0u;
+#pragma unroll
+    for (int dd = 16; dd > 0; dd >>= 1) {
+        my_total += __shfl_xor_sync(0xffffffffu, my_total, dd);
+        my_cov += __shfl_xor_sync(0xffffffffu, my_cov, dd);
+    }
+    if ((tid & 31) == 0) {
+        atomicAdd(&s.acc[0], my_total);
+        atomicAdd(&s.acc[1], my_cov);
+    }
+    __syncthreads();
+    if (tid < 4 && ((done >> tid) & 1)) {
+        unsigned long long cov = s.acc[1];
+        for (int m = 0; m < 8; ++m)
+            if ((zones_of(tid) >> m) & 1) cov += (unsigned long long)s.zbits[m] - s.zuw[m];
+        s.gres[tid][0] = s.acc[0];
+        s.gres[tid][1] = cov;
+    }
+    __syncthreads();
+    return done;
 }
 
 // One candidate's coverage by the T threads of a CTA (cover_kernel, or one listed item of cover_work_kernel).
 __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *__restrict__ recs,
                                            const TrigTables *__restrict__ trig, fcpp_summary *__restrict__ summary,
                                            int pc, int mode, const int32_t *__restrict__ rep /*[2][n_cand]*/,
+                                           const uint32_t *__restrict__ band_mask, longlong2 *__restrict__ band_out,
                                            uint32_t *__restrict__ corner_bits, int64_t corner_bits_stride,
                                            const int64_t cand)
 {
     // a part (A10 corner windows / A11 band) whose inputs equal those of an earlier candidate is
     // skipped: the candidate takes that one's counts afterwards (cover_copy_kernel).  A10 does not
-    // depend on the start corner or the heading, A11 not on the heading.
+    // depend on the start corner or the heading, A11 not on the heading.  A band representative writes the band of
+    // every start corner it evaluates to band_out[4 cand + start corner]; band_mask (band_group records) names them.
     const bool do10 = !rep || rep[cand] == (int32_t)cand;
     const bool do11 = !rep || rep[b.n_cand + cand] == (int32_t)cand;
     if (!do10 && !do11) return;
@@ -871,6 +1068,8 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
     if (r.status != 0 || r.n_total == 0) {
         if (tid == 0) {
             if (do11) sum->cov_cells = sum->cov_total = 0;
+            if (do11 && band_out)
+                for (int k = 0; k < 4; ++k) band_out[4 * cand + k] = make_longlong2(0, 0);
             if (do10)
                 for (int k = 0; k < 4; ++k) sum->corner_before[k] = sum->corner_after[k] = 0;
         }
@@ -1019,145 +1218,202 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
         const int64_t Xc0 = X0 + H64 / 2, Yc0 = Y0 + H64 / 2;  // lattice origin: centre of cell (0, 0)
         const int H = (int)H64, nx = (int)nx64, ny = (int)ny64;
         const double invH = 1.0 / (double)H;
-        const int nh = r.n_head;
         // relative coordinates must fit int32 with headroom (extent + r < 2^30 units = 107 km)
-        const bool ok = (nh <= pc) && nx64 > 0 && ny64 > 0 && nx64 * H64 < (1ll << 30) && ny64 * H64 < (1ll << 30) &&
-                        H64 < (1 << 20);
-        if (!ok) err11 = 1;
-        __syncthreads();
-        if (ok) {
-            if (tid == 0) s.nrect = 0;
+        const bool lat_ok = nx64 > 0 && ny64 > 0 && nx64 * H64 < (1ll << 30) && ny64 * H64 < (1ll << 30) && H64 < (1 << 20);
+        // the start corners to evaluate: this candidate's own, or (band_group) those of its whole group
+        const int own = r.flags & FCPP_FLAG_CORNER_MASK;
+        const bool grp = band_mask && r.band_group;
+        unsigned todo = grp ? band_mask[cand] : (1u << own);
+        auto put = [&](int sc, unsigned long long total, unsigned long long cells, bool err) {
+            if (tid != 0) return;
+            if (sc == own) {
+                sum->cov_total = err ? 0 : (int64_t)total;
+                sum->cov_cells = err ? 0 : (int64_t)cells;
+                if (err) err11 = 1;
+            }
+            if (band_out) band_out[4 * cand + sc] = make_longlong2(err ? -1 : (long long)total, err ? 0 : (long long)cells);
+        };
+        if (tid < 4) {  // reverse fill of physical corner tid: rev[t] is the fill of corner (own + t + 1) & 3
+            const int t = (tid - own - 1) & 3;
+            double f[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+            int n = 0;
+            if (t < 3) {
+                n = r.n_rev[t];
+                for (int q = 0; q < 5; ++q) f[q] = r.rev[t][q];
+            } else if (grp && r.K > 0 && (r.flags & FCPP_FLAG_GAP_GATE) && ((b.field_flags[r.field] >> tid) & 1)) {
+                // the fill at this candidate's own start corner (on the paths of the group's other start corners),
+                // as the layout kernel computes it
+                n = reverse_fill(s.tt, tm, r.corners[0][tid][0], r.corners[0][tid][1], tid, r.R,
+                                 b.field_extent[2 * r.field], b.field_extent[2 * r.field + 1], f);
+            }
+            s.pn[tid] = n;
+            for (int q = 0; q < 5; ++q) s.pfill[tid][q] = f[q];
+        }
+        if (lat_ok) {
             if (tid < 4) {
                 s.fq[tid] = make_int2((int)(qfix(b.field_verts[(int64_t)r.field * 8 + 2 * tid]) - Xc0),
                                       (int)(qfix(b.field_verts[(int64_t)r.field * 8 + 2 * tid + 1]) - Yc0));
                 s.mq[tid] = make_int2((int)(qfix(r.main_quad[tid][0]) - Xc0), (int)(qfix(r.main_quad[tid][1]) - Yc0));
             }
-            for (int k = tid; k < nh; k += T) {
-                double x, y;
-                uint8_t c;
-                gen_point(r, s.tt, tm, W, r.n_main + k, x, y, c);
-                d.ent(k).erow = make_int2((int)(qfix(x) - Xc0), (int)(qfix(y) - Yc0));
-            }
             __syncthreads();
             if (tid < 4) quad_edges_setup(s.fq, s.qedge[0], s.qtype[0], tid);
             if (tid >= 4 && tid < 8) quad_edges_setup(s.mq, s.qedge[1], s.qtype[1], tid - 4);
-            setup_entries<true, FCPP_COVER_RECT != 0>(s, d, 0, nh - 1, rd, rq, H, invH);
             __syncthreads();
-            // entries whose whole capsule (bounding box grown by r) lies in the closed R-inset cannot
-            // cover a band cell — the inner ends of the inner loops' turn arcs, most of the joins
-            for (int e = tid; e < nh - 1; e += T) {
-                const int4 sg = d.ent(e).seg;
-                if (sg.y > sg.w) continue;
-                const int x0 = min(sg.x, sg.z) - rq, x1 = max(sg.x, sg.z) + rq, y0 = sg.y - rq, y1 = sg.w + rq;
-                if (in_quad(s.mq, x0, y0) && in_quad(s.mq, x1, y0) && in_quad(s.mq, x1, y1) && in_quad(s.mq, x0, y1))
-                    write_dead_entry(d, e);
+            if (grp && FCPP_COVER_RECT && !(mode & 1)) {
+                const unsigned done = band_grouped(s, d, todo, pc, tm, rq, rd, H, invH, nx, ny, Xc0, Yc0);
+                for (int sc = 0; sc < 4; ++sc)
+                    if ((done >> sc) & 1) put(sc, s.gres[sc][0], s.gres[sc][1], false);
+                todo &= ~done;
+            }
+        }
+        // the others one start corner at a time, from the record patched to that start corner
+        while (todo) {
+            const int sc = __ffs(todo) - 1;
+            todo &= todo - 1;
+            __syncthreads();  // the previous start corner is done with the record and the accumulators
+            if (tid == 0) {
+                if (grp) {  // (otherwise sc is the record's own start corner)
+                    CandRec &w = s.rec;
+                    int nhs = FCPP_POINTS_PER_LOOP * w.K;
+                    for (int t = 0; t < 3; ++t) {
+                        const int c = (sc + t + 1) & 3;
+                        w.n_rev[t] = s.pn[c];
+                        for (int q = 0; q < 5; ++q) w.rev[t][q] = s.pfill[c][q];
+                        nhs += s.pn[c];
+                    }
+                    w.flags = (w.flags & ~FCPP_FLAG_CORNER_MASK) | sc;
+                    w.n_head = nhs;
+                }
+                s.acc[0] = s.acc[1] = 0ull;
             }
             __syncthreads();
-            unsigned long long my_total = 0ull, my_cov = 0ull;
-            int j0 = 0;
-            if (tid == 0) s.next_w0 = 0;
-            // axis-aligned straights: bitmap only around the corners, the rest in closed form
-            if (FCPP_COVER_RECT && !(mode & 1) && s.nrect > 0 &&
-                band_zoned(s, d, nh - 1, rq, H, invH, nx, ny, my_total, my_cov))
-                j0 = ny;
-            while (j0 < ny) {
-                // --- how many rows to try: from the word count of the first row.  The previous pass
-                // has usually computed it already (its first row that did not fit) ---
-                if (tid == 0) {
-                    int w0 = s.next_w0;
-                    if (w0 <= 0) {
-                        int a0, b0, a1, b1;
-                        quad_row_interval(s.fq, s.qedge[0], s.qtype[0], j0 * H, H, invH, nx, a0, b0);
-                        quad_row_interval(s.mq, s.qedge[1], s.qtype[1], j0 * H, H, invH, nx, a1, b1);
-                        w0 = (a1 <= b1) ? words_of(a0, a1 - 1) + words_of(b1 + 1, b0) : words_of(a0, b0);
-                    }
-                    const int rt = (5 * TW) / (4 * (w0 > 0 ? w0 : 1)) + 8;
-                    s.cnt[0] = min(max(rt, 8), min(ROWCAP, ny - j0));
-                    s.next_w0 = 0;
-                    s.nrows = 0;
-                    s.total_words = 0;
+            const int nh = r.n_head;
+            const bool ok = lat_ok && nh <= pc;
+            bool e11 = !ok;
+            if (ok) {
+                if (tid == 0) s.nrect = 0;
+                for (int k = tid; k < nh; k += T) {
+                    double x, y;
+                    uint8_t c;
+                    gen_point(r, s.tt, tm, W, r.n_main + k, x, y, c);
+                    d.ent(k).erow = make_int2((int)(qfix(x) - Xc0), (int)(qfix(y) - Yc0));
                 }
                 __syncthreads();
-                const int rows_try = s.cnt[0];
-                // --- row windows + word counts: one row per thread and round (rows k = tid + round*T) ---
-                constexpr int ROUNDS = ROWCAP / T;
-                int wcnt[ROUNDS], cells[ROUNDS];
-                int fit_rows = 0, fit_words = 0, carry = 0;
-#pragma unroll
-                for (int q = 0; q < ROUNDS; ++q) {
-                    const int k = tid + q * T;
-                    wcnt[q] = 0;
-                    cells[q] = 0;
-                    if (q * T >= rows_try) continue;  // uniform
-                    int4 win = make_int4(1, 0, 1, 0);
-                    int n1 = 0;
-                    if (k < rows_try) {
-                        win = band_row_windows(s, (j0 + k) * H, H, invH, nx);
-                        n1 = words_of(win.x, win.y);
-                        wcnt[q] = n1 + words_of(win.z, win.w);
-                        cells[q] = max(win.y - win.x + 1, 0) + max(win.w - win.z + 1, 0);
+                setup_entries<true, FCPP_COVER_RECT != 0>(s, d, 0, nh - 1, rd, rq, H, invH);
+                __syncthreads();
+                // entries whose whole capsule (bounding box grown by r) lies in the closed R-inset cannot
+                // cover a band cell — the inner ends of the inner loops' turn arcs, most of the joins
+                for (int e = tid; e < nh - 1; e += T) {
+                    const int4 sg = d.ent(e).seg;
+                    if (sg.y > sg.w) continue;
+                    const int x0 = min(sg.x, sg.z) - rq, x1 = max(sg.x, sg.z) + rq, y0 = sg.y - rq, y1 = sg.w + rq;
+                    if (in_quad(s.mq, x0, y0) && in_quad(s.mq, x1, y0) && in_quad(s.mq, x1, y1) && in_quad(s.mq, x0, y1))
+                        write_dead_entry(d, e);
+                }
+                __syncthreads();
+                unsigned long long my_total = 0ull, my_cov = 0ull;
+                int j0 = 0;
+                if (tid == 0) s.next_w0 = 0;
+                // axis-aligned straights: bitmap only around the corners, the rest in closed form
+                if (FCPP_COVER_RECT && !(mode & 1) && s.nrect > 0 &&
+                    band_zoned<4>(s, d, nh - 1, rq, H, invH, nx, ny, my_total, my_cov))
+                    j0 = ny;
+                while (j0 < ny) {
+                    // --- how many rows to try: from the word count of the first row.  The previous pass
+                    // has usually computed it already (its first row that did not fit) ---
+                    if (tid == 0) {
+                        int w0 = s.next_w0;
+                        if (w0 <= 0) {
+                            int a0, b0, a1, b1;
+                            quad_row_interval(s.fq, s.qedge[0], s.qtype[0], j0 * H, H, invH, nx, a0, b0);
+                            quad_row_interval(s.mq, s.qedge[1], s.qtype[1], j0 * H, H, invH, nx, a1, b1);
+                            w0 = (a1 <= b1) ? words_of(a0, a1 - 1) + words_of(b1 + 1, b0) : words_of(a0, b0);
+                        }
+                        const int rt = (5 * TW) / (4 * (w0 > 0 ? w0 : 1)) + 8;
+                        s.cnt[0] = min(max(rt, 8), min(ROWCAP, ny - j0));
+                        s.next_w0 = 0;
+                        s.nrows = 0;
+                        s.total_words = 0;
                     }
-                    int v[1] = {wcnt[q]};
-                    const int round_total = block_scan<1>(v, s.scan);  // inclusive prefix (syncs inside)
-                    const int wsum = carry + v[0];
-                    carry += round_total;
-                    if (k < rows_try) {
-                        const int base = wsum - wcnt[q];
-                        s.rwin[k] = win;
-                        s.rbias[k] = make_int2(base - (win.x >> 5), base + n1 - (win.z >> 5));
-                        if (wsum <= TW) {
-                            fit_rows = k + 1;
-                            fit_words = wsum;
+                    __syncthreads();
+                    const int rows_try = s.cnt[0];
+                    // --- row windows + word counts: one row per thread and round (rows k = tid + round*T) ---
+                    constexpr int ROUNDS = ROWCAP / T;
+                    int wcnt[ROUNDS], cells[ROUNDS];
+                    int fit_rows = 0, fit_words = 0, carry = 0;
+    #pragma unroll
+                    for (int q = 0; q < ROUNDS; ++q) {
+                        const int k = tid + q * T;
+                        wcnt[q] = 0;
+                        cells[q] = 0;
+                        if (q * T >= rows_try) continue;  // uniform
+                        int4 win = make_int4(1, 0, 1, 0);
+                        int n1 = 0;
+                        if (k < rows_try) {
+                            win = band_row_windows(s, (j0 + k) * H, H, invH, nx);
+                            n1 = words_of(win.x, win.y);
+                            wcnt[q] = n1 + words_of(win.z, win.w);
+                            cells[q] = max(win.y - win.x + 1, 0) + max(win.w - win.z + 1, 0);
+                        }
+                        int v[1] = {wcnt[q]};
+                        const int round_total = block_scan<1>(v, s.scan);  // inclusive prefix (syncs inside)
+                        const int wsum = carry + v[0];
+                        carry += round_total;
+                        if (k < rows_try) {
+                            const int base = wsum - wcnt[q];
+                            s.rwin[k] = win;
+                            s.rbias[k] = make_int2(base - (win.x >> 5), base + n1 - (win.z >> 5));
+                            if (wsum <= TW) {
+                                fit_rows = k + 1;
+                                fit_words = wsum;
+                            }
                         }
                     }
+                    if (fit_rows) {
+                        atomicMax(&s.nrows, fit_rows);
+                        atomicMax(&s.total_words, fit_words);
+                    }
+                    __syncthreads();
+                    const int nrows = s.nrows, nwords = s.total_words;
+                    if (nrows == 0) {  // a single row does not fit the tile
+                        e11 = true;
+                        break;
+                    }
+                    zero_words(s.tile, nwords);
+    #pragma unroll
+                    for (int q = 0; q < ROUNDS; ++q) {
+                        const int k = tid + q * T;
+                        if (k < nrows) my_total += (unsigned long long)cells[q];
+                        if (k == nrows && k < rows_try) s.next_w0 = wcnt[q];  // first row of the next pass
+                    }
+                    if (tid == 0) {
+                        Target &t = s.tg[0];
+                        t.j0 = j0;
+                        t.nrows = nrows;
+                        t.koff = 0;
+                    }
+                    __syncthreads();
+                    {
+                        fill_rects(s, j0, nrows, 0);
+                        auto tgt = [&](int) { return 0; };
+                        raster_entries(s, d, 0, nh - 1, tgt, rq, H, invH);
+                    }
+                    my_cov += (unsigned long long)count_words(s.tile, nwords);
+                    __syncthreads();
+                    j0 += nrows;
                 }
-                if (fit_rows) {
-                    atomicMax(&s.nrows, fit_rows);
-                    atomicMax(&s.total_words, fit_words);
-                }
-                __syncthreads();
-                const int nrows = s.nrows, nwords = s.total_words;
-                if (nrows == 0) {  // a single row does not fit the tile
-                    err11 = 1;
-                    break;
-                }
-                zero_words(s.tile, nwords);
 #pragma unroll
-                for (int q = 0; q < ROUNDS; ++q) {
-                    const int k = tid + q * T;
-                    if (k < nrows) my_total += (unsigned long long)cells[q];
-                    if (k == nrows && k < rows_try) s.next_w0 = wcnt[q];  // first row of the next pass
+                for (int dd = 16; dd > 0; dd >>= 1) {
+                    my_total += __shfl_xor_sync(0xffffffffu, my_total, dd);
+                    my_cov += __shfl_xor_sync(0xffffffffu, my_cov, dd);
                 }
-                if (tid == 0) {
-                    Target &t = s.tg[0];
-                    t.j0 = j0;
-                    t.nrows = nrows;
-                    t.koff = 0;
+                if ((tid & 31) == 0) {
+                    atomicAdd(&s.acc[0], my_total);
+                    atomicAdd(&s.acc[1], my_cov);
                 }
                 __syncthreads();
-                {
-                    fill_rects(s, j0, nrows, 0);
-                    auto tgt = [&](int) { return 0; };
-                    raster_entries(s, d, 0, nh - 1, tgt, rq, H, invH);
-                }
-                my_cov += (unsigned long long)count_words(s.tile, nwords);
-                __syncthreads();
-                j0 += nrows;
             }
-#pragma unroll
-            for (int dd = 16; dd > 0; dd >>= 1) {
-                my_total += __shfl_xor_sync(0xffffffffu, my_total, dd);
-                my_cov += __shfl_xor_sync(0xffffffffu, my_cov, dd);
-            }
-            if ((tid & 31) == 0) {
-                atomicAdd(&s.acc[0], my_total);
-                atomicAdd(&s.acc[1], my_cov);
-            }
-            __syncthreads();
-        }
-        if (tid == 0) {
-            sum->cov_total = (ok && !err11) ? (int64_t)s.acc[0] : 0;
-            sum->cov_cells = (ok && !err11) ? (int64_t)s.acc[1] : 0;
+            put(sc, s.acc[0], s.acc[1], e11);
         }
     }
     if (tid == 0 && (err10 | err11))
@@ -1169,10 +1425,12 @@ __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_kernel(const fc
                                                                         const TrigTables *__restrict__ trig,
                                                                         fcpp_summary *__restrict__ summary, int pc, int mode,
                                                                         const int32_t *__restrict__ rep,
+                                                                        const uint32_t *__restrict__ band_mask,
+                                                                        longlong2 *__restrict__ band_out,
                                                                         uint32_t *__restrict__ corner_bits,
                                                                         int64_t corner_bits_stride)
 {
-    cover_body(b, recs, trig, summary, pc, mode, rep, corner_bits, corner_bits_stride, blockIdx.x);
+    cover_body(b, recs, trig, summary, pc, mode, rep, band_mask, band_out, corner_bits, corner_bits_stride, blockIdx.x);
 }
 
 // De-duplicated batches: the candidates that rasterise at least one part are listed (cover_list_kernel) and a
@@ -1182,6 +1440,8 @@ __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_work_kernel(con
                                                                              const TrigTables *__restrict__ trig,
                                                                              fcpp_summary *__restrict__ summary, int pc, int mode,
                                                                              const int32_t *__restrict__ rep,
+                                                                             const uint32_t *__restrict__ band_mask,
+                                                                             longlong2 *__restrict__ band_out,
                                                                              uint32_t *__restrict__ corner_bits,
                                                                              int64_t corner_bits_stride,
                                                                              const int32_t *__restrict__ work,
@@ -1199,7 +1459,7 @@ __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_work_kernel(con
         __syncthreads();
         const int w = s_item;
         if (w >= counters[0]) return;
-        cover_body(b, recs, trig, summary, pc, mode, rep, corner_bits, corner_bits_stride, work[w]);
+        cover_body(b, recs, trig, summary, pc, mode, rep, band_mask, band_out, corner_bits, corner_bits_stride, work[w]);
     }
 }
 
@@ -1230,10 +1490,12 @@ namespace {
 __global__ void __launch_bounds__(128) cover_key_kernel(const CandRec *__restrict__ recs, int64_t n,
                                                         unsigned long long *__restrict__ keys,
                                                         unsigned int *__restrict__ vals, uint32_t cap_mask,
-                                                        unsigned long long *__restrict__ hash /*[2][n]*/)
+                                                        unsigned long long *__restrict__ hash /*[2][n]*/,
+                                                        uint32_t *__restrict__ band_mask)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n) return;
+    band_mask[c] = 0u;
 #pragma unroll
     for (int part = 0; part < 2; ++part) {
         const unsigned long long h = recs[c].cover_key[part];  // hashed by the layout kernel
@@ -1254,7 +1516,8 @@ __global__ void __launch_bounds__(128) cover_rep_kernel(const CandRec *__restric
                                                         const unsigned long long *__restrict__ keys,
                                                         const unsigned int *__restrict__ vals, uint32_t cap_mask,
                                                         unsigned long long *__restrict__ hash /*[2][n]*/,
-                                                        int32_t *__restrict__ rep /*[2][n]*/)
+                                                        int32_t *__restrict__ rep /*[2][n]*/,
+                                                        uint32_t *__restrict__ band_mask)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n) return;
@@ -1265,7 +1528,10 @@ __global__ void __launch_bounds__(128) cover_rep_kernel(const CandRec *__restric
         while (keys[slot] != h) slot = (slot + 1) & cap_mask;
         hash[part * n + c] = slot;  // remembered for the clean-up
         const int64_t first = (int64_t)(0x7fffffffu - vals[slot]);
-        rep[part * n + c] = (first < c && cover_same(recs[c], recs[first], part)) ? (int32_t)first : (int32_t)c;
+        const int64_t q = (first < c && cover_same(recs[c], recs[first], part)) ? first : c;
+        rep[part * n + c] = (int32_t)q;
+        // the start corners a band representative evaluates
+        if (part == 1 && recs[c].band_group) atomicOr(&band_mask[q], 1u << (recs[c].flags & FCPP_FLAG_CORNER_MASK));
     }
 }
 
@@ -1284,8 +1550,9 @@ __global__ void __launch_bounds__(128) cover_list_kernel(int64_t n, const int32_
     if (on) work[base + __popc(m & ((1u << lane) - 1))] = (int32_t)c;
 }
 
-__global__ void __launch_bounds__(128) cover_copy_kernel(fcpp_summary *__restrict__ summary, int64_t n,
-                                                         const int32_t *__restrict__ rep /*[2][n]*/,
+__global__ void __launch_bounds__(128) cover_copy_kernel(const CandRec *__restrict__ recs, fcpp_summary *__restrict__ summary,
+                                                         int64_t n, const int32_t *__restrict__ rep /*[2][n]*/,
+                                                         const longlong2 *__restrict__ band_out /*[n][4]*/,
                                                          unsigned long long *__restrict__ keys,
                                                          unsigned int *__restrict__ vals,
                                                          const unsigned long long *__restrict__ slot_of /*[2][n]*/)
@@ -1311,11 +1578,11 @@ __global__ void __launch_bounds__(128) cover_copy_kernel(fcpp_summary *__restric
         if (src.status & FCPP_CAND_CORNER_GRID_TOO_LARGE)
             dst.status |= FCPP_CAND_GRID_TOO_LARGE | FCPP_CAND_CORNER_GRID_TOO_LARGE;
     }
-    if (q1 != (int32_t)c) {
-        const fcpp_summary &src = summary[q1];
-        dst.cov_cells = src.cov_cells;
-        dst.cov_total = src.cov_total;
-        if (src.status & FCPP_CAND_BAND_GRID_TOO_LARGE) dst.status |= FCPP_CAND_GRID_TOO_LARGE | FCPP_CAND_BAND_GRID_TOO_LARGE;
+    if (q1 != (int32_t)c) {  // the representative's band of this candidate's start corner (-1: too large)
+        const longlong2 src = band_out[4 * (int64_t)q1 + (recs[c].flags & FCPP_FLAG_CORNER_MASK)];
+        dst.cov_cells = src.x < 0 ? 0 : src.y;
+        dst.cov_total = src.x < 0 ? 0 : src.x;
+        if (src.x < 0) dst.status |= FCPP_CAND_GRID_TOO_LARGE | FCPP_CAND_BAND_GRID_TOO_LARGE;
     }
 }
 
@@ -1343,6 +1610,8 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
     unsigned long long *keys = nullptr, *hash = nullptr;
     unsigned int *vals = nullptr;
     int32_t *work = nullptr, *counters = nullptr;  // de-duplicated batches: the listed candidates (cover_work_kernel)
+    uint32_t *band_mask = nullptr;                 // start corners per band representative
+    longlong2 *band_out = nullptr;                 // bands per (representative, start corner)
     cudaError_t e;
     // de-duplication (asked for by the batch, unless switched off by cover mode bit 1)
     const int64_t n = b.n_cand;
@@ -1351,7 +1620,7 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
     if (b.cover_dedupe && n > 1 && !(h->cover_mode & 2) && n < (1ll << 28)) {
         uint32_t cap = 1024;
         while ((int64_t)cap < 4 * n) cap <<= 1;  // two keys per candidate, load factor <= 1/2
-        const size_t need = (size_t)cap * 12 + (size_t)n * 28 + 64;
+        const size_t need = (size_t)cap * 12 + (size_t)n * 96 + 64;
         if (need > h->dedupe_bytes) {
             if (h->d_dedupe) cudaFree(h->d_dedupe);
             h->d_dedupe = nullptr;
@@ -1361,23 +1630,25 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
             h->dedupe_bytes = need;
             h->dedupe_cap = 0;
         }
-        // layout: keys [cap] | vals [cap] | hash / slot [2][n] | rep [2][n] | work [n] | counters [2]; a different
-        // capacity moves the arrays, so the table is zeroed again
+        // layout: keys [cap] | vals [cap] | hash / slot [2][n] | band_out [n][4] | rep [2][n] | band_mask [n] | work [n] |
+        // counters [2]; a different capacity moves the arrays, so the table is zeroed again
         keys = (unsigned long long *)h->d_dedupe;
         vals = (unsigned int *)(keys + cap);
         hash = (unsigned long long *)(vals + cap);
-        d_rep = (int32_t *)(hash + 2 * n);
+        band_out = (longlong2 *)(hash + 2 * n);
+        d_rep = (int32_t *)(band_out + 4 * n);
+        band_mask = (uint32_t *)(d_rep + 2 * n);
         if (h->dedupe_cap != cap) {
             e = cudaMemsetAsync(h->d_dedupe, 0, (size_t)cap * 12, st);
             if (e != cudaSuccess) return e;
             h->dedupe_cap = cap;
         }
         const unsigned g = (unsigned)((n + th - 1) / th);
-        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash);
-        cover_rep_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, d_rep);
+        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, band_mask);
+        cover_rep_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, d_rep, band_mask);
         h->launches += 2;
         if (cover_use_work_list(h, b)) {
-            work = d_rep + 2 * n;
+            work = (int32_t *)(band_mask + n);
             counters = work + n;
             e = cudaMemsetAsync(counters, 0, 2 * sizeof(int32_t), st);
             if (e != cudaSuccess) return e;
@@ -1393,17 +1664,17 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
         int64_t grid = (int64_t)FCPP_COVER_MINBLOCKS * h->sm_count;
         if (grid > n) grid = n;
         cover_work_kernel<<<(unsigned)grid, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
-                                                            o.corner_bits, o.corner_bits_stride, work, counters);
+                                                            band_mask, band_out, o.corner_bits, o.corner_bits_stride, work, counters);
     } else {
         e = cudaFuncSetAttribute(cover_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         if (e != cudaSuccess) return e;
         cover_kernel<<<(unsigned)n, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
-                                                    o.corner_bits, o.corner_bits_stride);
+                                                    band_mask, band_out, o.corner_bits, o.corner_bits_stride);
     }
     h->launches++;
     e = cudaGetLastError();
     if (e != cudaSuccess || !d_rep) return e;
-    cover_copy_kernel<<<(unsigned)((n + th - 1) / th), th, 0, st>>>(o.summary, n, d_rep, keys, vals, hash);
+    cover_copy_kernel<<<(unsigned)((n + th - 1) / th), th, 0, st>>>(h->d_rec, o.summary, n, d_rep, band_out, keys, vals, hash);
     h->launches++;
     return cudaGetLastError();
 }

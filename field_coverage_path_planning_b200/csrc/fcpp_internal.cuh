@@ -50,7 +50,10 @@ struct __align__(16) CandRec {
     double cx, cy;                      // rotation centre (work-area centroid, mlp3:690, :710)
     double cos_a, sin_a;                // rotate-back (mlp3:709-714)
     uint64_t cover_key[2];              // hashes of the fields A10 (corner windows) / A11 (band) read (de-duplication)
-    uint64_t pad1;
+    int32_t band_group;                 // 1: every headland straight is axis-aligned on the 1e-4 m lattice (de-duplicated
+                                        // batches only): the bands of all four start corners are evaluated together
+                                        // (fcpp_cover.cu: band_grouped)
+    int32_t pad1;
     double main_quad[4][2];             // R-inset of the field (mlp3:594-595), D1
     double rev[3][5];                   // loop-0 reverse fills: ex, ey, dx, dy, length (mlp3:1154-1218)
     double vrev[4][5];                  // verification corners (mlp3:1531-1554)
@@ -106,7 +109,10 @@ constexpr int COVER_FLAG_MASK = FCPP_FLAG_CORNER_MASK | FCPP_FLAG_GAP_GATE;
 
 // hashes of the CandRec fields the coverage kernel reads (fcpp_cover.cu: coverage de-duplication).
 // part 0 = A10, the four corner windows: field, R, window size, verification reverse fills — NOT the
-// start corner; part 1 = A11, the headland band: field, R, loops, start corner, rings, reverse fills
+// start corner; part 1 = A11, the headland band: field, R, loops, rings, reverse fills and the start corner,
+// except for records with band_group set: their four start corners share one key and one CTA evaluates the
+// bands of all of them.  Their reverse fills are left out: the fill at a corner is a function of the field,
+// R, the gap gate and the first ring (reverse_fill), all of which are in the key
 __device__ __forceinline__ bool cover_dead(const CandRec &r) { return r.status != 0 || r.n_total == 0; }
 __device__ __forceinline__ uint64_t cover_key(const CandRec &r, int part)
 {
@@ -120,6 +126,11 @@ __device__ __forceinline__ uint64_t cover_key(const CandRec &r, int part)
         h = mix64(h, (uint32_t)r.corner_g);
         for (int k = 0; k < 4; ++k) h = mix64(h, (uint32_t)r.vn_rev[k]);
         for (int k = 0; k < 20; ++k) h = mix64(h, dbits((&r.vrev[0][0])[k]));
+    } else if (r.band_group) {
+        h = mix64(h, ((uint64_t)(uint32_t)r.K << 32) | 0x80000000u);
+        h = mix64(h, (uint32_t)(r.flags & FCPP_FLAG_GAP_GATE));
+        for (int k = 0; k < 8; ++k) h = mix64(h, dbits((&r.main_quad[0][0])[k]));
+        for (int k = 0; k < 8 * r.K; ++k) h = mix64(h, dbits((&r.corners[0][0][0])[k]));
     } else {
         h = mix64(h, ((uint64_t)(uint32_t)r.K << 32) | (uint32_t)r.n_head);
         h = mix64(h, (uint32_t)(r.flags & COVER_FLAG_MASK));
@@ -140,14 +151,19 @@ __device__ __forceinline__ bool cover_same(const CandRec &a, const CandRec &b, i
         same = same && a.corner_g == b.corner_g;
         for (int k = 0; k < 4; ++k) same = same && a.vn_rev[k] == b.vn_rev[k];
         for (int k = 0; k < 20; ++k) same = same && dbits((&a.vrev[0][0])[k]) == dbits((&b.vrev[0][0])[k]);
-    } else {
-        same = same && a.K == b.K && a.n_head == b.n_head && (a.flags & COVER_FLAG_MASK) == (b.flags & COVER_FLAG_MASK);
-        for (int k = 0; k < 3; ++k) same = same && a.n_rev[k] == b.n_rev[k];
-        for (int k = 0; k < 8; ++k) same = same && dbits((&a.main_quad[0][0])[k]) == dbits((&b.main_quad[0][0])[k]);
-        for (int k = 0; k < 15; ++k) same = same && dbits((&a.rev[0][0])[k]) == dbits((&b.rev[0][0])[k]);
-        for (int k = 0; same && k < 8 * a.K; ++k)
-            same = dbits((&a.corners[0][0][0])[k]) == dbits((&b.corners[0][0][0])[k]);
+        return same;
     }
+    same = same && a.K == b.K && a.band_group == b.band_group;
+    if (a.band_group) {
+        same = same && (a.flags & FCPP_FLAG_GAP_GATE) == (b.flags & FCPP_FLAG_GAP_GATE);
+    } else {
+        same = same && a.n_head == b.n_head && (a.flags & COVER_FLAG_MASK) == (b.flags & COVER_FLAG_MASK);
+        for (int k = 0; k < 3; ++k) same = same && a.n_rev[k] == b.n_rev[k];
+        for (int k = 0; k < 15; ++k) same = same && dbits((&a.rev[0][0])[k]) == dbits((&b.rev[0][0])[k]);
+    }
+    for (int k = 0; k < 8; ++k) same = same && dbits((&a.main_quad[0][0])[k]) == dbits((&b.main_quad[0][0])[k]);
+    for (int k = 0; same && k < 8 * a.K; ++k)
+        same = dbits((&a.corners[0][0][0])[k]) == dbits((&b.corners[0][0][0])[k]);
     return same;
 }
 
@@ -421,6 +437,56 @@ __device__ __forceinline__ void corner_arc_pt(const TrigTables &tt, const TurnMo
 
 // 1e-4 m fixed point (D5): one FP64 multiply, round-half-even
 __device__ __forceinline__ int64_t qfix(double x) { return __double2ll_rn(x * FCPP_FIXED_UNIT); }
+
+// ---- reverse fills (layout kernel; the coverage kernel for the start corner of another candidate) ----
+// mlp3:1220-1288 — ray to the bbox lines x=0, x=field_length, y=0, y=field_width
+__device__ inline double distance_to_boundary(double x, double y, double dx, double dy, double fl, double fw, double R)
+{
+    double best = -1.0;
+    if (fabs(dx) > 1e-6) {
+        double t = (0.0 - x) / dx;
+        if (t > 0 && (best < 0 || t < best)) best = t;
+        t = (fl - x) / dx;
+        if (t > 0 && (best < 0 || t < best)) best = t;
+    }
+    if (fabs(dy) > 1e-6) {
+        double t = (0.0 - y) / dy;
+        if (t > 0 && (best < 0 || t < best)) best = t;
+        t = (fw - y) / dy;
+        if (t > 0 && (best < 0 || t < best)) best = t;
+    }
+    if (best < 0) return 2.0 * R;
+    const double cap = FCPP_REV_CAP * R;
+    return best < cap ? best : cap;
+}
+
+// mlp3:1154-1218: chord direction of the last two arc samples, length, sample count
+__device__ inline int reverse_fill(const TrigTables &tt, const TurnModel &tm, double cx, double cy, int ci, double R,
+                            double fl, double fw, double *rev /*[5]*/)
+{
+    double ex, ey, sx, sy;
+    corner_arc_pt(tt, tm, cx, cy, R, ci, FCPP_CORNER_POINTS - 1, ex, ey);
+    corner_arc_pt(tt, tm, cx, cy, R, ci, FCPP_CORNER_POINTS - 2, sx, sy);
+    const double tx = ex - sx, ty = ey - sy;
+    const double nrm = sqrt(tx * tx + ty * ty);
+    double dx, dy;
+    if (nrm > 1e-6) {
+        dx = -tx / nrm;
+        dy = -ty / nrm;
+    } else {
+        dx = -1.0;
+        dy = 0.0;
+    }
+    const double len = distance_to_boundary(ex, ey, dx, dy, fl, fw, R);
+    int n = (int)(len / FCPP_REV_SPACING);
+    if (n < FCPP_REV_MIN_PTS) n = FCPP_REV_MIN_PTS;
+    rev[0] = ex;
+    rev[1] = ey;
+    rev[2] = dx;
+    rev[3] = dy;
+    rev[4] = len;
+    return n;
+}
 
 // ---------------------------------------------------------------------------------------------
 // point generation: index -> (x, y, speed class, structure tag)

@@ -11,54 +11,6 @@
 
 namespace {
 
-// mlp3:1220-1288 — ray to the bbox lines x=0, x=field_length, y=0, y=field_width
-__device__ double distance_to_boundary(double x, double y, double dx, double dy, double fl, double fw, double R)
-{
-    double best = -1.0;
-    if (fabs(dx) > 1e-6) {
-        double t = (0.0 - x) / dx;
-        if (t > 0 && (best < 0 || t < best)) best = t;
-        t = (fl - x) / dx;
-        if (t > 0 && (best < 0 || t < best)) best = t;
-    }
-    if (fabs(dy) > 1e-6) {
-        double t = (0.0 - y) / dy;
-        if (t > 0 && (best < 0 || t < best)) best = t;
-        t = (fw - y) / dy;
-        if (t > 0 && (best < 0 || t < best)) best = t;
-    }
-    if (best < 0) return 2.0 * R;
-    const double cap = FCPP_REV_CAP * R;
-    return best < cap ? best : cap;
-}
-
-// mlp3:1154-1218: chord direction of the last two arc samples, length, sample count
-__device__ int reverse_fill(const TrigTables &tt, const TurnModel &tm, double cx, double cy, int ci, double R,
-                            double fl, double fw, double *rev /*[5]*/)
-{
-    double ex, ey, sx, sy;
-    corner_arc_pt(tt, tm, cx, cy, R, ci, FCPP_CORNER_POINTS - 1, ex, ey);
-    corner_arc_pt(tt, tm, cx, cy, R, ci, FCPP_CORNER_POINTS - 2, sx, sy);
-    const double tx = ex - sx, ty = ey - sy;
-    const double nrm = sqrt(tx * tx + ty * ty);
-    double dx, dy;
-    if (nrm > 1e-6) {
-        dx = -tx / nrm;
-        dy = -ty / nrm;
-    } else {
-        dx = -1.0;
-        dy = 0.0;
-    }
-    const double len = distance_to_boundary(ex, ey, dx, dy, fl, fw, R);
-    int n = (int)(len / FCPP_REV_SPACING);
-    if (n < FCPP_REV_MIN_PTS) n = FCPP_REV_MIN_PTS;
-    rev[0] = ex;
-    rev[1] = ey;
-    rev[2] = dx;
-    rev[3] = dy;
-    rev[4] = len;
-    return n;
-}
 
 __device__ int layout_one(const fcpp_batch &b, const TrigTables *__restrict__ trig, CandRec *__restrict__ recs,
                           int32_t *__restrict__ n_pts, int64_t c)
@@ -208,6 +160,17 @@ __device__ int layout_one(const fcpp_batch &b, const TrigTables *__restrict__ tr
         r.n_rev[t] = n;
         n_head += n;
     }
+    // every straight of every loop axis-aligned on the lattice: the band's corner zones do not depend on the
+    // start corner (fcpp_cover.cu: band_grouped); only de-duplicated batches group bands
+    const bool dd = b.cover_dedupe && b.do_coverage;
+    bool axis = dd && K > 0;
+    for (int k = 0; axis && k < K; ++k)
+        for (int q = 0; q < 4; ++q) {
+            const int q1 = (q + 1) & 3;
+            const bool vx = qfix(r.corners[k][q][0]) == qfix(r.corners[k][q1][0]);
+            const bool vy = qfix(r.corners[k][q][1]) == qfix(r.corners[k][q1][1]);
+            axis = axis && (vx != vy);
+        }
     // ---- verification corners (mlp3:1531-1554): main-area corners (hw,hw)… with hw = R ----
     for (int ci = 0; ci < 4; ++ci) {
         const double qx = (ci == 0 || ci == 3) ? R : fl - R;
@@ -235,6 +198,7 @@ __device__ int layout_one(const fcpp_batch &b, const TrigTables *__restrict__ tr
         r.n_total = n_main + n_head;
     }
     r.status = status;
+    r.band_group = (axis && status == 0) ? 1 : 0;
     r.P = P;
     r.K = K;
     r.flags = flags;
@@ -253,10 +217,9 @@ __device__ int layout_one(const fcpp_batch &b, const TrigTables *__restrict__ tr
         r.main_quad[k][0] = mq[k][0];
         r.main_quad[k][1] = mq[k][1];
     }
-    const bool dd = b.cover_dedupe && b.do_coverage;
     r.cover_key[0] = dd ? cover_key(r, 0) : 0ull;
     r.cover_key[1] = dd ? cover_key(r, 1) : 0ull;
-    r.pad1 = 0ull;
+    r.pad1 = 0;
     if (n_pts) n_pts[c] = r.n_total;
     return r.n_total;
 }
