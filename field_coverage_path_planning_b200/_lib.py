@@ -115,6 +115,14 @@ class GAResultC(C.Structure):
     ]
 
 
+class SelectionC(C.Structure):
+    """fcpp_selection (include/fcpp.h): weights, cell area, limits (< 0: none), top_k."""
+    _fields_ = [(n, C.c_double) for n in (
+        "w_length", "w_time", "w_boundary", "w_obstacle", "w_accel", "w_uncovered", "cell_area", "min_coverage")] + [
+        (n, C.c_int32) for n in ("max_boundary_viol", "max_obstacle_viol", "max_accel_viol", "top_k")]
+
+
+SELECT_MAX_K = 32
 GA_TRACE_INTS = 48
 GA_MAX_TOURNAMENT = 16
 
@@ -132,7 +140,7 @@ assert SUMMARY_DTYPE.itemsize == 176, SUMMARY_DTYPE.itemsize
 
 EXPORTS = [
     "fcpp_abi_version", "fcpp_create", "fcpp_destroy", "fcpp_last_error", "fcpp_set_trig_tables",
-    "fcpp_layout", "fcpp_plan_batch", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
+    "fcpp_layout", "fcpp_plan_batch", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
     "fcpp_tour_lengths", "fcpp_distance_matrix", "fcpp_connection_matrix", "fcpp_ga_init_population", "fcpp_ga_next_size", "fcpp_ga_generation", "fcpp_ga_solve", "fcpp_kmeans_lloyd", "fcpp_tsp_two_opt",
     "fcpp_launch_count", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
 ]
@@ -175,6 +183,10 @@ def load():
         L.fcpp_field_argmin.argtypes = [vp, vp, vp, i64, i32, C.c_int, i64, vp, vp, vp]
         L.fcpp_field_argmin_merge.restype = C.c_int
         L.fcpp_field_argmin_merge.argtypes = [vp, vp, i32, i32, vp, vp, vp]
+        L.fcpp_field_select.restype = C.c_int
+        L.fcpp_field_select.argtypes = [vp, vp, vp, i64, i32, C.POINTER(SelectionC), i64, vp, vp, vp]
+        L.fcpp_field_select_merge.restype = C.c_int
+        L.fcpp_field_select_merge.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp]
         L.fcpp_winner_records.restype = C.c_int
         L.fcpp_winner_records.argtypes = [vp, vp, i64, i64, vp, i32, vp, vp]
         L.fcpp_status_count.restype = C.c_int

@@ -223,6 +223,69 @@ def expand_axes(ax, index: Optional[np.ndarray] = None) -> Dict[str, np.ndarray]
     return out
 
 
+@dataclass(frozen=True)
+class Selection:
+    """How ``plan_batch(..., select=...)`` ranks the candidates of each field (include/fcpp.h, fcpp_selection).
+
+    A candidate is eligible when its status is 0, every limit that is set holds (``n_*_viol <= max_*``) and, with
+    ``min_coverage`` set, its headland band has cells and ``cov_cells >= min_coverage * cov_total`` (FP64).  Its cost,
+    in FP64, left to right::
+
+        w_length * (len_main + len_head) + w_time * (time_main + time_head) + w_boundary * n_boundary_viol
+        + w_obstacle * n_obstacle_viol + w_accel * n_accel_viol + w_uncovered * (cov_total - cov_cells) * grid_h**2
+
+    Per field the eligible candidates are ranked by (cost, candidate index) and the first ``top_k`` are returned.
+    The defaults are ``cost='length'``'s argmin exactly: same winner, same cost bits."""
+    w_length: float = 1.0
+    w_time: float = 0.0
+    w_boundary: float = 0.0
+    w_obstacle: float = 0.0
+    w_accel: float = 0.0
+    w_uncovered: float = 0.0          # per m² of the headland band left uncovered
+    max_boundary_viol: Optional[int] = None
+    max_obstacle_viol: Optional[int] = None
+    max_accel_viol: Optional[int] = None
+    min_coverage: Optional[float] = None    # share of the headland band's cells, in [0, 1]
+    top_k: int = 1
+
+    WEIGHTS = ("w_length", "w_time", "w_boundary", "w_obstacle", "w_accel", "w_uncovered")
+    LIMITS = ("max_boundary_viol", "max_obstacle_viol", "max_accel_viol")
+
+    def __post_init__(self):
+        for n in self.WEIGHTS:
+            w = getattr(self, n)
+            if isinstance(w, bool) or not isinstance(w, (int, float, np.floating, np.integer)) or \
+                    not math.isfinite(float(w)) or float(w) < 0:
+                raise ValueError(f"Selection.{n} must be a finite number >= 0, not {w!r}")
+        k = self.top_k
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= int(k) <= _lib.SELECT_MAX_K:
+            raise ValueError(f"Selection.top_k must be an integer in 1..{_lib.SELECT_MAX_K}, not {k!r}")
+        for n in self.LIMITS:
+            v = getattr(self, n)
+            if v is not None and (isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 0 <= int(v) < 2**31):
+                raise ValueError(f"Selection.{n} must be None or an integer >= 0, not {v!r}")
+        c = self.min_coverage
+        if c is not None and (isinstance(c, bool) or not isinstance(c, (int, float, np.floating, np.integer)) or
+                              not 0.0 <= float(c) <= 1.0):
+            raise ValueError(f"Selection.min_coverage must be None or in [0, 1], not {c!r}")
+
+    def check_batch(self, coverage: bool, cost: str):
+        """The combinations ``plan_batch`` refuses."""
+        if cost != "length":
+            raise ValueError("select= replaces cost=: weight the time with Selection(w_length=0, w_time=1)")
+        if not coverage and (self.min_coverage is not None or self.w_uncovered > 0):
+            raise ValueError("min_coverage and w_uncovered need coverage=True: without it the coverage counts are 0, "
+                             "not measured")
+
+    def c_struct(self, grid_h: float) -> "_lib.SelectionC":
+        def lim(v):
+            return -1 if v is None else int(v)
+        return _lib.SelectionC(*[float(getattr(self, n)) for n in self.WEIGHTS], float(grid_h) * float(grid_h),
+                               -1.0 if self.min_coverage is None else float(self.min_coverage),
+                               lim(self.max_boundary_viol), lim(self.max_obstacle_viol), lim(self.max_accel_viol),
+                               int(self.top_k))
+
+
 @dataclass
 class PreparedBatch:
     """Host (numpy) side of one batch, ready to be copied to a device."""
@@ -440,6 +503,11 @@ class BatchResult:
     # plan_batch(..., winners=True): field -> (path [n,2], speeds [n] km/h, n_main) of the field's best candidate, on
     # the host (in a distributed run: the fields whose winner this rank owns)
     winner_paths: Optional[Dict[int, tuple]] = None
+    # plan_batch(..., select=Selection(top_k=k)): per field the k best eligible candidates (global indices, -1 = none),
+    # their costs (+inf = none) and summary records (zeros = none); best_cand / best_cost are column 0
+    topk_cand: Optional[np.ndarray] = None      # [F, k] int64
+    topk_cost: Optional[np.ndarray] = None      # [F, k] float64
+    topk_summary: Optional[np.ndarray] = None   # [F, k] SUMMARY_DTYPE
 
     def path(self, b: int):
         """(path [n,2], speeds [n], n_main) of local candidate ``b`` copied to the host."""
@@ -466,6 +534,8 @@ class BatchBuffers:
         self.d_cb = torch.empty(2 * nf, dtype=torch.int64, device=dev)
         self.d_cost = self.d_cb[:nf].view(torch.float64)
         self.d_best = self.d_cb[nf:]
+        self.top_k = 0               # > 0: the batch is ranked by fcpp_field_select into d_tk (use_top_k)
+        self.d_tk = self.d_tk_cost = self.d_tk_cand = None
         self.d_off = self.d_path = self.d_spd = self.d_kap = None
         self.speculative = False     # sized from remembered maxima (_Hints), not from this batch's layout pass
         if total_points > 0:
@@ -477,6 +547,17 @@ class BatchBuffers:
                 self.d_spd = torch.empty(total_points, dtype=torch.float64, device=dev)
                 if want_curvature:
                     self.d_kap = torch.empty(total_points, dtype=torch.float64, device=dev)
+
+
+    def use_top_k(self, k: int):
+        """k > 0: this batch's ranking goes to d_tk = costs [F, k] (double bits) then candidates [F, k], back to back
+        in ONE allocation (the multi-GPU merge all-gathers both at once); k = 0: the per-field argmin."""
+        self.top_k = int(k)
+        nfk = max(self.n_fields, 1) * self.top_k
+        if self.top_k and (self.d_tk is None or self.d_tk.numel() != 2 * nfk):
+            self.d_tk = torch.empty(2 * nfk, dtype=torch.int64, device=self.dev)
+            self.d_tk_cost = self.d_tk[:nfk].view(torch.float64)
+            self.d_tk_cand = self.d_tk[nfk:]
 
 
 def corner_grids(words: np.ndarray, g: int) -> np.ndarray:
@@ -525,13 +606,13 @@ class _Hints:
 
 def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, cost: str, cand_base: int,
                          buffers: Optional["BatchBuffers"], path_alloc=None, corner_bits: bool = False,
-                         speculate: bool = False):
+                         speculate: bool = False, select: Optional[Selection] = None):
     """Enqueue layout, prefix sum, plan, coverage and argmin kernels of one batch on torch's current
     stream.  Returns (buffers, offsets or None).  Without ``buffers`` the path storage is sized from
     the layout pass (one small synchronous read-back) — or, with ``speculate`` and a batch of this shape seen
     before, from the remembered sizes with no synchronisation at all (``buffers.speculative`` is then True and the
     caller must check the status flags, see ``_Hints``); ``path_alloc(total) -> BatchBuffers | None`` lets the
-    caller provide the storage."""
+    caller provide the storage.  ``select``: the per-field top-k of fcpp_field_select instead of the argmin."""
     if outputs not in ("summary", "paths"):
         raise ValueError("outputs must be 'summary' or 'paths'")
     dev = db.dev
@@ -600,9 +681,16 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, co
             if hint_key is not None:
                 _Hints.update(hint_key, db.max_points, db.max_head_points, buffers.total_points)
         cf = db.t.get("cand_field")     # factored sets: the library's candidate records carry the field
-        h.check(L.fcpp_field_argmin(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B, F,
-                                    0 if cost == "length" else 1, cand_base, buffers.d_cost.data_ptr(),
-                                    buffers.d_best.data_ptr(), stream))
+        buffers.use_top_k(select.top_k if select is not None else 0)
+        if select is None:
+            h.check(L.fcpp_field_argmin(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B,
+                                        F, 0 if cost == "length" else 1, cand_base, buffers.d_cost.data_ptr(),
+                                        buffers.d_best.data_ptr(), stream))
+        else:
+            sc = select.c_struct(db.pb.grid_h)
+            h.check(L.fcpp_field_select(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B,
+                                        F, C.byref(sc), cand_base, buffers.d_tk_cost.data_ptr(),
+                                        buffers.d_tk_cand.data_ptr(), stream))
     return buffers, offsets
 
 
@@ -613,18 +701,20 @@ class _PendingFetch:
 
 def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
                    cand_base: int, win: Optional[torch.Tensor] = None) -> _PendingFetch:
-    """Enqueue the copies of summaries + argmin (+ offsets) (+ ``win``: the winners' records and flag-count word
-    of a sharded batch, see dist.gather_winner_records) into ONE pooled pinned buffer on torch's current stream and
-    record an event behind them; nothing is waited for."""
+    """Enqueue the copies of summaries + argmin or top-k ranking (+ offsets) (+ ``win``: the winners' records and
+    flag-count word of a sharded batch, see dist.gather_winner_records) into ONE pooled pinned buffer on torch's
+    current stream and record an event behind them; nothing is waited for."""
     dev = db.dev
     B, F = db.pb.n_cand, db.pb.n_fields
+    nk = buffers.top_k or 1             # entries per field: the argmin's 1 or the ranking's k
+    d_cost, d_best = (buffers.d_tk_cost, buffers.d_tk_cand) if buffers.top_k else (buffers.d_cost, buffers.d_best)
     pf = _PendingFetch()
     with torch.cuda.device(dev):
         nb_sum = B * _lib.SUMMARY_DTYPE.itemsize if copy_summary else 0
         need_off = outputs == "paths" and offsets is None
         o_cost = (nb_sum + 255) & ~255
-        o_best = o_cost + ((F * 8 + 255) & ~255)
-        o_off = o_best + ((F * 8 + 255) & ~255)
+        o_best = o_cost + ((F * nk * 8 + 255) & ~255)
+        o_off = o_best + ((F * nk * 8 + 255) & ~255)
         total_out = o_off + ((B + 1) * 8 if need_off else 0)
         o_win = (total_out + 255) & ~255
         if win is not None:
@@ -646,8 +736,8 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
             if nb_sum:
                 ho[:nb_sum].copy_(buffers.d_sum[:nb_sum], non_blocking=True)
             if F:
-                ho[o_cost:o_cost + F * 8].view(torch.float64).copy_(buffers.d_cost[:F], non_blocking=True)
-                ho[o_best:o_best + F * 8].view(torch.int64).copy_(buffers.d_best[:F], non_blocking=True)
+                ho[o_cost:o_cost + F * nk * 8].view(torch.float64).copy_(d_cost[:F * nk], non_blocking=True)
+                ho[o_best:o_best + F * nk * 8].view(torch.int64).copy_(d_best[:F * nk], non_blocking=True)
             if need_off:
                 ho[o_off:o_off + (B + 1) * 8].view(torch.int64).copy_(buffers.d_off[:B + 1], non_blocking=True)
             if win is not None:
@@ -666,15 +756,21 @@ def _finish_fetch(pf: _PendingFetch) -> "BatchResult":
     db, buffers, offsets, hv = pf.db, pf.buffers, pf.offsets, pf.hv
     B, F = db.pb.n_cand, db.pb.n_fields
     nb_sum, need_off, o_cost, o_best, o_off = pf.lay
+    k = buffers.top_k
+    nk = k or 1
     pf.event.synchronize()
     summary = hv[:nb_sum].view(_lib.SUMMARY_DTYPE)[:B] if nb_sum else np.zeros(0, dtype=_lib.SUMMARY_DTYPE)
-    best_cost = hv[o_cost:o_cost + F * 8].view(np.float64)
-    best_cand = hv[o_best:o_best + F * 8].view(np.int64)
+    best_cost = hv[o_cost:o_cost + F * nk * 8].view(np.float64)
+    best_cand = hv[o_best:o_best + F * nk * 8].view(np.int64)
+    topk_cost = topk_cand = None
+    if k:
+        topk_cost, topk_cand = best_cost.reshape(F, k), best_cand.reshape(F, k)
+        best_cost, best_cand = np.ascontiguousarray(topk_cost[:, 0]), np.ascontiguousarray(topk_cand[:, 0])
     if need_off:
         offsets = hv[o_off:o_off + (B + 1) * 8].view(np.int64)
     res = BatchResult(summary=summary, best_cand=best_cand, best_cost=best_cost, n_fields=F, offsets=offsets,
                       d_path=buffers.d_path, d_speeds=buffers.d_spd, d_curvature=buffers.d_kap,
-                      d_summary=buffers.d_sum, cand_base=pf.cand_base)
+                      d_summary=buffers.d_sum, cand_base=pf.cand_base, topk_cand=topk_cand, topk_cost=topk_cost)
     res.extras["buffers"] = buffers
     return res
 
@@ -797,9 +893,9 @@ class PendingBatch:
     all ranks repeat the batch together."""
 
     def __init__(self, db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                 speculate, shard):
+                 speculate, shard, select=None):
         self.db, self.pf, self.outputs = db, pf, outputs
-        self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits)
+        self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select)
         self.speculate, self.shard = speculate, shard
         self._res = None
 
@@ -816,9 +912,11 @@ class PendingBatch:
         if self._res is not None:
             return self._res
         db, pf, outputs = self.db, self.pf, self.outputs
-        want_curvature, cost, cand_base, copy_summary, winners, corner_bits = self.args
+        want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select = self.args
         buffers = pf.buffers
         B, F = db.pb.n_cand, db.pb.n_fields
+        k = select.top_k if select is not None else 0
+        nk = k or 1
         rec = _lib.SUMMARY_DTYPE.itemsize
         res = _finish_fetch(pf)
         if self.shard is None:
@@ -826,23 +924,30 @@ class PendingBatch:
         else:
             # the number of flagged candidates OF ALL RANKS: every rank reads the same word and decides alike, also
             # a rank that had no remembered sizes itself
-            redo = self.speculate and int(pf.hwin[F * rec:F * rec + 4].view(np.int32)[0]) != 0
+            redo = self.speculate and int(pf.hwin[F * nk * rec:F * nk * rec + 4].view(np.int32)[0]) != 0
         if redo:
             # remembered sizes (see _Hints) did not fit this batch, or cannot be checked: once more, sized from its
             # own layout pass.  (A batch with candidates that are genuinely too large takes this path too and comes
             # back with the same flags.)
             _Hints.drop(_Hints.key(db, outputs, want_curvature))
             self._res = run_device_batch(db, outputs, want_curvature, cost, cand_base, copy_summary, None, True,
-                                         winners, corner_bits, speculate=False, shard=self.shard)
+                                         winners, corner_bits, speculate=False, shard=self.shard, select=select)
             return self._res
         if corner_bits:   # [B, stride] words on the device; batch.corner_grids() unpacks one candidate's
             res.extras["corner_bits"] = buffers.d_cbits[:B * buffers.cbits_stride].view(B, -1)
         res.extras["h2d_bytes"] = db.pb.h2d_bytes()
-        res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F + ((B + 1) * 8 if outputs == "paths" else 0)
+        res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F * nk + ((B + 1) * 8 if outputs == "paths" else 0)
         if self.shard is not None:
-            res.extras["winner_summary"] = pf.hwin[:F * rec].view(_lib.SUMMARY_DTYPE)
+            records = pf.hwin[:F * nk * rec].view(_lib.SUMMARY_DTYPE)
+            res.extras["winner_summary"] = records.reshape(F, k)[:, 0].copy() if k else records
             res.extras["shard"] = self.shard
-            res.extras["d2h_bytes"] += F * rec + 16
+            res.extras["d2h_bytes"] += F * nk * rec + 16
+            if k:
+                res.topk_summary = records.reshape(F, k)
+        elif k and len(res.summary) == B:
+            res.topk_summary = np.zeros((F, k), dtype=_lib.SUMMARY_DTYPE)
+            own = res.topk_cand >= 0
+            res.topk_summary[own] = res.summary[res.topk_cand[own] - cand_base]
         res.extras["speculative"] = bool(buffers.speculative)
         if winners:
             # on the side stream: behind this batch (its event has completed), not behind later batches in flight
@@ -856,7 +961,7 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
                      cost: str = "length", cand_base: int = 0, copy_summary: bool = True,
                      buffers: Optional[BatchBuffers] = None, fetch: bool = True,
                      winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True,
-                     shard: Optional[tuple] = None):
+                     shard: Optional[tuple] = None, select: Optional[Selection] = None):
     """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + argmin back.
 
     With ``buffers`` (from a previous run of the same batch shape) and ``db.max_points`` known the
@@ -866,20 +971,29 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
     read-back (``_Hints``; checked and repeated when the sizes do not fit).  ``wait=False`` returns a
     ``PendingBatch``.  ``shard=(lo, hi)``: the batch is this rank's candidates [lo, hi) of a batch sharded over the
     default process group; before the read-back the per-field argmin is merged over the ranks and every field's
-    winning summary record gathered (``dist.reduce_best``, ``dist.gather_winner_records``)."""
+    winning summary record gathered (``dist.reduce_best``, ``dist.gather_winner_records``).  ``select``: the per-field
+    top-k ranking instead of the argmin (merged over the ranks with ``dist.reduce_topk``; the records of every
+    ranked candidate gathered)."""
     buffers, offsets = _launch_device_batch(db, outputs, want_curvature, cost, cand_base, buffers,
-                                            corner_bits=corner_bits, speculate=speculate and copy_summary)
+                                            corner_bits=corner_bits, speculate=speculate and copy_summary,
+                                            select=select)
     if not fetch:
         return None
     win = None
     if shard is not None:
         from . import dist
-        dist.reduce_best(buffers.d_cost, buffers.d_best)       # in place: now the GLOBAL per-field argmin
+        if select is None:
+            dist.reduce_best(buffers.d_cost, buffers.d_best)       # in place: now the GLOBAL per-field argmin
+            best = buffers.d_best
+        else:
+            nfk = db.pb.n_fields * select.top_k
+            best = buffers.d_tk_cand[:nfk]
+            dist.reduce_topk(buffers.d_tk_cost[:nfk], best, select.top_k)     # in place: the GLOBAL ranking
         # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
-        win = dist.gather_winner_records(buffers.d_sum, buffers.d_best, shard[0], shard[1], count_mask=_SIZE_FLAGS)
+        win = dist.gather_winner_records(buffers.d_sum, best, shard[0], shard[1], count_mask=_SIZE_FLAGS)
     pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win)
     pend = PendingBatch(db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                        speculate and copy_summary, shard)
+                        speculate and copy_summary, shard, select)
     return pend if not wait else pend.result()
 
 
@@ -887,7 +1001,7 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
                obstacles=None, start_points=None, outputs: str = "summary", grid_h: float = 0.1,
                coverage: bool = True, cost: str = "length", device=None, want_curvature: bool = False,
                distributed: bool = False, turn_model: str = "arc", clothoid_share: float = 0.5,
-               winners: bool = False, wait: bool = True):
+               winners: bool = False, wait: bool = True, select: Optional[Selection] = None):
     """Evaluate B candidate plans.  See ``prepare_batch`` for the inputs.
 
     Returns a ``BatchResult``: per-candidate ``summary`` records (layout counts, path lengths and
@@ -909,6 +1023,11 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     ``winners=True`` also returns every field's winning path and speed profile on the host
     (``BatchResult.winner_paths``) — what a search caller needs from a batch.
 
+    ``select=Selection(...)`` ranks each field's candidates under a weighted cost among those that respect the
+    selection's limits (see ``Selection``) instead of the plain argmin: ``BatchResult.topk_cand`` / ``topk_cost`` /
+    ``topk_summary`` hold the ``top_k`` best per field, ``best_cand`` / ``best_cost`` (and ``winners``) the first.
+    It replaces ``cost``, which must stay 'length'.
+
     ``wait=False`` returns a ``PendingBatch`` as soon as the batch is enqueued; its ``result()`` gives the
     BatchResult.  Submitting the next batch before collecting the previous one overlaps the host side of a call with
     the kernels of the other (see ``PendingBatch``).
@@ -919,14 +1038,20 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     ``winner_paths`` then holds the fields whose winner this rank owns."""
     if cost not in ("length", "time"):
         raise ValueError(f"cost must be 'length' or 'time', not {cost!r}")
+    if select is not None:
+        if not isinstance(select, Selection):
+            raise ValueError(f"select must be a Selection, not {type(select).__name__}")
+        select.check_batch(coverage, cost)
     vehicle = vehicle or VehicleParams()
     if distributed:
         from . import dist
         return dist.plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h,
-                                       coverage, cost, device, want_curvature, turn_model, clothoid_share, winners, wait)
+                                       coverage, cost, device, want_curvature, turn_model, clothoid_share, winners, wait,
+                                       select)
     dev = _dev(device)
     pb = prepare_batch(fields, vehicle, candidates, obstacles, start_points, grid_h, coverage, turn_model,
                        clothoid_share)
     db = DeviceBatch(pb, dev)
-    return run_device_batch(db, outputs, want_curvature, cost, winners=winners, speculate=True, wait=wait)
+    return run_device_batch(db, outputs, want_curvature, cost, winners=winners, speculate=True, wait=wait,
+                            select=select)
 

@@ -152,6 +152,7 @@ void fcpp_destroy(fcpp_handle *h)
     if (h->h_maxn) cudaFreeHost(h->h_maxn);
     if (h->d_ga) cudaFree(h->d_ga);
     if (h->d_dedupe) cudaFree(h->d_dedupe);
+    if (h->d_sel) cudaFree(h->d_sel);
     if (h->h_ga_state) cudaFreeHost(h->h_ga_state);
     if (h->ga_stream) cudaStreamDestroy(h->ga_stream);
     for (int k = 0; k < 4; ++k)
@@ -318,6 +319,46 @@ int fcpp_field_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t w
     cudaError_t e = fcpp_launch_argmin_merge(h, d_gathered, world, n_fields, d_best_cost, d_best_cand,
                                              (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(h, e, "argmin merge kernel");
+    return FCPP_OK;
+}
+
+int fcpp_field_select(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
+                      int32_t n_fields, const fcpp_selection *sel, int64_t cand_base, double *d_cost, int64_t *d_cand,
+                      void *stream)
+{
+    if (!h) return FCPP_ERR_INVALID;
+    if (!sel || n_cand < 0 || n_fields < 0 || cand_base < 0 || (n_fields > 0 && (!d_cost || !d_cand)) ||
+        (n_cand > 0 && !d_summary))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_field_select: bad argument");
+    if (sel->top_k < 1 || sel->top_k > FCPP_SELECT_MAX_K)
+        return fail(h, FCPP_ERR_INVALID, "fcpp_field_select: top_k must be in 1..%d (got %d)", FCPP_SELECT_MAX_K,
+                    sel->top_k);
+    const double w[7] = {sel->w_length, sel->w_time, sel->w_boundary, sel->w_obstacle, sel->w_accel, sel->w_uncovered,
+                         sel->cell_area};
+    for (double x : w)
+        if (!(x >= 0.0 && isfinite(x)))
+            return fail(h, FCPP_ERR_INVALID, "fcpp_field_select: weights and cell_area must be finite and >= 0");
+    if (!(sel->min_coverage <= 1.0))  // NaN too; < 0 = no limit
+        return fail(h, FCPP_ERR_INVALID, "fcpp_field_select: min_coverage must be <= 1");
+    if (n_cand > 0 && !d_cand_field && (n_cand > h->rec_cap || !h->d_rec))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_field_select: no cand_field and no candidate records of this batch");
+    cudaSetDevice(h->device);
+    cudaError_t e = fcpp_launch_select(h, d_summary, d_cand_field, n_cand, n_fields, *sel, cand_base, d_cost, d_cand,
+                                       (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "selection kernels");
+    return FCPP_OK;
+}
+
+int fcpp_field_select_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t world, int32_t n_fields, int32_t k,
+                            double *d_cost, int64_t *d_cand, void *stream)
+{
+    if (!h) return FCPP_ERR_INVALID;
+    if (world < 1 || n_fields < 0 || k < 1 || k > FCPP_SELECT_MAX_K ||
+        (n_fields > 0 && (!d_gathered || !d_cost || !d_cand)))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_field_select_merge: bad argument");
+    cudaSetDevice(h->device);
+    cudaError_t e = fcpp_launch_select_merge(h, d_gathered, world, n_fields, k, d_cost, d_cand, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "selection merge kernel");
     return FCPP_OK;
 }
 

@@ -95,6 +95,8 @@ struct fcpp_handle {
     size_t ga_bytes;
     void *h_ga_state;        // pinned host copy of the GA state
     cudaStream_t ga_stream;  // capture stream of the generation graph
+    void *d_sel;             // top-k selection workspace (fcpp_select.cu): field counts, keys sorted by field, unit lists
+    size_t sel_bytes;
     char err[512];
 };
 
@@ -185,6 +187,18 @@ __device__ __forceinline__ uint32_t fcpp_dynamic_smem_bytes()
 #else
 #define FCPP_ASSERT(c) ((void)0)
 #endif
+
+// doubles as unsigned keys with the same order (per-field argmin and top-k selection)
+__device__ __forceinline__ unsigned long long order_bits(double x)
+{
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double unorder_bits(unsigned long long o)
+{
+    const unsigned long long b = (o >> 63) ? (o & 0x7fffffffffffffffull) : ~o;
+    return __longlong_as_double((long long)b);
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p)
 {
@@ -777,6 +791,11 @@ cudaError_t fcpp_launch_connection_matrix(fcpp_handle *h, const double *d_verts,
                                           double depot_y, double *d_C, int32_t *d_arg, cudaStream_t st);
 cudaError_t fcpp_launch_status_count(fcpp_handle *h, const fcpp_summary *d_summary, int64_t n, int mask, int32_t *d_count,
                                      cudaStream_t st);
+cudaError_t fcpp_launch_select(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
+                               int64_t n_cand, int32_t n_fields, const fcpp_selection &sel, int64_t cand_base,
+                               double *d_cost, int64_t *d_cand, cudaStream_t st);
+cudaError_t fcpp_launch_select_merge(fcpp_handle *h, const int64_t *d_gathered, int world, int32_t n_fields, int k,
+                                     double *d_cost, int64_t *d_cand, cudaStream_t st);
 cudaError_t fcpp_launch_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
                                int64_t n_cand, int32_t n_fields, int cost_kind, int64_t cand_base,
                                double *d_best_cost, int64_t *d_best_cand, cudaStream_t st);

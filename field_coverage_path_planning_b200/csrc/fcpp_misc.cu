@@ -55,17 +55,6 @@ __global__ void __launch_bounds__(TOUR_THREADS) tour_kernel(const double *__rest
     }
 }
 
-__device__ __forceinline__ unsigned long long order_bits(double x)
-{
-    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
-    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-__device__ __forceinline__ double unorder_bits(unsigned long long o)
-{
-    const unsigned long long b = (o >> 63) ? (o & 0x7fffffffffffffffull) : ~o;
-    return __longlong_as_double((long long)b);
-}
-
 __device__ __forceinline__ double cand_cost(const fcpp_summary &s, int kind)
 {
     return kind == 0 ? s.len_main + s.len_head : s.time_main + s.time_head;

@@ -7,6 +7,9 @@ The reduction is exact and deterministic (ties go to the lowest global candidate
        all_reduce(MIN) of the candidate index where the local best equals the global minimum;
     3. the winner's 176-byte summary record is contributed by its owner (fcpp_winner_records) and summed
        as int32 words (every other rank contributes zeros), i.e. an all-gather of one record per field.
+A top-k ranking (plan_batch(select=...)) is merged the same way: ONE all-gather of every rank's [F, k] costs and
+candidates and the library's merge kernel (fcpp_field_select_merge) — CPU/gloo: an all-gather and a sort — then the
+records of all F * k ranked candidates in step 3.
 Works on NCCL (CUDA tensors) and gloo (CPU tensors — used by the world_size-2 CPU tests).
 """
 from __future__ import annotations
@@ -77,6 +80,53 @@ def reduce_best(best_cost: torch.Tensor, best_cand: torch.Tensor, group=None) ->
     return best_cost, best_cand
 
 
+def reduce_topk(top_cost: torch.Tensor, top_cand: torch.Tensor, k: int, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Global per-field top-k from the ranks' local ones, in place.  ``top_cost`` / ``top_cand`` hold [F, k] (flat
+    or 2-D) sorted by (cost, GLOBAL candidate index), padded with +inf / -1; the result is the k lowest
+    (cost, index) of the union, padded the same way.
+
+    CUDA tensors: one NCCL all-gather of the 2 F k words + the library's merge kernel (fcpp_field_select_merge).
+    CPU tensors (gloo tests): the same rule with torch ops."""
+    n = top_cost.numel()
+    F = n // k if k else 0
+    world = dist.get_world_size(group)
+    if top_cost.is_cuda:
+        import ctypes as C
+        dev = top_cost.device
+        adjacent = (top_cost.dtype == torch.float64 and top_cand.dtype == torch.int64 and top_cost.is_contiguous()
+                    and top_cand.is_contiguous() and top_cand.data_ptr() == top_cost.data_ptr() + 8 * n
+                    and top_cost.untyped_storage().data_ptr() == top_cand.untyped_storage().data_ptr())
+        if adjacent:   # BatchBuffers.use_top_k lays them out back to back
+            send = torch.empty(0, dtype=torch.int64, device=dev).set_(
+                top_cost.untyped_storage(), top_cost.storage_offset(), (2 * n,))
+        else:
+            send = torch.cat([top_cost.reshape(-1).view(torch.int64), top_cand.reshape(-1)])
+        gathered = torch.empty(world * 2 * n, dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(gathered, send, group=group)
+        h = _lib.handle(dev.index)
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        h.check(h.lib.fcpp_field_select_merge(h.h, gathered.data_ptr(), world, F, k, top_cost.data_ptr(),
+                                              top_cand.data_ptr(), st))
+        return top_cost, top_cand
+    costs = [torch.empty_like(top_cost) for _ in range(world)]
+    cands = [torch.empty_like(top_cand) for _ in range(world)]
+    dist.all_gather(costs, top_cost.contiguous(), group=group)
+    dist.all_gather(cands, top_cand.contiguous(), group=group)
+    c = torch.cat([x.reshape(F, k) for x in costs], dim=1)           # [F, world k]
+    i = torch.cat([x.reshape(F, k) for x in cands], dim=1)
+    i = torch.where(i < 0, torch.full_like(i, I64_MAX), i)           # padding after every real entry
+    c = torch.where(i == I64_MAX, torch.full_like(c, float("inf")), c)
+    # (cost, index) order: by index, then STABLY by cost
+    o = torch.argsort(i, dim=1, stable=True)
+    c, i = torch.gather(c, 1, o), torch.gather(i, 1, o)
+    o = torch.argsort(c, dim=1, stable=True)
+    c, i = torch.gather(c, 1, o)[:, :k], torch.gather(i, 1, o)[:, :k]
+    none = i == I64_MAX
+    top_cost.copy_(torch.where(none, torch.full_like(c, float("inf")), c).reshape(top_cost.shape))
+    top_cand.copy_(torch.where(none, torch.full_like(i, -1), i).reshape(top_cand.shape))
+    return top_cost, top_cand
+
+
 def gather_winner_records(summary_bytes: torch.Tensor, best_cand: torch.Tensor, lo: int, hi: int,
                           group=None, count_mask: int = 0) -> torch.Tensor:
     """[F, 176] uint8: the summary record of every field's global winner.
@@ -114,12 +164,14 @@ def gather_winner_records(summary_bytes: torch.Tensor, best_cand: torch.Tensor, 
 
 
 def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h, coverage, cost,
-                       device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True):
+                       device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True,
+                       select=None):
     """plan_batch over all ranks of the default process group (see batch.plan_batch): every rank plans its
     contiguous shard; ONE all-gather + merge kernel gives every rank the per-field argmin, one kernel + one
     all-reduce every winner's summary record; the local summaries, the merged argmin and the winners' records
     come back to the host with ONE synchronisation.  Launch sizes are remembered from earlier batches of the same
-    shape (no layout read-back); ``wait=False`` returns a ``batch.PendingBatch``."""
+    shape (no layout read-back); ``wait=False`` returns a ``batch.PendingBatch``.  With ``select`` the ranks' top-k
+    rankings are merged instead of the argmin, and the records of every ranked candidate gathered."""
     from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch, run_device_batch
     if not dist.is_initialized():
         raise RuntimeError("distributed=True needs torch.distributed.init_process_group (backend 'nccl')")
@@ -135,4 +187,4 @@ def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, out
     pb = prepare_batch(fv, vehicle, local, obstacles, sp, grid_h, coverage, turn_model, clothoid_share)
     db = DeviceBatch(pb, dev)
     return run_device_batch(db, outputs, want_curvature, cost, lo, winners=winners, speculate=True, wait=wait,
-                            shard=(lo, hi))
+                            shard=(lo, hi), select=select)

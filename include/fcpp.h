@@ -243,6 +243,41 @@ int fcpp_field_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32
 int fcpp_field_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t world, int32_t n_fields,
                             double *d_best_cost, int64_t *d_best_cand, void *stream);
 
+/* ---- per-field top-k under a constraint-aware cost (DESIGN.md §3.8) ---- */
+#define FCPP_SELECT_MAX_K 32
+
+/* A candidate is ELIGIBLE when status == 0, every limit that is set holds (n_*_viol <= max_*), and, with
+ * min_coverage set, cov_total > 0 and (double)cov_cells >= min_coverage * (double)cov_total.  Its cost, in FP64
+ * left to right (the library is built with -fmad=false):
+ *   L = len_main + len_head;  T = time_main + time_head;  U = (double)(cov_total - cov_cells) * cell_area;
+ *   cost = w_length*L + w_time*T + w_boundary*n_boundary_viol + w_obstacle*n_obstacle_viol
+ *        + w_accel*n_accel_viol + w_uncovered*U
+ * w_length = 1 with every other weight 0 and no limits is exactly fcpp_field_argmin's cost_kind 0. */
+typedef struct {
+    double w_length, w_time, w_boundary, w_obstacle, w_accel, w_uncovered; /* finite, >= 0 */
+    double cell_area;          /* m^2 of a headland-band cell: grid_h * grid_h */
+    double min_coverage;       /* in [0, 1]; < 0: no limit */
+    int32_t max_boundary_viol; /* < 0: no limit */
+    int32_t max_obstacle_viol; /* < 0: no limit */
+    int32_t max_accel_viol;    /* < 0: no limit */
+    int32_t top_k;             /* 1 .. FCPP_SELECT_MAX_K */
+} fcpp_selection;
+
+/* Per field, the eligible candidates ranked by (cost, candidate index) ascending, the first top_k of them:
+ * d_cost [F][k] double (+inf where fewer than k are eligible), d_cand [F][k] int64 global indices (cand_base added;
+ * -1 where none).  d_cand_field as in fcpp_field_argmin (NULL: the candidate records of the last fcpp_plan_batch).
+ * Exact and deterministic for any order of the candidates' fields; scratch space is the handle's workspace. */
+int fcpp_field_select(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
+                      int32_t n_fields, const fcpp_selection *sel, int64_t cand_base, double *d_cost,
+                      int64_t *d_cand, void *stream);
+
+/* Multi-GPU merge of the ranks' rankings: d_gathered [world][2*F*k] 8-byte words = every rank's d_cost [F][k] (as
+ * double bits) then d_cand [F][k], e.g. ONE all-gather of the two arrays laid out back to back.  Per field the k
+ * lowest (cost, index) of the union; +inf / -1 pad.  The winners' records of the ranking: fcpp_winner_records
+ * with n_fields = F * k on the flattened d_cand. */
+int fcpp_field_select_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t world, int32_t n_fields, int32_t k,
+                            double *d_cost, int64_t *d_cand, void *stream);
+
 /* Multi-GPU: this rank's contribution to the exchange of the winners' records after the merge: d_out [F][176 bytes]
  * = the summary record of every field whose global winner d_best_cand[f] lies in this rank's candidate range
  * [cand_lo, cand_hi) (d_summary holds that range), zeros for every other field — summing the ranks' buffers as
