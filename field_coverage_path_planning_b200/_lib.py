@@ -138,9 +138,14 @@ SUMMARY_DTYPE = np.dtype([
 ], align=True)
 assert SUMMARY_DTYPE.itemsize == 176, SUMMARY_DTYPE.itemsize
 
+# numpy mirror of fcpp_sweep (24 bytes): per layer, the segments that enter the obstacle region and the metres inside
+SWEEP_DTYPE = np.dtype([("n_seg_main", "<i4"), ("n_seg_head", "<i4"), ("len_main", "<f8"), ("len_head", "<f8")],
+                       align=True)
+assert SWEEP_DTYPE.itemsize == 24, SWEEP_DTYPE.itemsize
+
 EXPORTS = [
     "fcpp_abi_version", "fcpp_create", "fcpp_destroy", "fcpp_last_error", "fcpp_set_trig_tables",
-    "fcpp_layout", "fcpp_plan_batch", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
+    "fcpp_layout", "fcpp_plan_batch", "fcpp_obstacle_sweep", "fcpp_obstacle_sweep_paths", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
     "fcpp_tour_lengths", "fcpp_distance_matrix", "fcpp_connection_matrix", "fcpp_ga_init_population", "fcpp_ga_next_size", "fcpp_ga_generation", "fcpp_ga_solve", "fcpp_kmeans_lloyd", "fcpp_tsp_two_opt",
     "fcpp_launch_count", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
 ]
@@ -179,6 +184,10 @@ def load():
         L.fcpp_layout.argtypes = [vp, C.POINTER(Batch), vp, vp, vp]
         L.fcpp_plan_batch.restype = C.c_int
         L.fcpp_plan_batch.argtypes = [vp, C.POINTER(Batch), C.POINTER(Outputs), vp]
+        L.fcpp_obstacle_sweep.restype = C.c_int
+        L.fcpp_obstacle_sweep.argtypes = [vp, C.POINTER(Batch), vp, vp]
+        L.fcpp_obstacle_sweep_paths.restype = C.c_int
+        L.fcpp_obstacle_sweep_paths.argtypes = [vp, vp, vp, i64, vp, vp, vp, i32, dbl, vp, vp]
         L.fcpp_field_argmin.restype = C.c_int
         L.fcpp_field_argmin.argtypes = [vp, vp, vp, i64, i32, C.c_int, i64, vp, vp, vp]
         L.fcpp_field_argmin_merge.restype = C.c_int

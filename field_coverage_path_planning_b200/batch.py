@@ -508,6 +508,9 @@ class BatchResult:
     topk_cand: Optional[np.ndarray] = None      # [F, k] int64
     topk_cost: Optional[np.ndarray] = None      # [F, k] float64
     topk_summary: Optional[np.ndarray] = None   # [F, k] SUMMARY_DTYPE
+    # plan_batch(..., obstacle_sweep=True): per candidate the segments that drive through the obstacle region and the
+    # metres inside, per layer (include/fcpp.h fcpp_sweep)
+    sweep: Optional[np.ndarray] = None          # [B] SWEEP_DTYPE
 
     def path(self, b: int):
         """(path [n,2], speeds [n], n_main) of local candidate ``b`` copied to the host."""
@@ -537,6 +540,7 @@ class BatchBuffers:
         self.top_k = 0               # > 0: the batch is ranked by fcpp_field_select into d_tk (use_top_k)
         self.d_tk = self.d_tk_cost = self.d_tk_cand = None
         self.d_off = self.d_path = self.d_spd = self.d_kap = None
+        self.d_sweep = None          # [B] fcpp_sweep records of the last batch run with obstacle_sweep=True
         self.speculative = False     # sized from remembered maxima (_Hints), not from this batch's layout pass
         if total_points > 0:
             self.d_off = torch.empty(n_cand + 1, dtype=torch.int64, device=dev)
@@ -606,13 +610,14 @@ class _Hints:
 
 def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, cost: str, cand_base: int,
                          buffers: Optional["BatchBuffers"], path_alloc=None, corner_bits: bool = False,
-                         speculate: bool = False, select: Optional[Selection] = None):
+                         speculate: bool = False, select: Optional[Selection] = None, sweep: bool = False):
     """Enqueue layout, prefix sum, plan, coverage and argmin kernels of one batch on torch's current
     stream.  Returns (buffers, offsets or None).  Without ``buffers`` the path storage is sized from
     the layout pass (one small synchronous read-back) — or, with ``speculate`` and a batch of this shape seen
     before, from the remembered sizes with no synchronisation at all (``buffers.speculative`` is then True and the
     caller must check the status flags, see ``_Hints``); ``path_alloc(total) -> BatchBuffers | None`` lets the
-    caller provide the storage.  ``select``: the per-field top-k of fcpp_field_select instead of the argmin."""
+    caller provide the storage.  ``select``: the per-field top-k of fcpp_field_select instead of the argmin.
+    ``sweep``: also the segment-level obstacle sweep of every candidate (fcpp_obstacle_sweep) into buffers.d_sweep."""
     if outputs not in ("summary", "paths"):
         raise ValueError("outputs must be 'summary' or 'paths'")
     dev = db.dev
@@ -675,6 +680,11 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, co
             if buffers.d_kap is not None:
                 out.curvature = buffers.d_kap.data_ptr()
         h.check(L.fcpp_plan_batch(h.h, C.byref(db.c), C.byref(out), stream))
+        if sweep:
+            nb = max(B, 1) * _lib.SWEEP_DTYPE.itemsize
+            if buffers.d_sweep is None or buffers.d_sweep.numel() < nb:
+                buffers.d_sweep = torch.empty(nb, dtype=torch.uint8, device=dev)
+            h.check(L.fcpp_obstacle_sweep(h.h, C.byref(db.c), buffers.d_sweep.data_ptr(), stream))
         if db.c.max_points_hint == 0:
             db.max_points = int(L.fcpp_last_max_points(h.h))
             db.max_head_points = int(L.fcpp_last_max_head_points(h.h))
@@ -696,14 +706,14 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, co
 
 class _PendingFetch:
     """The read-back of a launched batch, enqueued but not waited for."""
-    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "hv", "lay", "win", "hwin", "event")
+    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "hv", "lay", "win", "hwin", "event", "o_sweep")
 
 
 def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
-                   cand_base: int, win: Optional[torch.Tensor] = None) -> _PendingFetch:
+                   cand_base: int, win: Optional[torch.Tensor] = None, sweep: bool = False) -> _PendingFetch:
     """Enqueue the copies of summaries + argmin or top-k ranking (+ offsets) (+ ``win``: the winners' records and
-    flag-count word of a sharded batch, see dist.gather_winner_records) into ONE pooled pinned buffer on torch's
-    current stream and record an event behind them; nothing is waited for."""
+    flag-count word of a sharded batch, see dist.gather_winner_records) (+ ``sweep``: the obstacle sweep records)
+    into ONE pooled pinned buffer on torch's current stream and record an event behind them; nothing is waited for."""
     dev = db.dev
     B, F = db.pb.n_cand, db.pb.n_fields
     nk = buffers.top_k or 1             # entries per field: the argmin's 1 or the ranking's k
@@ -719,6 +729,10 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
         o_win = (total_out + 255) & ~255
         if win is not None:
             total_out = o_win + win.numel()
+        o_sweep = (total_out + 255) & ~255
+        nb_sweep = B * _lib.SWEEP_DTYPE.itemsize if sweep else 0
+        if sweep:
+            total_out = o_sweep + nb_sweep
         ho, hv = _ResultPool.get(total_out)
         # the copies run on a COPY stream behind an event of the launching stream: the next batch's kernels (already
         # enqueued by a pipelining caller) must not wait for PCIe — at 737 280 candidates the 130 MB of summaries
@@ -741,12 +755,15 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
             if need_off:
                 ho[o_off:o_off + (B + 1) * 8].view(torch.int64).copy_(buffers.d_off[:B + 1], non_blocking=True)
             if win is not None:
-                ho[o_win:total_out].copy_(win, non_blocking=True)
+                ho[o_win:o_win + win.numel()].copy_(win, non_blocking=True)
+            if nb_sweep:
+                ho[o_sweep:o_sweep + nb_sweep].copy_(buffers.d_sweep[:nb_sweep], non_blocking=True)
             pf.event = torch.cuda.Event()
             pf.event.record(cs)
     pf.db, pf.buffers, pf.outputs, pf.offsets, pf.cand_base = db, buffers, outputs, offsets, cand_base
     pf.hv, pf.lay = hv, (nb_sum, need_off, o_cost, o_best, o_off)
-    pf.win, pf.hwin = win, (hv[o_win:total_out] if win is not None else None)
+    pf.win, pf.hwin = win, (hv[o_win:o_win + win.numel()] if win is not None else None)
+    pf.o_sweep = (o_sweep, B) if sweep else None
     return pf
 
 
@@ -771,6 +788,9 @@ def _finish_fetch(pf: _PendingFetch) -> "BatchResult":
     res = BatchResult(summary=summary, best_cand=best_cand, best_cost=best_cost, n_fields=F, offsets=offsets,
                       d_path=buffers.d_path, d_speeds=buffers.d_spd, d_curvature=buffers.d_kap,
                       d_summary=buffers.d_sum, cand_base=pf.cand_base, topk_cand=topk_cand, topk_cost=topk_cost)
+    if pf.o_sweep is not None:
+        o, n = pf.o_sweep
+        res.sweep = hv[o:o + n * _lib.SWEEP_DTYPE.itemsize].view(_lib.SWEEP_DTYPE)
     res.extras["buffers"] = buffers
     return res
 
@@ -893,9 +913,9 @@ class PendingBatch:
     all ranks repeat the batch together."""
 
     def __init__(self, db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                 speculate, shard, select=None):
+                 speculate, shard, select=None, sweep=False):
         self.db, self.pf, self.outputs = db, pf, outputs
-        self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select)
+        self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select, sweep)
         self.speculate, self.shard = speculate, shard
         self._res = None
 
@@ -912,7 +932,7 @@ class PendingBatch:
         if self._res is not None:
             return self._res
         db, pf, outputs = self.db, self.pf, self.outputs
-        want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select = self.args
+        want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select, sweep = self.args
         buffers = pf.buffers
         B, F = db.pb.n_cand, db.pb.n_fields
         k = select.top_k if select is not None else 0
@@ -931,12 +951,15 @@ class PendingBatch:
             # back with the same flags.)
             _Hints.drop(_Hints.key(db, outputs, want_curvature))
             self._res = run_device_batch(db, outputs, want_curvature, cost, cand_base, copy_summary, None, True,
-                                         winners, corner_bits, speculate=False, shard=self.shard, select=select)
+                                         winners, corner_bits, speculate=False, shard=self.shard, select=select,
+                                         obstacle_sweep=sweep)
             return self._res
         if corner_bits:   # [B, stride] words on the device; batch.corner_grids() unpacks one candidate's
             res.extras["corner_bits"] = buffers.d_cbits[:B * buffers.cbits_stride].view(B, -1)
         res.extras["h2d_bytes"] = db.pb.h2d_bytes()
         res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F * nk + ((B + 1) * 8 if outputs == "paths" else 0)
+        if sweep:
+            res.extras["d2h_bytes"] += B * _lib.SWEEP_DTYPE.itemsize
         if self.shard is not None:
             records = pf.hwin[:F * nk * rec].view(_lib.SUMMARY_DTYPE)
             res.extras["winner_summary"] = records.reshape(F, k)[:, 0].copy() if k else records
@@ -961,7 +984,7 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
                      cost: str = "length", cand_base: int = 0, copy_summary: bool = True,
                      buffers: Optional[BatchBuffers] = None, fetch: bool = True,
                      winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True,
-                     shard: Optional[tuple] = None, select: Optional[Selection] = None):
+                     shard: Optional[tuple] = None, select: Optional[Selection] = None, obstacle_sweep: bool = False):
     """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + argmin back.
 
     With ``buffers`` (from a previous run of the same batch shape) and ``db.max_points`` known the
@@ -973,10 +996,11 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
     default process group; before the read-back the per-field argmin is merged over the ranks and every field's
     winning summary record gathered (``dist.reduce_best``, ``dist.gather_winner_records``).  ``select``: the per-field
     top-k ranking instead of the argmin (merged over the ranks with ``dist.reduce_topk``; the records of every
-    ranked candidate gathered)."""
+    ranked candidate gathered).  ``obstacle_sweep``: also each candidate's segment-level obstacle sweep
+    (``BatchResult.sweep``; in a sharded batch, of this rank's candidates)."""
     buffers, offsets = _launch_device_batch(db, outputs, want_curvature, cost, cand_base, buffers,
                                             corner_bits=corner_bits, speculate=speculate and copy_summary,
-                                            select=select)
+                                            select=select, sweep=obstacle_sweep)
     if not fetch:
         return None
     win = None
@@ -991,9 +1015,9 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
             dist.reduce_topk(buffers.d_tk_cost[:nfk], best, select.top_k)     # in place: the GLOBAL ranking
         # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
         win = dist.gather_winner_records(buffers.d_sum, best, shard[0], shard[1], count_mask=_SIZE_FLAGS)
-    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win)
+    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win, obstacle_sweep)
     pend = PendingBatch(db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                        speculate and copy_summary, shard, select)
+                        speculate and copy_summary, shard, select, obstacle_sweep)
     return pend if not wait else pend.result()
 
 
@@ -1001,7 +1025,8 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
                obstacles=None, start_points=None, outputs: str = "summary", grid_h: float = 0.1,
                coverage: bool = True, cost: str = "length", device=None, want_curvature: bool = False,
                distributed: bool = False, turn_model: str = "arc", clothoid_share: float = 0.5,
-               winners: bool = False, wait: bool = True, select: Optional[Selection] = None):
+               winners: bool = False, wait: bool = True, select: Optional[Selection] = None,
+               obstacle_sweep: bool = False):
     """Evaluate B candidate plans.  See ``prepare_batch`` for the inputs.
 
     Returns a ``BatchResult``: per-candidate ``summary`` records (layout counts, path lengths and
@@ -1028,6 +1053,12 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     ``topk_summary`` hold the ``top_k`` best per field, ``best_cand`` / ``best_cost`` (and ``winners``) the first.
     It replaces ``cost``, which must stay 'length'.
 
+    ``obstacle_sweep=True`` also measures how far each plan drives through the obstacles (DESIGN.md §3.9): D3's
+    ``n_obstacle_viol`` counts path POINTS in the W/2-buffered obstacles, and a swath's two points can lie on either
+    side of an obstacle; the sweep measures every SEGMENT.  ``BatchResult.sweep`` [B] (``_lib.SWEEP_DTYPE``) holds per
+    layer the segments with metres inside the obstacle region and the sum of those metres.  It is read back with the
+    summaries (no extra synchronisation) and changes no other output.
+
     ``wait=False`` returns a ``PendingBatch`` as soon as the batch is enqueued; its ``result()`` gives the
     BatchResult.  Submitting the next batch before collecting the previous one overlaps the host side of a call with
     the kernels of the other (see ``PendingBatch``).
@@ -1047,11 +1078,57 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
         from . import dist
         return dist.plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h,
                                        coverage, cost, device, want_curvature, turn_model, clothoid_share, winners, wait,
-                                       select)
+                                       select, obstacle_sweep)
     dev = _dev(device)
     pb = prepare_batch(fields, vehicle, candidates, obstacles, start_points, grid_h, coverage, turn_model,
                        clothoid_share)
     db = DeviceBatch(pb, dev)
     return run_device_batch(db, outputs, want_curvature, cost, winners=winners, speculate=True, wait=wait,
-                            select=select)
+                            select=select, obstacle_sweep=obstacle_sweep)
+
+
+def obstacle_sweep(paths, obstacles, working_width: float, n_main=None, device=None) -> np.ndarray:
+    """The segment-level obstacle sweep of caller-supplied paths (DESIGN.md §3.9) on the GPU.
+
+    ``paths``: one [n, 2] array or a sequence of them; ``obstacles``: one list of polygons (each a sequence of (x, y))
+    that every path is checked against; the radius is ``working_width / 2``.  ``n_main`` (an int per path, or one int
+    for a single path) splits a path into main work (its first n_main points) and headland, as a plan's
+    ``main_work.path`` + ``headland.path``; without it the whole path counts as main work.  Returns a [n_paths]
+    ``_lib.SWEEP_DTYPE`` array: per layer the segments that enter the obstacle region and the metres inside."""
+    single = isinstance(paths, np.ndarray) and paths.ndim == 2
+    plist = [paths] if single else list(paths)
+    pts = [np.ascontiguousarray(np.asarray(p, dtype=np.float64).reshape(-1, 2)) for p in plist]
+    n = len(pts)
+    if n_main is not None:
+        nm = np.atleast_1d(np.asarray(n_main, dtype=np.int64))
+        if len(nm) != n:
+            raise ValueError("n_main needs one value per path")
+        if any(not 0 <= int(m) <= len(p) for m, p in zip(nm, pts)):
+            raise ValueError("n_main must lie in [0, len(path)]")
+        nm = nm.astype(np.int32)
+    if not working_width > 0:
+        raise ValueError("working_width must be > 0")
+    polys = [np.asarray(o, dtype=np.float64).reshape(-1, 2) for o in (obstacles or []) if len(o)]
+    out = np.zeros(n, dtype=_lib.SWEEP_DTYPE)
+    if n == 0:
+        return out
+    dev = _dev(device)
+    h = _lib.handle(dev.index)
+    offs = np.zeros(n + 1, dtype=np.int64)
+    offs[1:] = np.cumsum([len(p) for p in pts])
+    arrays = {"path": np.concatenate(pts) if offs[-1] else np.zeros((1, 2)), "offsets": offs,
+              "vs": np.concatenate([[0], np.cumsum([len(o) for o in polys])]).astype(np.int32),
+              "verts": np.concatenate(polys) if polys else np.zeros((1, 2))}
+    if n_main is not None:
+        arrays["n_main"] = nm
+    with torch.cuda.device(dev):
+        t = _pack_to_dev(arrays, dev)
+        d_out = torch.empty(n * _lib.SWEEP_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        h.check(h.lib.fcpp_obstacle_sweep_paths(h.h, t["path"].data_ptr(), t["offsets"].data_ptr(), n,
+                                                t["n_main"].data_ptr() if n_main is not None else None,
+                                                t["vs"].data_ptr(), t["verts"].data_ptr(), len(polys),
+                                                float(working_width) / 2, d_out.data_ptr(), stream))
+        out[:] = d_out.cpu().numpy().view(_lib.SWEEP_DTYPE)
+    return out
 

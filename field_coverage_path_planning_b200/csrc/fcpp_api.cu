@@ -220,6 +220,7 @@ int fcpp_layout(fcpp_handle *h, const fcpp_batch *batch, int32_t *d_n_pts, int64
     if (rc) return rc;
     cudaSetDevice(h->device);
     cudaStream_t st = (cudaStream_t)stream;
+    h->rec_valid = false;
     rc = ensure_workspace(h, batch->n_cand);
     if (rc) return rc;
     cudaError_t e = fcpp_launch_layout(h, *batch, d_n_pts, d_offsets, st);
@@ -247,6 +248,7 @@ int fcpp_layout(fcpp_handle *h, const fcpp_batch *batch, int32_t *d_n_pts, int64
     }
     h->cover_pcap = maxhead;
     h->layout_valid = true;
+    h->rec_valid = true;
     h->layout_ncand = batch->n_cand;
     h->layout_id[0] = batch->cand_field ? (const void *)batch->cand_R : (const void *)batch->ax_radii;
     h->layout_id[1] = batch->cand_field ? (const void *)batch->cand_flags : (const void *)(intptr_t)batch->cand_first;
@@ -290,6 +292,39 @@ int fcpp_plan_batch(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outputs 
     }
     if (prof) cudaEventRecord(h->ev[3], st);
     h->layout_valid = false;  // one layout per plan call
+    return FCPP_OK;
+}
+
+int fcpp_obstacle_sweep(fcpp_handle *h, const fcpp_batch *batch, fcpp_sweep *d_out, void *stream)
+{
+    int rc = check_batch(h, batch);
+    if (rc) return rc;
+    if (batch->n_cand > 0 && !d_out) return fail(h, FCPP_ERR_INVALID, "fcpp_obstacle_sweep: d_out is NULL");
+    // the records must be those of this batch: the stamp of its layout pass, which fcpp_plan_batch leaves in place
+    const void *id0 = batch->cand_field ? (const void *)batch->cand_R : (const void *)batch->ax_radii;
+    const void *id1 = batch->cand_field ? (const void *)batch->cand_flags : (const void *)(intptr_t)batch->cand_first;
+    if (!h->rec_valid || h->layout_ncand != batch->n_cand || h->layout_id[0] != id0 || h->layout_id[1] != id1 ||
+        h->layout_id[2] != batch->field_verts || h->layout_id[3] != stream)
+        return fail(h, FCPP_ERR_INVALID, "fcpp_layout must be called for this batch (same arrays, same stream) "
+                                         "before fcpp_obstacle_sweep");
+    cudaSetDevice(h->device);
+    cudaError_t e = fcpp_launch_sweep(h, *batch, d_out, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "obstacle sweep kernel");
+    return FCPP_OK;
+}
+
+int fcpp_obstacle_sweep_paths(fcpp_handle *h, const double *d_path_xy, const int64_t *d_offsets, int64_t n_paths,
+                              const int32_t *d_n_main, const int32_t *d_obs_vert_start, const double *d_obs_verts,
+                              int32_t n_polys, double radius, fcpp_sweep *d_out, void *stream)
+{
+    if (!h) return FCPP_ERR_INVALID;
+    if (n_paths < 0 || n_paths > 0x7fffffff || n_polys < 0 || !(radius >= 0.0) || !isfinite(radius) ||
+        (n_paths > 0 && (!d_path_xy || !d_offsets || !d_out)) || (n_polys > 0 && (!d_obs_vert_start || !d_obs_verts)))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_obstacle_sweep_paths: bad argument");
+    cudaSetDevice(h->device);
+    cudaError_t e = fcpp_launch_sweep_paths(h, d_path_xy, d_offsets, n_paths, d_n_main, d_obs_vert_start, d_obs_verts,
+                                            n_polys, radius, d_out, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "obstacle sweep kernel (paths)");
     return FCPP_OK;
 }
 

@@ -77,6 +77,7 @@ struct fcpp_handle {
     int max_smem_sm;         // shared memory per SM
     int sm_count;
     bool layout_valid;
+    bool rec_valid;          // the candidate records belong to the batch of layout_id (kept after fcpp_plan_batch)
     bool profiling;
     cudaEvent_t ev[4];       // layout start, plan start, cover start, end
     int last_maxn;
@@ -796,6 +797,10 @@ cudaError_t fcpp_launch_select(fcpp_handle *h, const fcpp_summary *d_summary, co
                                double *d_cost, int64_t *d_cand, cudaStream_t st);
 cudaError_t fcpp_launch_select_merge(fcpp_handle *h, const int64_t *d_gathered, int world, int32_t n_fields, int k,
                                      double *d_cost, int64_t *d_cand, cudaStream_t st);
+cudaError_t fcpp_launch_sweep(fcpp_handle *h, const fcpp_batch &b, fcpp_sweep *d_out, cudaStream_t st);
+cudaError_t fcpp_launch_sweep_paths(fcpp_handle *h, const double *d_path, const int64_t *d_offsets, int64_t n_paths,
+                                    const int32_t *d_n_main, const int32_t *d_vert_start, const double *d_verts,
+                                    int32_t n_polys, double radius, fcpp_sweep *d_out, cudaStream_t st);
 cudaError_t fcpp_launch_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
                                int64_t n_cand, int32_t n_fields, int cost_kind, int64_t cand_base,
                                double *d_best_cost, int64_t *d_best_cand, cudaStream_t st);

@@ -165,13 +165,14 @@ def gather_winner_records(summary_bytes: torch.Tensor, best_cand: torch.Tensor, 
 
 def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h, coverage, cost,
                        device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True,
-                       select=None):
+                       select=None, obstacle_sweep=False):
     """plan_batch over all ranks of the default process group (see batch.plan_batch): every rank plans its
     contiguous shard; ONE all-gather + merge kernel gives every rank the per-field argmin, one kernel + one
     all-reduce every winner's summary record; the local summaries, the merged argmin and the winners' records
     come back to the host with ONE synchronisation.  Launch sizes are remembered from earlier batches of the same
     shape (no layout read-back); ``wait=False`` returns a ``batch.PendingBatch``.  With ``select`` the ranks' top-k
-    rankings are merged instead of the argmin, and the records of every ranked candidate gathered."""
+    rankings are merged instead of the argmin, and the records of every ranked candidate gathered.  With
+    ``obstacle_sweep`` each rank gets the sweep of its own candidates (``BatchResult.sweep``)."""
     from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch, run_device_batch
     if not dist.is_initialized():
         raise RuntimeError("distributed=True needs torch.distributed.init_process_group (backend 'nccl')")
@@ -187,4 +188,4 @@ def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, out
     pb = prepare_batch(fv, vehicle, local, obstacles, sp, grid_h, coverage, turn_model, clothoid_share)
     db = DeviceBatch(pb, dev)
     return run_device_batch(db, outputs, want_curvature, cost, lo, winners=winners, speculate=True, wait=wait,
-                            shard=(lo, hi), select=select)
+                            shard=(lo, hi), select=select, obstacle_sweep=obstacle_sweep)

@@ -22,7 +22,7 @@ import torch
 
 from . import _geometry as G
 from . import _lib
-from .batch import DeviceBatch, _dev, corner_grids, prepare_batch, run_device_batch
+from .batch import DeviceBatch, _dev, corner_grids, obstacle_sweep, prepare_batch, run_device_batch
 from .vehicle import VehicleParams
 
 APPROACH_POINTS = 50  # mlp3:1317
@@ -55,6 +55,7 @@ class TwoLayerPathPlannerV37:
         self.start_point = self._validate_point(start_point)
         self.end_point = self._validate_point(end_point)
         self._last = None
+        self._last_path = None     # (points [n, 2], n_main) of the last plan
         self._last_grids = None
 
     # ---- A2: field set-up (host, FP64) -----------------------------------------------------
@@ -173,6 +174,7 @@ class TwoLayerPathPlannerV37:
         if self.end_point:     # mlp3:443-447
             departure = self._generate_departure_path(head['path'][-1], self.end_point)
         self._last = s
+        self._last_path = (path, nm)
         self._last_grids = corner_grids(res.extras["corner_bits"][0].cpu().numpy().view(np.uint32), int(s["corner_g"])) \
             if not (s["status"] & _lib.CAND_GRID_TOO_LARGE) else None
         result = {'main_work': main, 'headland': head, 'approach_path': approach, 'departure_path': departure,
@@ -248,6 +250,30 @@ class TwoLayerPathPlannerV37:
         return {'max_curvature': float(s["max_curvature"]), 'max_lateral_accel': float(s["max_lateral_accel"]),
                 'max_allowed_accel': self.vehicle.max_lateral_accel, 'accel_violations': viol,
                 'accel_violation_rate': rate, 'max_jump': float(s["max_jump"]), 'pass': rate < 5}
+
+    def verify_obstacle_clearance(self, path=None, n_main: Optional[int] = None) -> Dict:
+        """How far a path drives through the obstacles buffered by W/2 (the segment-level sweep, DESIGN.md §3.9).
+
+        ``path=None``: the last plan (``main_work.path`` then ``headland.path``, planned first if there is none);
+        otherwise a caller-supplied [n, 2] path whose first ``n_main`` points are main work (default: all of them).
+        Returns per layer the segments that enter the obstacle region and the metres inside, their totals,
+        ``pass`` = no segment enters, and ``point_violations``: D3's count of path POINTS inside (the plan's
+        ``n_obstacle_viol``; None for a caller-supplied path) — a swath can cross an obstacle with both its points
+        outside, which the point count does not see."""
+        points = None
+        if path is None:
+            if self._last_path is None:
+                self.plan_complete_coverage()
+            path, n_main = self._last_path
+            points = int(self._last["n_obstacle_viol"])
+        path = np.ascontiguousarray(path, dtype=np.float64).reshape(-1, 2)
+        sw = obstacle_sweep(path, self.obstacles, self.vehicle.working_width,
+                            n_main=None if n_main is None else [int(n_main)], device=self._device)[0]
+        segs = int(sw["n_seg_main"]) + int(sw["n_seg_head"])
+        return {'segments_main': int(sw["n_seg_main"]), 'segments_head': int(sw["n_seg_head"]),
+                'metres_main': float(sw["len_main"]), 'metres_head': float(sw["len_head"]),
+                'segments': segs, 'metres': float(sw["len_main"]) + float(sw["len_head"]),
+                'point_violations': points, 'pass': segs == 0}
 
     def verify_corner_coverage_grid_based(self, corner, corner_index: int, turn_path, reverse_path=None) -> Dict:
         """mlp3:1426-1510 with the exact fixed-point predicate (D5)."""

@@ -304,6 +304,32 @@ int fcpp_speed_verify(fcpp_handle *h, const fcpp_vehicle *veh, const double *d_p
                       int64_t max_path_len, int do_speed_plan, double *d_speeds_out,
                       double *d_curvature, fcpp_summary *d_summary, void *stream);
 
+/* ---- segment-level obstacle sweep (DESIGN.md §3.9) ----
+ * The obstacle region O of a field is the set of points D3 counts in n_obstacle_viol: inside an obstacle polygon
+ * (even-odd crossing) or at distance < r from one of its edges.  For every segment a -> b of a path, m = metres of
+ * the segment inside O (exact up to rounding: the segment is cut at the boundaries of the edges' r-capsules and each
+ * piece classified at its midpoint; oracle/sweep.py states the rule).  Per candidate or path: the segments with
+ * m > 0 and the sum of m (left to right in segment order) of main_work.path and of headland.path; the segment
+ * from the last main point to the first headland point belongs to neither.  24 bytes. */
+typedef struct {
+    int32_t n_seg_main, n_seg_head; /* segments with m > 0 */
+    double len_main, len_head;      /* m, summed left to right */
+} fcpp_sweep;
+
+/* The sweep of every candidate of `batch` with r = working_width / 2, from the library's candidate records: must
+ * follow fcpp_layout of the same batch (same arrays, same stream) on this handle — before or after its
+ * fcpp_plan_batch — else FCPP_ERR_INVALID.  d_out [B].  Candidates whose layout failed (status != 0) and fields
+ * without obstacles (or a batch without obstacle tables) get zeros. */
+int fcpp_obstacle_sweep(fcpp_handle *h, const fcpp_batch *batch, fcpp_sweep *d_out, void *stream);
+
+/* The sweep of caller-supplied paths (ragged batch, path p = points d_offsets[p] .. d_offsets[p+1]) against ONE
+ * obstacle set (polygon q = vertices d_obs_vert_start[q] .. [q+1] of d_obs_verts [NV][2]).  d_n_main [n_paths] (or
+ * NULL: the whole path is main work) splits path p into main_work (its first n_main points) and headland.  d_out
+ * [n_paths]. */
+int fcpp_obstacle_sweep_paths(fcpp_handle *h, const double *d_path_xy, const int64_t *d_offsets, int64_t n_paths,
+                              const int32_t *d_n_main, const int32_t *d_obs_vert_start, const double *d_obs_verts,
+                              int32_t n_polys, double radius, fcpp_sweep *d_out, void *stream);
+
 /* Generic A10 window raster (mlp3:1426-1510): ORs the W/2 round buffer of a polyline into a
  * g x g lattice-point window (bit (j*g+i) of d_bits, row-major, 32-bit words, ceil(g*g/32) words,
  * caller-zeroed or carrying an earlier cover) and writes the number of set bits to d_count. */
