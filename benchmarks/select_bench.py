@@ -8,8 +8,9 @@ Per workload, one JSON line:
   step_ms          device time of one step (layout .. coverage + argmin or selection, inputs and buffers resident),
                    CUDA events over --steps steps; the two arms alternate --rounds times, the median is reported
   e2e_plans_s      plans/s through plan_batch(..., winners=True) with two calls in flight (wait=False), alternating
-  kernel_us        the selection kernels alone over the step's resident summaries (k = 1 and k = 8), and today's
-                   argmin for comparison, CUDA events over 200 calls each
+  kernel_us        fcpp_field_select alone over the step's resident summaries, CUDA events over 200 calls each:
+                   "argmin" = Selection() (a plain selection: the argmin kernels), "select_k1" = its twin with a
+                   limit no candidate reaches (the ranking pipeline at k = 1), "select_k8" = the selection above
   gpu, power_limit_w   read in the same run
 """
 from __future__ import annotations
@@ -137,10 +138,9 @@ def main():
             return lambda: h.check(h.lib.fcpp_field_select(h.h, bufs.d_sum.data_ptr(), cf, B, F, C.byref(sc), 0,
                                                            d_tk.data_ptr(), d_tk.data_ptr() + 8 * F * s.top_k, sptr))
 
-        def argmin_fn():
-            h.check(h.lib.fcpp_field_argmin(h.h, bufs.d_sum.data_ptr(), cf, B, F, 0, 0, bufs.d_cost.data_ptr(),
-                                             bufs.d_best.data_ptr(), sptr))
-        kern = {"argmin": kernel_us(argmin_fn), "select_k1": kernel_us(select_fn(fc.Selection())),
+        argmin_fn = select_fn(fc.Selection())
+        kern = {"argmin": kernel_us(argmin_fn),
+                "select_k1": kernel_us(select_fn(fc.Selection(max_accel_viol=2**31 - 1))),
                 "select_k8": kernel_us(select_fn(sel))}
         l0 = h.launches
         select_fn(sel)()

@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # FCPP_LIB selects another build of the same library (A/B timing of kernel variants); there is still
 # no fallback: the file must exist and export the ABI
 LIB_PATH = os.environ.get("FCPP_LIB") or os.path.join(_HERE, "libfcpp.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 FLAG_CORNER_MASK = 3
 FLAG_REVERSE_ORDER = 4
@@ -145,7 +145,7 @@ assert SWEEP_DTYPE.itemsize == 24, SWEEP_DTYPE.itemsize
 
 EXPORTS = [
     "fcpp_abi_version", "fcpp_create", "fcpp_destroy", "fcpp_last_error", "fcpp_set_trig_tables",
-    "fcpp_layout", "fcpp_plan_batch", "fcpp_obstacle_sweep", "fcpp_obstacle_sweep_paths", "fcpp_field_argmin", "fcpp_field_argmin_merge", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
+    "fcpp_layout", "fcpp_plan_batch", "fcpp_obstacle_sweep", "fcpp_obstacle_sweep_paths", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
     "fcpp_tour_lengths", "fcpp_distance_matrix", "fcpp_connection_matrix", "fcpp_ga_init_population", "fcpp_ga_next_size", "fcpp_ga_generation", "fcpp_ga_solve", "fcpp_kmeans_lloyd", "fcpp_tsp_two_opt",
     "fcpp_launch_count", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
 ]
@@ -188,10 +188,6 @@ def load():
         L.fcpp_obstacle_sweep.argtypes = [vp, C.POINTER(Batch), vp, vp]
         L.fcpp_obstacle_sweep_paths.restype = C.c_int
         L.fcpp_obstacle_sweep_paths.argtypes = [vp, vp, vp, i64, vp, vp, vp, i32, dbl, vp, vp]
-        L.fcpp_field_argmin.restype = C.c_int
-        L.fcpp_field_argmin.argtypes = [vp, vp, vp, i64, i32, C.c_int, i64, vp, vp, vp]
-        L.fcpp_field_argmin_merge.restype = C.c_int
-        L.fcpp_field_argmin_merge.argtypes = [vp, vp, i32, i32, vp, vp, vp]
         L.fcpp_field_select.restype = C.c_int
         L.fcpp_field_select.argtypes = [vp, vp, vp, i64, i32, C.POINTER(SelectionC), i64, vp, vp, vp]
         L.fcpp_field_select_merge.restype = C.c_int

@@ -532,13 +532,8 @@ class BatchBuffers:
         self.dev = dev
         self.n_cand, self.n_fields, self.total_points = n_cand, n_fields, total_points
         self.d_sum = torch.empty(max(n_cand, 1) * _lib.SUMMARY_DTYPE.itemsize, dtype=torch.uint8, device=dev)
-        # cost and candidate back to back in ONE allocation: the multi-GPU merge all-gathers both at once
-        nf = max(n_fields, 1)
-        self.d_cb = torch.empty(2 * nf, dtype=torch.int64, device=dev)
-        self.d_cost = self.d_cb[:nf].view(torch.float64)
-        self.d_best = self.d_cb[nf:]
-        self.top_k = 0               # > 0: the batch is ranked by fcpp_field_select into d_tk (use_top_k)
-        self.d_tk = self.d_tk_cost = self.d_tk_cand = None
+        self.d_cost = self.d_best = None
+        self.rank_k(1)
         self.d_off = self.d_path = self.d_spd = self.d_kap = None
         self.d_sweep = None          # [B] fcpp_sweep records of the last batch run with obstacle_sweep=True
         self.speculative = False     # sized from remembered maxima (_Hints), not from this batch's layout pass
@@ -552,16 +547,14 @@ class BatchBuffers:
                 if want_curvature:
                     self.d_kap = torch.empty(total_points, dtype=torch.float64, device=dev)
 
-
-    def use_top_k(self, k: int):
-        """k > 0: this batch's ranking goes to d_tk = costs [F, k] (double bits) then candidates [F, k], back to back
-        in ONE allocation (the multi-GPU merge all-gathers both at once); k = 0: the per-field argmin."""
-        self.top_k = int(k)
-        nfk = max(self.n_fields, 1) * self.top_k
-        if self.top_k and (self.d_tk is None or self.d_tk.numel() != 2 * nfk):
-            self.d_tk = torch.empty(2 * nfk, dtype=torch.int64, device=self.dev)
-            self.d_tk_cost = self.d_tk[:nfk].view(torch.float64)
-            self.d_tk_cand = self.d_tk[nfk:]
+    def rank_k(self, k: int):
+        """Size the per-field ranking for k entries per field: ``d_cost`` [F, k] (flat) then ``d_best`` [F, k] (global
+        candidate indices), back to back in ONE allocation (the multi-GPU merge all-gathers both at once); at k = 1
+        they are the per-field best.  Reallocated only when k changes."""
+        nfk = max(self.n_fields, 1) * int(k)
+        if self.d_cost is None or self.d_cost.numel() != nfk:
+            ranking = torch.empty(2 * nfk, dtype=torch.int64, device=self.dev)
+            self.d_cost, self.d_best = ranking[:nfk].view(torch.float64), ranking[nfk:]
 
 
 def corner_grids(words: np.ndarray, g: int) -> np.ndarray:
@@ -608,16 +601,17 @@ class _Hints:
         cls._c.pop(key, None)
 
 
-def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, cost: str, cand_base: int,
+def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, selection: Selection, cand_base: int,
                          buffers: Optional["BatchBuffers"], path_alloc=None, corner_bits: bool = False,
-                         speculate: bool = False, select: Optional[Selection] = None, sweep: bool = False):
-    """Enqueue layout, prefix sum, plan, coverage and argmin kernels of one batch on torch's current
+                         speculate: bool = False, sweep: bool = False):
+    """Enqueue layout, prefix sum, plan, coverage and ranking kernels of one batch on torch's current
     stream.  Returns (buffers, offsets or None).  Without ``buffers`` the path storage is sized from
     the layout pass (one small synchronous read-back) — or, with ``speculate`` and a batch of this shape seen
     before, from the remembered sizes with no synchronisation at all (``buffers.speculative`` is then True and the
     caller must check the status flags, see ``_Hints``); ``path_alloc(total) -> BatchBuffers | None`` lets the
-    caller provide the storage.  ``select``: the per-field top-k of fcpp_field_select instead of the argmin.
-    ``sweep``: also the segment-level obstacle sweep of every candidate (fcpp_obstacle_sweep) into buffers.d_sweep."""
+    caller provide the storage.  ``selection``: how fcpp_field_select ranks each field's candidates into
+    buffers.d_cost / d_best.  ``sweep``: also the segment-level obstacle sweep of every candidate
+    (fcpp_obstacle_sweep) into buffers.d_sweep."""
     if outputs not in ("summary", "paths"):
         raise ValueError("outputs must be 'summary' or 'paths'")
     dev = db.dev
@@ -691,16 +685,11 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, co
             if hint_key is not None:
                 _Hints.update(hint_key, db.max_points, db.max_head_points, buffers.total_points)
         cf = db.t.get("cand_field")     # factored sets: the library's candidate records carry the field
-        buffers.use_top_k(select.top_k if select is not None else 0)
-        if select is None:
-            h.check(L.fcpp_field_argmin(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B,
-                                        F, 0 if cost == "length" else 1, cand_base, buffers.d_cost.data_ptr(),
-                                        buffers.d_best.data_ptr(), stream))
-        else:
-            sc = select.c_struct(db.pb.grid_h)
-            h.check(L.fcpp_field_select(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B,
-                                        F, C.byref(sc), cand_base, buffers.d_tk_cost.data_ptr(),
-                                        buffers.d_tk_cand.data_ptr(), stream))
+        buffers.rank_k(selection.top_k)
+        sc = selection.c_struct(db.pb.grid_h)
+        h.check(L.fcpp_field_select(h.h, buffers.d_sum.data_ptr(), cf.data_ptr() if cf is not None else None, B, F,
+                                    C.byref(sc), cand_base, buffers.d_cost.data_ptr(), buffers.d_best.data_ptr(),
+                                    stream))
     return buffers, offsets
 
 
@@ -711,20 +700,19 @@ class _PendingFetch:
 
 def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
                    cand_base: int, win: Optional[torch.Tensor] = None, sweep: bool = False) -> _PendingFetch:
-    """Enqueue the copies of summaries + argmin or top-k ranking (+ offsets) (+ ``win``: the winners' records and
+    """Enqueue the copies of summaries + the per-field ranking (+ offsets) (+ ``win``: the winners' records and
     flag-count word of a sharded batch, see dist.gather_winner_records) (+ ``sweep``: the obstacle sweep records)
     into ONE pooled pinned buffer on torch's current stream and record an event behind them; nothing is waited for."""
     dev = db.dev
     B, F = db.pb.n_cand, db.pb.n_fields
-    nk = buffers.top_k or 1             # entries per field: the argmin's 1 or the ranking's k
-    d_cost, d_best = (buffers.d_tk_cost, buffers.d_tk_cand) if buffers.top_k else (buffers.d_cost, buffers.d_best)
+    k = buffers.d_cost.numel() // max(F, 1)     # entries per field of the ranking
     pf = _PendingFetch()
     with torch.cuda.device(dev):
         nb_sum = B * _lib.SUMMARY_DTYPE.itemsize if copy_summary else 0
         need_off = outputs == "paths" and offsets is None
         o_cost = (nb_sum + 255) & ~255
-        o_best = o_cost + ((F * nk * 8 + 255) & ~255)
-        o_off = o_best + ((F * nk * 8 + 255) & ~255)
+        o_best = o_cost + ((F * k * 8 + 255) & ~255)
+        o_off = o_best + ((F * k * 8 + 255) & ~255)
         total_out = o_off + ((B + 1) * 8 if need_off else 0)
         o_win = (total_out + 255) & ~255
         if win is not None:
@@ -750,8 +738,8 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
             if nb_sum:
                 ho[:nb_sum].copy_(buffers.d_sum[:nb_sum], non_blocking=True)
             if F:
-                ho[o_cost:o_cost + F * nk * 8].view(torch.float64).copy_(d_cost[:F * nk], non_blocking=True)
-                ho[o_best:o_best + F * nk * 8].view(torch.int64).copy_(d_best[:F * nk], non_blocking=True)
+                ho[o_cost:o_cost + F * k * 8].view(torch.float64).copy_(buffers.d_cost[:F * k], non_blocking=True)
+                ho[o_best:o_best + F * k * 8].view(torch.int64).copy_(buffers.d_best[:F * k], non_blocking=True)
             if need_off:
                 ho[o_off:o_off + (B + 1) * 8].view(torch.int64).copy_(buffers.d_off[:B + 1], non_blocking=True)
             if win is not None:
@@ -761,33 +749,31 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
             pf.event = torch.cuda.Event()
             pf.event.record(cs)
     pf.db, pf.buffers, pf.outputs, pf.offsets, pf.cand_base = db, buffers, outputs, offsets, cand_base
-    pf.hv, pf.lay = hv, (nb_sum, need_off, o_cost, o_best, o_off)
+    pf.hv, pf.lay = hv, (nb_sum, need_off, o_cost, o_best, o_off, k)
     pf.win, pf.hwin = win, (hv[o_win:o_win + win.numel()] if win is not None else None)
     pf.o_sweep = (o_sweep, B) if sweep else None
     return pf
 
 
-def _finish_fetch(pf: _PendingFetch) -> "BatchResult":
+def _finish_fetch(pf: _PendingFetch, ranked: bool) -> "BatchResult":
     """Wait for the read-back of ``_enqueue_fetch`` (ONE synchronisation, on its event) and assemble the result:
-    its arrays are views of the read-back's own pooled buffer."""
+    its arrays are views of the read-back's own pooled buffer.  ``ranked``: the caller asked for the ranking
+    (``topk_cand`` / ``topk_cost``); ``best_cand`` / ``best_cost`` are its first column either way."""
     db, buffers, offsets, hv = pf.db, pf.buffers, pf.offsets, pf.hv
     B, F = db.pb.n_cand, db.pb.n_fields
-    nb_sum, need_off, o_cost, o_best, o_off = pf.lay
-    k = buffers.top_k
-    nk = k or 1
+    nb_sum, need_off, o_cost, o_best, o_off, k = pf.lay
     pf.event.synchronize()
     summary = hv[:nb_sum].view(_lib.SUMMARY_DTYPE)[:B] if nb_sum else np.zeros(0, dtype=_lib.SUMMARY_DTYPE)
-    best_cost = hv[o_cost:o_cost + F * nk * 8].view(np.float64)
-    best_cand = hv[o_best:o_best + F * nk * 8].view(np.int64)
-    topk_cost = topk_cand = None
-    if k:
-        topk_cost, topk_cand = best_cost.reshape(F, k), best_cand.reshape(F, k)
-        best_cost, best_cand = np.ascontiguousarray(topk_cost[:, 0]), np.ascontiguousarray(topk_cand[:, 0])
+    topk_cost = hv[o_cost:o_cost + F * k * 8].view(np.float64).reshape(F, k)
+    topk_cand = hv[o_best:o_best + F * k * 8].view(np.int64).reshape(F, k)
     if need_off:
         offsets = hv[o_off:o_off + (B + 1) * 8].view(np.int64)
-    res = BatchResult(summary=summary, best_cand=best_cand, best_cost=best_cost, n_fields=F, offsets=offsets,
+    res = BatchResult(summary=summary, best_cand=np.ascontiguousarray(topk_cand[:, 0]),
+                      best_cost=np.ascontiguousarray(topk_cost[:, 0]), n_fields=F, offsets=offsets,
                       d_path=buffers.d_path, d_speeds=buffers.d_spd, d_curvature=buffers.d_kap,
-                      d_summary=buffers.d_sum, cand_base=pf.cand_base, topk_cand=topk_cand, topk_cost=topk_cost)
+                      d_summary=buffers.d_sum, cand_base=pf.cand_base)
+    if ranked:
+        res.topk_cand, res.topk_cost = topk_cand, topk_cost
     if pf.o_sweep is not None:
         o, n = pf.o_sweep
         res.sweep = hv[o:o + n * _lib.SWEEP_DTYPE.itemsize].view(_lib.SWEEP_DTYPE)
@@ -912,10 +898,10 @@ class PendingBatch:
     ``result()`` is COLLECTIVE in one case only: when some rank's remembered launch sizes did not fit its shard,
     all ranks repeat the batch together."""
 
-    def __init__(self, db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                 speculate, shard, select=None, sweep=False):
+    def __init__(self, db, pf, outputs, want_curvature, selection, ranked, cand_base, copy_summary, winners,
+                 corner_bits, speculate, shard, sweep=False):
         self.db, self.pf, self.outputs = db, pf, outputs
-        self.args = (want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select, sweep)
+        self.args = (want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep)
         self.speculate, self.shard = speculate, shard
         self._res = None
 
@@ -932,42 +918,41 @@ class PendingBatch:
         if self._res is not None:
             return self._res
         db, pf, outputs = self.db, self.pf, self.outputs
-        want_curvature, cost, cand_base, copy_summary, winners, corner_bits, select, sweep = self.args
+        want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep = self.args
         buffers = pf.buffers
         B, F = db.pb.n_cand, db.pb.n_fields
-        k = select.top_k if select is not None else 0
-        nk = k or 1
+        k = selection.top_k
         rec = _lib.SUMMARY_DTYPE.itemsize
-        res = _finish_fetch(pf)
+        res = _finish_fetch(pf, ranked)
         if self.shard is None:
             redo = buffers.speculative and (not copy_summary or (res.summary["status"] & _SIZE_FLAGS).any())
         else:
             # the number of flagged candidates OF ALL RANKS: every rank reads the same word and decides alike, also
             # a rank that had no remembered sizes itself
-            redo = self.speculate and int(pf.hwin[F * nk * rec:F * nk * rec + 4].view(np.int32)[0]) != 0
+            redo = self.speculate and int(pf.hwin[F * k * rec:F * k * rec + 4].view(np.int32)[0]) != 0
         if redo:
             # remembered sizes (see _Hints) did not fit this batch, or cannot be checked: once more, sized from its
             # own layout pass.  (A batch with candidates that are genuinely too large takes this path too and comes
             # back with the same flags.)
             _Hints.drop(_Hints.key(db, outputs, want_curvature))
-            self._res = run_device_batch(db, outputs, want_curvature, cost, cand_base, copy_summary, None, True,
-                                         winners, corner_bits, speculate=False, shard=self.shard, select=select,
-                                         obstacle_sweep=sweep)
+            self._res = _run_device_batch(db, outputs, want_curvature, selection, ranked, cand_base, copy_summary,
+                                          buffers=None, fetch=True, winners=winners, corner_bits=corner_bits,
+                                          speculate=False, wait=True, shard=self.shard, obstacle_sweep=sweep)
             return self._res
         if corner_bits:   # [B, stride] words on the device; batch.corner_grids() unpacks one candidate's
             res.extras["corner_bits"] = buffers.d_cbits[:B * buffers.cbits_stride].view(B, -1)
         res.extras["h2d_bytes"] = db.pb.h2d_bytes()
-        res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F * nk + ((B + 1) * 8 if outputs == "paths" else 0)
+        res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F * k + ((B + 1) * 8 if outputs == "paths" else 0)
         if sweep:
             res.extras["d2h_bytes"] += B * _lib.SWEEP_DTYPE.itemsize
         if self.shard is not None:
-            records = pf.hwin[:F * nk * rec].view(_lib.SUMMARY_DTYPE)
-            res.extras["winner_summary"] = records.reshape(F, k)[:, 0].copy() if k else records
+            records = pf.hwin[:F * k * rec].view(_lib.SUMMARY_DTYPE).reshape(F, k)
+            res.extras["winner_summary"] = records[:, 0].copy()
             res.extras["shard"] = self.shard
-            res.extras["d2h_bytes"] += F * nk * rec + 16
-            if k:
-                res.topk_summary = records.reshape(F, k)
-        elif k and len(res.summary) == B:
+            res.extras["d2h_bytes"] += F * k * rec + 16
+            if ranked:
+                res.topk_summary = records
+        elif ranked and len(res.summary) == B:
             res.topk_summary = np.zeros((F, k), dtype=_lib.SUMMARY_DTYPE)
             own = res.topk_cand >= 0
             res.topk_summary[own] = res.summary[res.topk_cand[own] - cand_base]
@@ -985,39 +970,49 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
                      buffers: Optional[BatchBuffers] = None, fetch: bool = True,
                      winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True,
                      shard: Optional[tuple] = None, select: Optional[Selection] = None, obstacle_sweep: bool = False):
-    """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + argmin back.
+    """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + the per-field best back.
 
     With ``buffers`` (from a previous run of the same batch shape) and ``db.max_points`` known the
-    whole step is asynchronous: layout, prefix sum, plan, coverage and argmin kernels only.
+    whole step is asynchronous: layout, prefix sum, plan, coverage and ranking kernels only.
     ``winners``: also bring every field's winning path and speeds to the host (``fetch_winner_paths``).
     ``speculate``: size the launch from remembered batches of the same shape instead of a synchronous layout
     read-back (``_Hints``; checked and repeated when the sizes do not fit).  ``wait=False`` returns a
     ``PendingBatch``.  ``shard=(lo, hi)``: the batch is this rank's candidates [lo, hi) of a batch sharded over the
-    default process group; before the read-back the per-field argmin is merged over the ranks and every field's
-    winning summary record gathered (``dist.reduce_best``, ``dist.gather_winner_records``).  ``select``: the per-field
-    top-k ranking instead of the argmin (merged over the ranks with ``dist.reduce_topk``; the records of every
-    ranked candidate gathered).  ``obstacle_sweep``: also each candidate's segment-level obstacle sweep
-    (``BatchResult.sweep``; in a sharded batch, of this rank's candidates)."""
-    buffers, offsets = _launch_device_batch(db, outputs, want_curvature, cost, cand_base, buffers,
+    default process group; before the read-back the per-field ranking is merged over the ranks and the summary
+    record of every ranked candidate gathered (``dist.reduce_topk``, ``dist.gather_winner_records``).  ``select``:
+    the per-field top-k ranking (``BatchResult.topk_*``) instead of the argmin of ``cost``.  ``obstacle_sweep``: also
+    each candidate's segment-level obstacle sweep (``BatchResult.sweep``; in a sharded batch, of this rank's
+    candidates)."""
+    if select is not None:
+        selection = select
+    else:   # the argmin of the length or of the time: the plain selections (include/fcpp.h)
+        selection = Selection() if cost == "length" else Selection(w_length=0.0, w_time=1.0)
+    return _run_device_batch(db, outputs, want_curvature, selection, select is not None, cand_base, copy_summary,
+                             buffers, fetch, winners, corner_bits, speculate, wait, shard, obstacle_sweep)
+
+
+def _run_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, selection: Selection, ranked: bool,
+                      cand_base: int, copy_summary: bool, buffers: Optional[BatchBuffers], fetch: bool, winners: bool,
+                      corner_bits: bool, speculate: bool, wait: bool, shard: Optional[tuple], obstacle_sweep: bool):
+    """``run_device_batch`` with the ranking resolved: ``selection`` ranks every field, ``ranked`` = the caller asked
+    for the ranking (``BatchResult.topk_*``)."""
+    buffers, offsets = _launch_device_batch(db, outputs, want_curvature, selection, cand_base, buffers,
                                             corner_bits=corner_bits, speculate=speculate and copy_summary,
-                                            select=select, sweep=obstacle_sweep)
+                                            sweep=obstacle_sweep)
     if not fetch:
         return None
     win = None
     if shard is not None:
         from . import dist
-        if select is None:
-            dist.reduce_best(buffers.d_cost, buffers.d_best)       # in place: now the GLOBAL per-field argmin
-            best = buffers.d_best
-        else:
-            nfk = db.pb.n_fields * select.top_k
-            best = buffers.d_tk_cand[:nfk]
-            dist.reduce_topk(buffers.d_tk_cost[:nfk], best, select.top_k)     # in place: the GLOBAL ranking
+        k = selection.top_k
+        nfk = db.pb.n_fields * k
+        dist.reduce_topk(buffers.d_cost[:nfk], buffers.d_best[:nfk], k)     # in place: the GLOBAL ranking
         # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
-        win = dist.gather_winner_records(buffers.d_sum, best, shard[0], shard[1], count_mask=_SIZE_FLAGS)
+        win = dist.gather_winner_records(buffers.d_sum, buffers.d_best[:nfk], shard[0], shard[1],
+                                         count_mask=_SIZE_FLAGS)
     pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win, obstacle_sweep)
-    pend = PendingBatch(db, pf, outputs, want_curvature, cost, cand_base, copy_summary, winners, corner_bits,
-                        speculate and copy_summary, shard, select, obstacle_sweep)
+    pend = PendingBatch(db, pf, outputs, want_curvature, selection, ranked, cand_base, copy_summary, winners,
+                        corner_bits, speculate and copy_summary, shard, obstacle_sweep)
     return pend if not wait else pend.result()
 
 

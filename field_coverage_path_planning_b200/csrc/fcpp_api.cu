@@ -328,35 +328,6 @@ int fcpp_obstacle_sweep_paths(fcpp_handle *h, const double *d_path_xy, const int
     return FCPP_OK;
 }
 
-int fcpp_field_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
-                      int32_t n_fields, int cost_kind, int64_t cand_base, double *d_best_cost,
-                      int64_t *d_best_cand, void *stream)
-{
-    if (!h) return FCPP_ERR_INVALID;
-    if (n_cand < 0 || n_fields < 0 || !d_best_cost || !d_best_cand || (n_cand > 0 && !d_summary))
-        return fail(h, FCPP_ERR_INVALID, "fcpp_field_argmin: bad argument");
-    if (n_cand > 0 && !d_cand_field && (n_cand > h->rec_cap || !h->d_rec))
-        return fail(h, FCPP_ERR_INVALID, "fcpp_field_argmin: no cand_field and no candidate records of this batch");
-    cudaSetDevice(h->device);
-    cudaError_t e = fcpp_launch_argmin(h, d_summary, d_cand_field, n_cand, n_fields, cost_kind, cand_base,
-                                       d_best_cost, d_best_cand, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(h, e, "argmin kernels");
-    return FCPP_OK;
-}
-
-int fcpp_field_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t world, int32_t n_fields,
-                            double *d_best_cost, int64_t *d_best_cand, void *stream)
-{
-    if (!h) return FCPP_ERR_INVALID;
-    if (world < 1 || n_fields < 0 || (n_fields > 0 && (!d_gathered || !d_best_cost || !d_best_cand)))
-        return fail(h, FCPP_ERR_INVALID, "fcpp_field_argmin_merge: bad argument");
-    cudaSetDevice(h->device);
-    cudaError_t e = fcpp_launch_argmin_merge(h, d_gathered, world, n_fields, d_best_cost, d_best_cand,
-                                             (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(h, e, "argmin merge kernel");
-    return FCPP_OK;
-}
-
 int fcpp_field_select(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
                       int32_t n_fields, const fcpp_selection *sel, int64_t cand_base, double *d_cost, int64_t *d_cand,
                       void *stream)

@@ -783,8 +783,6 @@ cudaError_t fcpp_launch_ga_rotate(fcpp_handle *h, const int32_t *d_route, int n,
 size_t fcpp_ga_state_bytes();
 void fcpp_ga_read_state(const void *host_copy, int &gen, int &stagnant, int &done, int &last_gen, double &best_fit,
                         double &best_len);
-cudaError_t fcpp_launch_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int world, int32_t n_fields,
-                                     double *d_best_cost, int64_t *d_best_cand, cudaStream_t st);
 cudaError_t fcpp_launch_winner_records(fcpp_handle *h, const fcpp_summary *d_summary, int64_t lo, int64_t hi,
                                        const int64_t *d_best_cand, int32_t n_fields, void *d_out, cudaStream_t st);
 cudaError_t fcpp_launch_distance_matrix(fcpp_handle *h, const double *d_pos, int32_t n, double *d_D, cudaStream_t st);
@@ -801,6 +799,3 @@ cudaError_t fcpp_launch_sweep(fcpp_handle *h, const fcpp_batch &b, fcpp_sweep *d
 cudaError_t fcpp_launch_sweep_paths(fcpp_handle *h, const double *d_path, const int64_t *d_offsets, int64_t n_paths,
                                     const int32_t *d_n_main, const int32_t *d_vert_start, const double *d_verts,
                                     int32_t n_polys, double radius, fcpp_sweep *d_out, cudaStream_t st);
-cudaError_t fcpp_launch_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
-                               int64_t n_cand, int32_t n_fields, int cost_kind, int64_t cand_base,
-                               double *d_best_cost, int64_t *d_best_cand, cudaStream_t st);

@@ -1,10 +1,9 @@
-// fcpp_misc.cu — batched GA tour-length fitness (A12) and the per-field argmin of plan costs.
+// fcpp_misc.cu — batched GA tour-length fitness (A12), the multi-GPU exchange of the winners' records and the
+// multi-field distance / connection matrices.
 //
 // Reference code replaced:
 //   genetic_algorithm_solver.py:168-181  _calculate_fitness / _calculate_distance
 //   (distance-matrix layout: multi_field_planner.py:263-288, node 0 = depot)
-// The per-field argmin has no reference counterpart (SURVEY.md §8(b): build-defined cost
-// len_main + len_head, ties to the lowest candidate index).
 #include "fcpp_internal.cuh"
 
 namespace {
@@ -53,142 +52,6 @@ __global__ void __launch_bounds__(TOUR_THREADS) tour_kernel(const double *__rest
         out[me] = s;
         if (fit) fit[me] = 1.0 / (s + 1e-6);  // ga:172
     }
-}
-
-__device__ __forceinline__ double cand_cost(const fcpp_summary &s, int kind)
-{
-    return kind == 0 ? s.len_main + s.len_head : s.time_main + s.time_head;
-}
-
-__global__ void argmin_init(unsigned long long *key, int64_t *cand, int n_fields)
-{
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f < n_fields) {
-        key[f] = ~0ull;
-        cand[f] = 0x7fffffffffffffffll;
-    }
-}
-// field of candidate c: the caller's array, or (factored candidate sets) the library's candidate record
-__device__ __forceinline__ int cand_field_of(const int32_t *__restrict__ cf, const CandRec *__restrict__ recs, int64_t c)
-{
-    return cf ? cf[c] : recs[c].field;
-}
-
-__global__ void argmin_cost(const fcpp_summary *__restrict__ sm, const int32_t *__restrict__ cf,
-                            const CandRec *__restrict__ recs, int64_t n, int kind, unsigned long long *key)
-{
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < n && sm[c].status == 0) atomicMin(&key[cand_field_of(cf, recs, c)], order_bits(cand_cost(sm[c], kind)));
-}
-__global__ void argmin_index(const fcpp_summary *__restrict__ sm, const int32_t *__restrict__ cf,
-                             const CandRec *__restrict__ recs, int64_t n, int kind, int64_t base,
-                             const unsigned long long *__restrict__ key, int64_t *cand)
-{
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n || sm[c].status != 0) return;
-    const int f = cand_field_of(cf, recs, c);
-    if (order_bits(cand_cost(sm[c], kind)) == key[f]) atomicMin((long long *)&cand[f], (long long)(base + c));
-}
-__global__ void argmin_final(unsigned long long *key, int64_t *cand, int n_fields)
-{
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f < n_fields) {
-        const unsigned long long k = key[f];
-        double *out = reinterpret_cast<double *>(key);
-        if (k == ~0ull) {
-            out[f] = INFINITY;
-            cand[f] = -1;
-        } else {
-            out[f] = unorder_bits(k);
-        }
-    }
-}
-
-// atomicMin(&table[f], v) for the active lanes of a warp (all 32 lanes call it): one atomic per warp when its active
-// lanes share the field, else one per lane.  Values are unsigned-ordered (candidate indices are >= 0).
-__device__ __forceinline__ void warp_field_min(unsigned long long *table, int f, unsigned long long v, bool active)
-{
-    const unsigned m = __ballot_sync(0xffffffffu, active);
-    if (m == 0) return;
-    const int f0 = __shfl_sync(0xffffffffu, f, __ffs(m) - 1);
-    if (__all_sync(0xffffffffu, !active || f == f0)) {
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d);
-            v = o < v ? o : v;
-        }
-        if ((threadIdx.x & 31) == 0) atomicMin(&table[f0], v);
-    } else if (active) {
-        atomicMin(&table[f], v);
-    }
-}
-
-// the four phases in ONE CTA (small batches: four dependent launches cost more than the work)
-constexpr int ARGMIN_SMALL_THREADS = 1024;
-__global__ void __launch_bounds__(ARGMIN_SMALL_THREADS) argmin_small(const fcpp_summary *__restrict__ sm,
-                                                                      const int32_t *__restrict__ cf,
-                                                                      const CandRec *__restrict__ recs, int64_t n, int kind,
-                                                                      int64_t base, unsigned long long *key, int64_t *cand,
-                                                                      int n_fields)
-{
-    for (int f = threadIdx.x; f < n_fields; f += ARGMIN_SMALL_THREADS) {
-        key[f] = ~0ull;
-        cand[f] = 0x7fffffffffffffffll;
-    }
-    __threadfence();
-    __syncthreads();
-    // candidates of one field are contiguous (field-major order), so a warp usually holds ONE field: its minimum is
-    // reduced by shuffles and costs one atomic instead of 32 on the same address (config 2: 4096 candidates, 1 field)
-    for (int64_t c0 = 0; c0 < n; c0 += ARGMIN_SMALL_THREADS) {
-        const int64_t c = c0 + threadIdx.x;
-        const bool on = c < n && sm[c].status == 0;
-        const int f = on ? cand_field_of(cf, recs, c) : -1;
-        warp_field_min(key, f, on ? order_bits(cand_cost(sm[c], kind)) : ~0ull, on);
-    }
-    __threadfence();
-    __syncthreads();
-    for (int64_t c0 = 0; c0 < n; c0 += ARGMIN_SMALL_THREADS) {
-        const int64_t c = c0 + threadIdx.x;
-        bool on = c < n && sm[c].status == 0;
-        const int f = on ? cand_field_of(cf, recs, c) : -1;
-        on = on && order_bits(cand_cost(sm[c], kind)) == __ldcg(&key[f]);
-        warp_field_min(reinterpret_cast<unsigned long long *>(cand), on ? f : -1,
-                       on ? (unsigned long long)(base + c) : ~0ull, on);
-    }
-    __threadfence();
-    __syncthreads();
-    for (int f = threadIdx.x; f < n_fields; f += ARGMIN_SMALL_THREADS) {
-        const unsigned long long k = __ldcg(&key[f]);
-        double *out = reinterpret_cast<double *>(key);
-        if (k == ~0ull) {
-            out[f] = INFINITY;
-            cand[f] = -1;
-        } else {
-            out[f] = unorder_bits(k);
-        }
-    }
-}
-
-// multi-GPU: per-field merge of the ranks' local bests after ONE all-gather of (cost, candidate)
-// words; lowest cost wins, ties go to the lowest global candidate index, -1 = no candidate
-__global__ void argmin_merge_kernel(const long long *__restrict__ g, int world, int n_fields,
-                                    double *__restrict__ best_cost, long long *__restrict__ best_cand)
-{
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f >= n_fields) return;
-    double bc = INFINITY;
-    long long bi = -1;
-    for (int r = 0; r < world; ++r) {
-        const long long *row = g + (int64_t)r * 2 * n_fields;
-        const double c = __longlong_as_double(row[f]);
-        const long long i = row[n_fields + f];
-        if (i >= 0 && (bi < 0 || c < bc || (c == bc && i < bi))) {
-            bc = c;
-            bi = i;
-        }
-    }
-    best_cost[f] = bc;
-    best_cand[f] = bi;
 }
 
 // multi-GPU: this rank's contribution to the all-gather of the winners' summary records — the 176-byte record of
@@ -249,16 +112,6 @@ __global__ void connection_matrix_kernel(const double *__restrict__ verts, int n
 
 }  // namespace
 
-cudaError_t fcpp_launch_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int world, int32_t n_fields,
-                                     double *d_best_cost, int64_t *d_best_cand, cudaStream_t st)
-{
-    if (n_fields == 0) return cudaSuccess;
-    argmin_merge_kernel<<<(n_fields + 255) / 256, 256, 0, st>>>((const long long *)d_gathered, world, n_fields,
-                                                                d_best_cost, (long long *)d_best_cand);
-    h->launches++;
-    return cudaGetLastError();
-}
-
 // number of candidates whose status has one of the bits of `mask`
 __global__ void status_count_kernel(const fcpp_summary *__restrict__ sm, int64_t n, int mask, int32_t *__restrict__ count)
 {
@@ -316,33 +169,6 @@ cudaError_t fcpp_launch_tours(fcpp_handle *h, const double *d_D, int32_t n, cons
     if (pop_size == 0) return cudaSuccess;
     const unsigned blocks = (unsigned)((pop_size + TOUR_THREADS - 1) / TOUR_THREADS);
     tour_kernel<<<blocks, TOUR_THREADS, 0, st>>>(d_D, n, d_pop, pop_size, d_out, d_fit);
-    h->launches++;
-    return cudaGetLastError();
-}
-
-cudaError_t fcpp_launch_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
-                               int64_t n_cand, int32_t n_fields, int cost_kind, int64_t cand_base,
-                               double *d_best_cost, int64_t *d_best_cand, cudaStream_t st)
-{
-    if (n_fields == 0) return cudaSuccess;
-    unsigned long long *key = reinterpret_cast<unsigned long long *>(d_best_cost);
-    if (n_cand <= 16384 && n_fields <= 16384) {
-        argmin_small<<<1, ARGMIN_SMALL_THREADS, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, cost_kind, cand_base,
-                                                           key, d_best_cand, n_fields);
-        h->launches++;
-        return cudaGetLastError();
-    }
-    const int th = 256;
-    const unsigned fb = (unsigned)((n_fields + th - 1) / th);
-    argmin_init<<<fb, th, 0, st>>>(key, d_best_cand, n_fields);
-    h->launches++;
-    if (n_cand > 0) {
-        const unsigned cb = (unsigned)((n_cand + th - 1) / th);
-        argmin_cost<<<cb, th, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, cost_kind, key);
-        argmin_index<<<cb, th, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, cost_kind, cand_base, key, d_best_cand);
-        h->launches += 2;
-    }
-    argmin_final<<<fb, th, 0, st>>>(key, d_best_cand, n_fields);
     h->launches++;
     return cudaGetLastError();
 }

@@ -1,6 +1,10 @@
 // fcpp_select.cu — per-field top-k of the candidates under a constraint-aware cost (fcpp_field_select) and the
 // multi-GPU merge of the ranks' rankings (fcpp_field_select_merge).  No reference counterpart: build-defined
-// selection on top of the per-candidate summaries (DESIGN.md §3.8).
+// selection on top of the per-candidate summaries (DESIGN.md §3.8; SURVEY.md §8(b): ties to the lowest index).
+//
+// A PLAIN selection (top_k 1, no limit, the weights of length alone or time alone) is the per-field argmin and runs
+// the argmin kernels: one CTA up to 16 384 candidates and fields, else four kernels — one launch where the pipeline
+// below takes five.  Every other selection runs the pipeline.
 //
 // Pipeline (every stage exact, the order of the results independent of the order of the candidates):
 //   1. select_keys      1 thread / candidate: eligibility, FP64 cost, key = order_bits(cost); the candidate's rank
@@ -374,6 +378,189 @@ __global__ void __launch_bounds__(256) select_merge_kernel(const long long *__re
     }
 }
 
+// ---- per-field argmin: the plain selections (cost kind 0: len_main + len_head, 1: time_main + time_head).  As in
+// select_keys, a candidate whose field lies outside [0, n_fields) is skipped ----
+__device__ __forceinline__ double cand_cost(const fcpp_summary &s, int kind)
+{
+    return kind == 0 ? s.len_main + s.len_head : s.time_main + s.time_head;
+}
+
+__global__ void argmin_init(unsigned long long *key, int64_t *cand, int n_fields)
+{
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f < n_fields) {
+        key[f] = ~0ull;
+        cand[f] = 0x7fffffffffffffffll;
+    }
+}
+// field of candidate c: the caller's array, or (factored candidate sets) the library's candidate record
+__device__ __forceinline__ int cand_field_of(const int32_t *__restrict__ cf, const CandRec *__restrict__ recs, int64_t c)
+{
+    return cf ? cf[c] : recs[c].field;
+}
+
+__global__ void argmin_cost(const fcpp_summary *__restrict__ sm, const int32_t *__restrict__ cf,
+                            const CandRec *__restrict__ recs, int64_t n, int n_fields, int kind, unsigned long long *key)
+{
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n || sm[c].status != 0) return;
+    const int f = cand_field_of(cf, recs, c);
+    if (f >= 0 && f < n_fields) atomicMin(&key[f], order_bits(cand_cost(sm[c], kind)));
+}
+__global__ void argmin_index(const fcpp_summary *__restrict__ sm, const int32_t *__restrict__ cf,
+                             const CandRec *__restrict__ recs, int64_t n, int n_fields, int kind, int64_t base,
+                             const unsigned long long *__restrict__ key, int64_t *cand)
+{
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n || sm[c].status != 0) return;
+    const int f = cand_field_of(cf, recs, c);
+    if (f >= 0 && f < n_fields && order_bits(cand_cost(sm[c], kind)) == key[f])
+        atomicMin((long long *)&cand[f], (long long)(base + c));
+}
+__global__ void argmin_final(unsigned long long *key, int64_t *cand, int n_fields)
+{
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f < n_fields) {
+        const unsigned long long k = key[f];
+        double *out = reinterpret_cast<double *>(key);
+        if (k == ~0ull) {
+            out[f] = INFINITY;
+            cand[f] = -1;
+        } else {
+            out[f] = unorder_bits(k);
+        }
+    }
+}
+
+// atomicMin(&table[f], v) for the active lanes of a warp (all 32 lanes call it): one atomic per warp when its active
+// lanes share the field, else one per lane.  Values are unsigned-ordered (candidate indices are >= 0).
+__device__ __forceinline__ void warp_field_min(unsigned long long *table, int f, unsigned long long v, bool active)
+{
+    const unsigned m = __ballot_sync(0xffffffffu, active);
+    if (m == 0) return;
+    const int f0 = __shfl_sync(0xffffffffu, f, __ffs(m) - 1);
+    if (__all_sync(0xffffffffu, !active || f == f0)) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d);
+            v = o < v ? o : v;
+        }
+        if ((threadIdx.x & 31) == 0) atomicMin(&table[f0], v);
+    } else if (active) {
+        atomicMin(&table[f], v);
+    }
+}
+
+// the four phases in ONE CTA (small batches: four dependent launches cost more than the work)
+constexpr int ARGMIN_SMALL_THREADS = 1024;
+constexpr int ARGMIN_SMALL_MAX = 16384;  // candidates and fields
+__global__ void __launch_bounds__(ARGMIN_SMALL_THREADS) argmin_small(const fcpp_summary *__restrict__ sm,
+                                                                      const int32_t *__restrict__ cf,
+                                                                      const CandRec *__restrict__ recs, int64_t n, int kind,
+                                                                      int64_t base, unsigned long long *key, int64_t *cand,
+                                                                      int n_fields)
+{
+    for (int f = threadIdx.x; f < n_fields; f += ARGMIN_SMALL_THREADS) {
+        key[f] = ~0ull;
+        cand[f] = 0x7fffffffffffffffll;
+    }
+    __threadfence();
+    __syncthreads();
+    // candidates of one field are contiguous (field-major order), so a warp usually holds ONE field: its minimum is
+    // reduced by shuffles and costs one atomic instead of 32 on the same address (config 2: 4096 candidates, 1 field)
+    for (int64_t c0 = 0; c0 < n; c0 += ARGMIN_SMALL_THREADS) {
+        const int64_t c = c0 + threadIdx.x;
+        bool on = c < n && sm[c].status == 0;
+        const int f = on ? cand_field_of(cf, recs, c) : -1;
+        on = on && f >= 0 && f < n_fields;
+        warp_field_min(key, f, on ? order_bits(cand_cost(sm[c], kind)) : ~0ull, on);
+    }
+    __threadfence();
+    __syncthreads();
+    for (int64_t c0 = 0; c0 < n; c0 += ARGMIN_SMALL_THREADS) {
+        const int64_t c = c0 + threadIdx.x;
+        bool on = c < n && sm[c].status == 0;
+        const int f = on ? cand_field_of(cf, recs, c) : -1;
+        on = on && f >= 0 && f < n_fields && order_bits(cand_cost(sm[c], kind)) == __ldcg(&key[f]);
+        warp_field_min(reinterpret_cast<unsigned long long *>(cand), on ? f : -1,
+                       on ? (unsigned long long)(base + c) : ~0ull, on);
+    }
+    __threadfence();
+    __syncthreads();
+    for (int f = threadIdx.x; f < n_fields; f += ARGMIN_SMALL_THREADS) {
+        const unsigned long long k = __ldcg(&key[f]);
+        double *out = reinterpret_cast<double *>(key);
+        if (k == ~0ull) {
+            out[f] = INFINITY;
+            cand[f] = -1;
+        } else {
+            out[f] = unorder_bits(k);
+        }
+    }
+}
+
+// multi-GPU merge at k = 1: one thread per field over the ranks' (cost, candidate) words (layout of
+// select_merge_kernel); lowest cost wins, ties go to the lowest global candidate index, -1 = no candidate.  Kept next
+// to select_merge_kernel because it is faster for few fields (DESIGN.md §3.8)
+__global__ void argmin_merge_kernel(const long long *__restrict__ g, int world, int n_fields,
+                                    double *__restrict__ best_cost, long long *__restrict__ best_cand)
+{
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_fields) return;
+    double bc = INFINITY;
+    long long bi = -1;
+    for (int r = 0; r < world; ++r) {
+        const long long *row = g + (int64_t)r * 2 * n_fields;
+        const double c = __longlong_as_double(row[f]);
+        const long long i = row[n_fields + f];
+        if (i >= 0 && (bi < 0 || c < bc || (c == bc && i < bi))) {
+            bc = c;
+            bi = i;
+        }
+    }
+    best_cost[f] = bc;
+    best_cand[f] = bi;
+}
+
+// the cost kind of a plain selection (include/fcpp.h: its cost is L or T, bit for bit), -1 for any other
+int plain_cost_kind(const fcpp_selection &s)
+{
+    if (s.top_k != 1 || s.max_boundary_viol >= 0 || s.max_obstacle_viol >= 0 || s.max_accel_viol >= 0 ||
+        s.min_coverage >= 0.0 || s.w_boundary != 0.0 || s.w_obstacle != 0.0 || s.w_accel != 0.0 ||
+        s.w_uncovered != 0.0)
+        return -1;
+    if (s.w_length == 1.0 && s.w_time == 0.0) return 0;
+    if (s.w_length == 0.0 && s.w_time == 1.0) return 1;
+    return -1;
+}
+
+cudaError_t launch_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
+                          int32_t n_fields, int cost_kind, int64_t cand_base, double *d_best_cost,
+                          int64_t *d_best_cand, cudaStream_t st)
+{
+    unsigned long long *key = reinterpret_cast<unsigned long long *>(d_best_cost);
+    if (n_cand <= ARGMIN_SMALL_MAX && n_fields <= ARGMIN_SMALL_MAX) {
+        argmin_small<<<1, ARGMIN_SMALL_THREADS, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, cost_kind, cand_base,
+                                                           key, d_best_cand, n_fields);
+        h->launches++;
+        return cudaGetLastError();
+    }
+    const int th = 256;
+    const unsigned fb = (unsigned)((n_fields + th - 1) / th);
+    argmin_init<<<fb, th, 0, st>>>(key, d_best_cand, n_fields);
+    h->launches++;
+    if (n_cand > 0) {
+        const unsigned cb = (unsigned)((n_cand + th - 1) / th);
+        argmin_cost<<<cb, th, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, n_fields, cost_kind, key);
+        argmin_index<<<cb, th, 0, st>>>(d_summary, d_cand_field, h->d_rec, n_cand, n_fields, cost_kind, cand_base, key,
+                                        d_best_cand);
+        h->launches += 2;
+    }
+    argmin_final<<<fb, th, 0, st>>>(key, d_best_cand, n_fields);
+    h->launches++;
+    return cudaGetLastError();
+}
+
 size_t al256(size_t x) { return (x + 255) & ~size_t(255); }
 
 }  // namespace
@@ -383,6 +570,8 @@ cudaError_t fcpp_launch_select(fcpp_handle *h, const fcpp_summary *d_summary, co
                                double *d_cost, int64_t *d_cand, cudaStream_t st)
 {
     if (n_fields == 0) return cudaSuccess;
+    const int kind = plain_cost_kind(sel);
+    if (kind >= 0) return launch_argmin(h, d_summary, d_cand_field, n_cand, n_fields, kind, cand_base, d_cost, d_cand, st);
     const int k = sel.top_k;
     const int64_t n = n_cand, m = (int64_t)n_fields + 1;
     const int64_t scan_tiles = (m + SCAN_TILE - 1) / SCAN_TILE;
@@ -462,6 +651,12 @@ cudaError_t fcpp_launch_select_merge(fcpp_handle *h, const int64_t *d_gathered, 
                                      double *d_cost, int64_t *d_cand, cudaStream_t st)
 {
     if (n_fields == 0) return cudaSuccess;
+    if (k == 1) {
+        argmin_merge_kernel<<<(n_fields + 255) / 256, 256, 0, st>>>((const long long *)d_gathered, world, n_fields,
+                                                                    d_cost, (long long *)d_cand);
+        h->launches++;
+        return cudaGetLastError();
+    }
     const int64_t threads = (int64_t)n_fields * 32;
     select_merge_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>((const long long *)d_gathered, world,
                                                                           n_fields, k, d_cost, (long long *)d_cand);

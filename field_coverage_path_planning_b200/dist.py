@@ -1,15 +1,11 @@
 """Multi-GPU: one process per GPU (torch.distributed), candidates sharded in contiguous ranges,
-NO data-path collective — the only exchange is the final per-field argmin (SURVEY.md §8(e)).
+NO data-path collective — the only exchange is the final per-field ranking (SURVEY.md §8(e)).
 
 The reduction is exact and deterministic (ties go to the lowest global candidate index):
-    1+2. CUDA: ONE all-gather of every rank's (best cost, best candidate) words and the library's
-       merge kernel (fcpp_field_argmin_merge).  CPU/gloo (tests): all_reduce(MIN) of the cost, then
-       all_reduce(MIN) of the candidate index where the local best equals the global minimum;
-    3. the winner's 176-byte summary record is contributed by its owner (fcpp_winner_records) and summed
-       as int32 words (every other rank contributes zeros), i.e. an all-gather of one record per field.
-A top-k ranking (plan_batch(select=...)) is merged the same way: ONE all-gather of every rank's [F, k] costs and
-candidates and the library's merge kernel (fcpp_field_select_merge) — CPU/gloo: an all-gather and a sort — then the
-records of all F * k ranked candidates in step 3.
+    1+2. CUDA: ONE all-gather of every rank's [F, k] costs and candidates and the library's merge kernel
+       (fcpp_field_select_merge; k = 1 is the per-field argmin).  CPU/gloo (tests): an all-gather and a sort;
+    3. the records of the F * k ranked candidates are contributed by their owners (fcpp_winner_records) and summed
+       as int32 words (every other rank contributes zeros), i.e. an all-gather of k records per field.
 Works on NCCL (CUDA tensors) and gloo (CPU tensors — used by the world_size-2 CPU tests).
 """
 from __future__ import annotations
@@ -46,38 +42,9 @@ def shard_candidates(cands: Dict[str, np.ndarray], world: int, rank: int) -> Tup
 
 
 def reduce_best(best_cost: torch.Tensor, best_cand: torch.Tensor, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Global per-field (cost, candidate) from the local ones.  ``best_cand`` holds GLOBAL
-    candidate indices (-1 = this rank has no valid candidate for the field).  In place.
-
-    CUDA tensors: one NCCL all-gather of the (cost, candidate) words + the library's merge kernel
-    (fcpp_field_argmin_merge).  CPU tensors (gloo tests): the same rule with torch ops."""
-    if best_cost.is_cuda:
-        import ctypes as C
-        F = best_cost.numel()
-        world = dist.get_world_size(group)
-        dev = best_cost.device
-        adjacent = (best_cost.dtype == torch.float64 and best_cand.dtype == torch.int64 and best_cost.is_contiguous()
-                    and best_cand.is_contiguous() and best_cand.data_ptr() == best_cost.data_ptr() + 8 * F
-                    and best_cost.untyped_storage().data_ptr() == best_cand.untyped_storage().data_ptr())
-        if adjacent:   # BatchBuffers lays them out back to back
-            send = torch.empty(0, dtype=torch.int64, device=dev).set_(
-                best_cost.untyped_storage(), best_cost.storage_offset(), (2 * F,))
-        else:
-            send = torch.cat([best_cost.view(torch.int64), best_cand])
-        gathered = torch.empty(world * 2 * F, dtype=torch.int64, device=dev)
-        dist.all_gather_into_tensor(gathered, send, group=group)
-        h = _lib.handle(dev.index)
-        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        h.check(h.lib.fcpp_field_argmin_merge(h.h, gathered.data_ptr(), world, F, best_cost.data_ptr(),
-                                              best_cand.data_ptr(), st))
-        return best_cost, best_cand
-    local_cost = best_cost.clone()
-    dist.all_reduce(best_cost, op=dist.ReduceOp.MIN, group=group)
-    mine = (local_cost == best_cost) & (best_cand >= 0)
-    key = torch.where(mine, best_cand, torch.full_like(best_cand, I64_MAX))
-    dist.all_reduce(key, op=dist.ReduceOp.MIN, group=group)
-    best_cand.copy_(torch.where(key == I64_MAX, torch.full_like(key, -1), key))
-    return best_cost, best_cand
+    """Global per-field (cost, candidate) [F] from the local ones (``best_cand``: GLOBAL candidate indices, -1 = none),
+    in place: ``reduce_topk`` at k = 1."""
+    return reduce_topk(best_cost, best_cand, 1, group)
 
 
 def reduce_topk(top_cost: torch.Tensor, top_cand: torch.Tensor, k: int, group=None) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -96,7 +63,7 @@ def reduce_topk(top_cost: torch.Tensor, top_cand: torch.Tensor, k: int, group=No
         adjacent = (top_cost.dtype == torch.float64 and top_cand.dtype == torch.int64 and top_cost.is_contiguous()
                     and top_cand.is_contiguous() and top_cand.data_ptr() == top_cost.data_ptr() + 8 * n
                     and top_cost.untyped_storage().data_ptr() == top_cand.untyped_storage().data_ptr())
-        if adjacent:   # BatchBuffers.use_top_k lays them out back to back
+        if adjacent:   # BatchBuffers lays them out back to back
             send = torch.empty(0, dtype=torch.int64, device=dev).set_(
                 top_cost.untyped_storage(), top_cost.storage_offset(), (2 * n,))
         else:
@@ -167,12 +134,12 @@ def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, out
                        device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True,
                        select=None, obstacle_sweep=False):
     """plan_batch over all ranks of the default process group (see batch.plan_batch): every rank plans its
-    contiguous shard; ONE all-gather + merge kernel gives every rank the per-field argmin, one kernel + one
-    all-reduce every winner's summary record; the local summaries, the merged argmin and the winners' records
-    come back to the host with ONE synchronisation.  Launch sizes are remembered from earlier batches of the same
-    shape (no layout read-back); ``wait=False`` returns a ``batch.PendingBatch``.  With ``select`` the ranks' top-k
-    rankings are merged instead of the argmin, and the records of every ranked candidate gathered.  With
-    ``obstacle_sweep`` each rank gets the sweep of its own candidates (``BatchResult.sweep``)."""
+    contiguous shard; ONE all-gather + merge kernel gives every rank the per-field ranking (the argmin of ``cost``, or
+    the top-k of ``select``), one kernel + one all-reduce the summary record of every ranked candidate; the local
+    summaries, the merged ranking and the records come back to the host with ONE synchronisation.  Launch sizes are
+    remembered from earlier batches of the same shape (no layout read-back); ``wait=False`` returns a
+    ``batch.PendingBatch``.  With ``obstacle_sweep`` each rank gets the sweep of its own candidates
+    (``BatchResult.sweep``)."""
     from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch, run_device_batch
     if not dist.is_initialized():
         raise RuntimeError("distributed=True needs torch.distributed.init_process_group (backend 'nccl')")

@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define FCPP_ABI_VERSION 4
+#define FCPP_ABI_VERSION 5
 
 /* hard-coded sample counts of the reference (SURVEY.md §5) */
 #define FCPP_UTURN_POINTS 20      /* mlp3:807  */
@@ -226,23 +226,6 @@ int fcpp_layout(fcpp_handle *h, const fcpp_batch *batch, int32_t *d_n_pts, int64
  * rasterisation (mlp3:1357-1371, :1426-1578) for all candidates. */
 int fcpp_plan_batch(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outputs *out, void *stream);
 
-/* Per-field argmin over candidates of cost = len_main + len_head (cost_kind 0) or
- * time_main + time_head (cost_kind 1); candidates with status != 0 are skipped; ties go to the
- * lowest candidate index.  d_best_cost [F] double (+inf when no valid candidate),
- * d_best_cand [F] int64 (-1 when none).  cand_base is added to the indices (multi-GPU shards). */
-/* d_cand_field may be NULL right after fcpp_plan_batch of the same batch on this handle: the candidates' fields
- * are then taken from the library's candidate records (factored candidate sets have no cand_field array). */
-int fcpp_field_argmin(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field,
-                      int64_t n_cand, int32_t n_fields, int cost_kind, int64_t cand_base,
-                      double *d_best_cost, int64_t *d_best_cand, void *stream);
-
-/* Multi-GPU merge of the per-field argmin (SURVEY.md §8(e)): d_gathered [world][2*F] 8-byte words =
- * every rank's (best_cost[F] as double bits, best_cand[F] as int64 global indices, -1 = none), e.g.
- * the result of ONE all-gather of the two arrays laid out back to back.  Lowest cost wins, ties go
- * to the lowest candidate index; d_best_cost = +inf and d_best_cand = -1 when no rank has one. */
-int fcpp_field_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t world, int32_t n_fields,
-                            double *d_best_cost, int64_t *d_best_cand, void *stream);
-
 /* ---- per-field top-k under a constraint-aware cost (DESIGN.md §3.8) ---- */
 #define FCPP_SELECT_MAX_K 32
 
@@ -252,7 +235,8 @@ int fcpp_field_argmin_merge(fcpp_handle *h, const int64_t *d_gathered, int32_t w
  *   L = len_main + len_head;  T = time_main + time_head;  U = (double)(cov_total - cov_cells) * cell_area;
  *   cost = w_length*L + w_time*T + w_boundary*n_boundary_viol + w_obstacle*n_obstacle_viol
  *        + w_accel*n_accel_viol + w_uncovered*U
- * w_length = 1 with every other weight 0 and no limits is exactly fcpp_field_argmin's cost_kind 0. */
+ * A PLAIN selection: top_k = 1, no limit set, and the weights (w_length = 1, every other 0) or (w_time = 1, every
+ * other 0).  Its cost is L or T exactly (for finite L, T >= 0): the per-field argmin of the length or of the time. */
 typedef struct {
     double w_length, w_time, w_boundary, w_obstacle, w_accel, w_uncovered; /* finite, >= 0 */
     double cell_area;          /* m^2 of a headland-band cell: grid_h * grid_h */
@@ -265,8 +249,12 @@ typedef struct {
 
 /* Per field, the eligible candidates ranked by (cost, candidate index) ascending, the first top_k of them:
  * d_cost [F][k] double (+inf where fewer than k are eligible), d_cand [F][k] int64 global indices (cand_base added;
- * -1 where none).  d_cand_field as in fcpp_field_argmin (NULL: the candidate records of the last fcpp_plan_batch).
- * Exact and deterministic for any order of the candidates' fields; scratch space is the handle's workspace. */
+ * -1 where none).  Candidates whose field lies outside [0, n_fields) are skipped.  d_cand_field [n_cand] is the field
+ * of each candidate; it may be NULL right after fcpp_plan_batch of the same batch on this handle: the fields are
+ * then taken from the library's candidate records (factored candidate sets have no cand_field array).
+ * Exact and deterministic for any order of the candidates' fields; scratch space is the handle's workspace.
+ * A plain selection runs the argmin kernels: one launch up to 16 384 candidates and fields, else four (two without
+ * candidates), with no workspace; any other selection runs the ranking pipeline (DESIGN.md §3.8). */
 int fcpp_field_select(fcpp_handle *h, const fcpp_summary *d_summary, const int32_t *d_cand_field, int64_t n_cand,
                       int32_t n_fields, const fcpp_selection *sel, int64_t cand_base, double *d_cost,
                       int64_t *d_cand, void *stream);

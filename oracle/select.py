@@ -131,4 +131,7 @@ def adversarial_selections():
             sel(min_coverage=0.9, max_accel_viol=3, w_boundary=10.0, w_obstacle=2.5, w_accel=0.125, w_time=1.0,
                 top_k=7),
             sel(w_length=0.0, top_k=32),                       # every eligible cost 0: ranked by index alone
-            sel(min_coverage=1.0, max_boundary_viol=0, max_obstacle_viol=0, max_accel_viol=0, top_k=2)]
+            sel(min_coverage=1.0, max_boundary_viol=0, max_obstacle_viol=0, max_accel_viol=0, top_k=2),
+            # sel()'s twin with a limit no candidate reaches: the same ranking, but not a plain selection, so the
+            # library ranks it with the general pipeline at k = 1 instead of the argmin kernels
+            sel(max_accel_viol=2**31 - 1)]

@@ -1,7 +1,7 @@
 """torchrun worker of tests/test_gpu_multi.py (needs >= 2 GPUs): results of the multi-GPU path on hardware.
 
-1. reduce_best (NCCL all-gather + fcpp_field_argmin_merge) against the numpy rule, 40 back-to-back calls with
-   many ties, F = 1, 7, 4096;
+1. reduce_best (NCCL all-gather + fcpp_field_select_merge at k = 1) against the numpy rule, 40 back-to-back calls
+   with many ties, F = 1, 7, 4096;
 2. plan_batch(distributed=True) over the whole job == the single-process plan_batch of the same global
    candidate set (merged per-field argmin, costs, the winner's summary record), for config 2 at 512
    candidates per rank and a 3-field batch with a field that has no valid candidate.

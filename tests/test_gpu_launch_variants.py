@@ -2,7 +2,8 @@
 
 Many entry points pick a kernel instance from a path length, a batch size or a grid size: the caller-supplied-path
 kernels run in up to three shared-memory tiers plus an HBM-staged kernel, the prefix sum of the path offsets goes
-multi-tile beyond 4096 candidates, the per-field argmin switches kernels at 16384 candidates or fields, the coverage
+multi-tile beyond 4096 candidates, the per-field argmin (the plain selection of fcpp_field_select) switches kernels
+at 16384 candidates or fields, the coverage
 kernel runs one CTA per candidate or a persistent work list, and the window raster splits large windows into row
 tiles and long polylines into point chunks.  Every test here builds inputs that sit on both sides of such a switch
 and compares the result with the float64 / integer oracle (``oracle/``), or, where two variants must agree, checks
@@ -392,18 +393,35 @@ def _argmin_rule(status, cost, field, n_fields, base):
     return best_c, best_i
 
 
-def _device_argmin(h, sm, cand_field, n_fields, kind, base):
+def _device_argmin(h, sm, cand_field, n_fields, kind, base, twin=False):
+    """fcpp_field_select with the plain selection of cost kind ``kind`` (0: length, 1: time), which runs the argmin
+    kernels; ``twin``: the same selection with a limit no candidate reaches, which runs the ranking pipeline at
+    k = 1.  -> (cost [F], cand [F], kernel launches of the call)."""
+    import dataclasses
     import torch
     from field_coverage_path_planning_b200 import _lib
+    from field_coverage_path_planning_b200.batch import Selection
+    sel = Selection() if kind == 0 else Selection(w_length=0.0, w_time=1.0)
+    if twin:
+        sel = dataclasses.replace(sel, max_accel_viol=2**31 - 1)
+    sc = sel.c_struct(0.1)
     d_sum = torch.from_numpy(np.ascontiguousarray(sm).view(np.uint8).reshape(-1) if len(sm) else
                              np.zeros(_lib.SUMMARY_DTYPE.itemsize, dtype=np.uint8)).cuda()
     d_cf = torch.from_numpy(np.ascontiguousarray(cand_field, dtype=np.int32) if len(sm) else
                             np.zeros(1, dtype=np.int32)).cuda()
     d_cost = _nan(max(n_fields, 1))
     d_best = _nan(max(n_fields, 1)).view(torch.int64)
-    h.check(h.lib.fcpp_field_argmin(h.h, d_sum.data_ptr(), d_cf.data_ptr(), len(sm), n_fields, kind, base,
+    l0 = h.launches
+    h.check(h.lib.fcpp_field_select(h.h, d_sum.data_ptr(), d_cf.data_ptr(), len(sm), n_fields, C.byref(sc), base,
                                     d_cost.data_ptr(), d_best.data_ptr(), _stream()))
-    return d_cost.cpu().numpy()[:n_fields], d_best.cpu().numpy()[:n_fields]
+    launches = h.launches - l0
+    return d_cost.cpu().numpy()[:n_fields], d_best.cpu().numpy()[:n_fields], launches
+
+
+def _argmin_launches(n_cand, n_fields):
+    """The argmin kernels' launches: one CTA up to 16384 candidates and fields, else init, cost, index and final
+    (init and final alone without candidates)."""
+    return 1 if n_cand <= 16384 and n_fields <= 16384 else (4 if n_cand else 2)
 
 
 def _argmin_summaries(rng, n):
@@ -420,39 +438,67 @@ def _argmin_summaries(rng, n):
 
 @pytest.mark.parametrize("n_fields", [1, 7, 16384, 16385])
 @pytest.mark.parametrize("n_cand", [0, 1, 33, 16384, 16385, 200003])
-def test_field_argmin_both_kernels_vs_numpy_rule(fc, h, n_cand, n_fields):
+def test_plain_selection_both_argmin_kernels_vs_numpy_rule(fc, h, n_cand, n_fields):
     """Explicit cand_field in random order (nearly every warp holds several fields), quantised costs (exact ties
-    across warps), dead candidates, both cost kinds, candidate bases 0 and 3 * 2^32."""
+    across warps), dead candidates, both cost kinds, candidate bases 0 and 3 * 2^32.  The plain selection takes the
+    argmin kernels (their launch count), and its non-binding-limit twin, ranked by the pipeline, gives the same
+    bytes."""
     rng = np.random.default_rng(n_cand * 31 + n_fields)
     sm = _argmin_summaries(rng, n_cand)
     field = rng.integers(0, n_fields, n_cand).astype(np.int32)
     for kind in (0, 1):
         cost = sm["len_main"] + sm["len_head"] if kind == 0 else sm["time_main"] + sm["time_head"]
         for base in (0, 3 << 32):
-            got_c, got_i = _device_argmin(h, sm, field, n_fields, kind, base)
+            got_c, got_i, launches = _device_argmin(h, sm, field, n_fields, kind, base)
             want_c, want_i = _argmin_rule(sm["status"], cost, field, n_fields, base)
             assert np.array_equal(got_i, want_i), (kind, base, np.nonzero(got_i != want_i)[0][:5])
             assert np.array_equal(got_c, want_c), (kind, base)
+            assert launches == _argmin_launches(n_cand, n_fields), (kind, base, launches)
+            tw_c, tw_i, _ = _device_argmin(h, sm, field, n_fields, kind, base, twin=True)
+            assert tw_c.tobytes() == got_c.tobytes() and tw_i.tobytes() == got_i.tobytes(), (kind, base)
 
 
-def test_field_argmin_switch_does_not_change_the_answer(fc, h):
+def test_plain_selection_kernel_switch_does_not_change_the_answer(fc, h):
     """One dead candidate more (16384 -> 16385 candidates) or one empty field more (16384 -> 16385 fields) moves the
     argmin from the one-CTA kernel to the four-kernel path; the answer is the same bytes."""
     rng = np.random.default_rng(77)
     n = 16384
     sm = _argmin_summaries(rng, n)
     field = rng.integers(0, 512, n).astype(np.int32)
-    a_c, a_i = _device_argmin(h, sm, field, 512, 0, 0)
+    a_c, a_i, _ = _device_argmin(h, sm, field, 512, 0, 0)
     dead = np.concatenate([sm, sm[:1]])
     dead["status"][-1] = 1
     dead["len_main"][-1] = -1.0                 # would win every field if it were counted
-    b_c, b_i = _device_argmin(h, dead, np.concatenate([field, [0]]), 512, 0, 0)
+    b_c, b_i, _ = _device_argmin(h, dead, np.concatenate([field, [0]]), 512, 0, 0)
     assert a_c.tobytes() == b_c.tobytes() and a_i.tobytes() == b_i.tobytes()
     field = rng.integers(0, n, n).astype(np.int32)
-    a_c, a_i = _device_argmin(h, sm, field, n, 1, 5)
-    b_c, b_i = _device_argmin(h, sm, field, n + 1, 1, 5)
+    a_c, a_i, _ = _device_argmin(h, sm, field, n, 1, 5)
+    b_c, b_i, _ = _device_argmin(h, sm, field, n + 1, 1, 5)
     assert a_c.tobytes() == b_c[:n].tobytes() and a_i.tobytes() == b_i[:n].tobytes()
     assert np.isinf(b_c[n]) and b_i[n] == -1
+
+
+@pytest.mark.parametrize("n_cand,n_fields", [(5000, 7), (40000, 7), (5000, 20000)])
+def test_field_argmin_skips_fields_out_of_range(fc, h, n_cand, n_fields):
+    """Candidates of field -1 or F, mixed into both argmin kernel variants and costing less than any other, are skipped
+    as oracle/select.rank states; the pipeline's twin agrees."""
+    from oracle import select as osel
+    from field_coverage_path_planning_b200.batch import Selection
+    rng = np.random.default_rng(n_cand + n_fields)
+    sm = _argmin_summaries(rng, n_cand)
+    field = rng.integers(0, n_fields, n_cand).astype(np.int32)
+    out = rng.random(n_cand) < 0.1
+    field[out] = rng.choice([-1, n_fields], int(out.sum()))
+    sm["status"][out] = 0
+    for col in ("len_main", "len_head", "time_main", "time_head"):
+        sm[col][out] = 0.0
+    for kind, sel in ((0, Selection()), (1, Selection(w_length=0.0, w_time=1.0))):
+        want_c, want_i = osel.rank(sm, field, n_fields, sel, 0.01, base=7)
+        got_c, got_i, launches = _device_argmin(h, sm, field, n_fields, kind, 7)
+        assert launches == _argmin_launches(n_cand, n_fields)
+        assert np.array_equal(got_i, want_i[:, 0]) and got_c.tobytes() == want_c[:, 0].tobytes(), kind
+        tw_c, tw_i, _ = _device_argmin(h, sm, field, n_fields, kind, 7, twin=True)
+        assert tw_c.tobytes() == got_c.tobytes() and tw_i.tobytes() == got_i.tobytes(), kind
 
 
 def test_plan_batch_shuffled_field_order_argmin(fc):

@@ -529,9 +529,9 @@ def test_clothoid_turn_model_vs_scipy_oracle(fc):
         fc.plan_batch(fields, fc.VehicleParams(), cand, turn_model="bezier")
 
 
-def test_argmin_merge_kernel_vs_numpy_rule(fc):
-    """fcpp_field_argmin_merge (the multi-GPU merge after ONE all-gather): lowest cost wins, ties go
-    to the lowest global candidate index, ranks without a candidate (-1) are skipped."""
+def test_select_merge_at_k1_vs_numpy_rule(fc):
+    """fcpp_field_select_merge at k = 1 (the multi-GPU merge of the per-field argmin after ONE all-gather): lowest
+    cost wins, ties go to the lowest global candidate index, ranks without a candidate (-1) are skipped."""
     import ctypes as C
     import torch
     from field_coverage_path_planning_b200 import _lib
@@ -551,7 +551,7 @@ def test_argmin_merge_kernel_vs_numpy_rule(fc):
         oc = torch.empty(F, dtype=torch.float64, device="cuda")
         ob_ = torch.empty(F, dtype=torch.int64, device="cuda")
         st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        h.check(h.lib.fcpp_field_argmin_merge(h.h, dg.data_ptr(), world, F, oc.data_ptr(), ob_.data_ptr(), st))
+        h.check(h.lib.fcpp_field_select_merge(h.h, dg.data_ptr(), world, F, 1, oc.data_ptr(), ob_.data_ptr(), st))
         want_c, want_i = np.full(F, np.inf), np.full(F, -1, dtype=np.int64)
         for f in range(F):
             for r in range(world):

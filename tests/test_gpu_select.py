@@ -79,7 +79,7 @@ def test_select_kernel_skewed_fields(fc):
 def test_select_kernel_one_field_of_a_million(fc):
     from oracle import select as osel
     summ, fid = osel.adversarial_summaries(8, 1 << 20, 1)
-    for ns in (osel.adversarial_selections()[0], osel.adversarial_selections()[3]):
+    for ns in (osel.adversarial_selections()[0], osel.adversarial_selections()[3], osel.adversarial_selections()[-1]):
         _check(fc, summ, fid, 1, ns)
 
 
@@ -97,19 +97,24 @@ def test_select_kernel_c3_shape(fc):
 
 
 def _same_as_argmin(fc, fields, cands, obstacles, outputs, grid_h=0.1):
+    """cost= and the plain selection (the argmin kernels), and the plain selection's twin with a limit no candidate
+    reaches (the ranking pipeline at k = 1): the same bytes."""
     veh = fc.VehicleParams()
-    for cost, sel in (("length", fc.Selection()), ("time", fc.Selection(w_length=0.0, w_time=1.0))):
+    for cost, plain in (("length", fc.Selection()), ("time", fc.Selection(w_length=0.0, w_time=1.0))):
         want = fc.plan_batch(fields, veh, cands, obstacles=obstacles, outputs=outputs, grid_h=grid_h, cost=cost)
-        got = fc.plan_batch(fields, veh, cands, obstacles=obstacles, outputs=outputs, grid_h=grid_h, select=sel)
-        assert got.summary.tobytes() == want.summary.tobytes()
-        assert np.array_equal(got.best_cand, want.best_cand), cost
-        assert got.best_cost.tobytes() == want.best_cost.tobytes(), cost
-        assert got.topk_cand.shape == (len(fields), 1)
+        assert want.topk_cand is None and want.topk_cost is None and want.topk_summary is None
+        for sel in (plain, fc.Selection(**{**plain.__dict__, "max_accel_viol": 2**31 - 1})):
+            got = fc.plan_batch(fields, veh, cands, obstacles=obstacles, outputs=outputs, grid_h=grid_h, select=sel)
+            assert got.summary.tobytes() == want.summary.tobytes()
+            assert np.array_equal(got.best_cand, want.best_cand), (cost, sel)
+            assert got.best_cost.tobytes() == want.best_cost.tobytes(), (cost, sel)
+            assert got.topk_cand.shape == (len(fields), 1)
 
 
 def test_default_selections_equal_the_argmin(fc):
-    """Selection() is cost='length' and the time-only selection cost='time', bit for bit: config 2's shape (explicit
-    arrays and factored) and a heading search over parallelograms (factored, coverage de-duplicated per heading)."""
+    """Selection() is cost='length' and the time-only selection cost='time', bit for bit, through the argmin kernels
+    and through the ranking pipeline: config 2's shape (explicit arrays and factored) and a heading search over
+    parallelograms (factored, coverage de-duplicated per heading)."""
     from benchmarks import workloads as wl
     w = wl.c2(1, radii_per_gpu=256)
     _same_as_argmin(fc, w.fields, w.cands, w.obstacles, "paths")

@@ -35,9 +35,9 @@ for name in (sys.argv[1:] or ["c2", "c3", "c5"]):
                                              grid_h=w.grid_h, device=dev, winners=True), n)
         t_prep, pb = T(lambda: B.prepare_batch(w.fields, veh, cands, w.obstacles, None, w.grid_h, True), n)
         t_h2d, db = T(lambda: B.DeviceBatch(pb, dev), n)
-        t_launch, lb = T(lambda: B._launch_device_batch(db, w.outputs, False, "length", 0, None), n)
+        t_launch, lb = T(lambda: B._launch_device_batch(db, w.outputs, False, B.Selection(), 0, None), n)
         bufs, offs = lb
-        t_fetch, r = T(lambda: B._finish_fetch(B._enqueue_fetch(db, bufs, w.outputs, offs, True, 0)), n)
+        t_fetch, r = T(lambda: B._finish_fetch(B._enqueue_fetch(db, bufs, w.outputs, offs, True, 0), False), n)
         t_win, _ = T(lambda: B.fetch_winner_paths(db, r, w.outputs), n)
         t_nosum, _ = T(lambda: B.run_device_batch(db, w.outputs, copy_summary=False), n)
         print(f"{name} {form:8s} plan_batch(winners) {t_all:8.3f} ms = prepare {t_prep:.3f} + DeviceBatch/H2D {t_h2d:.3f} "
