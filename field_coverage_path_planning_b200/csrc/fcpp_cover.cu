@@ -108,6 +108,35 @@ static_assert(sizeof(Entry) == 48, "Entry layout");
 
 extern __shared__ __align__(16) unsigned char cover_smem[];
 
+#ifdef FCPP_COVER_TRACE
+// Diagnostic build (benchmarks/cover_balance.py, tests/test_cover_tasks.py): every coverage task a CTA runs records
+// [%globaltimer at start, at end, %smid | cost bucket << 16 | (task list position + 1) << 32, candidate << 2 | part]
+// (part 1 = A10, 2 = A11; position 0: not from the task list).  Read and reset by fcpp_cover_trace_take; the
+// default build has none of it.
+constexpr int TRACE_CAP = 1 << 18;
+__device__ unsigned long long g_trace[TRACE_CAP][4];
+__device__ unsigned int g_trace_n;
+__device__ __forceinline__ unsigned long long trace_clock()
+{
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ void trace_put(unsigned long long t0, int64_t cand, int part, int pos, int bucket)
+{
+    if (threadIdx.x != 0) return;
+    unsigned sm;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
+    const unsigned k = atomicAdd(&g_trace_n, 1u);
+    if (k < TRACE_CAP) {
+        g_trace[k][0] = t0;
+        g_trace[k][1] = trace_clock();
+        g_trace[k][2] = sm | ((unsigned long long)bucket << 16) | ((unsigned long long)(pos + 1) << 32);
+        g_trace[k][3] = ((unsigned long long)cand << 2) | (unsigned)part;
+    }
+}
+#endif
+
 __host__ __device__ constexpr size_t a16(size_t x) { return (x + 15) & ~size_t(15); }
 constexpr size_t OFF_APRE = a16(sizeof(CoverFixed));                 // int [EBATCH + 16]: exclusive (entry,row)-pair
                                                                      // prefix over the ACTIVE entries
@@ -1032,21 +1061,46 @@ __device__ __noinline__ unsigned band_grouped(CoverFixed &s, const CoverDyn &d, 
     return done;
 }
 
-// One candidate's coverage by the T threads of a CTA (cover_kernel, or one listed item of cover_work_kernel).
+// Coverage task list of a de-duplicated batch: one item per (representative, part) a CTA must run, in
+// non-increasing estimated cost.  An item is candidate << 1 | part (0 = A10 corner windows, 1 = A11 band).
+constexpr int COVER_BUCKETS = 48;
+
+// Estimated duration of coverage task `part` of record r in ns (B200, two CTAs per SM), as a cost bucket: six
+// buckets per octave from 4 us.  A rough fit to the task durations benchmarks/cover_balance.py traces on configs 2,
+// 3 and 5; only the ORDER in which the tasks are dispatched follows it, never a result.  A10: the four windows grow
+// with corner_g (2R / 0.1 m), plus their reverse fills.  A11: the (entry, row) pairs of the headland points, the
+// zone bitmaps around the corners (they grow as ((R + W) / h)^2) and, for a band without group (slanted straights,
+// evaluated row by row), the rows and words of the whole band.
+__device__ __forceinline__ int cover_task_bucket(const fcpp_batch &b, const CandRec &r, int part)
+{
+    if (cover_dead(r)) return 0;
+    double ns;
+    if (part == 0) {
+        ns = 12000.0 + 60.0 * r.corner_g + 100.0 * (r.vn_rev[0] + r.vn_rev[1] + r.vn_rev[2] + r.vn_rev[3]);
+    } else {
+        const double W = b.vehicle.working_width, h = b.grid_h, z = (r.R + W) / h;
+        ns = 30000.0 + 2.0 * r.n_head * (W / h) + 0.75 * z * z;
+        if (!r.band_group) ns += 10.0 * (b.field_extent[2 * r.field] + b.field_extent[2 * r.field + 1]) / h;
+    }
+    const int k = ns < 4096.0 ? 0 : (int)(6.0 * log2(ns / 4096.0)) + 1;
+    return min(k, COVER_BUCKETS - 1);
+}
+
+// Coverage of one candidate by the T threads of a CTA: the parts of `parts` (bit 0 A10 corner windows, bit 1 A11
+// band).  In a de-duplicated batch a CTA runs one part of a representative (a task), and the other candidates of its
+// group take that part's counts afterwards (cover_copy_kernel); both parts of one candidate may run in two CTAs at
+// once, so each writes only its own outputs and ORs its status bits atomically.  A band representative writes the
+// band of every start corner it evaluates to band_out[4 cand + start corner]; band_mask (band_group records) names them.
 __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *__restrict__ recs,
                                            const TrigTables *__restrict__ trig, fcpp_summary *__restrict__ summary,
-                                           int pc, int mode, const int32_t *__restrict__ rep /*[2][n_cand]*/,
-                                           const uint32_t *__restrict__ band_mask, longlong2 *__restrict__ band_out,
-                                           uint32_t *__restrict__ corner_bits, int64_t corner_bits_stride,
-                                           const int64_t cand)
+                                           int pc, int mode, const int parts, const uint32_t *__restrict__ band_mask,
+                                           longlong2 *__restrict__ band_out, uint32_t *__restrict__ corner_bits,
+                                           int64_t corner_bits_stride, const int64_t cand, const int pos)
 {
-    // a part (A10 corner windows / A11 band) whose inputs equal those of an earlier candidate is
-    // skipped: the candidate takes that one's counts afterwards (cover_copy_kernel).  A10 does not
-    // depend on the start corner or the heading, A11 not on the heading.  A band representative writes the band of
-    // every start corner it evaluates to band_out[4 cand + start corner]; band_mask (band_group records) names them.
-    const bool do10 = !rep || rep[cand] == (int32_t)cand;
-    const bool do11 = !rep || rep[b.n_cand + cand] == (int32_t)cand;
-    if (!do10 && !do11) return;
+    const bool do10 = parts & 1, do11 = parts & 2;
+#ifdef FCPP_COVER_TRACE
+    unsigned long long t0 = trace_clock();
+#endif
     CoverFixed &s = *reinterpret_cast<CoverFixed *>(cover_smem);
     const CoverDyn d;
     const int tid = threadIdx.x;
@@ -1065,6 +1119,9 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
     mbar_wait_block(&s.bar, 0);
     __syncthreads();
     const CandRec &r = s.rec;
+#ifdef FCPP_COVER_TRACE
+    const int tb10 = cover_task_bucket(b, r, 0), tb11 = cover_task_bucket(b, r, 1);
+#endif
     if (r.status != 0 || r.n_total == 0) {
         if (tid == 0) {
             if (do11) sum->cov_cells = sum->cov_total = 0;
@@ -1073,6 +1130,10 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
             if (do10)
                 for (int k = 0; k < 4; ++k) sum->corner_before[k] = sum->corner_after[k] = 0;
         }
+#ifdef FCPP_COVER_TRACE
+        if (do10) trace_put(t0, cand, 1, pos, tb10);
+        if (do11) trace_put(t0, cand, 2, pos, tb11);
+#endif
         return;
     }
     const double W = b.vehicle.working_width;
@@ -1196,6 +1257,10 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
                 sum->corner_before[k] = okc ? before[k] : 0;
                 sum->corner_after[k] = okc ? after[k] : 0;
             }
+#ifdef FCPP_COVER_TRACE
+        trace_put(t0, cand, 1, pos, tb10);
+        t0 = trace_clock();
+#endif
     }
 
     // =====================================================================================
@@ -1415,31 +1480,45 @@ __device__ __forceinline__ void cover_body(const fcpp_batch &b, const CandRec *_
             }
             put(sc, s.acc[0], s.acc[1], e11);
         }
+#ifdef FCPP_COVER_TRACE
+        trace_put(t0, cand, 2, pos, tb11);
+#endif
     }
     if (tid == 0 && (err10 | err11))
-        sum->status |= FCPP_CAND_GRID_TOO_LARGE | (err10 ? FCPP_CAND_CORNER_GRID_TOO_LARGE : 0) |
-                       (err11 ? FCPP_CAND_BAND_GRID_TOO_LARGE : 0);
+        atomicOr(&sum->status, FCPP_CAND_GRID_TOO_LARGE | (err10 ? FCPP_CAND_CORNER_GRID_TOO_LARGE : 0) |
+                                   (err11 ? FCPP_CAND_BAND_GRID_TOO_LARGE : 0));
 }
 
+// One CTA per candidate, both parts (no task list), or one CTA per listed task of a de-duplicated batch in list
+// order (the grid is sized to the 2 n_cand tasks there can be; the CTAs past the listed count exit at once).
 __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_kernel(const fcpp_batch b, const CandRec *__restrict__ recs,
                                                                         const TrigTables *__restrict__ trig,
                                                                         fcpp_summary *__restrict__ summary, int pc, int mode,
-                                                                        const int32_t *__restrict__ rep,
                                                                         const uint32_t *__restrict__ band_mask,
                                                                         longlong2 *__restrict__ band_out,
                                                                         uint32_t *__restrict__ corner_bits,
-                                                                        int64_t corner_bits_stride)
+                                                                        int64_t corner_bits_stride,
+                                                                        const int32_t *__restrict__ work,
+                                                                        const int32_t *__restrict__ counters /*[0] listed*/)
 {
-    cover_body(b, recs, trig, summary, pc, mode, rep, band_mask, band_out, corner_bits, corner_bits_stride, blockIdx.x);
+    int parts = 3, pos = -1;
+    int64_t cand = blockIdx.x;
+    if (work) {
+        pos = blockIdx.x;
+        if (pos >= counters[0]) return;
+        const int32_t it = work[pos];
+        parts = 1 << (it & 1);
+        cand = it >> 1;
+    }
+    cover_body(b, recs, trig, summary, pc, mode, parts, band_mask, band_out, corner_bits, corner_bits_stride, cand, pos);
 }
 
-// De-duplicated batches: the candidates that rasterise at least one part are listed (cover_list_kernel) and a
-// PERSISTENT grid of two CTAs per SM takes them from the list with an atomic counter — a heading search of
-// 737 280 candidates has ~4 096 of them, and launching 737 280 mostly empty 512-thread / 105 KB CTAs cost 4 ms.
+// The same task list taken by a PERSISTENT grid of two CTAs per SM with an atomic counter, in list order — a heading
+// search of 737 280 candidates has ~8 192 tasks, and launching one mostly empty 512-thread / 105 KB CTA per possible
+// task cost milliseconds.
 __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_work_kernel(const fcpp_batch b, const CandRec *__restrict__ recs,
                                                                              const TrigTables *__restrict__ trig,
                                                                              fcpp_summary *__restrict__ summary, int pc, int mode,
-                                                                             const int32_t *__restrict__ rep,
                                                                              const uint32_t *__restrict__ band_mask,
                                                                              longlong2 *__restrict__ band_out,
                                                                              uint32_t *__restrict__ corner_bits,
@@ -1459,7 +1538,9 @@ __global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) cover_work_kernel(con
         __syncthreads();
         const int w = s_item;
         if (w >= counters[0]) return;
-        cover_body(b, recs, trig, summary, pc, mode, rep, band_mask, band_out, corner_bits, corner_bits_stride, work[w]);
+        const int32_t it = work[w];
+        cover_body(b, recs, trig, summary, pc, mode, 1 << (it & 1), band_mask, band_out, corner_bits, corner_bits_stride,
+                   it >> 1, w);
     }
 }
 
@@ -1483,17 +1564,35 @@ int cover_point_capacity(int max_head)
 // ---------------------------------------------------------------------------------------------
 namespace {
 
+// task list counters: [0] listed tasks, [1] next task of the persistent grid, then per cost bucket the tasks
+// (histogram) and the tasks placed so far
+constexpr int COVER_COUNTERS = 2 + 2 * COVER_BUCKETS;
+
+// warp-aggregated atomicAdd(&ctr[key], 1) of the lanes with key >= 0 (all 32 lanes call it): the old value plus
+// the lane's rank among the lanes of the same key
+__device__ __forceinline__ int warp_add(int32_t *ctr, int key)
+{
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+    int base = 0;
+    if (key >= 0 && lane == leader) base = atomicAdd(&ctr[key], __popc(peers));
+    base = __shfl_sync(peers, base, leader);
+    return base + __popc(peers & ((1u << lane) - 1));
+}
+
 // table slot: key (0 = empty) and 0x7fffffff - (lowest candidate index) kept with atomicMax.  The
 // table is zeroed when it is allocated and every batch clears the slots it used (cover_copy_kernel),
 // so the steady state has no memset.  Both parts share the table (different hash seeds; a cross-part
-// collision is caught by the verification like any other).
+// collision is caught by the verification like any other).  Also zeroes the task list counters.
 __global__ void __launch_bounds__(128) cover_key_kernel(const CandRec *__restrict__ recs, int64_t n,
                                                         unsigned long long *__restrict__ keys,
                                                         unsigned int *__restrict__ vals, uint32_t cap_mask,
                                                         unsigned long long *__restrict__ hash /*[2][n]*/,
-                                                        uint32_t *__restrict__ band_mask)
+                                                        uint32_t *__restrict__ band_mask, int32_t *__restrict__ counters)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c == 0)
+        for (int k = 0; k < COVER_COUNTERS; ++k) counters[k] = 0;
     if (c >= n) return;
     band_mask[c] = 0u;
 #pragma unroll
@@ -1512,42 +1611,60 @@ __global__ void __launch_bounds__(128) cover_key_kernel(const CandRec *__restric
     }
 }
 
-__global__ void __launch_bounds__(128) cover_rep_kernel(const CandRec *__restrict__ recs, int64_t n,
+// the representative of each part of every candidate, and the histogram of the tasks' cost buckets
+__global__ void __launch_bounds__(128) cover_rep_kernel(const fcpp_batch b, const CandRec *__restrict__ recs, int64_t n,
                                                         const unsigned long long *__restrict__ keys,
                                                         const unsigned int *__restrict__ vals, uint32_t cap_mask,
                                                         unsigned long long *__restrict__ hash /*[2][n]*/,
                                                         int32_t *__restrict__ rep /*[2][n]*/,
-                                                        uint32_t *__restrict__ band_mask)
+                                                        uint32_t *__restrict__ band_mask, int32_t *__restrict__ counters)
 {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n) return;
 #pragma unroll
     for (int part = 0; part < 2; ++part) {
-        const unsigned long long h = hash[part * n + c];
-        uint32_t slot = (uint32_t)(h >> 17) & cap_mask;
-        while (keys[slot] != h) slot = (slot + 1) & cap_mask;
-        hash[part * n + c] = slot;  // remembered for the clean-up
-        const int64_t first = (int64_t)(0x7fffffffu - vals[slot]);
-        const int64_t q = (first < c && cover_same(recs[c], recs[first], part)) ? first : c;
-        rep[part * n + c] = (int32_t)q;
-        // the start corners a band representative evaluates
-        if (part == 1 && recs[c].band_group) atomicOr(&band_mask[q], 1u << (recs[c].flags & FCPP_FLAG_CORNER_MASK));
+        int bucket = -1;  // (lanes past n take part in the warp's histogram update)
+        if (c < n) {
+            const unsigned long long h = hash[part * n + c];
+            uint32_t slot = (uint32_t)(h >> 17) & cap_mask;
+            while (keys[slot] != h) slot = (slot + 1) & cap_mask;
+            const int64_t first = (int64_t)(0x7fffffffu - vals[slot]);
+            const int64_t q = (first < c && cover_same(recs[c], recs[first], part)) ? first : c;
+            rep[part * n + c] = (int32_t)q;
+            // the start corners a band representative evaluates
+            if (part == 1 && recs[c].band_group) atomicOr(&band_mask[q], 1u << (recs[c].flags & FCPP_FLAG_CORNER_MASK));
+            if (q == c) bucket = cover_task_bucket(b, recs[c], part);
+            // remembered: the slot for the clean-up, the task's bucket (+1, 0 = no task) for cover_list_kernel
+            hash[part * n + c] = slot | (unsigned long long)(bucket + 1) << 32;
+        }
+        warp_add(counters + 2, bucket);
     }
 }
 
-// the candidates that rasterise a part, in any order
-__global__ void __launch_bounds__(128) cover_list_kernel(int64_t n, const int32_t *__restrict__ rep /*[2][n]*/,
+// the task list: every (representative, part), by a counting sort over the cost buckets, costliest bucket first
+// (within a bucket in the order of the atomic placement, which no output depends on)
+__global__ void __launch_bounds__(128) cover_list_kernel(int64_t n, const unsigned long long *__restrict__ slot_of /*[2][n]*/,
                                                          int32_t *__restrict__ work, int32_t *__restrict__ counters)
 {
+    __shared__ int start[COVER_BUCKETS];
+    for (int k = threadIdx.x; k < COVER_BUCKETS; k += blockDim.x) start[k] = counters[2 + k];  // (32-thread CTAs too)
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int acc = 0;
+        for (int k = COVER_BUCKETS - 1; k >= 0; --k) {
+            const int m = start[k];
+            start[k] = acc;
+            acc += m;
+        }
+        if (blockIdx.x == 0) counters[0] = acc;
+    }
+    __syncthreads();
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool on = c < n && (rep[c] == (int32_t)c || rep[n + c] == (int32_t)c);
-    const unsigned m = __ballot_sync(0xffffffffu, on);
-    if (m == 0) return;
-    const int lane = threadIdx.x & 31;
-    int base = 0;
-    if (lane == 0) base = atomicAdd(&counters[0], __popc(m));
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (on) work[base + __popc(m & ((1u << lane) - 1))] = (int32_t)c;
+#pragma unroll
+    for (int part = 0; part < 2; ++part) {
+        const int bucket = c < n ? (int)(slot_of[part * n + c] >> 32) - 1 : -1;
+        const int k = warp_add(counters + 2 + COVER_BUCKETS, bucket);
+        if (bucket >= 0) work[start[bucket] + k] = (int32_t)(c << 1 | part);
+    }
 }
 
 __global__ void __launch_bounds__(128) cover_copy_kernel(const CandRec *__restrict__ recs, fcpp_summary *__restrict__ summary,
@@ -1588,9 +1705,9 @@ __global__ void __launch_bounds__(128) cover_copy_kernel(const CandRec *__restri
 
 }  // namespace
 
-// few representatives expected (a heading search): persistent grid over the listed candidates.  (Measured: config 3
-// coverage 4.0 -> 2.8 ms per 737 280 candidates; batches where most candidates rasterise a part — configs 2 and 5 —
-// run 1.5-2.5 % slower that way, hence the hint.  Cover mode bits 6 / 7 force either.)
+// few tasks expected (a heading search): the persistent grid over the task list.  (Measured: config 3 coverage
+// 4.0 -> 2.8 ms per 737 280 candidates against one CTA per candidate.)  Other de-duplicated batches launch one CTA per
+// possible task.  Cover mode bits 6 / 7 force either.
 static bool cover_use_work_list(const fcpp_handle *h, const fcpp_batch &b)
 {
     return (b.cover_dedupe >= 2 || (h->cover_mode & 128)) && !(h->cover_mode & 64);
@@ -1598,8 +1715,9 @@ static bool cover_use_work_list(const fcpp_handle *h, const fcpp_batch &b)
 
 static int dedupe_threads(const fcpp_handle *h, int64_t n) { return n <= 2 * 32 * (int64_t)h->sm_count ? 32 : 128; }
 
-// Coverage of a batch: (when the batch asks for it) the de-duplication kernels, the coverage kernel, then the copy of
-// the representatives' counts to the other members of their groups, which also empties the hash table.
+// Coverage of a batch: (when the batch asks for it) the de-duplication kernels, which also list the coverage tasks
+// costliest first, the coverage kernel, then the copy of the representatives' counts to the other members of their
+// groups, which also empties the hash table.
 cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_outputs &o, cudaStream_t st)
 {
     if (b.n_cand == 0) return cudaSuccess;
@@ -1609,7 +1727,7 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
     int32_t *d_rep = nullptr;
     unsigned long long *keys = nullptr, *hash = nullptr;
     unsigned int *vals = nullptr;
-    int32_t *work = nullptr, *counters = nullptr;  // de-duplicated batches: the listed candidates (cover_work_kernel)
+    int32_t *work = nullptr, *counters = nullptr;  // de-duplicated batches: the task list and its counters
     uint32_t *band_mask = nullptr;                 // start corners per band representative
     longlong2 *band_out = nullptr;                 // bands per (representative, start corner)
     cudaError_t e;
@@ -1620,7 +1738,7 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
     if (b.cover_dedupe && n > 1 && !(h->cover_mode & 2) && n < (1ll << 28)) {
         uint32_t cap = 1024;
         while ((int64_t)cap < 4 * n) cap <<= 1;  // two keys per candidate, load factor <= 1/2
-        const size_t need = (size_t)cap * 12 + (size_t)n * 96 + 64;
+        const size_t need = (size_t)cap * 12 + (size_t)n * 100 + sizeof(int32_t) * COVER_COUNTERS + 64;
         if (need > h->dedupe_bytes) {
             if (h->d_dedupe) cudaFree(h->d_dedupe);
             h->d_dedupe = nullptr;
@@ -1630,46 +1748,43 @@ cudaError_t fcpp_launch_cover(fcpp_handle *h, const fcpp_batch &b, const fcpp_ou
             h->dedupe_bytes = need;
             h->dedupe_cap = 0;
         }
-        // layout: keys [cap] | vals [cap] | hash / slot [2][n] | band_out [n][4] | rep [2][n] | band_mask [n] | work [n] |
-        // counters [2]; a different capacity moves the arrays, so the table is zeroed again
+        // layout: keys [cap] | vals [cap] | hash / slot [2][n] | band_out [n][4] | rep [2][n] | band_mask [n] |
+        // work [2n] | counters [COVER_COUNTERS]; a different capacity moves the arrays, so the table is zeroed again
         keys = (unsigned long long *)h->d_dedupe;
         vals = (unsigned int *)(keys + cap);
         hash = (unsigned long long *)(vals + cap);
         band_out = (longlong2 *)(hash + 2 * n);
         d_rep = (int32_t *)(band_out + 4 * n);
         band_mask = (uint32_t *)(d_rep + 2 * n);
+        work = (int32_t *)(band_mask + n);
+        counters = work + 2 * n;
         if (h->dedupe_cap != cap) {
             e = cudaMemsetAsync(h->d_dedupe, 0, (size_t)cap * 12, st);
             if (e != cudaSuccess) return e;
             h->dedupe_cap = cap;
         }
         const unsigned g = (unsigned)((n + th - 1) / th);
-        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, band_mask);
-        cover_rep_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, d_rep, band_mask);
-        h->launches += 2;
-        if (cover_use_work_list(h, b)) {
-            work = (int32_t *)(band_mask + n);
-            counters = work + n;
-            e = cudaMemsetAsync(counters, 0, 2 * sizeof(int32_t), st);
-            if (e != cudaSuccess) return e;
-            cover_list_kernel<<<g, th, 0, st>>>(n, d_rep, work, counters);
-            h->launches++;
-        }
+        cover_key_kernel<<<g, th, 0, st>>>(h->d_rec, n, keys, vals, cap - 1, hash, band_mask, counters);
+        cover_rep_kernel<<<g, th, 0, st>>>(b, h->d_rec, n, keys, vals, cap - 1, hash, d_rep, band_mask, counters);
+        cover_list_kernel<<<g, th, 0, st>>>(n, hash, work, counters);
+        h->launches += 3;
         e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
-    if (work) {
+    if (work && cover_use_work_list(h, b)) {
         e = cudaFuncSetAttribute(cover_work_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         if (e != cudaSuccess) return e;
         int64_t grid = (int64_t)FCPP_COVER_MINBLOCKS * h->sm_count;
-        if (grid > n) grid = n;
-        cover_work_kernel<<<(unsigned)grid, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
-                                                            band_mask, band_out, o.corner_bits, o.corner_bits_stride, work, counters);
+        if (grid > 2 * n) grid = 2 * n;
+        cover_work_kernel<<<(unsigned)grid, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode,
+                                                            band_mask, band_out, o.corner_bits, o.corner_bits_stride, work,
+                                                            counters);
     } else {
         e = cudaFuncSetAttribute(cover_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         if (e != cudaSuccess) return e;
-        cover_kernel<<<(unsigned)n, T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode, d_rep,
-                                                    band_mask, band_out, o.corner_bits, o.corner_bits_stride);
+        cover_kernel<<<(unsigned)(work ? 2 * n : n), T, bytes, st>>>(b, h->d_rec, h->d_trig, o.summary, pc, h->cover_mode,
+                                                                     band_mask, band_out, o.corner_bits,
+                                                                     o.corner_bits_stride, work, counters);
     }
     h->launches++;
     e = cudaGetLastError();
@@ -1756,6 +1871,21 @@ __global__ void __launch_bounds__(T) window_kernel(const double *__restrict__ pa
 }
 
 }  // namespace
+
+#ifdef FCPP_COVER_TRACE
+// the trace records of the coverage tasks since the previous call (at most cap of them are copied); resets the trace
+extern "C" int fcpp_cover_trace_take(unsigned long long *host, int cap)
+{
+    unsigned n = 0;
+    if (cudaDeviceSynchronize() != cudaSuccess || cudaMemcpyFromSymbol(&n, g_trace_n, sizeof(n)) != cudaSuccess) return -1;
+    n = n < (unsigned)TRACE_CAP ? n : (unsigned)TRACE_CAP;
+    const unsigned m = n < (unsigned)cap ? n : (unsigned)cap;
+    if (m && cudaMemcpyFromSymbol(host, g_trace, (size_t)m * 4 * sizeof(unsigned long long)) != cudaSuccess) return -1;
+    const unsigned zero = 0;
+    if (cudaMemcpyToSymbol(g_trace_n, &zero, sizeof(zero)) != cudaSuccess) return -1;
+    return (int)n;
+}
+#endif
 
 cudaError_t fcpp_launch_raster_window(fcpp_handle *h, const double *d_path, int32_t n_pts, double radius,
                                       double ox, double oy, double hc, int32_t g, uint32_t *d_bits,

@@ -86,7 +86,7 @@ struct fcpp_handle {
     int cover_pcap;          // point capacity of the coverage kernel's staging for the next launch
     int cover_mode;          // diagnostics (fcpp_set_cover_mode): bit 0 = never use the zoned band evaluation,
                              // bit 1 = no coverage de-duplication, bits 6 / 7 = de-duplicated batches: force one
-                             // coverage CTA per candidate / the persistent work list
+                             // coverage CTA per listed task / the persistent grid over the task list
     void *d_dedupe;          // coverage de-duplication: hash table, hashes, representatives
     size_t dedupe_bytes;
     uint32_t dedupe_cap;     // slots of the (currently zeroed) table inside d_dedupe; 0 = not initialised

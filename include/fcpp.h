@@ -115,8 +115,8 @@ typedef struct {
                                * headland band (A11) of candidates with the same field, R and start corner (any
                                * heading); 0: every candidate is rasterised.  2: as 1, and the caller expects FEW
                                * representatives (a heading search: many headings per field): the coverage kernel then
-                               * runs as a persistent grid over the list of representatives instead of one (mostly
-                               * empty) CTA per candidate.  Same integers either way. */
+                               * runs as a persistent grid over the list of coverage tasks instead of one (mostly
+                               * empty) CTA per possible task.  Same integers either way. */
     double clothoid_share;         /* share of a turn's deflection spent on the two clothoids, (0, 1] */
     /* ---- factored candidate set (optional): cand_field == NULL selects it.  The candidates are the Cartesian
      * product field x heading x radius x start corner, field-major (the order of make_candidates): candidate c of
@@ -454,7 +454,7 @@ int fcpp_kernel_times(fcpp_handle *h, float *ms3);
  * row-tiled.  Bit 1 set = no coverage de-duplication (by default candidates whose coverage inputs are
  * identical — same field, R, start corner; e.g. the headings of a heading search — are rasterised once
  * and share the counts).  Bits 6 / 7 override fcpp_batch.cover_dedupe's choice between one coverage CTA per
- * candidate (bit 6) and the persistent grid over the listed representatives (bit 7).  Any other bit is
+ * listed task (bit 6) and the persistent grid over the task list (bit 7).  Any other bit is
  * FCPP_ERR_INVALID and leaves the mode unchanged.  All modes give identical results (tests/test_gpu_parity.py
  * compares them). */
 int fcpp_set_cover_mode(fcpp_handle *h, int mode);

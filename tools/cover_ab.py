@@ -1,4 +1,4 @@
-"""A/B of coverage launch modes (fcpp_set_cover_mode: 0 default, 64 one coverage CTA per candidate, 128 the persistent
+"""A/B of coverage launch modes (fcpp_set_cover_mode: 0 default, 64 one coverage CTA per listed task, 128 the persistent
 work list over the listed representatives, ...) per workload and output mode.
 python tools/cover_ab.py [mode ...]"""
 import os
