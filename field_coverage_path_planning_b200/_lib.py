@@ -29,6 +29,8 @@ CAND_LOOP_SKIPPED = 2
 CAND_TOO_MANY_LOOPS = 4
 CAND_TOO_LARGE = 8
 CAND_GRID_TOO_LARGE = 16
+CAND_BAND_GRID_TOO_LARGE = 64
+PATH_OUT_OF_RANGE = 128     # fcpp_path_cover.status: a point 2^30 lattice units or more from the field's lattice origin
 
 
 class FcppError(RuntimeError):
@@ -143,9 +145,16 @@ SWEEP_DTYPE = np.dtype([("n_seg_main", "<i4"), ("n_seg_head", "<i4"), ("len_main
                        align=True)
 assert SWEEP_DTYPE.itemsize == 24, SWEEP_DTYPE.itemsize
 
+# numpy mirror of fcpp_path_cover (48 bytes): D3 point counts, the headland band's and the whole field's cells and
+# covered cells
+PATH_COVER_DTYPE = np.dtype([("status", "<i4"), ("n_boundary_viol", "<i4"), ("n_obstacle_viol", "<i4"),
+                             ("reserved", "<i4"), ("band_total", "<i8"), ("band_cells", "<i8"), ("field_total", "<i8"),
+                             ("field_cells", "<i8")], align=True)
+assert PATH_COVER_DTYPE.itemsize == 48, PATH_COVER_DTYPE.itemsize
+
 EXPORTS = [
     "fcpp_abi_version", "fcpp_create", "fcpp_destroy", "fcpp_last_error", "fcpp_set_trig_tables",
-    "fcpp_layout", "fcpp_plan_batch", "fcpp_obstacle_sweep", "fcpp_obstacle_sweep_paths", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
+    "fcpp_layout", "fcpp_plan_batch", "fcpp_obstacle_sweep", "fcpp_obstacle_sweep_paths", "fcpp_path_coverage", "fcpp_plan_coverage", "fcpp_field_select", "fcpp_field_select_merge", "fcpp_winner_records", "fcpp_status_count", "fcpp_speed_verify", "fcpp_raster_window",
     "fcpp_tour_lengths", "fcpp_distance_matrix", "fcpp_connection_matrix", "fcpp_ga_init_population", "fcpp_ga_next_size", "fcpp_ga_generation", "fcpp_ga_solve", "fcpp_kmeans_lloyd", "fcpp_tsp_two_opt",
     "fcpp_launch_count", "fcpp_last_max_points", "fcpp_last_max_head_points", "fcpp_last_total_points", "fcpp_set_profiling", "fcpp_kernel_times", "fcpp_set_cover_mode",
 ]
@@ -188,6 +197,10 @@ def load():
         L.fcpp_obstacle_sweep.argtypes = [vp, C.POINTER(Batch), vp, vp]
         L.fcpp_obstacle_sweep_paths.restype = C.c_int
         L.fcpp_obstacle_sweep_paths.argtypes = [vp, vp, vp, i64, vp, vp, vp, i32, dbl, vp, vp]
+        L.fcpp_path_coverage.restype = C.c_int
+        L.fcpp_path_coverage.argtypes = [vp, vp, vp, i64, vp, vp, vp, i32, vp, vp, vp, vp, dbl, dbl, vp, vp]
+        L.fcpp_plan_coverage.restype = C.c_int
+        L.fcpp_plan_coverage.argtypes = [vp, C.POINTER(Batch), C.POINTER(Outputs), vp, vp]
         L.fcpp_field_select.restype = C.c_int
         L.fcpp_field_select.argtypes = [vp, vp, vp, i64, i32, C.POINTER(SelectionC), i64, vp, vp, vp]
         L.fcpp_field_select_merge.restype = C.c_int

@@ -314,6 +314,35 @@ class PreparedBatch:
         return float(self.vehicle.min_turn_radius)
 
 
+def _obstacle_tables(obstacles, F: int, W: float, arrays: Dict[str, np.ndarray]):
+    """Obstacles (mlp3:600-609), one polygon list per field, as the flattened fcpp_batch tables + D2 round-buffer
+    moments, added to ``arrays`` (nothing when there is no obstacle).  -> (max vertices, max polygons) of a field."""
+    max_v = max_p = 0
+    if obstacles is not None and any(len(o) for o in obstacles):
+        if len(obstacles) != F:
+            raise ValueError("obstacles must have one (possibly empty) polygon list per field")
+        poly_start = [0]
+        vert_start = [0]
+        verts: List[Sequence[float]] = []
+        moms = []
+        for polys in obstacles:
+            nv_field = 0
+            for poly in polys:
+                pts = [tuple(map(float, p)) for p in poly]
+                verts.extend(pts)
+                nv_field += len(pts)
+                vert_start.append(len(verts))
+                moms.append(G.round_buffer_moments(pts, W / 2))
+            poly_start.append(len(vert_start) - 1)
+            max_v = max(max_v, nv_field)
+            max_p = max(max_p, len(polys))
+        arrays["obs_poly_start"] = np.asarray(poly_start, dtype=np.int32)
+        arrays["obs_vert_start"] = np.asarray(vert_start, dtype=np.int32)
+        arrays["obs_verts"] = np.asarray(verts, dtype=np.float64).reshape(-1, 2)
+        arrays["obs_moments"] = np.asarray(moms, dtype=np.float64).reshape(-1, 3)
+    return max_v, max_p
+
+
 def prepare_batch(fields, vehicle: VehicleParams, candidates: Optional[Dict[str, np.ndarray]] = None,
                   obstacles: Optional[Sequence[Sequence[Sequence[Sequence[float]]]]] = None,
                   start_points: Optional[np.ndarray] = None, grid_h: float = 0.1,
@@ -410,30 +439,7 @@ def prepare_batch(fields, vehicle: VehicleParams, candidates: Optional[Dict[str,
         dedupe = B > F and ("heading" in candidates or "start_corner" in candidates)
         if dedupe and "heading" in candidates and B >= 4 * F:
             dedupe = 2          # a heading search: few coverage representatives (fcpp_batch.cover_dedupe = 2)
-    # ---- obstacles (mlp3:600-609): flattened polygon tables + D2 round-buffer moments ----
-    max_v = max_p = 0
-    if obstacles is not None and any(len(o) for o in obstacles):
-        if len(obstacles) != F:
-            raise ValueError("obstacles must have one (possibly empty) polygon list per field")
-        poly_start = [0]
-        vert_start = [0]
-        verts: List[Sequence[float]] = []
-        moms = []
-        for polys in obstacles:
-            nv_field = 0
-            for poly in polys:
-                pts = [tuple(map(float, p)) for p in poly]
-                verts.extend(pts)
-                nv_field += len(pts)
-                vert_start.append(len(verts))
-                moms.append(G.round_buffer_moments(pts, W / 2))
-            poly_start.append(len(vert_start) - 1)
-            max_v = max(max_v, nv_field)
-            max_p = max(max_p, len(polys))
-        arrays["obs_poly_start"] = np.asarray(poly_start, dtype=np.int32)
-        arrays["obs_vert_start"] = np.asarray(vert_start, dtype=np.int32)
-        arrays["obs_verts"] = np.asarray(verts, dtype=np.float64).reshape(-1, 2)
-        arrays["obs_moments"] = np.asarray(moms, dtype=np.float64).reshape(-1, 3)
+    max_v, max_p = _obstacle_tables(obstacles, F, W, arrays)
     if turn_model not in ("arc", "clothoid", "omega"):
         raise ValueError("turn_model must be 'arc' (the reference's sampled arcs), 'clothoid' or 'omega'")
     return PreparedBatch(vehicle, F, B, arrays, max_v, max_p, float(grid_h), bool(coverage), turn_model,
@@ -511,6 +517,9 @@ class BatchResult:
     # plan_batch(..., obstacle_sweep=True): per candidate the segments that drive through the obstacle region and the
     # metres inside, per layer (include/fcpp.h fcpp_sweep)
     sweep: Optional[np.ndarray] = None          # [B] SWEEP_DTYPE
+    # plan_batch(..., field_coverage=True): per candidate the D3 counts and the cells of the headland band and of the
+    # whole field with those the plan covers (include/fcpp.h fcpp_path_cover)
+    field_cover: Optional[np.ndarray] = None    # [B] PATH_COVER_DTYPE
 
     def path(self, b: int):
         """(path [n,2], speeds [n], n_main) of local candidate ``b`` copied to the host."""
@@ -536,6 +545,7 @@ class BatchBuffers:
         self.rank_k(1)
         self.d_off = self.d_path = self.d_spd = self.d_kap = None
         self.d_sweep = None          # [B] fcpp_sweep records of the last batch run with obstacle_sweep=True
+        self.d_fcov = None           # [B] fcpp_path_cover records of the last batch run with field_coverage=True
         self.speculative = False     # sized from remembered maxima (_Hints), not from this batch's layout pass
         if total_points > 0:
             self.d_off = torch.empty(n_cand + 1, dtype=torch.int64, device=dev)
@@ -603,7 +613,7 @@ class _Hints:
 
 def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, selection: Selection, cand_base: int,
                          buffers: Optional["BatchBuffers"], path_alloc=None, corner_bits: bool = False,
-                         speculate: bool = False, sweep: bool = False):
+                         speculate: bool = False, sweep: bool = False, field_cover: bool = False):
     """Enqueue layout, prefix sum, plan, coverage and ranking kernels of one batch on torch's current
     stream.  Returns (buffers, offsets or None).  Without ``buffers`` the path storage is sized from
     the layout pass (one small synchronous read-back) — or, with ``speculate`` and a batch of this shape seen
@@ -611,7 +621,8 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, se
     caller must check the status flags, see ``_Hints``); ``path_alloc(total) -> BatchBuffers | None`` lets the
     caller provide the storage.  ``selection``: how fcpp_field_select ranks each field's candidates into
     buffers.d_cost / d_best.  ``sweep``: also the segment-level obstacle sweep of every candidate
-    (fcpp_obstacle_sweep) into buffers.d_sweep."""
+    (fcpp_obstacle_sweep) into buffers.d_sweep.  ``field_cover`` (paths mode): also the whole-field and headland-band
+    coverage of the materialised paths (fcpp_plan_coverage) into buffers.d_fcov."""
     if outputs not in ("summary", "paths"):
         raise ValueError("outputs must be 'summary' or 'paths'")
     dev = db.dev
@@ -679,6 +690,11 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, se
             if buffers.d_sweep is None or buffers.d_sweep.numel() < nb:
                 buffers.d_sweep = torch.empty(nb, dtype=torch.uint8, device=dev)
             h.check(L.fcpp_obstacle_sweep(h.h, C.byref(db.c), buffers.d_sweep.data_ptr(), stream))
+        if field_cover:
+            nb = max(B, 1) * _lib.PATH_COVER_DTYPE.itemsize
+            if buffers.d_fcov is None or buffers.d_fcov.numel() < nb:
+                buffers.d_fcov = torch.empty(nb, dtype=torch.uint8, device=dev)
+            h.check(L.fcpp_plan_coverage(h.h, C.byref(db.c), C.byref(out), buffers.d_fcov.data_ptr(), stream))
         if db.c.max_points_hint == 0:
             db.max_points = int(L.fcpp_last_max_points(h.h))
             db.max_head_points = int(L.fcpp_last_max_head_points(h.h))
@@ -695,13 +711,16 @@ def _launch_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, se
 
 class _PendingFetch:
     """The read-back of a launched batch, enqueued but not waited for."""
-    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "hv", "lay", "win", "hwin", "event", "o_sweep")
+    __slots__ = ("db", "buffers", "outputs", "offsets", "cand_base", "hv", "lay", "win", "hwin", "event", "o_sweep",
+                 "o_fcov")
 
 
 def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offsets, copy_summary: bool,
-                   cand_base: int, win: Optional[torch.Tensor] = None, sweep: bool = False) -> _PendingFetch:
+                   cand_base: int, win: Optional[torch.Tensor] = None, sweep: bool = False,
+                   field_cover: bool = False) -> _PendingFetch:
     """Enqueue the copies of summaries + the per-field ranking (+ offsets) (+ ``win``: the winners' records and
     flag-count word of a sharded batch, see dist.gather_winner_records) (+ ``sweep``: the obstacle sweep records)
+    (+ ``field_cover``: the field coverage records)
     into ONE pooled pinned buffer on torch's current stream and record an event behind them; nothing is waited for."""
     dev = db.dev
     B, F = db.pb.n_cand, db.pb.n_fields
@@ -721,6 +740,10 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
         nb_sweep = B * _lib.SWEEP_DTYPE.itemsize if sweep else 0
         if sweep:
             total_out = o_sweep + nb_sweep
+        o_fcov = (total_out + 255) & ~255
+        nb_fcov = B * _lib.PATH_COVER_DTYPE.itemsize if field_cover else 0
+        if field_cover:
+            total_out = o_fcov + nb_fcov
         ho, hv = _ResultPool.get(total_out)
         # the copies run on a COPY stream behind an event of the launching stream: the next batch's kernels (already
         # enqueued by a pipelining caller) must not wait for PCIe — at 737 280 candidates the 130 MB of summaries
@@ -746,12 +769,15 @@ def _enqueue_fetch(db: DeviceBatch, buffers: "BatchBuffers", outputs: str, offse
                 ho[o_win:o_win + win.numel()].copy_(win, non_blocking=True)
             if nb_sweep:
                 ho[o_sweep:o_sweep + nb_sweep].copy_(buffers.d_sweep[:nb_sweep], non_blocking=True)
+            if nb_fcov:
+                ho[o_fcov:o_fcov + nb_fcov].copy_(buffers.d_fcov[:nb_fcov], non_blocking=True)
             pf.event = torch.cuda.Event()
             pf.event.record(cs)
     pf.db, pf.buffers, pf.outputs, pf.offsets, pf.cand_base = db, buffers, outputs, offsets, cand_base
     pf.hv, pf.lay = hv, (nb_sum, need_off, o_cost, o_best, o_off, k)
     pf.win, pf.hwin = win, (hv[o_win:o_win + win.numel()] if win is not None else None)
     pf.o_sweep = (o_sweep, B) if sweep else None
+    pf.o_fcov = (o_fcov, B) if field_cover else None
     return pf
 
 
@@ -777,6 +803,9 @@ def _finish_fetch(pf: _PendingFetch, ranked: bool) -> "BatchResult":
     if pf.o_sweep is not None:
         o, n = pf.o_sweep
         res.sweep = hv[o:o + n * _lib.SWEEP_DTYPE.itemsize].view(_lib.SWEEP_DTYPE)
+    if pf.o_fcov is not None:
+        o, n = pf.o_fcov
+        res.field_cover = hv[o:o + n * _lib.PATH_COVER_DTYPE.itemsize].view(_lib.PATH_COVER_DTYPE)
     res.extras["buffers"] = buffers
     return res
 
@@ -899,9 +928,10 @@ class PendingBatch:
     all ranks repeat the batch together."""
 
     def __init__(self, db, pf, outputs, want_curvature, selection, ranked, cand_base, copy_summary, winners,
-                 corner_bits, speculate, shard, sweep=False):
+                 corner_bits, speculate, shard, sweep=False, field_cover=False):
         self.db, self.pf, self.outputs = db, pf, outputs
-        self.args = (want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep)
+        self.args = (want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep,
+                     field_cover)
         self.speculate, self.shard = speculate, shard
         self._res = None
 
@@ -918,7 +948,7 @@ class PendingBatch:
         if self._res is not None:
             return self._res
         db, pf, outputs = self.db, self.pf, self.outputs
-        want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep = self.args
+        want_curvature, selection, ranked, cand_base, copy_summary, winners, corner_bits, sweep, field_cover = self.args
         buffers = pf.buffers
         B, F = db.pb.n_cand, db.pb.n_fields
         k = selection.top_k
@@ -937,7 +967,8 @@ class PendingBatch:
             _Hints.drop(_Hints.key(db, outputs, want_curvature))
             self._res = _run_device_batch(db, outputs, want_curvature, selection, ranked, cand_base, copy_summary,
                                           buffers=None, fetch=True, winners=winners, corner_bits=corner_bits,
-                                          speculate=False, wait=True, shard=self.shard, obstacle_sweep=sweep)
+                                          speculate=False, wait=True, shard=self.shard, obstacle_sweep=sweep,
+                                          field_coverage=field_cover)
             return self._res
         if corner_bits:   # [B, stride] words on the device; batch.corner_grids() unpacks one candidate's
             res.extras["corner_bits"] = buffers.d_cbits[:B * buffers.cbits_stride].view(B, -1)
@@ -945,6 +976,8 @@ class PendingBatch:
         res.extras["d2h_bytes"] = len(res.summary) * rec + 16 * F * k + ((B + 1) * 8 if outputs == "paths" else 0)
         if sweep:
             res.extras["d2h_bytes"] += B * _lib.SWEEP_DTYPE.itemsize
+        if field_cover:
+            res.extras["d2h_bytes"] += B * _lib.PATH_COVER_DTYPE.itemsize
         if self.shard is not None:
             records = pf.hwin[:F * k * rec].view(_lib.SUMMARY_DTYPE).reshape(F, k)
             res.extras["winner_summary"] = records[:, 0].copy()
@@ -969,7 +1002,8 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
                      cost: str = "length", cand_base: int = 0, copy_summary: bool = True,
                      buffers: Optional[BatchBuffers] = None, fetch: bool = True,
                      winners: bool = False, corner_bits: bool = False, speculate: bool = False, wait: bool = True,
-                     shard: Optional[tuple] = None, select: Optional[Selection] = None, obstacle_sweep: bool = False):
+                     shard: Optional[tuple] = None, select: Optional[Selection] = None, obstacle_sweep: bool = False,
+                     field_coverage: bool = False):
     """Enqueue one batch on torch's current stream and (``fetch``) copy summaries + the per-field best back.
 
     With ``buffers`` (from a previous run of the same batch shape) and ``db.max_points`` known the
@@ -982,23 +1016,27 @@ def run_device_batch(db: DeviceBatch, outputs: str = "summary", want_curvature: 
     record of every ranked candidate gathered (``dist.reduce_topk``, ``dist.gather_winner_records``).  ``select``:
     the per-field top-k ranking (``BatchResult.topk_*``) instead of the argmin of ``cost``.  ``obstacle_sweep``: also
     each candidate's segment-level obstacle sweep (``BatchResult.sweep``; in a sharded batch, of this rank's
-    candidates)."""
+    candidates).  ``field_coverage`` (``outputs='paths'``): each candidate's whole-field and headland-band coverage
+    (``BatchResult.field_cover``, likewise of this rank's candidates)."""
+    if field_coverage and outputs != "paths":
+        raise ValueError("field_coverage=True needs outputs='paths': it measures the materialised paths")
     if select is not None:
         selection = select
     else:   # the argmin of the length or of the time: the plain selections (include/fcpp.h)
         selection = Selection() if cost == "length" else Selection(w_length=0.0, w_time=1.0)
     return _run_device_batch(db, outputs, want_curvature, selection, select is not None, cand_base, copy_summary,
-                             buffers, fetch, winners, corner_bits, speculate, wait, shard, obstacle_sweep)
+                             buffers, fetch, winners, corner_bits, speculate, wait, shard, obstacle_sweep, field_coverage)
 
 
 def _run_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, selection: Selection, ranked: bool,
                       cand_base: int, copy_summary: bool, buffers: Optional[BatchBuffers], fetch: bool, winners: bool,
-                      corner_bits: bool, speculate: bool, wait: bool, shard: Optional[tuple], obstacle_sweep: bool):
+                      corner_bits: bool, speculate: bool, wait: bool, shard: Optional[tuple], obstacle_sweep: bool,
+                      field_coverage: bool = False):
     """``run_device_batch`` with the ranking resolved: ``selection`` ranks every field, ``ranked`` = the caller asked
     for the ranking (``BatchResult.topk_*``)."""
     buffers, offsets = _launch_device_batch(db, outputs, want_curvature, selection, cand_base, buffers,
                                             corner_bits=corner_bits, speculate=speculate and copy_summary,
-                                            sweep=obstacle_sweep)
+                                            sweep=obstacle_sweep, field_cover=field_coverage)
     if not fetch:
         return None
     win = None
@@ -1010,9 +1048,9 @@ def _run_device_batch(db: DeviceBatch, outputs: str, want_curvature: bool, selec
         # every rank passes the mask whether or not IT speculated: the all-reduce must have the same shape everywhere
         win = dist.gather_winner_records(buffers.d_sum, buffers.d_best[:nfk], shard[0], shard[1],
                                          count_mask=_SIZE_FLAGS)
-    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win, obstacle_sweep)
+    pf = _enqueue_fetch(db, buffers, outputs, offsets, copy_summary, cand_base, win, obstacle_sweep, field_coverage)
     pend = PendingBatch(db, pf, outputs, want_curvature, selection, ranked, cand_base, copy_summary, winners,
-                        corner_bits, speculate and copy_summary, shard, obstacle_sweep)
+                        corner_bits, speculate and copy_summary, shard, obstacle_sweep, field_coverage)
     return pend if not wait else pend.result()
 
 
@@ -1021,7 +1059,7 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
                coverage: bool = True, cost: str = "length", device=None, want_curvature: bool = False,
                distributed: bool = False, turn_model: str = "arc", clothoid_share: float = 0.5,
                winners: bool = False, wait: bool = True, select: Optional[Selection] = None,
-               obstacle_sweep: bool = False):
+               obstacle_sweep: bool = False, field_coverage: bool = False):
     """Evaluate B candidate plans.  See ``prepare_batch`` for the inputs.
 
     Returns a ``BatchResult``: per-candidate ``summary`` records (layout counts, path lengths and
@@ -1054,6 +1092,12 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     layer the segments with metres inside the obstacle region and the sum of those metres.  It is read back with the
     summaries (no extra synchronisation) and changes no other output.
 
+    ``field_coverage=True`` (needs ``outputs='paths'``) also measures how much of each field its plan covers
+    (DESIGN.md §3.10): ``BatchResult.field_cover`` [B] (``_lib.PATH_COVER_DTYPE``) holds the cells of the whole field
+    covered by the W/2 buffer of both layers, the headland band's cells covered by the headland layer (the
+    summary's ``cov_total`` / ``cov_cells``) and D3's point counts, as ``verify_paths`` measures them on the same
+    path.  Read back with the summaries; no other output changes.
+
     ``wait=False`` returns a ``PendingBatch`` as soon as the batch is enqueued; its ``result()`` gives the
     BatchResult.  Submitting the next batch before collecting the previous one overlaps the host side of a call with
     the kernels of the other (see ``PendingBatch``).
@@ -1064,6 +1108,8 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
     ``winner_paths`` then holds the fields whose winner this rank owns."""
     if cost not in ("length", "time"):
         raise ValueError(f"cost must be 'length' or 'time', not {cost!r}")
+    if field_coverage and outputs != "paths":
+        raise ValueError("field_coverage=True needs outputs='paths': it measures the materialised paths")
     if select is not None:
         if not isinstance(select, Selection):
             raise ValueError(f"select must be a Selection, not {type(select).__name__}")
@@ -1073,13 +1119,13 @@ def plan_batch(fields, vehicle: Optional[VehicleParams] = None, candidates: Opti
         from . import dist
         return dist.plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h,
                                        coverage, cost, device, want_curvature, turn_model, clothoid_share, winners, wait,
-                                       select, obstacle_sweep)
+                                       select, obstacle_sweep, field_coverage)
     dev = _dev(device)
     pb = prepare_batch(fields, vehicle, candidates, obstacles, start_points, grid_h, coverage, turn_model,
                        clothoid_share)
     db = DeviceBatch(pb, dev)
     return run_device_batch(db, outputs, want_curvature, cost, winners=winners, speculate=True, wait=wait,
-                            select=select, obstacle_sweep=obstacle_sweep)
+                            select=select, obstacle_sweep=obstacle_sweep, field_coverage=field_coverage)
 
 
 def obstacle_sweep(paths, obstacles, working_width: float, n_main=None, device=None) -> np.ndarray:
@@ -1127,3 +1173,119 @@ def obstacle_sweep(paths, obstacles, working_width: float, n_main=None, device=N
         out[:] = d_out.cpu().numpy().view(_lib.SWEEP_DTYPE)
     return out
 
+
+
+def _fields_array(fields) -> np.ndarray:
+    fv = np.asarray(fields, dtype=np.float64)
+    if fv.shape == (4, 2):
+        fv = fv[None]
+    if fv.ndim != 3 or fv.shape[1:] != (4, 2) or len(fv) == 0:
+        raise ValueError("fields must be one [4, 2] quad or an [F, 4, 2] array of them")
+    if not np.isfinite(fv).all():
+        raise ValueError("field vertices must be finite")
+    e = np.roll(fv, -1, axis=1) - fv
+    cross = e[:, :, 0] * np.roll(e, -1, axis=1)[:, :, 1] - e[:, :, 1] * np.roll(e, -1, axis=1)[:, :, 0]
+    if not (cross > 0).all():
+        raise ValueError("every field must be a convex counter-clockwise quad")
+    return np.ascontiguousarray(fv)
+
+
+def _per_path(v, n: int, name: str, dtype) -> np.ndarray:
+    a = np.asarray(v, dtype=dtype)
+    if a.ndim == 0:
+        a = np.full(n, a, dtype=dtype)
+    if a.shape != (n,):
+        raise ValueError(f"{name} needs one value per path ({n}), not shape {a.shape}")
+    return np.ascontiguousarray(a)
+
+
+def verify_paths(paths, fields, vehicle: Optional[VehicleParams] = None, *, path_field=None, headland_width=None,
+                 obstacles=None, n_main=None, grid_h: float = 0.1, device=None) -> np.ndarray:
+    """The checks every generated plan carries, for caller-supplied paths on the GPU (DESIGN.md §3.10).
+
+    ``paths``: one [n, 2] array or a sequence of them (any lengths, 0 and 1 points too); ``fields``: one [4, 2] convex
+    CCW quad or [F, 4, 2] of them; ``path_field``: each path's field (may be omitted with one field);
+    ``headland_width`` (one value or one per path; default ``vehicle.min_turn_radius``): the band's R;
+    ``obstacles``: one (possibly empty) polygon list per field, as ``plan_batch``; the radius is
+    ``vehicle.working_width / 2``.  ``n_main`` (one int per path, or one int for a single path) splits a path into main
+    work (its first n_main points) and headland.  Without it n_main = 0: the whole path is the HEADLAND layer and counts
+    for both the band and the field (unlike ``obstacle_sweep``, whose default is all main work).
+
+    Returns a [n_paths] ``_lib.PATH_COVER_DTYPE`` array: D3's ``n_boundary_viol`` / ``n_obstacle_viol`` over every
+    point; ``band_total`` / ``band_cells``, the A11 headland band of (field, headland width) and its cells covered by
+    the headland layer (a plan's ``cov_total`` / ``cov_cells``); ``field_total`` / ``field_cells``, the whole field's
+    cells and those covered by both layers (the segment joining the layers counts for neither).  ``status``
+    ``_lib.PATH_OUT_OF_RANGE``: a point lies ~107 km or more from its field (every count 0).  Every input is checked
+    on the host before the device is touched: invalid input raises ValueError."""
+    vehicle = vehicle or VehicleParams()
+    fv = _fields_array(fields)
+    F = len(fv)
+    single = isinstance(paths, np.ndarray) and paths.ndim == 2
+    plist = [paths] if single else list(paths)
+    pts = []
+    for p in plist:
+        a = np.asarray(p, dtype=np.float64)
+        if a.size == 0:
+            a = a.reshape(0, 2)
+        if a.ndim != 2 or a.shape[1] != 2:
+            raise ValueError(f"every path must be an [n, 2] array, not shape {a.shape}")
+        if not np.isfinite(a).all():
+            raise ValueError("path coordinates must be finite")
+        pts.append(np.ascontiguousarray(a))
+    n = len(pts)
+    lens = np.array([len(p) for p in pts], dtype=np.int64)
+    if path_field is None:
+        if F != 1:
+            raise ValueError("path_field is required with more than one field")
+        path_field = 0
+    pf = _per_path(path_field, n, "path_field", np.int64)
+    if n and (pf.min() < 0 or pf.max() >= F):
+        raise ValueError(f"path_field must lie in [0, {F})")
+    hw = _per_path(vehicle.min_turn_radius if headland_width is None else headland_width, n, "headland_width",
+                   np.float64)
+    if not np.isfinite(hw).all():
+        raise ValueError("headland_width must be finite")
+    nm = np.zeros(n, dtype=np.int64)
+    if n_main is not None:
+        nm = np.atleast_1d(np.asarray(n_main))
+        if nm.ndim != 1 or len(nm) != n or not np.issubdtype(nm.dtype, np.integer):
+            raise ValueError("n_main needs one integer per path")
+        nm = nm.astype(np.int64)
+        if ((nm < 0) | (nm > lens)).any():
+            raise ValueError("n_main must lie in [0, len(path)]")
+    W = float(vehicle.working_width)
+    if not (W > 0 and math.isfinite(W)):
+        raise ValueError("working_width must be > 0")
+    hq = float(grid_h) * 1e4
+    if not (grid_h > 0 and math.isfinite(hq) and abs(hq - round(hq)) <= 1e-6 and round(hq) % 2 == 0):
+        raise ValueError(f"grid_h must be a positive even multiple of 1e-4 m, not {grid_h!r}")
+    if obstacles is not None:
+        for polys in obstacles:
+            for poly in polys:
+                o = np.asarray(poly, dtype=np.float64)
+                if o.ndim != 2 or o.shape[1] != 2 or len(o) < 3 or not np.isfinite(o).all():
+                    raise ValueError("every obstacle must be a polygon of >= 3 finite (x, y) vertices")
+    arrays: Dict[str, np.ndarray] = {}
+    _obstacle_tables(obstacles, F, W, arrays)
+    out = np.zeros(n, dtype=_lib.PATH_COVER_DTYPE)
+    if n == 0:
+        return out
+    offs = np.zeros(n + 1, dtype=np.int64)
+    offs[1:] = np.cumsum(lens)
+    arrays.update({"path": np.concatenate(pts) if offs[-1] else np.zeros((1, 2)), "offsets": offs,
+                   "field": pf.astype(np.int32), "hw": hw, "n_main": nm.astype(np.int32), "field_verts": fv})
+    dev = _dev(device)
+    h = _lib.handle(dev.index)
+    with torch.cuda.device(dev):
+        t = _pack_to_dev(arrays, dev)
+        d_out = torch.empty(n * _lib.PATH_COVER_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        obs = t.get("obs_poly_start")
+        h.check(h.lib.fcpp_path_coverage(h.h, t["path"].data_ptr(), t["offsets"].data_ptr(), n, t["n_main"].data_ptr(),
+                                         t["field"].data_ptr(), t["hw"].data_ptr(), F, t["field_verts"].data_ptr(),
+                                         obs.data_ptr() if obs is not None else None,
+                                         t["obs_vert_start"].data_ptr() if obs is not None else None,
+                                         t["obs_verts"].data_ptr() if obs is not None else None, W / 2, float(grid_h),
+                                         d_out.data_ptr(), stream))
+        out[:] = d_out.cpu().numpy().view(_lib.PATH_COVER_DTYPE)
+    return out

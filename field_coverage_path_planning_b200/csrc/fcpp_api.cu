@@ -153,6 +153,7 @@ void fcpp_destroy(fcpp_handle *h)
     if (h->d_ga) cudaFree(h->d_ga);
     if (h->d_dedupe) cudaFree(h->d_dedupe);
     if (h->d_sel) cudaFree(h->d_sel);
+    if (h->d_pcov) cudaFree(h->d_pcov);
     if (h->h_ga_state) cudaFreeHost(h->h_ga_state);
     if (h->ga_stream) cudaStreamDestroy(h->ga_stream);
     for (int k = 0; k < 4; ++k)
@@ -325,6 +326,83 @@ int fcpp_obstacle_sweep_paths(fcpp_handle *h, const double *d_path_xy, const int
     cudaError_t e = fcpp_launch_sweep_paths(h, d_path_xy, d_offsets, n_paths, d_n_main, d_obs_vert_start, d_obs_verts,
                                             n_polys, radius, d_out, (cudaStream_t)stream);
     if (e != cudaSuccess) return cuda_fail(h, e, "obstacle sweep kernel (paths)");
+    return FCPP_OK;
+}
+
+static bool grid_h_ok(double grid_h)
+{
+    const double hq = grid_h * FCPP_FIXED_UNIT;
+    const long long H = llrint(hq);
+    return isfinite(hq) && H >= 2 && !(H & 1) && fabs(hq - (double)H) <= 1e-6;
+}
+
+int fcpp_path_coverage(fcpp_handle *h, const double *d_path_xy, const int64_t *d_offsets, int64_t n_paths,
+                       const int32_t *d_n_main, const int32_t *d_path_field, const double *d_headland_width,
+                       int32_t n_fields, const double *d_field_verts, const int32_t *d_obs_poly_start,
+                       const int32_t *d_obs_vert_start, const double *d_obs_verts, double radius, double grid_h,
+                       fcpp_path_cover *d_out, void *stream)
+{
+    if (!h) return FCPP_ERR_INVALID;
+    if (n_paths < 0 || n_paths > 0x7fffffff || n_fields < 0 || !(radius >= 0.0) || !isfinite(radius) ||
+        (n_paths > 0 && (!d_path_xy || !d_offsets || !d_path_field || !d_headland_width || !d_out)) ||
+        (n_paths > 0 && n_fields > 0 && !d_field_verts) || (d_obs_poly_start && (!d_obs_vert_start || !d_obs_verts)))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_path_coverage: bad argument");
+    if (!grid_h_ok(grid_h))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_path_coverage: grid_h must be an even multiple of 1e-4 m (got %g)", grid_h);
+    cudaSetDevice(h->device);
+    PathCoverSrc src{};
+    src.path = d_path_xy;
+    src.offsets = d_offsets;
+    src.n = n_paths;
+    src.path_field = d_path_field;
+    src.headland_width = d_headland_width;
+    src.n_main = d_n_main;
+    src.n_fields = n_fields;
+    src.field_verts = d_field_verts;
+    src.obs_poly_start = d_obs_poly_start;
+    src.obs_vert_start = d_obs_vert_start;
+    src.obs_verts = d_obs_verts;
+    src.radius = radius;
+    src.grid_h = grid_h;
+    cudaError_t e = fcpp_launch_path_cover(h, src, d_out, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "path coverage kernels");
+    return FCPP_OK;
+}
+
+int fcpp_plan_coverage(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outputs *outputs, fcpp_path_cover *d_out,
+                       void *stream)
+{
+    int rc = check_batch(h, batch);
+    if (rc) return rc;
+    if (!outputs || !outputs->summary || !outputs->path_xy || !outputs->offsets)
+        return fail(h, FCPP_ERR_INVALID, "fcpp_plan_coverage: needs materialised paths (outputs.path_xy, offsets)");
+    if (batch->n_cand > 0 && !d_out) return fail(h, FCPP_ERR_INVALID, "fcpp_plan_coverage: d_out is NULL");
+    if (!grid_h_ok(batch->grid_h))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_plan_coverage: grid_h must be an even multiple of 1e-4 m (got %g)",
+                    batch->grid_h);
+    // the records must be those of this batch (the stamp of its layout pass, as fcpp_obstacle_sweep)
+    const void *id0 = batch->cand_field ? (const void *)batch->cand_R : (const void *)batch->ax_radii;
+    const void *id1 = batch->cand_field ? (const void *)batch->cand_flags : (const void *)(intptr_t)batch->cand_first;
+    if (!h->rec_valid || h->layout_ncand != batch->n_cand || h->layout_id[0] != id0 || h->layout_id[1] != id1 ||
+        h->layout_id[2] != batch->field_verts || h->layout_id[3] != stream)
+        return fail(h, FCPP_ERR_INVALID, "fcpp_layout and fcpp_plan_batch must be called for this batch (same arrays, "
+                                         "same stream) before fcpp_plan_coverage");
+    cudaSetDevice(h->device);
+    PathCoverSrc src{};
+    src.path = outputs->path_xy;
+    src.offsets = outputs->offsets;
+    src.n = batch->n_cand;
+    src.recs = h->d_rec;
+    src.summary = outputs->summary;
+    src.n_fields = batch->n_fields;
+    src.field_verts = batch->field_verts;
+    src.obs_poly_start = batch->obs_poly_start;
+    src.obs_vert_start = batch->obs_vert_start;
+    src.obs_verts = batch->obs_verts;
+    src.radius = batch->vehicle.working_width / 2;
+    src.grid_h = batch->grid_h;
+    cudaError_t e = fcpp_launch_path_cover(h, src, d_out, (cudaStream_t)stream);
+    if (e != cudaSuccess) return cuda_fail(h, e, "plan coverage kernels");
     return FCPP_OK;
 }
 

@@ -1870,7 +1870,439 @@ __global__ void __launch_bounds__(T) window_kernel(const double *__restrict__ pa
     if (tid == 0) *count = (int64_t)s.acc[0];
 }
 
+// ---------------------------------------------------------------------------------------------
+// Whole-field and headland-band coverage of polylines in device memory (include/fcpp.h fcpp_path_cover, DESIGN.md
+// §3.10): caller-supplied paths and materialised plans.  Three kernels:
+//   path_cover_prep_kernel  one CTA per path: D3 counts over every point, the lattice range check, the record's
+//                           status, and the number of row slabs of the path's field lattice;
+//   path_cover_scan_kernel  one CTA: the prefix sum of the slab counts (the work list), the work counter;
+//   path_cover_slab_kernel  a persistent grid over every (path, row slab): a slab is as many lattice rows as fit the
+//                           32 KB tile.  The CTA stages only the segments whose capsules can reach its rows,
+//                           rasterises the headland layer, counts the band windows, adds the main layer, counts the
+//                           field windows, and adds its four counts to the path's record with integer atomics.
+// ---------------------------------------------------------------------------------------------
+constexpr int PCOV_PC = 512;             // live segments staged per raster call
+constexpr int PCOV_PREP_T = 256;
+constexpr int PCOV_OBS = 256;            // obstacle boxes per staging round of the D3 counts
+constexpr int64_t PCOV_LIM = 1ll << 30;  // |point - lattice origin| in units (the rasteriser's int32 headroom)
+
+struct PcovExtra {
+    int4 bwin[ROWCAP];          // per slab row: band windows, cells [x, y] and [z, w] (empty: lo > hi)
+    unsigned long long acc[4];  // field cells, band cells, band cells covered, field cells covered
+    long long item;             // the (path, slab) work item
+    long long path;
+    int slab;
+    int n_live;                 // segments staged
+    int band;                   // 0 no band, 1 band = the whole field, 2 band = field minus the inset
+};
+constexpr size_t PCOV_OFF_X = a16(OFF_ENT + (size_t)PCOV_PC * sizeof(Entry));
+constexpr size_t PCOV_SMEM = PCOV_OFF_X + sizeof(PcovExtra);
+
+struct PathInfo {
+    int64_t o0;
+    int N, nm, field;
+    double hw;   // headland width
+    bool live;   // false: zero record
+    bool bad;    // field index outside [0, n_fields)
+};
+__device__ __forceinline__ PathInfo path_info(const PathCoverSrc &a, int64_t p)
+{
+    PathInfo q;
+    q.o0 = a.offsets[p];
+    q.N = (int)(a.offsets[p + 1] - q.o0);
+    q.bad = false;
+    if (a.recs) {
+        const CandRec &r = a.recs[p];
+        q.field = r.field;
+        q.hw = r.R;
+        q.nm = r.n_main;
+        q.live = r.status == 0 && r.n_total > 0 && !(a.summary[p].status & FCPP_CAND_TOO_LARGE);
+    } else {
+        q.field = a.path_field[p];
+        q.hw = a.headland_width[p];
+        q.nm = a.n_main ? a.n_main[p] : 0;
+        q.bad = q.field < 0 || q.field >= a.n_fields;
+        q.live = !q.bad;
+    }
+    q.nm = min(max(q.nm, 0), q.N);
+    return q;
+}
+
+// A11's lattice of a field (cover_body): cell centres (Xc0 + i H, Yc0 + j H), i < nx, j < ny; rows of rw words, `rows`
+// rows per slab
+struct PathLattice {
+    int64_t Xc0, Yc0;
+    int H, nx, ny, rw, rows, nslab;
+    bool ok;
+};
+__device__ __forceinline__ PathLattice path_lattice(const double *fv, double grid_h)
+{
+    double bx0 = 1e300, by0 = 1e300, bx1 = -1e300, by1 = -1e300;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        bx0 = fmin(bx0, fv[2 * k]);
+        by0 = fmin(by0, fv[2 * k + 1]);
+        bx1 = fmax(bx1, fv[2 * k]);
+        by1 = fmax(by1, fv[2 * k + 1]);
+    }
+    PathLattice L;
+    const int64_t H64 = qfix(grid_h);
+    const int64_t X0 = qfix(bx0), Y0 = qfix(by0);
+    const int64_t nx64 = ceil_div64(qfix(bx1) - X0, H64), ny64 = ceil_div64(qfix(by1) - Y0, H64);
+    L.Xc0 = X0 + H64 / 2;
+    L.Yc0 = Y0 + H64 / 2;
+    L.ok = nx64 > 0 && ny64 > 0 && nx64 * H64 < PCOV_LIM && ny64 * H64 < PCOV_LIM && H64 < (1 << 20) &&
+           (nx64 + 31) / 32 <= TW;
+    L.H = (int)H64;
+    L.nx = L.ok ? (int)nx64 : 0;
+    L.ny = L.ok ? (int)ny64 : 0;
+    L.rw = (L.nx + 31) >> 5;
+    L.rows = L.ok ? min(ROWCAP, TW / L.rw) : 1;
+    L.nslab = L.ok ? (L.ny + L.rows - 1) / L.rows : 0;
+    return L;
+}
+
+__global__ void __launch_bounds__(PCOV_PREP_T) path_cover_prep_kernel(const PathCoverSrc a, fcpp_path_cover *__restrict__ out,
+                                                                      int64_t *__restrict__ slabs)
+{
+    constexpr int TP = PCOV_PREP_T;
+    __shared__ double geo[20];
+    __shared__ double bb[4 * PCOV_OBS];
+    __shared__ int red[3][TP / 32];
+    const int tid = threadIdx.x;
+    const int64_t p = blockIdx.x;
+    const PathInfo q = path_info(a, p);
+    if (!q.live) {
+        if (tid == 0) {
+            out[p] = fcpp_path_cover{q.bad ? FCPP_PATH_OUT_OF_RANGE : 0, 0, 0, 0, 0, 0, 0, 0};
+            slabs[p] = 0;
+        }
+        return;
+    }
+    const double *fv = a.field_verts + 8 * (int64_t)q.field;
+    const PathLattice L = path_lattice(fv, a.grid_h);
+    if (tid < 4) {  // the plan kernel's geofence table: cross(e, p - v) < -eps*|e|
+        const int k = tid, k1 = (k + 1) & 3;
+        const double ax = fv[2 * k], ay = fv[2 * k + 1];
+        const double ex = fv[2 * k1] - ax, ey = fv[2 * k1 + 1] - ay;
+        geo[5 * k] = ax;
+        geo[5 * k + 1] = ay;
+        geo[5 * k + 2] = ex;
+        geo[5 * k + 3] = ey;
+        const double el = sqrt(ex * ex + ey * ey);
+        geo[5 * k + 4] = -FCPP_GEOFENCE_EPS * el;
+    }
+    int p0 = 0, np = 0;
+    if (a.obs_poly_start) {
+        p0 = a.obs_poly_start[q.field];
+        np = a.obs_poly_start[q.field + 1] - p0;
+    }
+    const int nchunk = np > 0 ? (np + PCOV_OBS - 1) / PCOV_OBS : 1;
+    const double rr = a.radius, r2 = rr * rr;
+    const double2 *pts = reinterpret_cast<const double2 *>(a.path) + q.o0;
+    int nb = 0, no = 0, far = 0;
+    for (int i0 = 0; i0 < q.N; i0 += TP) {
+        const int i = i0 + tid;
+        const bool have = i < q.N;
+        double x = 0.0, y = 0.0;
+        if (have) {
+            const double2 v = pts[i];
+            x = v.x;
+            y = v.y;
+            const int64_t rx = qfix(x) - L.Xc0, ry = qfix(y) - L.Yc0;
+            if (!(rx > -PCOV_LIM && rx < PCOV_LIM && ry > -PCOV_LIM && ry < PCOV_LIM)) far = 1;
+        }
+        int outb = 0, hit = 0;
+        for (int c = 0; c < nchunk; ++c) {
+            const int pc0 = c * PCOV_OBS, npc = max(min(PCOV_OBS, np - pc0), 0);
+            if (nchunk > 1 || i0 == 0) {  // the boxes of this chunk of polygons, as the plan kernel grows them
+                __syncthreads();
+                for (int u = tid; u < npc; u += TP) {
+                    double x0 = 1e300, y0 = 1e300, x1 = -1e300, y1 = -1e300;
+                    for (int v = a.obs_vert_start[p0 + pc0 + u]; v < a.obs_vert_start[p0 + pc0 + u + 1]; ++v) {
+                        x0 = fmin(x0, a.obs_verts[2 * (int64_t)v]);
+                        x1 = fmax(x1, a.obs_verts[2 * (int64_t)v]);
+                        y0 = fmin(y0, a.obs_verts[2 * (int64_t)v + 1]);
+                        y1 = fmax(y1, a.obs_verts[2 * (int64_t)v + 1]);
+                    }
+                    bb[4 * u] = x0 - rr - 1e-6;
+                    bb[4 * u + 1] = y0 - rr - 1e-6;
+                    bb[4 * u + 2] = x1 + rr + 1e-6;
+                    bb[4 * u + 3] = y1 + rr + 1e-6;
+                }
+                __syncthreads();
+            }
+            if (have) {
+                const int m = point_tests_impl(geo, a.obs_verts, bb, a.obs_vert_start ? a.obs_vert_start + p0 + pc0 : nullptr,
+                                               npc, r2, x, y);
+                if (c == 0) outb = m & 1;
+                hit |= m >> 1;
+            }
+        }
+        nb += outb;
+        no += hit;
+    }
+    nb = __reduce_add_sync(0xffffffffu, nb);
+    no = __reduce_add_sync(0xffffffffu, no);
+    far = __reduce_or_sync(0xffffffffu, far);
+    if ((tid & 31) == 0) {
+        red[0][tid >> 5] = nb;
+        red[1][tid >> 5] = no;
+        red[2][tid >> 5] = far;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < TP / 32; ++w) {
+            nb += red[0][w];
+            no += red[1][w];
+            far |= red[2][w];
+        }
+        fcpp_path_cover rec{0, 0, 0, 0, 0, 0, 0, 0};
+        int64_t ns = 0;
+        if (far) {
+            rec.status = FCPP_PATH_OUT_OF_RANGE;
+        } else {
+            rec.n_boundary_viol = nb;
+            rec.n_obstacle_viol = no;
+            if (!L.ok) rec.status = FCPP_CAND_GRID_TOO_LARGE | FCPP_CAND_BAND_GRID_TOO_LARGE;
+            ns = L.nslab;
+        }
+        out[p] = rec;
+        slabs[p] = ns;
+    }
+}
+
+// exclusive prefix sum of the slab counts in place (slabs[n] = total) and the work counter = 0; one CTA
+__global__ void __launch_bounds__(1024) path_cover_scan_kernel(int64_t n, int64_t *__restrict__ slabs,
+                                                               unsigned long long *__restrict__ counter)
+{
+    __shared__ long long wsum[32];
+    __shared__ long long carry;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid == 0) {
+        carry = 0;
+        *counter = 0ull;
+    }
+    for (int64_t b = 0; b < n; b += 1024) {
+        const int64_t i = b + tid;
+        const long long v = i < n ? slabs[i] : 0;
+        long long inc = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const long long o = __shfl_up_sync(0xffffffffu, inc, d);
+            if (lane >= d) inc += o;
+        }
+        __syncthreads();  // carry is final; wsum is free
+        if (lane == 31) wsum[warp] = inc;
+        __syncthreads();
+        long long pre = carry;
+        for (int w = 0; w < warp; ++w) pre += wsum[w];
+        if (i < n) slabs[i] = pre + inc - v;
+        __syncthreads();
+        if (tid == 1023) carry = pre + inc;
+    }
+    __syncthreads();
+    if (tid == 0) slabs[n] = carry;
+}
+
+// bits of the cells [lo, hi] in word wi of a row
+__device__ __forceinline__ uint32_t span_mask(int lo, int hi, int wi)
+{
+    const int c0 = wi << 5;
+    if (lo > hi || hi < c0 || lo > c0 + 31) return 0u;
+    const int a = max(lo - c0, 0), b = min(hi - c0, 31);
+    return (0xffffffffu << a) & (0xffffffffu >> (31 - b));
+}
+
+__device__ __forceinline__ unsigned long long block_sum_u64(unsigned long long v)
+{
+#pragma unroll
+    for (int dd = 16; dd > 0; dd >>= 1) v += __shfl_xor_sync(0xffffffffu, v, dd);
+    return v;
+}
+
+// one row slab of one path
+__device__ __forceinline__ void path_cover_slab(const PathCoverSrc &a, fcpp_path_cover *rec, int64_t p, int slab)
+{
+    CoverFixed &s = *reinterpret_cast<CoverFixed *>(cover_smem);
+    PcovExtra &x = *reinterpret_cast<PcovExtra *>(cover_smem + PCOV_OFF_X);
+    const CoverDyn d;
+    const int tid = threadIdx.x;
+    const PathInfo q = path_info(a, p);
+    const double *fv = a.field_verts + 8 * (int64_t)q.field;
+    const PathLattice L = path_lattice(fv, a.grid_h);
+    const int H = L.H, nx = L.nx, rw = L.rw;
+    const double invH = 1.0 / (double)H;
+    const int j0 = slab * L.rows, nrows = min(L.rows, L.ny - j0);
+    const int rq = (int)qfix(a.radius);
+    const double rd = (double)rq;
+    if (tid < 4) s.fq[tid] = make_int2((int)(qfix(fv[2 * tid]) - L.Xc0), (int)(qfix(fv[2 * tid + 1]) - L.Yc0));
+    if (tid == 0) {
+        int band = q.hw > 0.0 ? 1 : 0;
+        if (band) {  // D1 as the layout kernel: an inset that fails or has |area| < 1 m^2 leaves the whole field
+            double v[4][2], mq[4][2];
+            for (int k = 0; k < 4; ++k) {
+                v[k][0] = fv[2 * k];
+                v[k][1] = fv[2 * k + 1];
+            }
+            const bool ok = inset4(v, q.hw, mq);
+            if (ok && !(fabs(signed_area4(mq)) < 1.0)) {
+                band = 2;
+                for (int k = 0; k < 4; ++k) s.mq[k] = make_int2((int)(qfix(mq[k][0]) - L.Xc0), (int)(qfix(mq[k][1]) - L.Yc0));
+            }
+        }
+        x.band = band;
+        x.n_live = 0;
+        for (int k = 0; k < 4; ++k) x.acc[k] = 0ull;
+        s.tg[0].j0 = j0;
+        s.tg[0].nrows = nrows;
+        s.tg[0].koff = 0;
+    }
+    __syncthreads();
+    const int band = x.band;
+    if (tid < 4) quad_edges_setup(s.fq, s.qedge[0], s.qtype[0], tid);
+    if (tid >= 4 && tid < 8 && band == 2) quad_edges_setup(s.mq, s.qedge[1], s.qtype[1], tid - 4);
+    __syncthreads();
+    // row windows: the field interval is the only window the rasteriser writes (rows of rw words); the band windows
+    // (band_windows_of, as the coverage kernel) are counted from the same bits
+    unsigned long long ft = 0ull, bt = 0ull;
+    for (int k = tid; k < nrows; k += T) {
+        const int cy = (j0 + k) * H;
+        int4 v = make_int4(0, -1, 1, 0);
+        quad_row_interval(s.fq, s.qedge[0], s.qtype[0], cy, H, invH, nx, v.x, v.y);
+        if (band == 2) quad_row_interval(s.mq, s.qedge[1], s.qtype[1], cy, H, invH, nx, v.z, v.w);
+        s.rwin[k] = make_int4(v.x, v.y, 1, 0);
+        s.rbias[k] = make_int2(k * rw, 0);
+        const int4 bw = band ? band_windows_of(v) : make_int4(1, 0, 1, 0);
+        x.bwin[k] = bw;
+        ft += (unsigned long long)max(v.y - v.x + 1, 0);
+        bt += (unsigned long long)(max(bw.y - bw.x + 1, 0) + max(bw.w - bw.z + 1, 0));
+    }
+    zero_words(s.tile, nrows * rw);
+    unsigned long long bc = 0ull, fc = 0ull;
+    if (__syncthreads_or(ft != 0ull)) {
+        const double2 *pts = reinterpret_cast<const double2 *>(a.path) + q.o0;
+        // a capsule reaches a row of the slab only if its segment's box grown by r meets the slab's box
+        const int64_t ylo = (int64_t)j0 * H - rq, yhi = (int64_t)(j0 + nrows - 1) * H + rq;
+        const int64_t xlo = -(int64_t)rq, xhi = (int64_t)(nx - 1) * H + rq;
+        auto raster_layer = [&](int s0, int s1) {  // segments i -> i + 1, i in [s0, s1)
+            for (int b = s0; b < s1; b += T) {
+                const int i = b + tid;
+                bool take = false;
+                int2 pa = make_int2(0, 0), pb = make_int2(0, 0);
+                if (i < s1) {
+                    const double2 u = pts[i], w = pts[i + 1];
+                    const int64_t ax = qfix(u.x) - L.Xc0, ay = qfix(u.y) - L.Yc0;
+                    const int64_t bx = qfix(w.x) - L.Xc0, by = qfix(w.y) - L.Yc0;
+                    take = min(ay, by) < yhi && max(ay, by) > ylo && min(ax, bx) < xhi && max(ax, bx) > xlo;
+                    pa = make_int2((int)ax, (int)ay);
+                    pb = make_int2((int)bx, (int)by);
+                }
+                const unsigned m = __ballot_sync(0xffffffffu, take);
+                int base = 0;
+                if ((tid & 31) == 0 && m) base = atomicAdd(&x.n_live, __popc(m));
+                base = __shfl_sync(0xffffffffu, base, 0);
+                if (take) write_entry(d, base + __popc(m & ((1u << (tid & 31)) - 1u)), pa, pb, rd);
+                __syncthreads();
+                const int n_live = x.n_live;
+                __syncthreads();  // every thread has read the count before the next round adds to it
+                if (n_live > PCOV_PC - T || b + T >= s1) {
+                    if (n_live) raster_entries(s, d, 0, n_live, [](int) { return 0; }, rq, H, invH);
+                    __syncthreads();
+                    if (tid == 0) x.n_live = 0;
+                    __syncthreads();
+                }
+            }
+        };
+        raster_layer(q.nm, q.N - 1);  // the headland layer
+        if (band)
+            for (int w = tid; w < nrows * rw; w += T) {
+                const uint32_t bits = s.tile[w];
+                if (!bits) continue;
+                const int k = w / rw, wi = w - k * rw;
+                const int4 bw = x.bwin[k];
+                bc += (unsigned long long)(__popc(bits & span_mask(bw.x, bw.y, wi)) + __popc(bits & span_mask(bw.z, bw.w, wi)));
+            }
+        __syncthreads();
+        raster_layer(0, q.nm - 1);  // the main layer (the junction nm - 1 -> nm belongs to neither)
+        fc = (unsigned long long)count_words(s.tile, nrows * rw);
+    }
+    ft = block_sum_u64(ft);
+    bt = block_sum_u64(bt);
+    bc = block_sum_u64(bc);
+    fc = block_sum_u64(fc);
+    if ((tid & 31) == 0) {
+        if (ft) atomicAdd(&x.acc[0], ft);
+        if (bt) atomicAdd(&x.acc[1], bt);
+        if (bc) atomicAdd(&x.acc[2], bc);
+        if (fc) atomicAdd(&x.acc[3], fc);
+    }
+    __syncthreads();
+    if (tid == 0) {
+        if (x.acc[0]) atomicAdd(reinterpret_cast<unsigned long long *>(&rec->field_total), x.acc[0]);
+        if (x.acc[1]) atomicAdd(reinterpret_cast<unsigned long long *>(&rec->band_total), x.acc[1]);
+        if (x.acc[2]) atomicAdd(reinterpret_cast<unsigned long long *>(&rec->band_cells), x.acc[2]);
+        if (x.acc[3]) atomicAdd(reinterpret_cast<unsigned long long *>(&rec->field_cells), x.acc[3]);
+    }
+}
+
+// persistent grid over the work list: item k is slab k - slabs[p] of the last path p with slabs[p] <= k
+__global__ void __launch_bounds__(T, FCPP_COVER_MINBLOCKS) path_cover_slab_kernel(const PathCoverSrc a,
+                                                                                  fcpp_path_cover *__restrict__ out,
+                                                                                  const int64_t *__restrict__ slabs,
+                                                                                  unsigned long long *__restrict__ counter)
+{
+    PcovExtra &x = *reinterpret_cast<PcovExtra *>(cover_smem + PCOV_OFF_X);
+    const long long total = slabs[a.n];
+    while (true) {
+        __syncthreads();  // the previous item is done with the shared memory
+        if (threadIdx.x == 0) {
+            const long long item = (long long)atomicAdd(counter, 1ull);
+            x.item = item;
+            if (item < total) {
+                int64_t lo = 0, hi = a.n - 1;
+                while (lo < hi) {
+                    const int64_t mid = (lo + hi + 1) >> 1;
+                    if (slabs[mid] <= item)
+                        lo = mid;
+                    else
+                        hi = mid - 1;
+                }
+                x.path = lo;
+                x.slab = (int)(item - slabs[lo]);
+            }
+        }
+        __syncthreads();
+        if (x.item >= total) return;
+        const int64_t p = x.path;
+        path_cover_slab(a, out + p, p, x.slab);
+    }
+}
+
 }  // namespace
+
+cudaError_t fcpp_launch_path_cover(fcpp_handle *h, const PathCoverSrc &src, fcpp_path_cover *d_out, cudaStream_t st)
+{
+    if (src.n == 0) return cudaSuccess;
+    const size_t need = (size_t)(src.n + 2) * sizeof(int64_t);
+    if (need > h->pcov_bytes) {
+        if (h->d_pcov) cudaFree(h->d_pcov);
+        h->d_pcov = nullptr;
+        h->pcov_bytes = 0;
+        cudaError_t e = cudaMalloc(&h->d_pcov, need);
+        if (e != cudaSuccess) return e;
+        h->pcov_bytes = need;
+    }
+    int64_t *slabs = (int64_t *)h->d_pcov;
+    unsigned long long *counter = (unsigned long long *)(slabs + src.n + 1);
+    path_cover_prep_kernel<<<(unsigned)src.n, PCOV_PREP_T, 0, st>>>(src, d_out, slabs);
+    path_cover_scan_kernel<<<1, 1024, 0, st>>>(src.n, slabs, counter);
+    cudaError_t e = cudaFuncSetAttribute(path_cover_slab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PCOV_SMEM);
+    if (e != cudaSuccess) return e;
+    path_cover_slab_kernel<<<(unsigned)(FCPP_COVER_MINBLOCKS * h->sm_count), T, PCOV_SMEM, st>>>(src, d_out, slabs, counter);
+    h->launches += 3;
+    return cudaGetLastError();
+}
 
 #ifdef FCPP_COVER_TRACE
 // the trace records of the coverage tasks since the previous call (at most cap of them are copied); resets the trace

@@ -98,6 +98,8 @@ struct fcpp_handle {
     cudaStream_t ga_stream;  // capture stream of the generation graph
     void *d_sel;             // top-k selection workspace (fcpp_select.cu): field counts, keys sorted by field, unit lists
     size_t sel_bytes;
+    void *d_pcov;            // path coverage (fcpp_cover.cu): per-path first slab [n + 1], the slab counter
+    size_t pcov_bytes;
     char err[512];
 };
 
@@ -316,6 +318,48 @@ __device__ inline void centroid4(const double (*v)[2], double &cx, double &cy)
     }
     cx = ox + sx / (3.0 * a2);
     cy = oy + sy / (3.0 * a2);
+}
+
+// D3 geofence and obstacle (D2/D3) tests of one point, shared by the plan kernel and the path coverage kernels:
+// bit 0 = outside the field by more than 1e-9 m (geo [4][5]: edge start ax, ay, edge ex, ey, -1e-9 |e|), bit 1 = inside
+// an obstacle polygon or closer than r to one of its edges (obs_bb [n][4]: the polygons' boxes grown by r + 1e-6;
+// obs_vs [n + 1]: their vertex ranges in obs_xy).  The tables are handed over as four __restrict__ pointers instead
+// of through the plan kernel's shared-memory struct: measured 2-5 % on the plan kernel (a non-inlined single copy,
+// tried against the instruction-fetch stalls, cost 15-30 %).
+__device__ __forceinline__ int point_tests_impl(const double *__restrict__ geo, const double *__restrict__ obs_xy,
+                                                const double *__restrict__ obs_bb, const int32_t *__restrict__ obs_vs,
+                                                int n_obs_poly, double r2, double x, double y)
+{
+    bool outb = false;
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+        outb = outb || (geo[5 * k + 2] * (y - geo[5 * k + 1]) - geo[5 * k + 3] * (x - geo[5 * k]) < geo[5 * k + 4]);
+    bool hit = false;
+    for (int p = 0; p < n_obs_poly && !hit; ++p) {
+        if (x < obs_bb[4 * p] || y < obs_bb[4 * p + 1] || x > obs_bb[4 * p + 2] || y > obs_bb[4 * p + 3]) continue;
+        const int vs = obs_vs[p], ve = obs_vs[p + 1];
+        bool inside = false;
+        for (int q = vs; q < ve; ++q) {
+            const int q1 = (q + 1 < ve) ? q + 1 : vs;
+            const double ax = obs_xy[2 * q], ay = obs_xy[2 * q + 1];
+            const double bx = obs_xy[2 * q1], by = obs_xy[2 * q1 + 1];
+            // even-odd crossing (oracle/geom.py point_in_polygon_crossing)
+            if ((ay > y) != (by > y)) {
+                const double xi = ax + (y - ay) * (bx - ax) / (by - ay);
+                if (x < xi) inside = !inside;
+            }
+            // D2 distance test (oracle/geom.py dist2_point_segment)
+            const double dx = bx - ax, dy = by - ay, wx = x - ax, wy = y - ay;
+            const double dd = dx * dx + dy * dy;
+            const double tt_ = wx * dx + wy * dy;
+            double u = dd > 0.0 ? tt_ / dd : 0.0;
+            u = fmin(fmax(u, 0.0), 1.0);
+            const double qx = wx - u * dx, qy = wy - u * dy;
+            hit = hit || (qx * qx + qy * qy < r2);
+        }
+        hit = hit || inside;
+    }
+    return (outb ? 1 : 0) | (hit ? 2 : 0);
 }
 
 // x / y for a compile-time constant y, correctly rounded, in three instructions instead of the generic FP64
@@ -799,3 +843,23 @@ cudaError_t fcpp_launch_sweep(fcpp_handle *h, const fcpp_batch &b, fcpp_sweep *d
 cudaError_t fcpp_launch_sweep_paths(fcpp_handle *h, const double *d_path, const int64_t *d_offsets, int64_t n_paths,
                                     const int32_t *d_n_main, const int32_t *d_vert_start, const double *d_verts,
                                     int32_t n_polys, double radius, fcpp_sweep *d_out, cudaStream_t st);
+// whole-field / headland-band coverage and D3 counts of polylines in device memory (fcpp_cover.cu)
+struct PathCoverSrc {
+    const double *path;           // [total][2]
+    const int64_t *offsets;       // [n + 1]
+    int64_t n;
+    // caller paths: per path its field, headland width and main-work points (n_main NULL: 0)
+    const int32_t *path_field;
+    const double *headland_width;
+    const int32_t *n_main;
+    // materialised plans (recs != NULL): field, R and n_main from the candidate records; a record with a status, no
+    // points, or whose summary has FCPP_CAND_TOO_LARGE (its path was not written) is skipped
+    const CandRec *recs;
+    const fcpp_summary *summary;
+    int32_t n_fields;
+    const double *field_verts;    // [F][4][2]
+    const int32_t *obs_poly_start, *obs_vert_start;  // fcpp_batch layout; obs_poly_start NULL: no obstacles
+    const double *obs_verts;
+    double radius, grid_h;
+};
+cudaError_t fcpp_launch_path_cover(fcpp_handle *h, const PathCoverSrc &src, fcpp_path_cover *d_out, cudaStream_t st);

@@ -357,44 +357,7 @@ __device__ __forceinline__ double final_speed(bool act, double u, double u_lim, 
     return v;
 }
 
-// geofence (D3) and obstacle (D2/D3) point tests of one generated point.  The tables are handed over as four
-// __restrict__ pointers instead of through the GenSmem struct: measured 2-5 % on the plan kernel (a non-inlined
-// single copy, tried against the instruction-fetch stalls, cost 15-30 %).
-__device__ __forceinline__ int point_tests_impl(const double *__restrict__ geo, const double *__restrict__ obs_xy,
-                                                const double *__restrict__ obs_bb, const int32_t *__restrict__ obs_vs,
-                                                int n_obs_poly, double r2, double x, double y)
-{
-    bool outb = false;
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-        outb = outb || (geo[5 * k + 2] * (y - geo[5 * k + 1]) - geo[5 * k + 3] * (x - geo[5 * k]) < geo[5 * k + 4]);
-    bool hit = false;
-    for (int p = 0; p < n_obs_poly && !hit; ++p) {
-        if (x < obs_bb[4 * p] || y < obs_bb[4 * p + 1] || x > obs_bb[4 * p + 2] || y > obs_bb[4 * p + 3]) continue;
-        const int vs = obs_vs[p], ve = obs_vs[p + 1];
-        bool inside = false;
-        for (int q = vs; q < ve; ++q) {
-            const int q1 = (q + 1 < ve) ? q + 1 : vs;
-            const double ax = obs_xy[2 * q], ay = obs_xy[2 * q + 1];
-            const double bx = obs_xy[2 * q1], by = obs_xy[2 * q1 + 1];
-            // even-odd crossing (oracle/geom.py point_in_polygon_crossing)
-            if ((ay > y) != (by > y)) {
-                const double xi = ax + (y - ay) * (bx - ax) / (by - ay);
-                if (x < xi) inside = !inside;
-            }
-            // D2 distance test (oracle/geom.py dist2_point_segment)
-            const double dx = bx - ax, dy = by - ay, wx = x - ax, wy = y - ay;
-            const double dd = dx * dx + dy * dy;
-            const double tt_ = wx * dx + wy * dy;
-            double u = dd > 0.0 ? tt_ / dd : 0.0;
-            u = fmin(fmax(u, 0.0), 1.0);
-            const double qx = wx - u * dx, qy = wy - u * dy;
-            hit = hit || (qx * qx + qy * qy < r2);
-        }
-        hit = hit || inside;
-    }
-    return (outb ? 1 : 0) | (hit ? 2 : 0);
-}
+// geofence (D3) and obstacle (D2/D3) point tests of one generated point (point_tests_impl, fcpp_internal.cuh)
 __device__ __forceinline__ void point_tests(const GenSmem &s, int n_obs_poly, double r2, double x, double y, int &n_bviol,
                                             int &n_oviol)
 {

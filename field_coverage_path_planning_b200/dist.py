@@ -132,14 +132,14 @@ def gather_winner_records(summary_bytes: torch.Tensor, best_cand: torch.Tensor, 
 
 def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, outputs, grid_h, coverage, cost,
                        device, want_curvature, turn_model="arc", clothoid_share=0.5, winners=False, wait=True,
-                       select=None, obstacle_sweep=False):
+                       select=None, obstacle_sweep=False, field_coverage=False):
     """plan_batch over all ranks of the default process group (see batch.plan_batch): every rank plans its
     contiguous shard; ONE all-gather + merge kernel gives every rank the per-field ranking (the argmin of ``cost``, or
     the top-k of ``select``), one kernel + one all-reduce the summary record of every ranked candidate; the local
     summaries, the merged ranking and the records come back to the host with ONE synchronisation.  Launch sizes are
     remembered from earlier batches of the same shape (no layout read-back); ``wait=False`` returns a
     ``batch.PendingBatch``.  With ``obstacle_sweep`` each rank gets the sweep of its own candidates
-    (``BatchResult.sweep``)."""
+    (``BatchResult.sweep``), with ``field_coverage`` its own candidates' coverage records (``BatchResult.field_cover``)."""
     from .batch import DeviceBatch, _dev, axes_count, is_axes, prepare_batch, run_device_batch
     if not dist.is_initialized():
         raise RuntimeError("distributed=True needs torch.distributed.init_process_group (backend 'nccl')")
@@ -155,4 +155,4 @@ def plan_batch_sharded(fields, vehicle, candidates, obstacles, start_points, out
     pb = prepare_batch(fv, vehicle, local, obstacles, sp, grid_h, coverage, turn_model, clothoid_share)
     db = DeviceBatch(pb, dev)
     return run_device_batch(db, outputs, want_curvature, cost, lo, winners=winners, speculate=True, wait=wait,
-                            shard=(lo, hi), select=select, obstacle_sweep=obstacle_sweep)
+                            shard=(lo, hi), select=select, obstacle_sweep=obstacle_sweep, field_coverage=field_coverage)

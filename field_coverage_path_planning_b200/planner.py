@@ -22,7 +22,7 @@ import torch
 
 from . import _geometry as G
 from . import _lib
-from .batch import DeviceBatch, _dev, corner_grids, obstacle_sweep, prepare_batch, run_device_batch
+from .batch import DeviceBatch, _dev, corner_grids, obstacle_sweep, prepare_batch, run_device_batch, verify_paths
 from .vehicle import VehicleParams
 
 APPROACH_POINTS = 50  # mlp3:1317
@@ -274,6 +274,29 @@ class TwoLayerPathPlannerV37:
                 'metres_main': float(sw["len_main"]), 'metres_head': float(sw["len_head"]),
                 'segments': segs, 'metres': float(sw["len_main"]) + float(sw["len_head"]),
                 'point_violations': points, 'pass': segs == 0}
+
+    def verify_field_coverage(self, path=None, n_main: Optional[int] = None) -> Dict:
+        """How much of the field a path covers, on the A11 lattice (DESIGN.md §3.10).
+
+        ``path=None``: the last plan (``main_work.path`` then ``headland.path``, planned first if there is none);
+        otherwise a caller-supplied [n, 2] path whose first ``n_main`` points are main work — without ``n_main`` the
+        whole path is the headland layer (unlike ``verify_obstacle_clearance``, whose default is all main work).
+        Returns ``field_coverage_rate`` (cells of the whole field covered by the W/2 buffer of both layers),
+        ``band_coverage_rate`` (the headland band's cells covered by the headland layer: the plan's ``coverage_rate``),
+        their cells and totals, and D3's point counts ``boundary_violations`` / ``obstacle_violations``."""
+        if path is None:
+            if self._last_path is None:
+                self.plan_complete_coverage()
+            path, n_main = self._last_path
+        path = np.ascontiguousarray(path, dtype=np.float64).reshape(-1, 2)
+        r = verify_paths([path], [self.field_vertices], self.vehicle, headland_width=self.headland_width,
+                         obstacles=[self.obstacles], n_main=[0 if n_main is None else int(n_main)], grid_h=self.grid_h,
+                         device=self._device)[0]
+        ft, fc, bt, bc = (int(r[k]) for k in ("field_total", "field_cells", "band_total", "band_cells"))
+        return {'field_coverage_rate': fc / ft if ft else 0.0, 'band_coverage_rate': bc / bt if bt else 0.0,
+                'field_cells': fc, 'field_total': ft, 'band_cells': bc, 'band_total': bt,
+                'boundary_violations': int(r["n_boundary_viol"]), 'obstacle_violations': int(r["n_obstacle_viol"]),
+                'status': int(r["status"])}
 
     def verify_corner_coverage_grid_based(self, corner, corner_index: int, turn_path, reverse_path=None) -> Dict:
         """mlp3:1426-1510 with the exact fixed-point predicate (D5)."""

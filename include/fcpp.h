@@ -318,6 +318,51 @@ int fcpp_obstacle_sweep_paths(fcpp_handle *h, const double *d_path_xy, const int
                               const int32_t *d_n_main, const int32_t *d_obs_vert_start, const double *d_obs_verts,
                               int32_t n_polys, double radius, fcpp_sweep *d_out, void *stream);
 
+/* ---- whole-field and headland-band coverage of polylines in device memory (DESIGN.md §3.10) ----
+ * The lattice is A11's: cell centres q(bbox_min) + H/2 + (i H, j H) of the path's field, H = q(grid_h),
+ * q(x) = rint(x 1e4).  A cell is covered by a set of segments iff its centre lies strictly within r = W/2 of one of
+ * them (the exact 128-bit predicate, D2/D5).  A path is main work (its first n_main points) then headland; the
+ * segment from the last main point to the first headland point belongs to neither layer.
+ *   field cells: centre inside-or-on the field quad; field_cells counts those covered by the segments of BOTH layers.
+ *   band cells: A11's headland band, the field cells not inside-or-on the mitred inset of the field by the headland
+ *     width (D1); band_cells counts those covered by the HEADLAND layer only (as fcpp_summary.cov_cells).  An inset
+ *     that is empty or has |area| < 1 m^2 makes the band the whole field; a headland width <= 0 means no band (both
+ *     band counts 0).
+ *   n_boundary_viol / n_obstacle_viol: D3 over every point of the path (the plan kernel's point test).
+ * status: FCPP_CAND_GRID_TOO_LARGE | FCPP_CAND_BAND_GRID_TOO_LARGE when the field's lattice does not fit (a lattice
+ * row longer than the 32 KB tile, or an extent of 2^30 units); the four cell counts are then 0.
+ * FCPP_PATH_OUT_OF_RANGE when a point lies 2^30 lattice units (~107 km) or more from the field's lattice origin, or
+ * the path's field index is outside [0, n_fields): every count is 0.  Points are never clamped.
+ * The counts are sums of integer atomics over row slabs: deterministic.  48 bytes. */
+#define FCPP_PATH_OUT_OF_RANGE 128
+typedef struct {
+    int32_t status;
+    int32_t n_boundary_viol, n_obstacle_viol;
+    int32_t reserved;
+    int64_t band_total, band_cells;   /* cells of the headland band; of those, covered by the headland layer */
+    int64_t field_total, field_cells; /* cells of the field; of those, covered by either layer */
+} fcpp_path_cover;
+
+/* Coverage and D3 counts of caller-supplied paths (ragged batch, path p = points d_offsets[p] .. d_offsets[p+1] of
+ * d_path_xy [N][2]).  d_n_main [n_paths] splits path p into main work and headland; NULL means n_main = 0: the whole
+ * path is the headland layer and counts for both the band and the field.  d_path_field [n_paths] is each path's
+ * field (d_field_verts [n_fields][4][2], convex CCW), d_headland_width [n_paths] its headland width in m.  Obstacles
+ * as in fcpp_batch, per field (d_obs_poly_start [n_fields + 1], or NULL: none).  radius = W/2; grid_h an even
+ * multiple of 1e-4 m.  d_out [n_paths].  Asynchronous: no read-back. */
+int fcpp_path_coverage(fcpp_handle *h, const double *d_path_xy, const int64_t *d_offsets, int64_t n_paths,
+                       const int32_t *d_n_main, const int32_t *d_path_field, const double *d_headland_width,
+                       int32_t n_fields, const double *d_field_verts, const int32_t *d_obs_poly_start,
+                       const int32_t *d_obs_vert_start, const double *d_obs_verts, double radius, double grid_h,
+                       fcpp_path_cover *d_out, void *stream);
+
+/* The same for the materialised plans of the last fcpp_plan_batch of `batch` on this handle (outputs->path_xy and
+ * outputs->offsets are required, else FCPP_ERR_INVALID; the candidate records must be this batch's, as for
+ * fcpp_obstacle_sweep): field, headland width R and n_main from the candidate records, r = working_width / 2 and
+ * the batch's grid_h and obstacles.  Candidates whose layout failed, that have no points, or whose paths were not
+ * written (summary status FCPP_CAND_TOO_LARGE) get zero records.  d_out [B]. */
+int fcpp_plan_coverage(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outputs *outputs, fcpp_path_cover *d_out,
+                       void *stream);
+
 /* Generic A10 window raster (mlp3:1426-1510): ORs the W/2 round buffer of a polyline into a
  * g x g lattice-point window (bit (j*g+i) of d_bits, row-major, 32-bit words, ceil(g*g/32) words,
  * caller-zeroed or carrying an earlier cover) and writes the number of set bits to d_count. */
