@@ -492,6 +492,8 @@ int fcpp_raster_window(fcpp_handle *h, const double *d_path_xy, int32_t n_pts, d
     if (!d_path_xy || n_pts < 0 || g < 1 || g > 8192 || !d_bits || !d_count || !(h_cell > 0) || !(radius >= 0))
         return fail(h, FCPP_ERR_INVALID, "fcpp_raster_window: bad argument");
     if (llrint(h_cell * FCPP_FIXED_UNIT) < 1) return fail(h, FCPP_ERR_INVALID, "h_cell below the 1e-4 m lattice");
+    if (!(h_cell * FCPP_FIXED_UNIT < 1e15) || (int64_t)g * llrint(h_cell * FCPP_FIXED_UNIT) >= (1ll << 30))
+        return fail(h, FCPP_ERR_INVALID, "fcpp_raster_window: g * q(h_cell) must be below 2^30 lattice units");
     cudaSetDevice(h->device);
     cudaError_t e = fcpp_launch_raster_window(h, d_path_xy, n_pts, radius, origin_x, origin_y, h_cell, g, d_bits,
                                               d_count, (cudaStream_t)stream);

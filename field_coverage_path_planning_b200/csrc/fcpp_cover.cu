@@ -1816,7 +1816,19 @@ __global__ void __launch_bounds__(T) window_kernel(const double *__restrict__ pa
     const int rq = (int)qfix(radius);
     const int rw = (g + 31) >> 5;
     const int rows_per_tile = min(ROWCAP, TW / rw);
+    // range contract (as fcpp_path_coverage): every point within 2^30 units of the window origin, so that the
+    // rasteriser's int32 differences cannot overflow; otherwise count -1 and the caller's bits stay as they are.
+    // Points are never clamped: a clamped far end turns the segment about its near end.
     const int64_t lim = (1ll << 30);
+    int far = 0;
+    for (int k = tid; k < n_pts; k += T) {
+        const int64_t x = qfix(path[2 * k]) - X0, y = qfix(path[2 * k + 1]) - Y0;
+        if (!(x > -lim && x < lim && y > -lim && y < lim)) far = 1;
+    }
+    if (__syncthreads_or(far)) {
+        if (tid == 0) *count = -1;
+        return;
+    }
     for (int j0 = 0; j0 < g; j0 += rows_per_tile) {
         const int nrows = min(rows_per_tile, g - j0);
         for (int k = tid; k < nrows; k += T) {
@@ -1831,14 +1843,11 @@ __global__ void __launch_bounds__(T) window_kernel(const double *__restrict__ pa
             t.koff = 0;
         }
         __syncthreads();
-        // polyline in chunks of 1024 points (chunks overlap by one point); points far outside
-        // the window are clamped (they cannot reach it, the capsule radius is tiny against 2^30)
+        // polyline in chunks of 1024 points (chunks overlap by one point)
         for (int p0 = 0; p0 + 1 < n_pts; p0 += 1023) {
             const int np = min(1024, n_pts - p0);
             for (int k = tid; k < np; k += T) {
-                int64_t x = qfix(path[2 * (p0 + k)]) - X0, y = qfix(path[2 * (p0 + k) + 1]) - Y0;
-                x = x < -lim ? -lim : (x > lim ? lim : x);
-                y = y < -lim ? -lim : (y > lim ? lim : y);
+                const int64_t x = qfix(path[2 * (p0 + k)]) - X0, y = qfix(path[2 * (p0 + k) + 1]) - Y0;
                 d.ent(k).erow = make_int2((int)x, (int)y);
             }
             __syncthreads();

@@ -305,6 +305,16 @@ class TwoLayerPathPlannerV37:
         x, y = corner
         ox = x if corner_index in (0, 3) else x - 2 * R                    # mlp3:1461-1468
         oy = y if corner_index in (0, 1) else y - 2 * R
+        # the window raster's range contract (include/fcpp.h fcpp_raster_window), checked before the device is touched
+        o = np.rint(np.array([ox, oy], dtype=np.float64) * 1e4)
+        for name, p in (("turn_path", turn_path), ("reverse_path", reverse_path)):
+            if p is None or len(p) == 0:
+                continue
+            d = np.abs(np.rint(np.asarray(p, dtype=np.float64).reshape(-1, 2) * 1e4) - o)
+            bad = np.nonzero(~(d < 2.0 ** 30).all(axis=1))[0]
+            if len(bad):
+                raise ValueError(f"{name} point {int(bad[0])} lies 2^30 lattice units (~107 km) or more from the "
+                                 f"corner window's origin {(ox, oy)}")
         dev = _dev(self._device)
         h = _lib.handle(dev.index)
         nw = (g * g + 31) // 32

@@ -365,7 +365,10 @@ int fcpp_plan_coverage(fcpp_handle *h, const fcpp_batch *batch, const fcpp_outpu
 
 /* Generic A10 window raster (mlp3:1426-1510): ORs the W/2 round buffer of a polyline into a
  * g x g lattice-point window (bit (j*g+i) of d_bits, row-major, 32-bit words, ceil(g*g/32) words,
- * caller-zeroed or carrying an earlier cover) and writes the number of set bits to d_count. */
+ * caller-zeroed or carrying an earlier cover) and writes the number of set bits to d_count.
+ * Range contract (as fcpp_path_coverage): FCPP_ERR_INVALID when g * q(h_cell) >= 2^30 lattice units; when a point
+ * lies 2^30 units (~107 km) or more from q(origin) in x or y, *d_count = -1 and no bit of d_bits changes.  Points
+ * are never clamped. */
 int fcpp_raster_window(fcpp_handle *h, const double *d_path_xy, int32_t n_pts, double radius,
                        double origin_x, double origin_y, double h_cell, int32_t g,
                        uint32_t *d_bits, int64_t *d_count, void *stream);
